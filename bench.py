@@ -2,7 +2,7 @@
 """Benchmark of the message-passing hot path (BASELINE.json metric: aggregated edges/s +
 HBM GB/s vs roofline; GCN/GAT/SAGE epoch ms, 1-8 GPU) — ONE JSON line on stdout.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 Headline workload `sage_reddit` = BASELINE.json configs[2], the config the metric is quoted
@@ -32,6 +32,10 @@ T(1)/T(N) over the driver's N=1,2,4,8 runs is the strong scaling).  `--skip-extr
 
 `--impl reference` times the reference's CPU arithmetic for the same steps (the oracle port —
 the Python reference cannot travel to the GPU box) on the host cores.
+
+`--dump-outputs DIR` writes what the last timed step of the headline workload computed (hop-1 and layer-2
+means, a seeded 4,096-row sample of the hop-2 mean, the e2e logits) as float32 DIR/<name>.npy; every input is
+seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -165,6 +169,17 @@ def measured_traffic(kernel_key):
         return float(t["dram_bytes"]), t.get("source")
     except Exception:
         return None, None
+
+
+DUMP_HOP2_ROWS = 4096  # seeded sample of the 25,600 hop-2 rows (all of them would be 62 MB)
+
+
+def dump_outputs(path, arrays):
+    """Write each array as <path>/<name>.npy in float32, so that two builds can be compared output for output."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if torch.is_tensor(a) else a
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
 
 
 def sage_algorithmic_bytes(n_src, fanout, F, s=4):
@@ -311,6 +326,12 @@ def run_sage_b200(args, rank, world, dev):
         exact = model.forward_sampled(table, dev_blocks[(args.warmup + args.steps - 1) % pool])
     model.tensor_core_gemm = True
     gemm_rel_err = float(((eager - exact).abs().max() / exact.abs().max().clamp_min(1e-30)).item())
+    if args.dump_outputs and rank == 0:
+        # the last timed step of both legs: the kernels-only outputs hold minibatch warmup+steps-1 (the warm_l2
+        # pass repeats the same minibatches), the e2e runner's host logits the same minibatch's forward
+        rows = torch.from_numpy(np.sort(np.random.default_rng(0).choice(B * f1, DUMP_HOP2_ROWS, replace=False)))
+        dump_outputs(args.dump_outputs, {"hop2_mean_rows": out2[rows.to(dev)], "hop1_mean": out1,
+                                         "layer2_mean": out0, "e2e_logits": runner.logits_host})
 
     if world > 1:
         t = torch.tensor([ms_total, e2e_ms, k2_ms, warm_ms_total, k2_warm_ms, wall_ms_incl_flush], device=dev,
@@ -798,7 +819,11 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--skip-extra", action="store_true", help="headline workload only")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the headline workload's last-step outputs to DIR/<name>.npy (float32; rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -816,7 +841,13 @@ def main():
             ref = run_sage_reference(steps, args.warmup)
         except Exception as e:  # pragma: no cover
             print(f"reference snapshot arm failed ({e!r}); falling back to the port", file=sys.stderr)
-        pv, pms = run_sage_cpu(min(steps, 20), min(args.warmup, 3))  # the vectorised port, always reported beside it
+        else:
+            if ref is None:
+                print("no reference checkout (GNN_REFERENCE_ROOT) or oracle/_ref snapshot: the CPU arm times the "
+                      "vectorised port (cpu_baseline.kind = \"port\"), not the reference's own step", file=sys.stderr)
+        # the vectorised port, always reported beside the reference; it is the timed arm (all --steps) without one
+        port_steps = steps if ref is None else min(steps, 20)
+        pv, pms = run_sage_cpu(port_steps, min(args.warmup, 3))
         port = {"value": pv, "unit": "edges/s", "ms_per_step": pms, "kind": "port",
                 "what": "oracle/sage.py: the same step with a VECTORISED torch gather instead of the reference's "
                         "python list comprehension, full 1024-node minibatches"}
@@ -829,7 +860,7 @@ def main():
                       f"vectorised port of the same step runs at {pv:.3g} edges/s (`port`)")
         else:
             v, ms, kind = pv, pms, "port"
-            sample = (f"{min(steps, 20)} full minibatches on rank 0's host cores: torch-CPU feature gather of the 3 id "
+            sample = (f"{steps} full minibatches on rank 0's host cores: torch-CPU feature gather of the 3 id "
                       "blocks + GraphSage forward (oracle/sage.py restating GraphSAGE_Pytorch); no reference snapshot "
                       "(oracle/_ref) was available")
         line = {"impl": "reference", "metric": "aggregated_edges_per_sec", "value": v, "unit": "edges/s",

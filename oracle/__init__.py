@@ -12,8 +12,9 @@ cites the reference file:line it follows.
 
 Pinning: the reference ships no tests, golden vectors or fixtures ("parity unpinned" by the
 reference's own tests).  The oracle is therefore pinned against the reference ITSELF:
-`oracle/ref_loader.py` imports the unmodified modules from /root/reference (present in the
-build container only) and `tests/test_oracle_vs_reference.py` compares them with this
-restatement on seeded inputs; `tests/golden/make_golden.py` dumps reference outputs into
-`tests/golden/*.npz`, which travel to the GPU box where /root/reference does not exist.
+`oracle/ref_loader.py` imports the unmodified modules from a reference checkout named by
+$GNN_REFERENCE_ROOT (the reference is not part of this repository) and
+`tests/test_oracle_vs_reference_live.py` compares them with this restatement on seeded inputs;
+`tests/golden/make_golden.py` dumps reference outputs into `tests/golden/*.npz`, which pin the
+oracle wherever the reference is absent.
 """

@@ -1,7 +1,7 @@
 """CPU restatement of the GTN pieces next to the hot path (test infrastructure: imported by tests/ only).
 
-  norm      /root/reference GTN/models/GTN.py:7-19   column normalisation of the learned adjacency
-  gcn_conv  /root/reference GTN/models/GTN.py:49-52  GCN over the learned adjacency
+  norm      GTN/models/GTN.py:7-19   column normalisation of the learned adjacency
+  gcn_conv  GTN/models/GTN.py:49-52  GCN over the learned adjacency
 Pinned against the unmodified reference by tests/golden/gtn_small.npz (made by tests/golden/make_golden.py)
 and by tests/test_oracle_vs_reference_live.py on fresh seeds."""
 import torch

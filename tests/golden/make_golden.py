@@ -1,11 +1,11 @@
 """Generate the golden fixtures in tests/golden/*.npz from the UNMODIFIED reference.
 
-Run in the build container (where /root/reference exists):
-    python tests/golden/make_golden.py
+Run with a reference checkout (kaddly/GraphNeuralNetwork):
+    GNN_REFERENCE_ROOT=<checkout> python tests/golden/make_golden.py
 The reference modules are imported through oracle/ref_loader.py and driven with seeded
 synthetic inputs; inputs that are cheap to regenerate are stored as seeds + a checksum,
 everything else (weights, index blocks, outputs, gradients) is stored verbatim.  The
-fixtures travel to the GPU box, where the reference does not exist.
+fixtures pin the tests wherever the reference is absent.
 """
 import hashlib
 import os

@@ -2,8 +2,8 @@
 path substituted by import path (SURVEY.md §8b "installed by import-path substitution"), run on the GPU and
 are compared with the unmodified reference run on the CPU from the same seed.
 
-The reference modules come from the verbatim snapshot in the git-ignored oracle/_ref/ (tools/make_ref_snapshot.py,
-made by __graft_entry__.build(); /root/reference itself in the build container).  Skipped when neither exists.
+The reference modules come from the checkout $GNN_REFERENCE_ROOT names or from the verbatim snapshot in the
+git-ignored oracle/_ref/ (tools/make_ref_snapshot.py, made by __graft_entry__.build()).  Skipped when neither exists.
   * GCN   GCN/GCN.py:21-27 `GCN_Model` (dispatch on `_get_name() == 'Graph_conv_layer'`) built from the reference
           class with `Graph_conv_layer` replaced, trained by the reference's `train` (GCN/train_eval.py:20-66);
   * SAGE  GraphSAGE_Pytorch `GraphSage` / `SageGCN` with `NeighborAggregator` replaced, fed by the reference's own
