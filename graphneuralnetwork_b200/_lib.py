@@ -94,7 +94,8 @@ class SpmmOpts(C.Structure):
     _fields_ = [("struct_size", i32), ("accumulate", i32), ("accumulate_prefix", i64), ("rows_per_team", i32),
                 ("relu", i32), ("bias", ptr), ("row_map", ptr), ("X2", ptr), ("ldx2", i64), ("split", i64),
                 ("long_rows", ptr), ("n_long", i64), ("long_threshold", i64), ("chunk_off", ptr), ("n_chunks", i64),
-                ("chunk_edges", i32), ("exclusion_smem_bytes", i32), ("workspace", ptr), ("workspace_bytes", size_t)]
+                ("chunk_edges", i32), ("exclusion_smem_bytes", i32), ("workspace", ptr), ("workspace_bytes", size_t),
+                ("epilogue_skip_prefix", i64)]
 
 
 class GatDropout(C.Structure):

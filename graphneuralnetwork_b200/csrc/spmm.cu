@@ -12,7 +12,7 @@ int spmm_impl(const int64_t* rowptr, const int32_t* col, const float* val, const
               int64_t n_cols, int32_t F, int64_t ldx, int64_t ldy, const int64_t* long_rows, int64_t n_long,
               int64_t long_threshold, const int64_t* chunk_off, int64_t n_chunks, int32_t chunk_edges, int accumulate,
               int32_t rows_per_team, const float* bias, int32_t relu, void* workspace, size_t workspace_bytes,
-              cudaStream_t st, const gnn_spmm_opts* ex = nullptr) {
+              cudaStream_t st, const gnn_spmm_opts* ex = nullptr, int64_t epi_skip = 0) {
   GNN_REQUIRE(n_rows >= 0 && n_cols >= 0 && F >= 0, GNN_ERR_BAD_ARG, "negative size");
   if (n_rows == 0 || F == 0) return GNN_OK;
   // col may be null only for a graph without edges (nnz lives on the device; rowptr decides)
@@ -34,7 +34,9 @@ int spmm_impl(const int64_t* rowptr, const int32_t* col, const float* val, const
   a.skip_deg_gt = 0;
   a.accumulate = accumulate ? 1 : 0;
   GNN_REQUIRE(rows_per_team >= 0, GNN_ERR_BAD_ARG, "rows_per_team must be >= 0");
-  GNN_REQUIRE(!(accumulate && (bias || relu)), GNN_ERR_BAD_ARG, "the bias/ReLU epilogue belongs to the final pass");
+  // the planned entry keeps the epilogue on overwriting launches; the extended one also fuses it into the
+  // accumulating (last) pass of a two-pass row: y = relu?(y_prev + sum + b)
+  GNN_REQUIRE(ex || !(accumulate && (bias || relu)), GNN_ERR_BAD_ARG, "the bias/ReLU epilogue belongs to the final pass");
   a.bias = bias;
   a.relu = relu ? 1 : 0;
   a.rows_per_team = tuning("spmm.rows_per_team", 0) > 0 ? tuning("spmm.rows_per_team", 0) : rows_per_team;
@@ -43,15 +45,14 @@ int spmm_impl(const int64_t* rowptr, const int32_t* col, const float* val, const
     // row-subset / two-table form: the CSR is compact over the selected rows
     GNN_REQUIRE(ex->accumulate_prefix >= 0 && ex->accumulate_prefix <= n_rows, GNN_ERR_BAD_ARG,
                 "accumulate_prefix out of range");
-    GNN_REQUIRE(!(ex->accumulate_prefix > 0 && (bias || relu)), GNN_ERR_BAD_ARG,
-                "the bias/ReLU epilogue belongs to the final pass");
+    GNN_REQUIRE(epi_skip >= 0 && epi_skip <= n_rows, GNN_ERR_BAD_ARG, "epilogue_skip_prefix out of range");
     GNN_REQUIRE(ex->exclusion_smem_bytes >= 0 && ex->exclusion_smem_bytes <= 48 * 1024, GNN_ERR_BAD_ARG,
                 "exclusion_smem_bytes must be within [0, 48 KB]");
     a.row_map = ex->row_map;
     a.acc_prefix = ex->accumulate_prefix;
     a.excl_smem = ex->exclusion_smem_bytes;
+    a.epi_skip = epi_skip;
     if (ex->X2) {
-      GNN_REQUIRE(!(bias || relu), GNN_ERR_BAD_ARG, "two-table form has no bias/ReLU epilogue");
       GNN_REQUIRE(ex->split >= 0 && ex->split <= n_cols && ex->ldx2 >= F, GNN_ERR_BAD_ARG, "bad split / ldx2");
       GNN_REQUIRE(aligned_to(ex->X2, sizeof(T)), GNN_ERR_MISALIGNED, "X2 not element aligned");
       a.ldx2 = ex->ldx2;
@@ -71,6 +72,15 @@ int spmm_impl(const int64_t* rowptr, const int32_t* col, const float* val, const
     if (rc != GNN_OK) return rc;
   }
   return spmm_main<T>(a, st);
+}
+
+// struct_size is the version of gnn_spmm_opts: the current size, or the size before epilogue_skip_prefix was
+// appended (read as 0).  -1: missing or unknown version (the caller's struct must not be read past its end).
+int64_t spmm_opts_epilogue_skip(const gnn_spmm_opts* o) {
+  if (!o) return -1;
+  if (o->struct_size == (int32_t)sizeof(gnn_spmm_opts)) return o->epilogue_skip_prefix;
+  if (o->struct_size == (int32_t)offsetof(gnn_spmm_opts, epilogue_skip_prefix)) return 0;
+  return -1;
 }
 
 }  // namespace
@@ -119,22 +129,22 @@ int gnn_spmm_csr_planned_bf16(const int64_t* rowptr, const int32_t* col, const f
 int gnn_spmm_csr_ex_f32(const int64_t* rowptr, const int32_t* col, const float* val, const float* X, float* Y,
                         int64_t n_rows, int64_t n_cols, int32_t F, int64_t ldx, int64_t ldy, const gnn_spmm_opts* o,
                         gnn_stream_t stream) {
-  GNN_REQUIRE(o && o->struct_size == (int32_t)sizeof(gnn_spmm_opts), GNN_ERR_BAD_ARG,
-              "gnn_spmm_opts missing or struct_size mismatch (header/library version skew)");
+  const int64_t epi_skip = spmm_opts_epilogue_skip(o);
+  GNN_REQUIRE(epi_skip >= 0, GNN_ERR_BAD_ARG, "gnn_spmm_opts missing or struct_size mismatch (header/library version skew)");
   return spmm_impl<float>(rowptr, col, val, X, Y, n_rows, n_cols, F, ldx, ldy, o->long_rows, o->n_long,
                           o->long_threshold, o->chunk_off, o->n_chunks, o->chunk_edges, o->accumulate, o->rows_per_team,
-                          o->bias, o->relu, o->workspace, o->workspace_bytes, (cudaStream_t)stream, o);
+                          o->bias, o->relu, o->workspace, o->workspace_bytes, (cudaStream_t)stream, o, epi_skip);
 }
 
 int gnn_spmm_csr_ex_bf16(const int64_t* rowptr, const int32_t* col, const float* val, const void* X, void* Y,
                          int64_t n_rows, int64_t n_cols, int32_t F, int64_t ldx, int64_t ldy, const gnn_spmm_opts* o,
                          gnn_stream_t stream) {
-  GNN_REQUIRE(o && o->struct_size == (int32_t)sizeof(gnn_spmm_opts), GNN_ERR_BAD_ARG,
-              "gnn_spmm_opts missing or struct_size mismatch (header/library version skew)");
+  const int64_t epi_skip = spmm_opts_epilogue_skip(o);
+  GNN_REQUIRE(epi_skip >= 0, GNN_ERR_BAD_ARG, "gnn_spmm_opts missing or struct_size mismatch (header/library version skew)");
   return spmm_impl<__nv_bfloat16>(rowptr, col, val, (const __nv_bfloat16*)X, (__nv_bfloat16*)Y, n_rows, n_cols, F, ldx,
                                   ldy, o->long_rows, o->n_long, o->long_threshold, o->chunk_off, o->n_chunks,
                                   o->chunk_edges, o->accumulate, o->rows_per_team, o->bias, o->relu, o->workspace,
-                                  o->workspace_bytes, (cudaStream_t)stream, o);
+                                  o->workspace_bytes, (cudaStream_t)stream, o, epi_skip);
 }
 
 }  // extern "C"

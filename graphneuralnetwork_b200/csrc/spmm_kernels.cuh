@@ -41,6 +41,7 @@ struct SpmmArgs {
   int64_t ldx2;            //   the host passes X2 pre-offset by -split rows, so the row is X2 + c * ldx2
   int32_t split;
   int32_t excl_smem;       // host only: token dynamic shared memory per CTA (keeps CTAs off SMs a mover filled)
+  int64_t epi_skip;        // compact rows [0, epi_skip) get no bias/ReLU epilogue (first pass of two-pass rows)
 };
 
 // source row of column id c (SPLIT: two tables, [0, split) -> X, [split, ...) -> X2)
@@ -78,7 +79,9 @@ constexpr int kSpmmThreads = 256;
 // kernel is latency-bound and the third CTA is worth 4-11 % (F=602 fp32 34.1 -> 30.6 ms, bf16 23.6 ->
 // 21.7 ms; profiles/r01s2_kbench_spmm_reddit_ctas3_ab.jsonl).  "spmm.ctas3" = 0 selects the unconstrained
 // instantiation (100-140 registers, 2 CTAs/SM).
-template <typename T, int VEC, int GROUP, int CHUNKS, int U, bool EPI, int MINB = ((CHUNKS == 1) ? 4 : 1), bool SPLIT = false>
+// SKIP: the epilogue honours epi_skip (a separate instantiation, so the plain epilogue keeps its registers).
+template <typename T, int VEC, int GROUP, int CHUNKS, int U, bool EPI, int MINB = ((CHUNKS == 1) ? 4 : 1), bool SPLIT = false,
+          bool SKIP = false>
 __global__ void __launch_bounds__(kSpmmThreads, MINB) spmm_rbs_kernel(const SpmmArgs<T> a) {
   const int lane = threadIdx.x & 31;
   const int gl = threadIdx.x % GROUP;
@@ -118,7 +121,7 @@ __global__ void __launch_bounds__(kSpmmThreads, MINB) spmm_rbs_kernel(const Spmm
 #pragma unroll
           for (int i = 0; i < VEC; ++i) acc[ch][i] += prev[i];
         }
-        if (EPI) spmm_epilogue<VEC>(acc[ch], a.bias, a.relu, col0, a.F);
+        if (EPI && (!SKIP || (r0 + r) >= a.epi_skip)) spmm_epilogue<VEC>(acc[ch], a.bias, a.relu, col0, a.F);
         VecIO<T, VEC>::store(yr + col0, acc[ch]);
       }
 #pragma unroll
@@ -334,11 +337,15 @@ __global__ void __launch_bounds__(256)
     spmm_long_finalize_kernel(const int64_t* __restrict__ long_rows, const int64_t* __restrict__ chunk_off,
                               const float* __restrict__ partial, int ldp, int col_base, int Ftile, T* __restrict__ Y,
                               int64_t ldy, int accumulate, const float* __restrict__ bias, int relu,
-                              const int32_t* __restrict__ row_map, int64_t acc_prefix) {
+                              const int32_t* __restrict__ row_map, int64_t acc_prefix, int64_t epi_skip) {
   const int64_t r = blockIdx.x;
   const int64_t crow = __ldg(long_rows + r);  // (compact) CSR row
   const int64_t row = row_map ? (int64_t)__ldg(row_map + crow) : crow;
   accumulate = accumulate || crow < acc_prefix;
+  if (crow < epi_skip) {  // first pass of a two-pass row: its epilogue comes with the last contribution
+    bias = nullptr;
+    relu = 0;
+  }
   const int64_t c0 = __ldg(chunk_off + r), c1 = __ldg(chunk_off + r + 1);
   for (int f = threadIdx.x; f < Ftile; f += blockDim.x) {
     float sum = 0.f;
@@ -383,10 +390,18 @@ inline void spmm_rbs_launch(const SpmmArgs<T>& a, cudaStream_t st) {
   // dedicated halo push has claimed (peer.cu); 0 outside the partitioned SpMM's local pass
   const size_t sm = (size_t)(a.excl_smem > 0 ? a.excl_smem : 0);
   constexpr int MINB_DEF = (CHUNKS == 1) ? 4 : ((CHUNKS <= 5) ? 3 : 1);
+  // the partitioned SpMM's consumers with the GCN epilogue (two-table pass, first pass + finished rows in one
+  // launch): held to a register budget that does not spill
+  constexpr int MINB_EPI = (CHUNKS == 1) ? 2 : 1;
+  const bool epi = a.bias || a.relu;
   if (a.split != 0x7fffffff) {
-    // two-table form (never combined with the bias/ReLU epilogue: spmm_impl rejects that)
-    spmm_rbs_kernel<T, VEC, GROUP, CHUNKS, U, false, MINB_DEF, true><<<(unsigned)grid, kSpmmThreads, sm, st>>>(a);
-  } else if (a.bias || a.relu) {
+    if (epi)
+      spmm_rbs_kernel<T, VEC, GROUP, CHUNKS, U, true, MINB_EPI, true, true><<<(unsigned)grid, kSpmmThreads, sm, st>>>(a);
+    else
+      spmm_rbs_kernel<T, VEC, GROUP, CHUNKS, U, false, MINB_DEF, true><<<(unsigned)grid, kSpmmThreads, sm, st>>>(a);
+  } else if (epi && a.epi_skip > 0) {
+    spmm_rbs_kernel<T, VEC, GROUP, CHUNKS, U, true, MINB_EPI, false, true><<<(unsigned)grid, kSpmmThreads, sm, st>>>(a);
+  } else if (epi) {
     spmm_rbs_kernel<T, VEC, GROUP, CHUNKS, U, true><<<(unsigned)grid, kSpmmThreads, sm, st>>>(a);
   } else if (CHUNKS >= 2 && CHUNKS <= 5 && tuning("spmm.ctas3", 1)) {
     spmm_rbs_kernel<T, VEC, GROUP, CHUNKS, U, false, (CHUNKS >= 2 && CHUNKS <= 5) ? 3 : 1>
@@ -464,7 +479,7 @@ inline int spmm_long_vec(const SpmmArgs<T>& a0, const int64_t* long_rows, int64_
     GNN_LAUNCH_CHECK();
     spmm_long_finalize_kernel<T><<<(unsigned)n_long, 256, 0, st>>>(long_rows, chunk_off, partial, ldp, c0, a.F, a0.Y,
                                                                    a0.ldy, a0.accumulate, a0.bias, a0.relu,
-                                                                   a0.row_map, a0.acc_prefix);
+                                                                   a0.row_map, a0.acc_prefix, a0.epi_skip);
     GNN_LAUNCH_CHECK();
   }
   return GNN_OK;

@@ -78,13 +78,16 @@ def spmm_raw(g: CSRGraph, X: torch.Tensor, out: Optional[torch.Tensor] = None, p
 
 def spmm_ex(g: CSRGraph, X: torch.Tensor, out: torch.Tensor, row_map: Optional[torch.Tensor] = None,
             accumulate: bool = False, accumulate_prefix: int = 0, X2: Optional[torch.Tensor] = None, split: int = 0,
-            exclusion_smem: int = 0) -> torch.Tensor:
+            exclusion_smem: int = 0, bias: Optional[torch.Tensor] = None, relu: bool = False,
+            epilogue_skip_prefix: int = 0) -> torch.Tensor:
     """Row-subset / two-table SpMM (gnn_spmm_csr_ex_*, no autograd): `g` is a CSR that is COMPACT over the
     selected rows; compact row r writes `out[row_map[r]]` (row_map None: out[r]); rows below
     `accumulate_prefix` (or all, with accumulate) add into `out`; column ids >= `split` read row
-    (c - split) of X2.  The consumers of the partitioned SpMM's waves (partition.py)."""
+    (c - split) of X2.  bias / relu: the epilogue relu?(. + bias), applied after the add of accumulating rows,
+    except on compact rows below `epilogue_skip_prefix`.  The consumers of the partitioned SpMM's waves
+    (partition.py)."""
     import ctypes as C
-    _require_cuda(X, out, row_map, X2)
+    _require_cuda(X, out, row_map, X2, bias)
     lib = _lib.load()
     X = _rowmajor(X)
     if X.dtype not in (torch.float32, torch.bfloat16) or out.dtype != X.dtype:
@@ -100,6 +103,10 @@ def spmm_ex(g: CSRGraph, X: torch.Tensor, out: torch.Tensor, row_map: Optional[t
         raise _lib.GnnError("spmm_ex: row_map must be int32 with one entry per compact row")
     if out.stride(1) != 1 or out.shape[1] != F:
         raise _lib.GnnError("spmm_ex: `out` must be [*, F] with unit column stride")
+    if bias is not None:
+        if bias.dtype != torch.float32 or bias.numel() != F:
+            raise _lib.GnnError(f"spmm_ex: bias must be fp32 with {F} entries")
+        bias = bias.contiguous()
     plan = g.long_row_plan()
     lr, thr, chunk_off, n_chunks, chunk, ws = plan if plan is not None else (None, 0, None, 0, 0, None)
     o = _lib.SpmmOpts()
@@ -114,6 +121,7 @@ def spmm_ex(g: CSRGraph, X: torch.Tensor, out: torch.Tensor, row_map: Optional[t
     o.long_rows, o.n_long, o.long_threshold = _p(lr), 0 if lr is None else lr.numel(), thr
     o.chunk_off, o.n_chunks, o.chunk_edges = _p(chunk_off), n_chunks, chunk
     o.exclusion_smem_bytes = int(exclusion_smem)
+    o.bias, o.relu, o.epilogue_skip_prefix = _p(bias), 1 if relu else 0, int(epilogue_skip_prefix)
     o.workspace, o.workspace_bytes = _p(ws), 0 if ws is None else ws.numel()
     fn = lib.gnn_spmm_csr_ex_f32 if X.dtype == torch.float32 else lib.gnn_spmm_csr_ex_bf16
     _lib.check(fn(_p(g.rowptr), _p(g.col), _p(g.val), _p(X), _p(out), g.n_rows, max(g.n_cols, n_src), F, _ld(X),
@@ -220,6 +228,47 @@ def gcn_aggregate(g: CSRGraph, S: torch.Tensor, bias: Optional[torch.Tensor] = N
     if bias is not None and bias.dtype != torch.float32:
         bias = bias.float()
     return _GcnAggregateFn.apply(S, bias, g, relu)
+
+
+class _PartitionedGcnAggregateFn(torch.autograd.Function):
+    """The rank's rows of relu?(Â·S + b) on a row-partitioned graph (partition.PartitionedGraph), the contract of
+    _GcnAggregateFn: the halo exchange and the partitioned SpMM with the bias/ReLU epilogue fused into the launch
+    that writes each row's last contribution.  Backward: dZ = dY ⊙ [Y > 0];  dS = (Âᵀ·dZ)[own rows] (the
+    partitioned backward: every rank's dZ reaches the rows it reads);  db = Σ dZ over the OWN rows only — the sum
+    over the ranks (partition.allreduce_gradients) is the full bias gradient."""
+
+    @staticmethod
+    def forward(ctx, S, bias, op, relu: bool):
+        Y = op.forward(S, bias=bias, relu=relu)
+        ctx.op, ctx.relu, ctx.has_bias = op, relu, bias is not None
+        if relu:
+            ctx.save_for_backward(Y)
+        return Y
+
+    @staticmethod
+    def backward(ctx, dY):
+        dZ = dY
+        if ctx.relu:
+            (Y,) = ctx.saved_tensors
+            dZ = dY * (Y > 0).to(dY.dtype)
+        dZ = dZ.contiguous()
+        # always run: the backward exchange is a collective every rank takes part in
+        dS = ctx.op.backward(dZ)
+        db = dZ.sum(dim=0) if (ctx.has_bias and ctx.needs_input_grad[1]) else None
+        return (dS if ctx.needs_input_grad[0] else None), db, None, None
+
+
+def partitioned_gcn_aggregate(pg, S: torch.Tensor, bias: Optional[torch.Tensor] = None,
+                              relu: bool = False) -> torch.Tensor:
+    """relu?(Â·S + bias)[own rows] with autograd into S and bias, over a partition.PartitionedGraph `pg`; S = the
+    rank's own rows (fp32).  Collective: every rank calls it, and its backward, in the same order."""
+    _require_cuda(S, bias)
+    if S.dtype != torch.float32 or (bias is not None and bias.dtype != torch.float32):
+        raise _lib.GnnError("partitioned_gcn_aggregate: fp32 features and bias expected")
+    if S.dim() != 2 or S.shape[0] != pg.n_local:
+        raise _lib.GnnError(f"partitioned_gcn_aggregate: S must be [{pg.n_local}, F] (this rank's rows), "
+                            f"got {tuple(S.shape)}")
+    return _PartitionedGcnAggregateFn.apply(S.contiguous(), bias, pg.op(S.shape[1]), relu)
 
 
 # --------------------------------------------------------------------------------------

@@ -11,15 +11,23 @@ Re-designed for the device:
   * the `nn.ReLU` module that follows every hidden layer (GCN.py:12,19) is folded into the same
     launch: the model walks `gcn_blocks` with one step of lookahead and, when a graph layer is
     followed by a ReLU, asks the layer for the fused activation and skips the module;
-  * the COO adjacency is converted to CSR (+ transpose for the backward) once per graph.
+  * the COO adjacency is converted to CSR (+ transpose for the backward) once per graph;
+  * `adj` may also be a `partition.PartitionedGraph` (one rank's share of a graph split over GPUs): X is then the
+    rank's own rows, the aggregation is the partitioned SpMM with the same fused epilogue, and the module tree and
+    state_dict are unchanged, so a checkpoint moves between 1 and N GPUs.
 The dense `X·Wᵀ` stays a torch matmul (north_star): transform first, aggregate on the narrow
 width.
 """
 import torch
 from torch import nn
 
-from ..functional import gcn_aggregate
+from ..functional import gcn_aggregate, partitioned_gcn_aggregate
 from ..graph import adj_cache
+from ..partition import PartitionedGraph
+
+
+def _graph(adj):
+    return adj if isinstance(adj, PartitionedGraph) else adj_cache.get(adj)
 
 
 class Graph_conv_layer(nn.Module):
@@ -33,6 +41,8 @@ class Graph_conv_layer(nn.Module):
         self.register_parameter('bias', nn.Parameter(torch.zeros(out_features)) if is_bias else None)
 
     def forward(self, X_input, adj, fused_relu=False):
+        if isinstance(adj, PartitionedGraph):
+            return partitioned_gcn_aggregate(adj, self.dense(X_input), self.bias, relu=fused_relu)
         return gcn_aggregate(adj_cache.get(adj), self.dense(X_input), self.bias, relu=fused_relu)
 
     def __repr__(self):
@@ -55,7 +65,7 @@ class GCN_Model(nn.Module):
                 self.gcn_blocks.add_module(f'dropout{i}', nn.Dropout(dropout))
 
     def forward(self, X, adj):
-        graph = adj_cache.get(adj)
+        graph = _graph(adj)
         blocks = list(self.gcn_blocks)
         i = 0
         while i < len(blocks):

@@ -108,13 +108,16 @@ def select_rows(rowptr: torch.Tensor, col: torch.Tensor, val: Optional[torch.Ten
 class Consumer:
     """One SpMM launch of the step: a compact CSR over a row subset of the rank's block.
     mode "local": columns index X_local.  "remote": columns index the halo, accumulate into Y.
-    "combined": columns < n_local index X_local, the others (col - n_local) the halo; overwrite."""
+    "combined": columns < n_local index X_local, the others (col - n_local) the halo; overwrite.
+    With a bias/ReLU epilogue every row gets it in the launch that adds its last contribution: compact rows
+    [0, epilogue_skip) of P1 are the first pass of two-pass rows and get it later, in their "remote" pass."""
     mode: str
     rowptr: torch.Tensor
     col: torch.Tensor
     val: Optional[torch.Tensor]
     row_map: Optional[torch.Tensor]   # int32 compact row -> local row; None = every local row in order
     n_cols: int
+    epilogue_skip: int = 0
 
     @property
     def n_rows(self) -> int:
@@ -399,14 +402,19 @@ def build_halo_plan(rowptr: torch.Tensor, col: torch.Tensor, val: Optional[torch
                       rows_mixed=sum(m_rows), nnz_interior=nnz_interior)
     cut_row = chunk_bounds[c0]  # mixed rows at or beyond this row are single-pass
     all_rows = torch.arange(n_loc, dtype=torch.int64, device=dev)
-    # P1: local columns of every row except the single-pass mixed rows
-    if c0 == K:
-        plan.p1 = Consumer("local", rowptr_loc, col_loc, val_loc, None, n_loc)
+    # P1: local columns of every row except the single-pass mixed rows.  The two-pass mixed rows come first (their
+    # remote pass adds the rest, so a fused epilogue skips them: Consumer.epilogue_skip), then the interior rows.
+    # Every row is its own ordered reduction, so the order of the rows changes no result.
+    first = all_rows[mixed & (all_rows < cut_row)]
+    interior = all_rows[~mixed]
+    n_first = int(first.numel())
+    if n_first + int(interior.numel()) == n_loc and (n_first == 0 or n_first == n_loc):
+        plan.p1 = Consumer("local", rowptr_loc, col_loc, val_loc, None, n_loc, epilogue_skip=n_first)
     else:
-        keep = (~mixed) | (all_rows < cut_row)
-        rows = all_rows[keep]
+        rows = torch.cat([first, interior])
         rp, cc, vv = select_rows(rowptr_loc, col_loc, val_loc, rows)
-        plan.p1 = Consumer("local", rp, cc, vv, rows.to(torch.int32), n_loc) if rows.numel() else None
+        plan.p1 = (Consumer("local", rp, cc, vv, rows.to(torch.int32), n_loc, epilogue_skip=n_first)
+                   if rows.numel() else None)
     # combined column space of the single-pass rows: local col j -> j, remote -> n_loc + halo slot
     col_comb = None
     if c0 < K:
@@ -430,13 +438,21 @@ def build_halo_plan(rowptr: torch.Tensor, col: torch.Tensor, val: Optional[torch
     return plan
 
 
-def reference_step_cpu(plan: HaloPlan, X_local: torch.Tensor, halo: torch.Tensor) -> torch.Tensor:
+def reference_step_cpu(plan: HaloPlan, X_local: torch.Tensor, halo: torch.Tensor, bias: Optional[torch.Tensor] = None,
+                       relu: bool = False) -> torch.Tensor:
     """The step's arithmetic with torch ops in float64 (test-side: replays P1 and the wave consumers of a
-    plan exactly as `PartitionedSpmm.forward` schedules them).  `halo` = the received rows in slot order."""
+    plan exactly as `PartitionedSpmm.forward` schedules them).  `halo` = the received rows in slot order.
+    bias / relu: the fused epilogue, applied where the schedule applies it (P1 rows past its epilogue_skip,
+    after the add of a "remote" pass, on every "combined" row)."""
     n_loc, F = plan.n_local, X_local.shape[1]
     Y = torch.zeros((n_loc, F), dtype=torch.float64)
     Xl, Hl = X_local.double(), halo.double()
     table = torch.cat([Xl, Hl], 0)
+    b = None if bias is None else bias.double().view(1, -1)
+
+    def epilogue(y):
+        y = y if b is None else y + b
+        return y.clamp_min(0.0) if relu else y
 
     def product(c: Consumer, src):
         rows = torch.repeat_interleave(torch.arange(c.n_rows), c.rowptr[1:] - c.rowptr[:-1])
@@ -449,14 +465,17 @@ def reference_step_cpu(plan: HaloPlan, X_local: torch.Tensor, halo: torch.Tensor
         return torch.arange(n_loc) if c.row_map is None else c.row_map.long()
 
     if plan.p1 is not None:
-        Y[target(plan.p1)] = product(plan.p1, Xl)
+        y, k = product(plan.p1, Xl), plan.p1.epilogue_skip
+        y[k:] = epilogue(y[k:])
+        Y[target(plan.p1)] = y
     for c in plan.p2:
         if c is None:
             continue
         if c.mode == "remote":
-            Y[target(c)] += product(c, Hl)
+            t = target(c)
+            Y[t] = epilogue(Y[t] + product(c, Hl))
         else:
-            Y[target(c)] = product(c, table)
+            Y[target(c)] = epilogue(product(c, table))
     return Y
 
 
@@ -731,17 +750,22 @@ class PartitionedSpmm:
             self._exchange_wave(X, w, stream)
             self._signal(0, s * K + w + 1, stream)
 
-    def _run(self, c: Consumer, X, halo, out, excl: int = 0):
+    def _run(self, c: Consumer, X, halo, out, excl: int = 0, bias: Optional[torch.Tensor] = None, relu: bool = False):
         from .functional import spmm_ex
         g = self._graph(c)
         if c.mode == "local":
-            spmm_ex(g, X, out, row_map=g._row_map, exclusion_smem=excl)
+            spmm_ex(g, X, out, row_map=g._row_map, exclusion_smem=excl, bias=bias, relu=relu,
+                    epilogue_skip_prefix=c.epilogue_skip if (bias is not None or relu) else 0)
         elif c.mode == "remote":
-            spmm_ex(g, halo, out, row_map=g._row_map, accumulate=True)
+            spmm_ex(g, halo, out, row_map=g._row_map, accumulate=True, bias=bias, relu=relu)
         else:
-            spmm_ex(g, X, out, row_map=g._row_map, X2=halo, split=self.plan.n_local)
+            spmm_ex(g, X, out, row_map=g._row_map, X2=halo, split=self.plan.n_local, bias=bias, relu=relu)
 
-    def forward(self, X: torch.Tensor, out: Optional[torch.Tensor] = None, overlap: bool = True) -> torch.Tensor:
+    def forward(self, X: torch.Tensor, out: Optional[torch.Tensor] = None, overlap: bool = True,
+                bias: Optional[torch.Tensor] = None, relu: bool = False) -> torch.Tensor:
+        """Y_local = relu?((Â·X)[own rows] + bias).  bias (fp32 [F], nullable) / relu: the GCN epilogue, fused into
+        the launch that writes each row's last contribution (no extra pass over Y).  Collective: every rank of the
+        group runs the same sequence of forward / backward calls (the arrival flags count steps)."""
         from .functional import spmm_raw
         plan = self.plan
         assert X.shape == (plan.n_local, self.F) and X.dtype == self.dtype and X.is_cuda
@@ -749,27 +773,28 @@ class PartitionedSpmm:
         if out is None:
             out = torch.empty((plan.n_local, self.F), dtype=self.dtype, device=self.dev)
         if plan.world == 1:
-            return spmm_raw(self.A_loc, X, out=out)
+            return spmm_raw(self.A_loc, X, out=out, bias=bias, relu=relu)
         K, s = plan.waves, self._fstep
         flags = self.transport in ("p2p", "ce")
         comm = self.comm if overlap else main
         if overlap:
             self._ev_x.record(main)
             self.comm.wait_event(self._ev_x)  # X is ready (and everything earlier on the main stream is done)
+            X.record_stream(self.comm)  # the movers read X after the main stream is done with it
         with torch.cuda.stream(comm):
             self._exchange(X, comm)
             if not flags:
                 self._ev_halo.record(comm)
         excl = 28 * 1024 if (self.transport == "p2p" and self.dedicated > 0 and overlap) else 0
         if plan.p1 is not None:
-            self._run(plan.p1, X, self.halo, out, excl)
+            self._run(plan.p1, X, self.halo, out, excl, bias, relu)
         if not flags and overlap:
             main.wait_event(self._ev_halo)
         for w in range(K):
             if flags:
                 self._wait(0, s * K + w + 1, main)
             if plan.p2[w] is not None:
-                self._run(plan.p2[w], X, self.halo, out)
+                self._run(plan.p2[w], X, self.halo, out, 0, bias, relu)
         if flags:
             self._signal(1, s + 1, main)  # this rank is done reading its halo
         self._fstep += 1
@@ -882,3 +907,127 @@ class PartitionedSpmm:
             for b in self._bufs:
                 b.close()
             self._bufs = []
+
+
+class PartitionedGraph:
+    """This rank's share of a row-partitioned graph, in the form a GCN layer takes as `adj`
+    (`Graph_conv_layer.forward(X_local, pg)`, `GCN_Model.forward(X_local, pg)`; X_local = the rank's own rows).
+
+    Holds the row-block `bounds`, the `HaloPlan` (built once, at the widest width: only the schedule choice
+    depends on F) and one `PartitionedSpmm` per feature width in `widths`.  The operators are built here, not on
+    first use: creating one maps peer buffers and is a collective.
+
+    Lock-step: the halo exchange counts steps with flags in peer memory, so every rank of `group` must run the
+    same sequence of forward and backward calls (same layers, same order) — a model's forward / backward on every
+    rank, every step.  Ranks that own no training row still run both.
+
+    Constructors: `PartitionedGraph(rowptr, col, val, bounds, rank, world, widths, ...)` from the rank's own row
+    block (rowptr over its rows, GLOBAL column ids — what `build_halo_plan` takes), or `from_global(g, ...)` for a
+    graph every rank holds.  Keyword arguments other than the plan's go to every `PartitionedSpmm`."""
+
+    def __init__(self, rowptr: torch.Tensor, col: torch.Tensor, val: Optional[torch.Tensor], bounds: List[int],
+                 rank: int, world: int, widths, device=None, group=None, waves: Optional[int] = 1,
+                 two_pass_chunks: Optional[int] = None, transport: str = "p2p", dtype: torch.dtype = torch.float32,
+                 **op_kw):
+        self.bounds, self.rank, self.world, self.group = [int(b) for b in bounds], int(rank), int(world), group
+        self.dev = torch.device(device) if device is not None else col.device
+        widths = sorted({int(w) for w in widths})
+        if not widths or widths[0] <= 0:
+            raise ValueError("PartitionedGraph: at least one positive feature width is needed")
+        elem = 4 if dtype == torch.float32 else 2
+        self.plan = build_halo_plan(rowptr.to(self.dev), col.to(self.dev), None if val is None else val.to(self.dev),
+                                    self.bounds, self.rank, self.world, group=group, waves=waves,
+                                    two_pass_chunks=two_pass_chunks, F=widths[-1], elem_size=elem)
+        self.ops: Dict[int, PartitionedSpmm] = {}
+        try:
+            for F in widths:
+                self.ops[F] = PartitionedSpmm(self.plan, F, self.dev, group=group, transport=transport, dtype=dtype,
+                                              **op_kw)
+        except Exception:
+            self.close()
+            raise
+
+    @classmethod
+    def from_global(cls, g, rank: int, world: int, widths, group=None, **kw) -> "PartitionedGraph":
+        """From a whole `CSRGraph` every rank holds: row blocks balanced by nnz (`balanced_bounds`), this rank's
+        block cut out of it."""
+        bounds = balanced_bounds(g.rowptr, world)
+        lo, hi = bounds[rank], bounds[rank + 1]
+        rows = torch.arange(lo, hi, dtype=torch.int64, device=g.rowptr.device)
+        rp, cc, vv = select_rows(g.rowptr, g.col, g.val, rows)
+        return cls(rp, cc, vv, bounds, rank, world, widths, device=kw.pop("device", g.rowptr.device), group=group, **kw)
+
+    @property
+    def n_local(self) -> int:
+        return self.plan.n_local
+
+    @property
+    def row_range(self):
+        return self.bounds[self.rank], self.bounds[self.rank + 1]
+
+    def op(self, F: int) -> PartitionedSpmm:
+        op = self.ops.get(int(F))
+        if op is None:
+            raise _lib.GnnError(f"PartitionedGraph: no operator for feature width {F} (built for {sorted(self.ops)}); "
+                                "list every layer's output width in `widths`")
+        return op
+
+    def local_index(self, idx_global: torch.Tensor) -> torch.Tensor:
+        """The global node ids of `idx_global` (train / val / test ids) that this rank owns, as local row indices
+        (ascending where idx_global is)."""
+        lo, hi = self.row_range
+        idx = idx_global.to(torch.int64)
+        return idx[(idx >= lo) & (idx < hi)] - lo
+
+    def close(self):
+        """Free the peer buffers (collective: every rank calls it)."""
+        for op in self.ops.values():
+            op.close()
+        self.ops = {}
+
+
+# ---- training across ranks ------------------------------------------------------------------
+# A model holds replicated weights and rank-local activations.  With the loss rule below, the SUM over the ranks of
+# the per-rank gradients is the 1-GPU gradient, so one SUM all_reduce of the gradients before the optimizer step
+# keeps the replicas identical (given identical initial weights: broadcast_parameters).
+
+def broadcast_parameters(module: torch.nn.Module, group=None):
+    """Send the parameters and buffers of the group's first rank to every rank (call once, before training)."""
+    src = 0 if group is None else dist.get_global_rank(group, 0)
+    with torch.no_grad():
+        for t in list(module.parameters()) + list(module.buffers()):
+            dist.broadcast(t.data, src=src, group=group)
+
+
+def allreduce_gradients(module: torch.nn.Module, group=None):
+    """SUM every parameter's .grad over the ranks: one all_reduce of the gradients flattened in parameter order
+    (a missing .grad counts as zeros).  Call between backward() and optimizer.step()."""
+    params = [p for p in module.parameters() if p.requires_grad]
+    if not params:
+        return
+    flat = torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).reshape(-1) for p in params])
+    dist.all_reduce(flat, group=group)
+    off = 0
+    for p in params:
+        n = p.numel()
+        g = flat[off:off + n].view_as(p)
+        if p.grad is None:
+            p.grad = g.clone()
+        else:
+            p.grad.copy_(g)
+        off += n
+
+
+def global_count(n_local: int, device, group=None) -> int:
+    """Σ over the ranks of n_local (e.g. the global number of training rows): one all_reduce."""
+    t = torch.tensor([int(n_local)], dtype=torch.int64, device=device)
+    dist.all_reduce(t, group=group)
+    return int(t.item())
+
+
+def partitioned_cross_entropy(logits_local: torch.Tensor, target_local: torch.Tensor, n_global: int) -> torch.Tensor:
+    """The loss rule of partitioned training: Σ of the per-row cross-entropy over this rank's rows, divided by
+    the GLOBAL row count (`global_count`).  The sum of these losses over the ranks is the mean cross-entropy over
+    all rows — `nn.CrossEntropyLoss()(output[idx_train], labels[idx_train])` of the 1-GPU model — and the sum of
+    their gradients (`allreduce_gradients`) is its gradient."""
+    return torch.nn.functional.cross_entropy(logits_local, target_local, reduction="sum") / float(max(n_global, 1))

@@ -155,15 +155,23 @@ int gnn_spmm_csr_planned_bf16(const int64_t* rowptr, const int32_t* col, const f
 /* Extended form of the planned SpMM for ROW SUBSETS and TWO SOURCE TABLES — the consumers of the
  * wave-pipelined halo exchange of the partitioned SpMM (SURVEY.md §8e; reference seam GCN/GCN.py:43).
  * The CSR passed in is compact over the selected rows (rowptr has n_rows+1 entries):
- *   row_map (nullable, int32 [n_rows], ascending): compact row r writes Y row row_map[r];
+ *   row_map (nullable, int32 [n_rows], distinct rows in any order): compact row r writes Y row row_map[r];
  *   accumulate_prefix: compact rows [0, accumulate_prefix) add into Y (their local-column part was
  *     written by an earlier pass), the others overwrite — one launch serves both kinds of row;
  *   X2/ldx2/split: a column id c >= split reads row (c - split) of X2 (the halo buffer) instead of X,
  *     so rows that need local AND remote columns finish in ONE pass with no read-modify-write of Y;
+ *   bias/relu: the GCN epilogue y = relu?(. + bias) of the planned entry, here allowed in EVERY form:
+ *     with accumulate / accumulate_prefix it applies after the add, y = relu?(y_prev + sum + bias),
+ *     and with X2 to the two-table sum, so each output row gets it once, in the launch that writes
+ *     the row's last contribution (the planned entry still refuses accumulate with bias/relu);
+ *   epilogue_skip_prefix: compact rows [0, epilogue_skip_prefix) get NO epilogue even when bias/relu
+ *     are set — the first pass of two-pass rows, written in the same launch as finished rows;
  *   exclusion_smem_bytes: token dynamic shared memory per CTA (<= 48 KB), for callers that keep this
  *     kernel off SMs a shared-memory-filling mover kernel has claimed.  0 = none.
  * Every per-call choice is an argument: no process-global state is consulted.
- * struct_size = sizeof(gnn_spmm_opts) (ABI versioning); zero-initialise the rest. */
+ * struct_size = sizeof(gnn_spmm_opts) (ABI versioning); zero-initialise the rest.  A struct_size of
+ * offsetof(gnn_spmm_opts, epilogue_skip_prefix) (the layout before that field was appended) is also
+ * accepted and reads as epilogue_skip_prefix = 0; any other size is refused. */
 typedef struct gnn_spmm_opts {
   int32_t struct_size;
   int32_t accumulate;
@@ -184,6 +192,7 @@ typedef struct gnn_spmm_opts {
   int32_t exclusion_smem_bytes;
   void* workspace;
   size_t workspace_bytes;
+  int64_t epilogue_skip_prefix;
 } gnn_spmm_opts;
 int gnn_spmm_csr_ex_f32(const int64_t* rowptr, const int32_t* col, const float* val,
                         const float* X, float* Y, int64_t n_rows, int64_t n_cols, int32_t F,
