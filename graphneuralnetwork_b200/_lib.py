@@ -61,6 +61,9 @@ SIGNATURES = {
     "gnn_gat_fused_bwd_f32": (cint, [ptr, ptr, ptr, ptr, ptr, ptr, i64, ptr, ptr, ptr, ptr, ptr, ptr, i64, i64, i32,
                                      i32, f32, cint, ptr, ptr, i64, ptr, ptr, ptr, i64, ptr, i64, ptr, i64, i64, cint,
                                      ptr, ptr, i64, ptr]),
+    "gnn_gat_fused_bwd_ex_f32": (cint, [ptr, ptr, ptr, ptr, ptr, ptr, i64, ptr, ptr, ptr, ptr, ptr, ptr, i64, i64, i64,
+                                        i32, i32, f32, cint, ptr, ptr, i64, ptr, ptr, ptr, i64, ptr, i64, ptr, i64, i64,
+                                        cint, ptr, ptr, ptr]),
     "gnn_gat_fused_fwd_train_f32": (cint, [ptr, ptr, ptr, i64, ptr, ptr, i64, i64, i32, i32, f32, cint, cint, ptr, ptr,
                                            ptr, ptr, ptr, i64, ptr, ptr, ptr, i64, i64, i64, ptr]),
     "gnn_gat_fused_fwd_train_bf16": (cint, [ptr, ptr, ptr, i64, ptr, ptr, i64, i64, i32, i32, f32, cint, cint, ptr, ptr,
@@ -100,7 +103,7 @@ class SpmmOpts(C.Structure):
 
 class GatDropout(C.Structure):
     """gnn_gat_dropout of include/gnn_b200.h."""
-    _fields_ = [("struct_size", i32), ("p", f32), ("seed", u64), ("seed_dev", ptr)]
+    _fields_ = [("struct_size", i32), ("p", f32), ("seed", u64), ("seed_dev", ptr), ("edge_slot_base", i64)]
 
 
 class HaloOpts(C.Structure):

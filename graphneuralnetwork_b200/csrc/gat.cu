@@ -785,16 +785,25 @@ int gat_fwd_dispatch(const GatArgs& a, int cpl, unsigned grid, cudaStream_t st) 
   }
 }
 
+// struct_size is the version of gnn_gat_dropout: the current size, or the size before edge_slot_base was appended
+// (read as base 0); any other size is refused.  a.H must be set.
 inline int set_dropout(GatArgs& a, const float* edge_keep, const gnn_gat_dropout* d) {
   a.keep = edge_keep;
   if (d && d->p > 0.f) {
-    GNN_REQUIRE(d->struct_size == (int32_t)sizeof(gnn_gat_dropout), GNN_ERR_BAD_ARG,
+    const bool cur = d->struct_size == (int32_t)sizeof(gnn_gat_dropout);
+    GNN_REQUIRE(cur || d->struct_size == (int32_t)offsetof(gnn_gat_dropout, edge_slot_base), GNN_ERR_BAD_ARG,
                 "gnn_gat_dropout struct_size mismatch (header/library version skew)");
+    const int64_t base = cur ? d->edge_slot_base : 0;
+    GNN_REQUIRE(base >= 0, GNN_ERR_BAD_ARG, "negative edge_slot_base");
+    GNN_REQUIRE(base == 0 || !d->seed_dev, GNN_ERR_UNSUPPORTED,
+                "edge_slot_base needs the whole seed on the host (seed_dev = NULL)");
     GNN_REQUIRE(d->p < 1.f, GNN_ERR_BAD_ARG, "dropout probability must be below 1");
     GNN_REQUIRE(!edge_keep, GNN_ERR_BAD_ARG, "give either an explicit keep mask or a seeded dropout, not both");
     a.keep_prob = 1.f - d->p;
     a.drop_scale = 1.f / a.keep_prob;
-    a.drop_seed = d->seed;
+    // keep_factor hashes seed + (e*H + h + 1)*golden: slot e + base is slot e under seed + base*H*golden (mod 2^64),
+    // so the base is folded into the seed here and the kernels are unchanged
+    a.drop_seed = d->seed + (uint64_t)base * (uint64_t)a.H * 0x9E3779B97F4A7C15ULL;
     a.drop_seed_dev = d->seed_dev;
   }
   return GNN_OK;
@@ -902,14 +911,20 @@ int gat_bwd2_dispatch(const GatArgs& a, int cplr, unsigned grid, cudaStream_t st
 template <typename T>
 int gat_bwd_impl(const int64_t* rowptr, const int32_t* col, const int64_t* rowptr_t, const int32_t* col_t,
                  const int64_t* perm_t, const T* Wh, int64_t ldw, const float* s, const float* t, const float* row_max,
-                 const float* row_sum, const T* out_pre, const T* d_out, int64_t ldo, int64_t n, int32_t H, int32_t Fp,
+                 const float* row_sum, const T* out_pre, const T* d_out, int64_t ldo, int64_t n, int64_t n_cols,
+                 int32_t H, int32_t Fp,
                  float alpha, int mode, const float* edge_keep, T* d_Wh, int64_t ld_dwh, float* d_s, float* d_t,
                  float* row_scratch, int64_t nnz, const int64_t* long_rows, int64_t n_long, const int64_t* long_rows_t,
                  int64_t n_long_t, int64_t long_threshold, cudaStream_t st, int apply_elu = 0, T* d_pre = nullptr,
                  const gnn_gat_dropout* drop = nullptr, int64_t batch_nodes = 0) {
   int rc = check_common(n, H, Fp);
   if (rc != GNN_OK) return rc;
-  if (n == 0) return GNN_OK;
+  rc = check_common(n_cols, H, Fp);
+  if (rc != GNN_OK) return rc;
+  GNN_REQUIRE(n_cols >= n, GNN_ERR_BAD_ARG, "n_cols (%lld) below the forward row count (%lld)", (long long)n_cols,
+              (long long)n);
+  GNN_REQUIRE(n_cols == n || batch_nodes == 0, GNN_ERR_UNSUPPORTED, "batched graphs are square (n_cols == n)");
+  if (n == 0 && n_cols == 0) return GNN_OK;
   GNN_REQUIRE(rowptr && rowptr_t && Wh && s && t && row_max && row_sum && out_pre && d_out && d_Wh && d_s && d_t &&
                   row_scratch,
               GNN_ERR_BAD_ARG, "null pointer");
@@ -950,7 +965,7 @@ int gat_bwd_impl(const int64_t* rowptr, const int32_t* col, const int64_t* rowpt
   a.ld_dwh = ld_dwh;
   a.d_s = d_s;
   a.d_t = d_t;
-  {
+  if (n > 0) {
     int64_t grid = (n * H + 255) / 256;
     const int64_t cap = (int64_t)num_sms() * 16;
     grid = grid > cap ? cap : grid;
@@ -963,15 +978,19 @@ int gat_bwd_impl(const int64_t* rowptr, const int32_t* col, const int64_t* rowpt
   const int cpl = (HF + 31) / 32;
   int cplr = cpl <= 1 ? 1 : cpl <= 2 ? 2 : cpl <= 4 ? 4 : 8;
   if (a.packed && cplr < 2) cplr = 2;
-  const bool coop = cooperative(n, nnz);
+  // the row-record kernel and pass 1 walk the n forward rows; pass 2 the n_cols table rows (its own schedule)
+  const bool coop = cooperative(n, nnz), coop_t = cooperative(n_cols, nnz);
   const unsigned grid1 = (unsigned)((n + kGatWarps - 1) / kGatWarps);
+  const unsigned grid1_t = (unsigned)((n_cols + kGatWarps - 1) / kGatWarps);
   GNN_REQUIRE((n_long == 0 || long_rows) && (n_long_t == 0 || long_rows_t) &&
                   ((n_long == 0 && n_long_t == 0) || long_threshold > 0),
               GNN_ERR_BAD_ARG, "inconsistent long-row lists");
   // pass 1 over the forward CSR: d_s.  W: 1 warp per row, 4 = every row a CTA (dense graphs), 16 = listed hub rows
   a.rowptr = rowptr;
   a.col = col;
-  if (coop) {
+  if (n == 0) {
+    // no forward row: the table rows get zero gradients from pass 2 (every transposed row is empty)
+  } else if (coop) {
     rc = gat_bwd2_dispatch<T, 4, false>(a, cplr, (unsigned)n, st);
     if (rc != GNN_OK) return rc;
   } else {
@@ -989,9 +1008,10 @@ int gat_bwd_impl(const int64_t* rowptr, const int32_t* col, const int64_t* rowpt
   a.rowptr = rowptr_t;
   a.col = col_t;
   a.perm = perm_t;
+  a.n = n_cols;
   a.row_list = nullptr;
   a.skip_deg_gt = 0;
-  if (coop) return gat_bwd2_dispatch<T, 4, true>(a, cplr, (unsigned)n, st);
+  if (coop_t) return gat_bwd2_dispatch<T, 4, true>(a, cplr, (unsigned)n_cols, st);
   if (n_long_t > 0) {
     a.row_list = long_rows_t;
     rc = gat_bwd2_dispatch<T, 16, true>(a, cplr, (unsigned)n_long_t, st);
@@ -999,7 +1019,7 @@ int gat_bwd_impl(const int64_t* rowptr, const int32_t* col, const int64_t* rowpt
     a.row_list = nullptr;
     a.skip_deg_gt = long_threshold;
   }
-  return gat_bwd2_dispatch<T, 1, true>(a, cplr, grid1, st);
+  return gat_bwd2_dispatch<T, 1, true>(a, cplr, grid1_t, st);
 }
 
 }  // namespace
@@ -1076,7 +1096,7 @@ int gnn_gat_fused_bwd_f32(const int64_t* rowptr, const int32_t* col, const int64
                           const int64_t* long_rows_t, int64_t n_long_t, int64_t long_threshold, int apply_elu,
                           float* d_pre, const gnn_gat_dropout* dropout, int64_t batch_nodes, gnn_stream_t stream) {
   return gat_bwd_impl<float>(rowptr, col, rowptr_t, col_t, perm_t, Wh, ldw, s, t, row_max, row_sum, out_pre, d_out, ldo,
-                             n, H, Fp, alpha, mode, edge_keep, d_Wh, ld_dwh, d_s, d_t, row_scratch, nnz, long_rows,
+                             n, n, H, Fp, alpha, mode, edge_keep, d_Wh, ld_dwh, d_s, d_t, row_scratch, nnz, long_rows,
                              n_long, long_rows_t, n_long_t, long_threshold, (cudaStream_t)stream, apply_elu, d_pre,
                              dropout, batch_nodes);
 }
@@ -1090,10 +1110,24 @@ int gnn_gat_fused_bwd_bf16(const int64_t* rowptr, const int32_t* col, const int6
                            const int64_t* long_rows_t, int64_t n_long_t, int64_t long_threshold, int apply_elu,
                            void* d_pre, const gnn_gat_dropout* dropout, int64_t batch_nodes, gnn_stream_t stream) {
   return gat_bwd_impl<__nv_bfloat16>(rowptr, col, rowptr_t, col_t, perm_t, (const __nv_bfloat16*)Wh, ldw, s, t, row_max,
-                                     row_sum, (const __nv_bfloat16*)out_pre, (const __nv_bfloat16*)d_out, ldo, n, H, Fp,
+                                     row_sum, (const __nv_bfloat16*)out_pre, (const __nv_bfloat16*)d_out, ldo, n, n, H, Fp,
                                      alpha, mode, edge_keep, (__nv_bfloat16*)d_Wh, ld_dwh, d_s, d_t, row_scratch, nnz,
                                      long_rows, n_long, long_rows_t, n_long_t, long_threshold, (cudaStream_t)stream,
                                      apply_elu, (__nv_bfloat16*)d_pre, dropout, batch_nodes);
+}
+
+int gnn_gat_fused_bwd_ex_f32(const int64_t* rowptr, const int32_t* col, const int64_t* rowptr_t, const int32_t* col_t,
+                             const int64_t* perm_t, const float* Wh, int64_t ldw, const float* s, const float* t,
+                             const float* row_max, const float* row_sum, const float* out_pre, const float* d_out,
+                             int64_t ldo, int64_t n_rows, int64_t n_cols, int32_t H, int32_t Fp, float alpha, int mode,
+                             const float* edge_keep, float* d_Wh, int64_t ld_dwh, float* d_s, float* d_t,
+                             float* row_scratch, int64_t nnz, const int64_t* long_rows, int64_t n_long,
+                             const int64_t* long_rows_t, int64_t n_long_t, int64_t long_threshold, int apply_elu,
+                             float* d_pre, const gnn_gat_dropout* dropout, gnn_stream_t stream) {
+  return gat_bwd_impl<float>(rowptr, col, rowptr_t, col_t, perm_t, Wh, ldw, s, t, row_max, row_sum, out_pre, d_out, ldo,
+                             n_rows, n_cols, H, Fp, alpha, mode, edge_keep, d_Wh, ld_dwh, d_s, d_t, row_scratch, nnz,
+                             long_rows, n_long, long_rows_t, n_long_t, long_threshold, (cudaStream_t)stream, apply_elu,
+                             d_pre, dropout, 0);
 }
 
 }  // extern "C"

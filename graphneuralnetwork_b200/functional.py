@@ -271,6 +271,35 @@ def partitioned_gcn_aggregate(pg, S: torch.Tensor, bias: Optional[torch.Tensor] 
     return _PartitionedGcnAggregateFn.apply(S.contiguous(), bias, pg.op(S.shape[1]), relu)
 
 
+class _HaloExchangeFn(torch.autograd.Function):
+    """X_comb = [X_local ; halo rows] of a row-partitioned graph.  Backward: dX_local = dX_comb[:n_local] plus the
+    halo rows' gradients every peer returns, added in fixed (peer, slot) order (partition.PartitionedSpmm)."""
+
+    @staticmethod
+    def forward(ctx, X, op):
+        ctx.op = op
+        return op.gather_halo(X)
+
+    @staticmethod
+    def backward(ctx, dX_comb):
+        # always run: the gradient return is a collective every rank takes part in
+        return ctx.op.return_halo_grad(dX_comb.contiguous()), None
+
+
+def halo_exchange(pg, X_local: torch.Tensor) -> torch.Tensor:
+    """[X_local ; halo] ([n_local + n_halo, F], fp32) over a partition.PartitionedGraph `pg`: the table whose rows the
+    combined column ids of `pg.attention()` address, as a private copy (its backward needs the halo rows after
+    later exchanges may have reused the peer buffer).  Collective, with autograd: every rank calls it, and its
+    backward, in the same order."""
+    _require_cuda(X_local)
+    if X_local.dtype != torch.float32:
+        raise _lib.GnnError("halo_exchange: fp32 features expected")
+    if X_local.dim() != 2 or X_local.shape[0] != pg.n_local:
+        raise _lib.GnnError(f"halo_exchange: X_local must be [{pg.n_local}, F] (this rank's rows), "
+                            f"got {tuple(X_local.shape)}")
+    return _HaloExchangeFn.apply(X_local.contiguous(), pg.op(X_local.shape[1]))
+
+
 # --------------------------------------------------------------------------------------
 # GraphSAGE: fused gather + reduce
 # --------------------------------------------------------------------------------------
@@ -556,10 +585,13 @@ def _gat_groups(H: int, Fp: int):
 class AttentionDropout:
     """Seeded post-softmax attention dropout (GAT/models/layers.py:31) for the fused kernels: probability `p`, a host
     seed and a device int64 tensor mixed into it (so a captured CUDA graph draws a fresh mask per replay).  The
-    kernels recompute the keep factor of every (edge, head) from the stream — no [nnz, H] mask is materialised."""
+    kernels recompute the keep factor of every (edge, head) from the stream — no [nnz, H] mask is materialised.
+    edge_slot_base: local edge slot e draws the factor of slot e + edge_slot_base (a row block of a larger CSR passes
+    its first global slot and draws the whole graph's mask for its edges)."""
 
-    def __init__(self, p: float, seed: int, seed_dev: Optional[torch.Tensor] = None):
+    def __init__(self, p: float, seed: int, seed_dev: Optional[torch.Tensor] = None, edge_slot_base: int = 0):
         self.p, self.seed, self.seed_dev = float(p), int(seed) & 0xFFFFFFFFFFFFFFFF, seed_dev
+        self.edge_slot_base = int(edge_slot_base)
         assert seed_dev is None or (seed_dev.dtype == torch.int64 and seed_dev.is_cuda and seed_dev.numel() == 1)
 
     def c_struct(self):
@@ -567,7 +599,16 @@ class AttentionDropout:
         d = _lib.GatDropout()
         d.struct_size = C.sizeof(_lib.GatDropout)
         d.p, d.seed, d.seed_dev = self.p, self.seed, _p(self.seed_dev)
+        d.edge_slot_base = self.edge_slot_base
         return d
+
+    def with_slot_base(self, edge_slot_base: int) -> "AttentionDropout":
+        """The same stream for a row block whose first edge is global slot `edge_slot_base`.  The kernels take a slot
+        base only with the whole seed on the host, so the device half is read back here (one synchronisation)."""
+        seed = self.seed
+        if self.seed_dev is not None:
+            seed ^= (int(self.seed_dev.item()) * 0xD6E8FEB86659FD93) & 0xFFFFFFFFFFFFFFFF
+        return AttentionDropout(self.p, seed, None, edge_slot_base)
 
 
 _drop_counters = {}
@@ -602,7 +643,7 @@ def attention_keep_mask_from_seed(g: CSRGraph, H: int, drop: AttentionDropout) -
     seed = drop.seed
     if drop.seed_dev is not None:
         seed ^= (int(drop.seed_dev.item()) * 0xD6E8FEB86659FD93) & M64
-    idx = torch.arange(g.nnz * H, dtype=torch.int64, device=g.device) + 1
+    idx = torch.arange(g.nnz * H, dtype=torch.int64, device=g.device) + (drop.edge_slot_base * H + 1)
     z = idx * s64(0x9E3779B97F4A7C15) + s64(seed)
     z = (z ^ lsr(z, 30)) * s64(0xBF58476D1CE4E5B9)
     z = (z ^ lsr(z, 27)) * s64(0x94D049BB133111EB)
@@ -623,7 +664,9 @@ def gat_fwd_raw(g: CSRGraph, Wh, s, t, H, Fp, alpha, mode=_lib.GAT_SOFTMAX, elu=
     Training form (`out_act` given): `out` receives the PRE-activation aggregate and `out_act` the activated one
     (elu applied `elu` times) in the same launch.  `dropout`: seeded attention dropout (or `keep`: explicit mask).
     batch = M > 1: `g` is the block diagonal of M graphs over the same N nodes (CSRGraph.block_diagonal), Wh / out are
-    [N, M*H*Fp] (graph m's columns at m*H*Fp), s / t are [M*N, H] (batched-row major) — HAN's metapaths in one launch."""
+    [N, M*H*Fp] (graph m's columns at m*H*Fp), s / t are [M*N, H] (batched-row major) — HAN's metapaths in one launch.
+    Rectangular `g` (n_cols > n_rows, a row block whose columns address [own rows ; halo rows]): Wh and t have n_cols
+    rows, s and out n_rows; fp32, one graph, H*Fp <= 256 and no row without edges."""
     _require_cuda(Wh, s, t, keep)
     lib = _lib.load()
     Wh = _rowmajor(Wh)
@@ -631,12 +674,15 @@ def gat_fwd_raw(g: CSRGraph, Wh, s, t, H, Fp, alpha, mode=_lib.GAT_SOFTMAX, elu=
         raise _lib.GnnError(f"gat: unsupported dtype {Wh.dtype} (fp32 and bf16 only)")
     s = s.float().contiguous()
     t = t.float().contiguous()
-    n = g.n_rows
+    n, nc = g.n_rows, g.n_cols
     M = int(batch)
     nodes = n // M
-    if M < 1 or n % M or Wh.shape != (nodes, M * H * Fp) or g.n_cols != n or s.shape != (n, H) or t.shape != (n, H):
-        raise _lib.GnnError(f"gat: Wh {tuple(Wh.shape)} / s {tuple(s.shape)} do not match graph rows={n}, batch={M}, "
-                            f"H*Fp={H * Fp}")
+    if (M < 1 or n % M or nc < n or Wh.shape != (nc // M, M * H * Fp) or s.shape != (n, H)
+            or t.shape != (nc, H)):
+        raise _lib.GnnError(f"gat: Wh {tuple(Wh.shape)} / s {tuple(s.shape)} / t {tuple(t.shape)} do not match graph "
+                            f"rows={n}, cols={nc}, batch={M}, H*Fp={H * Fp}")
+    if nc != n and (M > 1 or H * Fp > 256 or Wh.dtype != torch.float32):
+        raise _lib.GnnError("gat: a rectangular graph (table rows != rows) takes one fp32 graph of H*Fp <= 256")
     if M > 1 and H * Fp > 256:
         raise _lib.GnnError("gat: batched graphs need H*Fp <= 256 per graph")
     if out is None:
@@ -648,6 +694,9 @@ def gat_fwd_raw(g: CSRGraph, Wh, s, t, H, Fp, alpha, mode=_lib.GAT_SOFTMAX, elu=
         raise _lib.GnnError("gat: `out_act` must match `out` in shape, dtype and strides")
     row_max = torch.empty((n, H), dtype=torch.float32, device=Wh.device) if save_stats else None
     row_sum = torch.empty((n, H), dtype=torch.float32, device=Wh.device) if save_stats else None
+    if nc != n and g.has_empty_rows():
+        raise _lib.GnnError("gat: rows without edges take the mean of ALL table rows (GAT/models/layers.py:28-30), "
+                            "which a rectangular graph does not define")
     col_mean = Wh.float().mean(dim=0).contiguous() if g.has_empty_rows() else None
     bn = nodes if M > 1 else 0
     lr, thr = g.gat_long_rows()
@@ -727,7 +776,7 @@ class _GatFn(torch.autograd.Function):
         keep = keep if keep.numel() > 0 else None
         drop = ctx.dropout if (ctx.dropout is not None and ctx.dropout.p > 0.0) else None
         dstruct = drop.c_struct() if drop is not None else None
-        n = g.n_rows
+        n, nc = g.n_rows, g.n_cols
         d_out = d_out.to(Wh.dtype)
         if d_out.stride(1) != 1 or d_out.stride(0) != out.stride(0):
             d_out = d_out.contiguous()  # out is contiguous [n, H*Fp]: one leading dimension for both
@@ -737,13 +786,22 @@ class _GatFn(torch.autograd.Function):
         bn = n // M if M > 1 else 0
         d_Wh = torch.empty_like(Wh)
         d_s = torch.empty((n, H), dtype=torch.float32, device=dev)
-        d_t = torch.empty((n, H), dtype=torch.float32, device=dev)
+        d_t = torch.empty((nc, H), dtype=torch.float32, device=dev)
         d_pre = torch.empty_like(out) if elu > 0 else None
         (lr, thr), (lrt, _) = g.gat_long_rows(), gt.gat_long_rows()
         fn = lib.gnn_gat_fused_bwd_f32 if Wh.dtype == torch.float32 else lib.gnn_gat_fused_bwd_bf16
         groups = list(_gat_groups(H, Fp))
         esz = Wh.element_size()
         need_perm = keep is not None or drop is not None
+        if nc != n:  # rectangular (one fp32 group, checked by the forward): table rows get d_Wh / d_t
+            row_scratch = torch.empty((n, 4, H), dtype=torch.float32, device=dev)
+            _lib.check(lib.gnn_gat_fused_bwd_ex_f32(
+                _p(g.rowptr), _p(g.col), _p(gt.rowptr), _p(gt.col), _p(g.perm_t) if need_perm else None, _p(Wh), _ld(Wh),
+                _p(s), _p(t), _p(row_max), _p(row_sum), _p(out), _p(d_out), _ld(out), n, nc, H, Fp, alpha, mode,
+                _p(keep), _p(d_Wh), _ld(d_Wh), _p(d_s), _p(d_t), _p(row_scratch), g.nnz, _p(lr), lr.numel(), _p(lrt),
+                lrt.numel(), thr, elu, _p(d_pre), C.byref(dstruct) if dstruct is not None else None, _stream_ptr()),
+                "gnn_gat_fused_bwd_ex_f32")
+            groups = []
         for gi, (h0, h1, f0, f1) in enumerate(groups):
             whole = len(groups) == 1
             Hg, Fg = h1 - h0, f1 - f0

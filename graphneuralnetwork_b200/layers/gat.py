@@ -13,8 +13,9 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from .. import _lib
-from ..functional import attention_keep_mask, gat_aggregate, next_attention_dropout, spmm_values
+from ..functional import attention_keep_mask, gat_aggregate, halo_exchange, next_attention_dropout, spmm_values
 from ..graph import CSRGraph, adj_cache
+from ..partition import PartitionedGraph
 
 # True: draw the attention dropout as an explicit [nnz, H] mask (attention_keep_mask) instead of the seeded
 # in-kernel stream — the parity tests replay reference masks through this hook
@@ -65,7 +66,10 @@ class SpecialSpmm(nn.Module):
 
 
 def _fused_heads(x, adj, Ws, a_srcs, a_dsts, alpha, mode, elu, dropout, training, out=None):
-    """All heads of one attention layer: x [N,in]; Ws list of [in,F']; a_* list of [F']."""
+    """All heads of one attention layer: x [N,in]; Ws list of [in,F']; a_* list of [F'].
+    adj may be a partition.PartitionedGraph: x is then the rank's own rows, and so is the result."""
+    if isinstance(adj, PartitionedGraph):
+        return _fused_heads_partitioned(x, adj, Ws, a_srcs, a_dsts, alpha, mode, elu, dropout, training)
     g = adj_cache.get(adj)
     H = len(Ws)
     Fp = Ws[0].shape[1]
@@ -84,6 +88,36 @@ def _fused_heads(x, adj, Ws, a_srcs, a_dsts, alpha, mode, elu, dropout, training
         else:
             drop = next_attention_dropout(dropout, Wh.device)  # seeded: no [nnz, H] mask is materialised
     return gat_aggregate(g, Wh, s, t, H, Fp, alpha, mode=mode, elu=elu, keep=keep, out=out, dropout=drop)
+
+
+def _fused_heads_partitioned(x, pg, Ws, a_srcs, a_dsts, alpha, mode, elu, dropout, training):
+    """`_fused_heads` on this rank's row block: Wh of the own rows, the halo rows' Wh from their owners
+    (functional.halo_exchange), s of the own rows, t of all table rows, and the fused kernels over the block in the
+    combined column space.  The backward returns d Wh of the halo rows (from the aggregation and from t) to their
+    owners; d a_src / d a_dst are this rank's share, summed over the ranks by partition.allreduce_gradients."""
+    H = len(Ws)
+    Fp = Ws[0].shape[1]
+    if x.dtype != torch.float32:
+        raise _lib.GnnError(f"GAT on a PartitionedGraph: fp32 features only (got {x.dtype})")
+    if H * Fp > 256:
+        raise _lib.GnnError(f"GAT on a PartitionedGraph: H*F' = {H * Fp} exceeds the 256 columns of one fused "
+                            "attention call")
+    g, edge_slot_base = pg.attention()
+    W_cat = Ws[0] if H == 1 else torch.cat(list(Ws), dim=1)
+    Wh = halo_exchange(pg, torch.mm(x, W_cat))  # [n_local + n_halo, H*F']
+    Wh3 = Wh.view(-1, H, Fp)
+    a_src = a_srcs[0].view(1, Fp) if H == 1 else torch.stack(list(a_srcs), dim=0)
+    a_dst = a_dsts[0].view(1, Fp) if H == 1 else torch.stack(list(a_dsts), dim=0)
+    s = (Wh3[:pg.n_local] * a_src.unsqueeze(0)).sum(-1)  # [n_local, H]
+    t = (Wh3 * a_dst.unsqueeze(0)).sum(-1)               # [n_local + n_halo, H]
+    keep = drop = None
+    if training and dropout > 0.0:
+        if EXPLICIT_DROPOUT_MASK:
+            keep = attention_keep_mask(g, H, dropout)
+        else:
+            # the whole graph's mask for this block's edges
+            drop = next_attention_dropout(dropout, Wh.device).with_slot_base(edge_slot_base)
+    return gat_aggregate(g, Wh, s, t, H, Fp, alpha, mode=mode, elu=elu, keep=keep, dropout=drop)
 
 
 class GraphAttentionLayer(nn.Module):
@@ -167,7 +201,8 @@ class GATBase(nn.Module):
         self.out_att = self._head_cls(nhid * nheads, nclass, self.dropout, alpha, False)
 
     def forward(self, x, adj):
-        graph = adj_cache.get(adj)  # CSR of adj > 0, built once per adjacency tensor
+        # CSR of adj > 0, built once per adjacency tensor; a PartitionedGraph is passed through (x = own rows)
+        graph = adj if isinstance(adj, PartitionedGraph) else adj_cache.get(adj)
         heads = list(self.attentions)
         halves = [head._halves() for head in heads]
         p_att = heads[0].dropout.p if isinstance(heads[0].dropout, nn.Dropout) else heads[0].dropout

@@ -25,6 +25,7 @@ from .. import _lib
 from ..functional import (SEMANTIC_MAX_K, SEMANTIC_MAX_M, gat_aggregate, next_attention_dropout,
                           semantic_attention)
 from ..graph import CSRGraph, adj_cache
+from ..partition import PartitionedGraph
 from .gat import GraphAttentionLayer, _fused_heads
 from . import gat as _gat
 
@@ -138,6 +139,9 @@ class HANLayer(nn.Module):
         return z.view(n, M, H * Fp)
 
     def forward(self, gs, h):
+        if any(isinstance(g, PartitionedGraph) for g in gs):
+            raise _lib.GnnError("HANLayer: metapath graphs on a PartitionedGraph are not supported (the batched "
+                                "metapath attention runs on one GPU)")
         convs = list(self.gat_layers)
         heads0 = list(convs[0].attentions)
         if (getattr(self, "batched", True) and len(convs) > 1 and all(c.num_class is None for c in convs)
@@ -163,7 +167,7 @@ class HANModel(nn.Module):
         self.predict = nn.Linear(widths[-1], out_size)
 
     def forward(self, g, h):
-        graphs = [adj_cache.get(a) for a in g]  # dense float64 masks -> CSR, once per graph
+        graphs = [a if isinstance(a, PartitionedGraph) else adj_cache.get(a) for a in g]  # dense float64 masks -> CSR, once per graph
         for layer in self.layers:
             h = layer(graphs, h)
         return self.predict(h)

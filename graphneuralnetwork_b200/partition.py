@@ -438,6 +438,51 @@ def build_halo_plan(rowptr: torch.Tensor, col: torch.Tensor, val: Optional[torch
     return plan
 
 
+@dataclass
+class AttentionView:
+    """This rank's row block in the COMBINED column space of `build_halo_plan`: local column c -> c - lo, remote
+    column -> n_local + its halo slot.  The columns address Wh_comb = [Wh_local ; Wh_halo] (functional.halo_exchange),
+    and every row keeps the edge order of the global CSR, so a fused attention row over it is the same ordered
+    reduction as over the whole graph.  edge_slot_base = the block's first global edge slot (global rowptr[lo]): the
+    seeded attention dropout of local slot e is the one of global slot e + edge_slot_base."""
+    rowptr: torch.Tensor
+    col: torch.Tensor             # int32 combined column ids
+    n_rows: int
+    n_cols: int                   # n_local + n_halo
+    edge_slot_base: int
+    any_empty_row: bool           # some row of the GLOBAL graph (any rank's block) has no edge
+
+    def require_edges(self):
+        """GAT's rule for a row without edges is the mean of ALL N rows of Wh (GAT/models/layers.py:28-30), which the
+        partitioned layer does not compute.  The flag is global, so every rank raises together."""
+        if self.any_empty_row:
+            raise _lib.GnnError("GAT on a PartitionedGraph: the graph has rows without edges (their output is the mean "
+                                "over all nodes, not supported across ranks); add self-loops")
+
+
+def build_attention_view(plan: HaloPlan, rowptr: torch.Tensor, col: torch.Tensor, group=None) -> AttentionView:
+    """The attention view of the block `plan` was built from (rowptr over the rank's rows, GLOBAL column ids).
+    Collective when world > 1: one all_gather of (nnz, has-empty-row) per rank gives the exclusive scan of the
+    ranks' nnz and the global empty-row flag."""
+    lo, hi = plan.bounds[plan.rank], plan.bounds[plan.rank + 1]
+    n_loc = hi - lo
+    col64 = col.to(torch.int64)
+    is_loc = (col64 >= lo) & (col64 < hi)
+    del col64
+    col_comb = torch.empty(col.numel(), dtype=torch.int32, device=col.device)
+    col_comb[is_loc] = plan.col_loc.to(col.device)
+    col_comb[~is_loc] = plan.col_rem.to(col.device) + n_loc
+    empty = bool((rowptr[1:] == rowptr[:-1]).any().item()) if n_loc > 0 else False
+    base, any_empty = 0, empty
+    if plan.world > 1:
+        mine = torch.tensor([col.numel(), int(empty)], dtype=torch.int64, device=col.device)
+        parts = [torch.empty_like(mine) for _ in range(plan.world)]
+        dist.all_gather(parts, mine, group=group)
+        base = sum(int(p[0].item()) for p in parts[:plan.rank])
+        any_empty = any(int(p[1].item()) for p in parts)
+    return AttentionView(rowptr, col_comb, n_loc, n_loc + plan.n_halo, base, any_empty)
+
+
 def reference_step_cpu(plan: HaloPlan, X_local: torch.Tensor, halo: torch.Tensor, bias: Optional[torch.Tensor] = None,
                        relu: bool = False) -> torch.Tensor:
     """The step's arithmetic with torch ops in float64 (test-side: replays P1 and the wave consumers of a
@@ -761,6 +806,32 @@ class PartitionedSpmm:
         else:
             spmm_ex(g, X, out, row_map=g._row_map, X2=halo, split=self.plan.n_local, bias=bias, relu=relu)
 
+    def _exchange_begin(self, X: torch.Tensor, overlap: bool):
+        """Start the exchange of this step: on the comm stream once X is ready (overlap) or on the main stream."""
+        main = torch.cuda.current_stream()
+        comm = self.comm if overlap else main
+        if overlap:
+            self._ev_x.record(main)
+            self.comm.wait_event(self._ev_x)  # X is ready (and everything earlier on the main stream is done)
+            X.record_stream(self.comm)  # the movers read X after the main stream is done with it
+        with torch.cuda.stream(comm):
+            self._exchange(X, comm)
+            if self.transport not in ("p2p", "ce"):
+                self._ev_halo.record(comm)
+
+    def _exchange_wait(self, w: int, stream):
+        """The halo rows of wave w are readable on `stream` (flags: per wave; nccl: the whole halo, at wave 0)."""
+        if self.transport in ("p2p", "ce"):
+            self._wait(0, self._fstep * self.plan.waves + w + 1, stream)
+        elif w == 0:
+            stream.wait_event(self._ev_halo)
+
+    def _exchange_end(self, stream):
+        """This rank is done reading its halo: the peers may overwrite it in the next step."""
+        if self.transport in ("p2p", "ce"):
+            self._signal(1, self._fstep + 1, stream)
+        self._fstep += 1
+
     def forward(self, X: torch.Tensor, out: Optional[torch.Tensor] = None, overlap: bool = True,
                 bias: Optional[torch.Tensor] = None, relu: bool = False) -> torch.Tensor:
         """Y_local = relu?((Â·X)[own rows] + bias).  bias (fp32 [F], nullable) / relu: the GCN epilogue, fused into
@@ -774,30 +845,33 @@ class PartitionedSpmm:
             out = torch.empty((plan.n_local, self.F), dtype=self.dtype, device=self.dev)
         if plan.world == 1:
             return spmm_raw(self.A_loc, X, out=out, bias=bias, relu=relu)
-        K, s = plan.waves, self._fstep
-        flags = self.transport in ("p2p", "ce")
-        comm = self.comm if overlap else main
-        if overlap:
-            self._ev_x.record(main)
-            self.comm.wait_event(self._ev_x)  # X is ready (and everything earlier on the main stream is done)
-            X.record_stream(self.comm)  # the movers read X after the main stream is done with it
-        with torch.cuda.stream(comm):
-            self._exchange(X, comm)
-            if not flags:
-                self._ev_halo.record(comm)
+        self._exchange_begin(X, overlap)
         excl = 28 * 1024 if (self.transport == "p2p" and self.dedicated > 0 and overlap) else 0
         if plan.p1 is not None:
             self._run(plan.p1, X, self.halo, out, excl, bias, relu)
-        if not flags and overlap:
-            main.wait_event(self._ev_halo)
-        for w in range(K):
-            if flags:
-                self._wait(0, s * K + w + 1, main)
+        for w in range(plan.waves):
+            self._exchange_wait(w, main)
             if plan.p2[w] is not None:
                 self._run(plan.p2[w], X, self.halo, out, 0, bias, relu)
-        if flags:
-            self._signal(1, s + 1, main)  # this rank is done reading its halo
-        self._fstep += 1
+        self._exchange_end(main)
+        return out
+
+    def gather_halo(self, X: torch.Tensor) -> torch.Tensor:
+        """X_comb = [X ; halo] ([n_local + n_halo, F]): the exchange of one step (waves, flags, transport as in
+        `forward`), then a private copy of the received rows in slot order.  Collective, like `forward`."""
+        plan = self.plan
+        assert X.shape == (plan.n_local, self.F) and X.dtype == self.dtype and X.is_cuda
+        out = torch.empty((plan.n_local + plan.n_halo, self.F), dtype=self.dtype, device=self.dev)
+        if plan.world > 1:
+            main = torch.cuda.current_stream()
+            self._exchange_begin(X, True)
+        out[:plan.n_local].copy_(X)
+        if plan.world == 1:
+            return out
+        for w in range(plan.waves):
+            self._exchange_wait(w, main)
+        out[plan.n_local:].copy_(self.halo[:plan.n_halo])
+        self._exchange_end(main)
         return out
 
     def exchange_only(self, X: torch.Tensor):
@@ -815,7 +889,7 @@ class PartitionedSpmm:
 
     # -- backward --------------------------------------------------------------------------
     def _backward_setup(self):
-        from .graph import CSRGraph, index_block_transpose
+        from .graph import CSRGraph
         plan = self.plan
         n_loc, n_halo = plan.n_local, max(plan.n_halo, 1)
         self._t_loc = self.A_loc.transpose()
@@ -825,6 +899,15 @@ class PartitionedSpmm:
         self._t_rem = A_rem.transpose()          # [n_halo, n_loc]: one partial row per halo slot
         self._t_rem._t = None
         del A_rem
+        if self._R is None:
+            self._return_setup()
+
+    def _return_setup(self):
+        """Buffers of the gradient return: the partial rows (one per halo slot), the receive buffer of the rows the
+        peers send back, and R, the pattern-only CSR that adds them to their local rows in (peer, slot) order."""
+        from .graph import CSRGraph, index_block_transpose
+        plan = self.plan
+        n_loc, n_halo = plan.n_local, max(plan.n_halo, 1)
         n_send = int(plan.send_rows.numel())
         # R: local row r <- the positions k of the send list with send_rows[k] == r, ascending k
         rowptr_t, pos_t = index_block_transpose(plan.send_rows, n_loc)
@@ -848,23 +931,48 @@ class PartitionedSpmm:
         """dX_local = (Âᵀ·dY)[own rows]: the autograd of GCN/GCN.py:43 on the partitioned graph.
         Remote partials first (they must travel), the local transposed product while they do, then the
         partials this rank's rows received are added in fixed (peer, slot) order."""
-        from .functional import spmm_ex, spmm_raw
-        plan, lib = self.plan, _lib.load()
+        from .functional import spmm_raw
+        plan = self.plan
         assert dY.shape == (plan.n_local, self.F) and dY.dtype == self.dtype and dY.is_cuda
         if self._t_loc is None:
             self._backward_setup()
-        main = torch.cuda.current_stream()
         if out is None:
             out = torch.empty((plan.n_local, self.F), dtype=self.dtype, device=self.dev)
         if plan.world == 1:
             return spmm_raw(self._t_loc, dY, out=out)
-        s, W = self._bstep, plan.world
         spmm_raw(self._t_rem, dY, out=self._partial)           # partial[h] = Σ_i Â[i, halo h] dY[i]
+        self._return_send(lambda: spmm_raw(self._t_loc, dY, out=out))  # local transposed product, under the copies
+        self._return_add(out)
+        return out
+
+    def return_halo_grad(self, dX_comb: torch.Tensor) -> torch.Tensor:
+        """Backward of `gather_halo`: dX_local = dX_comb[:n_local] + the gradients of this rank's rows that the peers
+        return (rows dX_comb[n_local:] travel to their owners), added in fixed (peer, slot) order."""
+        plan = self.plan
+        assert dX_comb.shape == (plan.n_local + plan.n_halo, self.F) and dX_comb.dtype == self.dtype
+        out = dX_comb[:plan.n_local].clone()
+        if plan.world == 1:
+            return out
+        if self._R is None:
+            self._return_setup()
+        self._partial[:plan.n_halo].copy_(dX_comb[plan.n_local:])
+        self._return_send()
+        self._return_add(out)
+        return out
+
+    def _return_send(self, local=None):
+        """Send the partial rows to their owners (copy engines + flags, or all_to_all); `local()` runs on the main
+        stream while they travel.  On return the rows this rank receives are in `self.back`, visible to the main
+        stream."""
+        plan, lib = self.plan, _lib.load()
+        main = torch.cuda.current_stream()
+        s, W = self._bstep, plan.world
         if self.transport == "nccl":
             dist.all_to_all_single(self.back[:int(plan.send_rows.numel())], self._partial[:plan.n_halo].contiguous(),
                                    output_split_sizes=plan.send_counts, input_split_sizes=plan.recv_counts,
                                    group=self.group)
-            spmm_raw(self._t_loc, dY, out=out)
+            if local is not None:
+                local()
         else:
             self._ev_partial.record(main)
             comm = self.comm
@@ -890,14 +998,19 @@ class PartitionedSpmm:
                     self._ev_bcopied[k].record(st)
                     comm.wait_event(self._ev_bcopied[k])
                 self._signal(2, s + 1, comm)
-            spmm_raw(self._t_loc, dY, out=out)                 # local transposed product, under the copies
+            if local is not None:
+                local()
             self._wait(2, s + 1, main)
+
+    def _return_add(self, out: torch.Tensor):
+        """out[r] += the received rows of local row r, in (peer, slot) order; frees the receive buffer for the
+        peers' next step."""
+        from .functional import spmm_ex
         if self._R.n_rows > 0:
             spmm_ex(self._R, self.back, out, row_map=self._R._row_map, accumulate=True)
         if self.transport != "nccl":
-            self._signal(3, s + 1, main)
+            self._signal(3, self._bstep + 1, torch.cuda.current_stream())
         self._bstep += 1
-        return out
 
     def close(self):
         if self._bufs:
@@ -921,6 +1034,9 @@ class PartitionedGraph:
     same sequence of forward and backward calls (same layers, same order) — a model's forward / backward on every
     rank, every step.  Ranks that own no training row still run both.
 
+    GAT layers take it as well (`GAT.forward(X_local, pg)`): `attention()` is the block in the combined column space
+    (AttentionView, built here: one more collective), and `widths` must then list every layer's H*F'.
+
     Constructors: `PartitionedGraph(rowptr, col, val, bounds, rank, world, widths, ...)` from the rank's own row
     block (rowptr over its rows, GLOBAL column ids — what `build_halo_plan` takes), or `from_global(g, ...)` for a
     graph every rank holds.  Keyword arguments other than the plan's go to every `PartitionedSpmm`."""
@@ -935,9 +1051,12 @@ class PartitionedGraph:
         if not widths or widths[0] <= 0:
             raise ValueError("PartitionedGraph: at least one positive feature width is needed")
         elem = 4 if dtype == torch.float32 else 2
-        self.plan = build_halo_plan(rowptr.to(self.dev), col.to(self.dev), None if val is None else val.to(self.dev),
+        rowptr, col = rowptr.to(self.dev), col.to(self.dev)
+        self.plan = build_halo_plan(rowptr, col, None if val is None else val.to(self.dev),
                                     self.bounds, self.rank, self.world, group=group, waves=waves,
                                     two_pass_chunks=two_pass_chunks, F=widths[-1], elem_size=elem)
+        self._att = build_attention_view(self.plan, rowptr, col, group)
+        self._att_graph = None
         self.ops: Dict[int, PartitionedSpmm] = {}
         try:
             for F in widths:
@@ -971,6 +1090,20 @@ class PartitionedGraph:
             raise _lib.GnnError(f"PartitionedGraph: no operator for feature width {F} (built for {sorted(self.ops)}); "
                                 "list every layer's output width in `widths`")
         return op
+
+    @property
+    def edge_slot_base(self) -> int:
+        return self._att.edge_slot_base
+
+    def attention(self):
+        """(CSRGraph of the block in the combined column space [n_local, n_local + n_halo], edge_slot_base) for the
+        fused attention kernels.  Raises on every rank when the graph has a row without edges."""
+        from .graph import CSRGraph
+        self._att.require_edges()
+        if self._att_graph is None:
+            a = self._att
+            self._att_graph = CSRGraph(a.rowptr, a.col, None, a.n_rows, a.n_cols)
+        return self._att_graph, self._att.edge_slot_base
 
     def local_index(self, idx_global: torch.Tensor) -> torch.Tensor:
         """The global node ids of `idx_global` (train / val / test ids) that this rank owns, as local row indices

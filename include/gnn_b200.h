@@ -300,7 +300,11 @@ int gnn_gat_scores_f32(const float* Wh, int64_t ldw, const float* a_src, const f
  * Schedule: one warp per row; the rows of long_rows[n_long] (those with more than
  * long_threshold edges: the caller's plan, CSRGraph.gat_long_rows) get one CTA each (4 warps on
  * alternate 128-edge chunks, merged in warp order); when nnz/n >= the "gat.coop_min_avg_deg"
- * knob (dense metapath adjacencies) every row gets a CTA and the list is ignored. */
+ * knob (dense metapath adjacencies) every row gets a CTA and the list is ignored.
+ * Rectangular use: Wh and t are read only through col, so col may address n_cols >= n table rows (Wh [n_cols, ldw],
+ * t [n_cols, H]; s, out and the row statistics stay [n, .]) — a row block of a partitioned graph whose columns index
+ * [own rows ; halo rows].  col_mean (rows without edges) and batch_nodes are not defined for that use: pass NULL / 0
+ * (gnn_gat_fused_bwd_ex_f32 is the matching backward). */
 int gnn_gat_fused_fwd_f32(const int64_t* rowptr, const int32_t* col, const float* Wh, int64_t ldw,
                           const float* s, const float* t, int64_t n, int64_t nnz /*schedule hint, 0 if unknown*/,
                           int32_t H, int32_t Fp,
@@ -322,12 +326,20 @@ int gnn_gat_fused_fwd_f32(const int64_t* rowptr, const int32_t* col, const float
  * (probability 1-p, kept weights scaled by 1/(1-p)) — identically in the forward and in both backward passes.
  * seed_dev (nullable) is a device int64 mixed into the seed at run time, so a captured CUDA graph draws a fresh
  * mask on every replay.  Semantically (not bit-) equal to F.dropout on the dense attention matrix; the explicit
- * `edge_keep` mask remains for parity tests.  struct_size = sizeof(gnn_gat_dropout). */
+ * `edge_keep` mask remains for parity tests.
+ * edge_slot_base: the keep factor of local edge slot e is the one of slot e + edge_slot_base.  A row block of a
+ * larger CSR (a contiguous edge range starting at global slot rowptr[lo]) passes rowptr[lo] and draws exactly the
+ * mask the whole graph draws for its edges.  It offsets the seeded stream only, not an explicit edge_keep mask, and
+ * needs seed_dev == NULL (GNN_ERR_UNSUPPORTED otherwise): the caller mixes the device half into seed itself.
+ * struct_size = sizeof(gnn_gat_dropout) (ABI versioning).  A struct_size of offsetof(gnn_gat_dropout,
+ * edge_slot_base) (the layout before that field was appended) is also accepted and reads as edge_slot_base = 0;
+ * any other size is refused. */
 typedef struct gnn_gat_dropout {
   int32_t struct_size;
   float p;
   uint64_t seed;
   const int64_t* seed_dev;
+  int64_t edge_slot_base;
 } gnn_gat_dropout;
 
 /* Training form of the forward: writes the PRE-activation aggregate to out_pre (saved for the backward) and, when
@@ -380,6 +392,25 @@ int gnn_gat_fused_bwd_f32(const int64_t* rowptr, const int32_t* col,
                           int apply_elu, float* d_pre /*nullable when apply_elu == 0*/,
                           const gnn_gat_dropout* dropout /*nullable*/, int64_t batch_nodes,
                           gnn_stream_t stream);
+/* Rectangular backward (fp32): the forward ran over n_rows CSR rows whose columns address n_cols >= n_rows table
+ * rows of Wh / t.  The row-record kernel and pass 1 (d_s [n_rows,H]) walk the n_rows forward rows; pass 2 walks the
+ * transposed [n_cols, n_rows] CSR (rowptr_t has n_cols + 1 entries) and writes d_Wh [n_cols, ld_dwh] and d_t
+ * [n_cols, H] for every table row (zero for a row no edge reads) — its grid, its long-row list (long_rows_t) and its
+ * cooperative-schedule choice follow n_cols.  row_scratch is [n_rows,4,H].  One graph only (no batch_nodes).
+ * gnn_gat_fused_bwd_f32 is this function with n_rows == n_cols == n. */
+int gnn_gat_fused_bwd_ex_f32(const int64_t* rowptr, const int32_t* col,
+                             const int64_t* rowptr_t, const int32_t* col_t, const int64_t* perm_t /*nullable*/,
+                             const float* Wh, int64_t ldw, const float* s, const float* t,
+                             const float* row_max, const float* row_sum,
+                             const float* out_pre, const float* d_out, int64_t ldo,
+                             int64_t n_rows, int64_t n_cols, int32_t H, int32_t Fp, float alpha, int mode,
+                             const float* edge_keep,
+                             float* d_Wh, int64_t ld_dwh, float* d_s, float* d_t, float* row_scratch,
+                             int64_t nnz,
+                             const int64_t* long_rows, int64_t n_long,
+                             const int64_t* long_rows_t, int64_t n_long_t, int64_t long_threshold,
+                             int apply_elu, float* d_pre, const gnn_gat_dropout* dropout /*nullable*/,
+                             gnn_stream_t stream);
 /* bf16-feature variants (north_star: "bf16-feature variants within 1e-2"): Wh, out, out_pre, d_out and
  * d_Wh are bf16; the scores s/t, the softmax statistics and every accumulation stay fp32.
  * Same reference call site (GAT/models/layers.py:22-37). */
