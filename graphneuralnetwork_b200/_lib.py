@@ -51,6 +51,10 @@ SIGNATURES = {
     "gnn_gather_reduce_multi_f32": (cint, [ptr, i64, i64, i32, cint, i32, ptr, cint, ptr, ptr, ptr, ptr, ptr]),
     "gnn_gather_reduce_multi_bf16": (cint, [ptr, i64, i64, i32, cint, i32, ptr, cint, ptr, ptr, ptr, ptr, ptr]),
     "gnn_gather_reduce_multi_f32_split": (cint, [ptr, i64, i64, i32, cint, i32, ptr, cint, ptr, ptr, ptr, ptr, ptr, ptr]),
+    "gnn_gather_reduce_multi_sharded_f32": (cint, [ptr, i64, i32, cint, i32, ptr, cint, ptr, ptr, ptr, ptr, ptr]),
+    "gnn_gather_reduce_multi_sharded_bf16": (cint, [ptr, i64, i32, cint, i32, ptr, cint, ptr, ptr, ptr, ptr, ptr]),
+    "gnn_gather_reduce_multi_sharded_f32_split": (cint, [ptr, i64, i32, cint, i32, ptr, cint, ptr, ptr, ptr, ptr, ptr,
+                                                         ptr]),
     "gnn_gather_reduce_typed_f32": (cint, [ptr, i64, i64, i32, ptr, cint, i64, i32, i32, cint, ptr, i64, ptr]),
     "gnn_gather_reduce_bwd_f32": (cint, [ptr, ptr, i64, i32, f32, ptr, i64, ptr, i64, i32, ptr]),
     "gnn_gather_reduce_bwd_dense_f32": (cint, [ptr, i64, ptr, i64, i32, i32, f32, ptr, ptr]),
@@ -104,6 +108,15 @@ class SpmmOpts(C.Structure):
 class GatDropout(C.Structure):
     """gnn_gat_dropout of include/gnn_b200.h."""
     _fields_ = [("struct_size", i32), ("p", f32), ("seed", u64), ("seed_dev", ptr), ("edge_slot_base", i64)]
+
+
+MAX_SHARDS = 8
+
+
+class ShardedTableDesc(C.Structure):
+    """gnn_sharded_table of include/gnn_b200.h."""
+    _fields_ = [("struct_size", i32), ("n_shards", i32), ("base", ptr * MAX_SHARDS),
+                ("row_begin", i64 * (MAX_SHARDS + 1))]
 
 
 class HaloOpts(C.Structure):

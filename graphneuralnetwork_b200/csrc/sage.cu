@@ -56,6 +56,25 @@ struct SageArgs {
   int64_t lo_off[kMaxBlocks];
 };
 
+// Sharded table (gnn_sharded_table): global row r of shard s = the largest s with row_begin[s] <= r lives at
+// base[s] + (r - row_begin[s]) * ld = origin[s] + r * ld, origin[s] the byte address base[s] - row_begin[s] * ld
+// (integer arithmetic: it may lie outside any allocation; only origin + r * ld is ever dereferenced).  Bounds fit
+// int32 (n_table_rows < 2^31).  `table` is unused; n_table_rows = row_begin[n_shards].
+template <typename T>
+struct SageShardedArgs : SageArgs<T> {
+  uint64_t origin[GNN_MAX_SHARDS];
+  int32_t row_begin[GNN_MAX_SHARDS];
+  int32_t n_shards;
+};
+template <typename T, bool SH>
+struct SageArgsOf {
+  using type = SageArgs<T>;
+};
+template <typename T>
+struct SageArgsOf<T, true> {
+  using type = SageShardedArgs<T>;
+};
+
 // Two fp32 adds in one instruction (SASS FADD2, sm_100): same round-to-nearest result as two
 // FADDs at half the issue slots.  The bf16 consumer loop was issue-bound (ncu r01: 195 warp
 // instructions per 1.2 KB row, 64 % issue-active with one scheduler idle).
@@ -119,8 +138,19 @@ __device__ __forceinline__ void cursor_next(Cursor& c, const SageArgs<T>& a) {
   if (c.c0 >= c.fan) cursor_set(c, a, c.g + gridDim.x);
 }
 
-template <typename T, int NV, int OP, bool PK = true>
-__global__ void __launch_bounds__(kSageThreads) sage_tma_kernel(const SageArgs<T> a) {
+// CTAs per SM the register allocation of the sharded kernel is held to (0: ptxas chooses, as for the unsharded
+// kernel).  4 x 192 threads caps it at 80 registers, what the unsharded twin uses or less; without the bound ptxas
+// spilled a few bytes in some sharded twins of spill-free kernels.  The bf16 max kernels with 3-4 vectors per thread
+// need 114-121 registers unsharded, so they keep ptxas's choice.
+template <typename T, int NV, int OP, bool SH>
+constexpr int sage_min_ctas() {
+  return (SH && !(sizeof(T) == 2 && OP == GNN_REDUCE_MAX && NV >= 3)) ? 4 : 0;
+}
+
+// SH: the table is sharded (SageShardedArgs); only the producer's source address depends on it.
+template <typename T, int NV, int OP, bool PK = true, bool SH = false>
+__global__ void __launch_bounds__(kSageThreads, (sage_min_ctas<T, NV, OP, SH>()))
+    sage_tma_kernel(const typename SageArgsOf<T, SH>::type a) {
   constexpr int E = Vec16<T>::E;
   extern __shared__ __align__(128) unsigned char smem[];
   const int S = a.stages;
@@ -181,9 +211,21 @@ __global__ void __launch_bounds__(kSageThreads) sage_tma_kernel(const SageArgs<T
           mbar_arrive_expect_tx(full + stage, (uint32_t)__popc(m) * (uint32_t)a.row_bytes);
         }
         __syncwarp();
-        if (valid)
-          bulk_g2s(smem + (size_t)stage * stage_bytes + (size_t)lane * a.row_bytes, a.table + r * a.ld,
-                   (uint32_t)a.row_bytes, full + stage);
+        if (valid) {
+          const T* src;
+          if constexpr (SH) {
+            // unrolled scan of the (uniform) shard bounds: no per-lane indexing into the parameter space
+            uint64_t origin = a.origin[0];
+#pragma unroll
+            for (int s = 1; s < GNN_MAX_SHARDS; ++s)
+              if (s < a.n_shards && (int32_t)r >= a.row_begin[s]) origin = a.origin[s];
+            src = reinterpret_cast<const T*>(origin + (uint64_t)(r * a.ld) * sizeof(T));
+          } else {
+            src = a.table + r * a.ld;
+          }
+          bulk_g2s(smem + (size_t)stage * stage_bytes + (size_t)lane * a.row_bytes, src, (uint32_t)a.row_bytes,
+                   full + stage);
+        }
         cursor_next(cur, a);
         if (++stage == S) {
           stage = 0;
@@ -329,41 +371,41 @@ __global__ void __launch_bounds__(kSageThreads) sage_tma_kernel(const SageArgs<T
   }
 }
 
-template <typename T, int NV, int OP, bool PK>
-int launch_tma_pk(const SageArgs<T>& a, size_t smem_bytes, int grid, cudaStream_t st) {
+template <typename T, int NV, int OP, bool PK, bool SH>
+int launch_tma_pk(const typename SageArgsOf<T, SH>::type& a, size_t smem_bytes, int grid, cudaStream_t st) {
   // function attributes belong to a device's context: remember the largest size set PER DEVICE (a process driving
   // several GPUs must not skip the call on the second one); benign race: setting the attribute is idempotent
   static size_t configured[64] = {};
   int dev = 0;
   const bool cached = cudaGetDevice(&dev) == cudaSuccess && dev >= 0 && dev < 64;
   if (!cached || smem_bytes > configured[dev]) {
-    GNN_CUDA(cudaFuncSetAttribute(sage_tma_kernel<T, NV, OP, PK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    GNN_CUDA(cudaFuncSetAttribute(sage_tma_kernel<T, NV, OP, PK, SH>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   (int)smem_bytes));
     if (cached) configured[dev] = smem_bytes;
   }
-  sage_tma_kernel<T, NV, OP, PK><<<grid, kSageThreads, smem_bytes, st>>>(a);
+  sage_tma_kernel<T, NV, OP, PK, SH><<<grid, kSageThreads, smem_bytes, st>>>(a);
   GNN_LAUNCH_CHECK();
   return GNN_OK;
 }
 
-template <typename T, int NV, int OP>
-int launch_tma_inst(const SageArgs<T>& a, size_t smem_bytes, int grid, cudaStream_t st) {
+template <typename T, int NV, int OP, bool SH>
+int launch_tma_inst(const typename SageArgsOf<T, SH>::type& a, size_t smem_bytes, int grid, cudaStream_t st) {
   // packed adds pay where the consumers are issue-bound (bf16: 8 unpack + 8 add per 16 bytes);
   // "sage.packed_add": -1 = by dtype, 0 / 1 = force
   const int knob = tuning("sage.packed_add", -1);
   const bool pk = (OP != GNN_REDUCE_MAX) && (knob < 0 ? sizeof(T) == 2 : knob != 0);
-  if (pk) return launch_tma_pk<T, NV, OP, true>(a, smem_bytes, grid, st);
-  return launch_tma_pk<T, NV, OP, false>(a, smem_bytes, grid, st);
+  if (pk) return launch_tma_pk<T, NV, OP, true, SH>(a, smem_bytes, grid, st);
+  return launch_tma_pk<T, NV, OP, false, SH>(a, smem_bytes, grid, st);
 }
 
-template <typename T, int OP>
-int launch_tma(const SageArgs<T>& a, size_t smem_bytes, int grid, cudaStream_t st) {
+template <typename T, int OP, bool SH>
+int launch_tma(const typename SageArgsOf<T, SH>::type& a, size_t smem_bytes, int grid, cudaStream_t st) {
   const int nv = (a.nvec + kConsumerThreads - 1) / kConsumerThreads;
   switch (nv) {
-    case 1: return launch_tma_inst<T, 1, OP>(a, smem_bytes, grid, st);
-    case 2: return launch_tma_inst<T, 2, OP>(a, smem_bytes, grid, st);
-    case 3: return launch_tma_inst<T, 3, OP>(a, smem_bytes, grid, st);
-    case 4: return launch_tma_inst<T, 4, OP>(a, smem_bytes, grid, st);
+    case 1: return launch_tma_inst<T, 1, OP, SH>(a, smem_bytes, grid, st);
+    case 2: return launch_tma_inst<T, 2, OP, SH>(a, smem_bytes, grid, st);
+    case 3: return launch_tma_inst<T, 3, OP, SH>(a, smem_bytes, grid, st);
+    case 4: return launch_tma_inst<T, 4, OP, SH>(a, smem_bytes, grid, st);
     default: break;
   }
   set_error("TMA gather: row too wide (nvec=%d)", a.nvec);
@@ -383,9 +425,38 @@ struct GatherBlock {
   int64_t lo_off = 0;
 };
 
+// Every field of a gnn_sharded_table, before anything is launched.
+int check_sharded_table(const gnn_sharded_table* sh, int64_t ld, int32_t F, int esz) {
+  GNN_REQUIRE(sh, GNN_ERR_BAD_ARG, "null sharded table");
+  GNN_REQUIRE(sh->struct_size == (int32_t)sizeof(gnn_sharded_table), GNN_ERR_BAD_ARG,
+              "gnn_sharded_table.struct_size %d, expected %d", sh->struct_size, (int)sizeof(gnn_sharded_table));
+  GNN_REQUIRE(sh->n_shards >= 1 && sh->n_shards <= GNN_MAX_SHARDS, GNN_ERR_BAD_ARG, "n_shards %d outside [1, %d]",
+              sh->n_shards, GNN_MAX_SHARDS);
+  GNN_REQUIRE(sh->row_begin[0] == 0, GNN_ERR_BAD_ARG, "row_begin[0] must be 0");
+  for (int s = 0; s < sh->n_shards; ++s) {
+    GNN_REQUIRE(sh->row_begin[s + 1] >= sh->row_begin[s], GNN_ERR_BAD_ARG, "row_begin decreases at shard %d", s);
+    if (sh->row_begin[s + 1] > sh->row_begin[s])
+      GNN_REQUIRE(sh->base[s] && aligned_to(sh->base[s], 16), GNN_ERR_MISALIGNED,
+                  "shard %d: base must be non-null and 16-byte aligned", s);
+  }
+  GNN_REQUIRE(ld >= F && F >= 0, GNN_ERR_BAD_ARG, "leading dimension smaller than F");
+  GNN_REQUIRE(ld * esz % 16 == 0, GNN_ERR_MISALIGNED, "sharded table: ld_table * elem must be a multiple of 16");
+  return GNN_OK;
+}
+
 template <typename T>
 int gather_reduce_impl(const T* table, int64_t ld, int64_t n_table_rows, int32_t F, int reduce,
-                       const GatherBlock<T>* blocks, int n_blocks, cudaStream_t st) {
+                       const GatherBlock<T>* blocks, int n_blocks, cudaStream_t st,
+                       const gnn_sharded_table* sh = nullptr) {
+  if (sh) {
+    const int rc = check_sharded_table(sh, ld, F, (int)sizeof(T));
+    if (rc != GNN_OK) return rc;
+    const size_t rb = round_up((size_t)F * sizeof(T), 16);
+    GNN_REQUIRE(F == 0 || (rb >= 256 && rb / 16 <= 4 * (size_t)kConsumerThreads), GNN_ERR_UNSUPPORTED,
+                "sharded table: TMA path only, rows of 256 to %d bytes (F=%d gives %d)", 64 * kConsumerThreads, F,
+                (int)rb);
+    n_table_rows = sh->row_begin[sh->n_shards];
+  }
   GNN_REQUIRE(F >= 0 && n_blocks >= 0 && n_blocks <= kMaxBlocks, GNN_ERR_BAD_ARG, "bad size (F=%d, blocks=%d, max %d)",
               F, n_blocks, kMaxBlocks);
   GNN_REQUIRE(reduce == GNN_REDUCE_MEAN || reduce == GNN_REDUCE_SUM || reduce == GNN_REDUCE_MAX, GNN_ERR_BAD_ARG,
@@ -397,7 +468,7 @@ int gather_reduce_impl(const T* table, int64_t ld, int64_t n_table_rows, int32_t
     GNN_REQUIRE(k.n_src >= 0 && k.fanout >= 0, GNN_ERR_BAD_ARG, "negative size");
     if (k.n_src == 0 || F == 0) continue;
     GNN_REQUIRE(k.fanout > 0, GNN_ERR_BAD_ARG, "fanout must be positive");
-    GNN_REQUIRE(table && k.out, GNN_ERR_BAD_ARG, "null table/out");
+    GNN_REQUIRE((table || sh) && k.out, GNN_ERR_BAD_ARG, "null table/out");
     GNN_REQUIRE(k.idx == nullptr || k.idx_bits == 32 || k.idx_bits == 64, GNN_ERR_BAD_ARG, "idx_bits must be 32 or 64");
     GNN_REQUIRE(ld >= F && k.ldo >= F, GNN_ERR_BAD_ARG, "leading dimension smaller than F");
     GNN_REQUIRE(!k.split || (sizeof(T) == 4 && reduce != GNN_REDUCE_MAX && k.lo_off >= F && k.ldo % 4 == 0 &&
@@ -411,10 +482,18 @@ int gather_reduce_impl(const T* table, int64_t ld, int64_t n_table_rows, int32_t
 
   const int esz = (int)sizeof(T);
   const int row_bytes = (int)round_up((size_t)F * esz, 16);
-  const bool tma_ok = !tuning("sage.force_ldg", 0) && aligned_to(table, 16) && ((ld * esz) % 16 == 0) &&
-                      (int64_t)row_bytes <= ld * esz && row_bytes >= 256 && (row_bytes / 16) <= 4 * kConsumerThreads;
+  // a sharded table has no vector-load form: its rows were checked for the TMA path above
+  const bool tma_ok = sh || (!tuning("sage.force_ldg", 0) && aligned_to(table, 16) && ((ld * esz) % 16 == 0) &&
+                             (int64_t)row_bytes <= ld * esz && row_bytes >= 256 && (row_bytes / 16) <= 4 * kConsumerThreads);
   if (tma_ok) {
-    SageArgs<T> a{};
+    SageShardedArgs<T> a{};
+    if (sh) {
+      for (int s = 0; s < sh->n_shards; ++s) {
+        a.origin[s] = (uint64_t)(uintptr_t)sh->base[s] - (uint64_t)(sh->row_begin[s] * ld) * sizeof(T);
+        a.row_begin[s] = (int32_t)sh->row_begin[s];
+      }
+      a.n_shards = sh->n_shards;
+    }
     a.table = table;
     a.ld = ld;
     a.F = F;
@@ -459,9 +538,14 @@ int gather_reduce_impl(const T* table, int64_t ld, int64_t n_table_rows, int32_t
     const size_t smem_bytes = (size_t)stages * stage_rows * row_bytes + (size_t)stages * (16 + 4) + 16;
     int64_t grid = (int64_t)num_sms() * tuning("sage.ctas_per_sm", 4);
     grid = grid > total_src ? total_src : grid;
+    const SageArgs<T>& flat = a;  // the unsharded kernels take the base part only
     switch (reduce) {
-      case GNN_REDUCE_MAX: return launch_tma<T, GNN_REDUCE_MAX>(a, smem_bytes, (int)grid, st);
-      default: return launch_tma<T, GNN_REDUCE_SUM>(a, smem_bytes, (int)grid, st);
+      case GNN_REDUCE_MAX:
+        return sh ? launch_tma<T, GNN_REDUCE_MAX, true>(a, smem_bytes, (int)grid, st)
+                  : launch_tma<T, GNN_REDUCE_MAX, false>(flat, smem_bytes, (int)grid, st);
+      default:
+        return sh ? launch_tma<T, GNN_REDUCE_SUM, true>(a, smem_bytes, (int)grid, st)
+                  : launch_tma<T, GNN_REDUCE_SUM, false>(flat, smem_bytes, (int)grid, st);
     }
   }
 
@@ -497,13 +581,31 @@ int gather_reduce_impl(const T* table, int64_t ld, int64_t n_table_rows, int32_t
 template <typename T>
 int gather_reduce_multi(const T* table, int64_t ld, int64_t n_table_rows, int32_t F, int reduce, int32_t n_blocks,
                         const void* const* idx, int idx_bits, const int64_t* n_src, const int32_t* fanout,
-                        void* const* out, const int64_t* ld_out, cudaStream_t st) {
+                        void* const* out, const int64_t* ld_out, cudaStream_t st,
+                        const gnn_sharded_table* sh = nullptr) {
   GNN_REQUIRE(n_blocks >= 0 && n_blocks <= kMaxBlocks, GNN_ERR_UNSUPPORTED, "at most %d blocks per launch", kMaxBlocks);
   GNN_REQUIRE(n_blocks == 0 || (idx && n_src && fanout && out && ld_out), GNN_ERR_BAD_ARG, "null block array");
   GatherBlock<T> blocks[kMaxBlocks];
   for (int b = 0; b < n_blocks; ++b)
     blocks[b] = GatherBlock<T>{idx[b], idx_bits, n_src[b], fanout[b], (T*)out[b], ld_out[b], nullptr};
-  return gather_reduce_impl<T>(table, ld, n_table_rows, F, reduce, blocks, n_blocks, st);
+  return gather_reduce_impl<T>(table, ld, n_table_rows, F, reduce, blocks, n_blocks, st, sh);
+}
+
+int gather_reduce_multi_split(const float* table, int64_t ld_table, int64_t n_table_rows, int32_t F, int reduce,
+                              int32_t n_blocks, const void* const* idx_host, int idx_bits, const int64_t* n_src_host,
+                              const int32_t* fanout_host, void* const* out_hi_host, const int64_t* ld_out_host,
+                              const int64_t* lo_off_host, cudaStream_t st, const gnn_sharded_table* sh = nullptr) {
+  GNN_REQUIRE(n_blocks >= 0 && n_blocks <= kMaxBlocks, GNN_ERR_UNSUPPORTED, "at most %d blocks per launch", kMaxBlocks);
+  GNN_REQUIRE(n_blocks == 0 || (idx_host && n_src_host && fanout_host && out_hi_host && ld_out_host && lo_off_host),
+              GNN_ERR_BAD_ARG, "null block array");
+  GatherBlock<float> blocks[kMaxBlocks];
+  for (int b = 0; b < n_blocks; ++b) {
+    blocks[b] = GatherBlock<float>{idx_host[b], idx_bits, n_src_host[b], fanout_host[b], (float*)out_hi_host[b],
+                                   ld_out_host[b], nullptr};
+    blocks[b].split = 1;
+    blocks[b].lo_off = lo_off_host[b];
+  }
+  return gather_reduce_impl<float>(table, ld_table, n_table_rows, F, reduce, blocks, n_blocks, st, sh);
 }
 
 __global__ void __launch_bounds__(256) bwd_dense_kernel(const float* __restrict__ d_out, int64_t ld,
@@ -554,17 +656,36 @@ int gnn_gather_reduce_multi_f32_split(const float* table, int64_t ld_table, int6
                                       int32_t n_blocks, const void* const* idx_host, int idx_bits,
                                       const int64_t* n_src_host, const int32_t* fanout_host, void* const* out_hi_host,
                                       const int64_t* ld_out_host, const int64_t* lo_off_host, gnn_stream_t stream) {
-  GNN_REQUIRE(n_blocks >= 0 && n_blocks <= kMaxBlocks, GNN_ERR_UNSUPPORTED, "at most %d blocks per launch", kMaxBlocks);
-  GNN_REQUIRE(n_blocks == 0 || (idx_host && n_src_host && fanout_host && out_hi_host && ld_out_host && lo_off_host),
-              GNN_ERR_BAD_ARG, "null block array");
-  GatherBlock<float> blocks[kMaxBlocks];
-  for (int b = 0; b < n_blocks; ++b) {
-    blocks[b] = GatherBlock<float>{idx_host[b], idx_bits, n_src_host[b], fanout_host[b], (float*)out_hi_host[b],
-                                   ld_out_host[b], nullptr};
-    blocks[b].split = 1;
-    blocks[b].lo_off = lo_off_host[b];
-  }
-  return gather_reduce_impl<float>(table, ld_table, n_table_rows, F, reduce, blocks, n_blocks, (cudaStream_t)stream);
+  return gather_reduce_multi_split(table, ld_table, n_table_rows, F, reduce, n_blocks, idx_host, idx_bits, n_src_host,
+                                   fanout_host, out_hi_host, ld_out_host, lo_off_host, (cudaStream_t)stream);
+}
+
+int gnn_gather_reduce_multi_sharded_f32(const gnn_sharded_table* table, int64_t ld_table, int32_t F, int reduce,
+                                        int32_t n_blocks, const void* const* idx_host, int idx_bits,
+                                        const int64_t* n_src_host, const int32_t* fanout_host, void* const* out_host,
+                                        const int64_t* ld_out_host, gnn_stream_t stream) {
+  GNN_REQUIRE(table, GNN_ERR_BAD_ARG, "null sharded table");
+  return gather_reduce_multi<float>(nullptr, ld_table, 0, F, reduce, n_blocks, idx_host, idx_bits, n_src_host,
+                                    fanout_host, out_host, ld_out_host, (cudaStream_t)stream, table);
+}
+
+int gnn_gather_reduce_multi_sharded_bf16(const gnn_sharded_table* table, int64_t ld_table, int32_t F, int reduce,
+                                         int32_t n_blocks, const void* const* idx_host, int idx_bits,
+                                         const int64_t* n_src_host, const int32_t* fanout_host, void* const* out_host,
+                                         const int64_t* ld_out_host, gnn_stream_t stream) {
+  GNN_REQUIRE(table, GNN_ERR_BAD_ARG, "null sharded table");
+  return gather_reduce_multi<__nv_bfloat16>(nullptr, ld_table, 0, F, reduce, n_blocks, idx_host, idx_bits, n_src_host,
+                                            fanout_host, out_host, ld_out_host, (cudaStream_t)stream, table);
+}
+
+int gnn_gather_reduce_multi_sharded_f32_split(const gnn_sharded_table* table, int64_t ld_table, int32_t F, int reduce,
+                                              int32_t n_blocks, const void* const* idx_host, int idx_bits,
+                                              const int64_t* n_src_host, const int32_t* fanout_host,
+                                              void* const* out_hi_host, const int64_t* ld_out_host,
+                                              const int64_t* lo_off_host, gnn_stream_t stream) {
+  GNN_REQUIRE(table, GNN_ERR_BAD_ARG, "null sharded table");
+  return gather_reduce_multi_split(nullptr, ld_table, 0, F, reduce, n_blocks, idx_host, idx_bits, n_src_host,
+                                   fanout_host, out_hi_host, ld_out_host, lo_off_host, (cudaStream_t)stream, table);
 }
 
 int gnn_gather_reduce_multi_bf16(const void* table, int64_t ld_table, int64_t n_table_rows, int32_t F, int reduce,

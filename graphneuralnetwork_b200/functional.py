@@ -12,6 +12,7 @@ import torch
 
 from . import _lib
 from .graph import CSRGraph, _p, _require_cuda, _stream_ptr, index_block_transpose
+from .partition import ShardedTable
 
 
 def _rowmajor(x: torch.Tensor) -> torch.Tensor:
@@ -341,17 +342,38 @@ def gather_reduce_raw(table: torch.Tensor, idx: Optional[torch.Tensor], n_src: i
     return out
 
 
-def gather_reduce_multi_raw(table: torch.Tensor, blocks, reduce: str = "mean", outs=None):
+def _table_head(table, plain, sharded):
+    """(C entry point, leading arguments) for a tensor table [N, F] or a ShardedTable: `plain` / `sharded` map the
+    dtype to the entry point of that form.  A sharded call takes (descriptor, ld, F), a plain one (ptr, ld, N, F)."""
+    import ctypes as C
+    if isinstance(table, ShardedTable):
+        fn = sharded.get(table.dtype)
+        head = (C.byref(table.desc), table.ld, table.F)
+    else:
+        _require_cuda(table)
+        table = _rowmajor(table)
+        fn = plain.get(table.dtype)
+        head = (_p(table), _ld(table), table.shape[0], table.shape[1])
+    if fn is None:
+        raise _lib.GnnError(f"gather_reduce: unsupported dtype {table.dtype}")
+    return fn, head
+
+
+def gather_reduce_multi_raw(table, blocks, reduce: str = "mean", outs=None):
     """Several fixed-fanout id blocks over the SAME table in ONE launch
     (gnn_gather_reduce_multi_*): `blocks` = [(idx, n_src, fanout), ...] (idx=None: identity).
-    The hops of a GraphSAGE minibatch (GraphSage.py:24-27) are such a set.  No autograd."""
+    The hops of a GraphSAGE minibatch (GraphSage.py:24-27) are such a set.  No autograd.
+    `table`: a tensor, or a partition.ShardedTable (gnn_gather_reduce_multi_sharded_*, the same result bit for bit)."""
     import ctypes as C
     if reduce not in _lib.REDUCE:
         raise ValueError("Unknown aggr type, expected sum, max, or mean, but got {}".format(reduce))
-    _require_cuda(table, *[b[0] for b in blocks])
+    _require_cuda(*[b[0] for b in blocks])
     lib = _lib.load()
-    table = _rowmajor(table)
-    N, F = table.shape
+    fn, head = _table_head(table, {torch.float32: lib.gnn_gather_reduce_multi_f32,
+                                   torch.bfloat16: lib.gnn_gather_reduce_multi_bf16},
+                           {torch.float32: lib.gnn_gather_reduce_multi_sharded_f32,
+                            torch.bfloat16: lib.gnn_gather_reduce_multi_sharded_bf16})
+    F = table.shape[1]
     nb = len(blocks)
     idxs, bits = [], None
     for idx, n_src, fanout in blocks:
@@ -368,30 +390,28 @@ def gather_reduce_multi_raw(table: torch.Tensor, blocks, reduce: str = "mean", o
         idxs.append(idx)
     if outs is None:
         outs = [_padded_empty(n_src, F, table.dtype, table.device) for _, n_src, _ in blocks]
-    fn = {torch.float32: lib.gnn_gather_reduce_multi_f32, torch.bfloat16: lib.gnn_gather_reduce_multi_bf16}.get(table.dtype)
-    if fn is None:
-        raise _lib.GnnError(f"gather_reduce: unsupported dtype {table.dtype}")
     idx_arr = (C.c_void_p * nb)(*[_p(i) for i in idxs])
     nsrc_arr = (C.c_int64 * nb)(*[int(b[1]) for b in blocks])
     fan_arr = (C.c_int32 * nb)(*[int(b[2]) for b in blocks])
     out_arr = (C.c_void_p * nb)(*[_p(o) for o in outs])
     ldo_arr = (C.c_int64 * nb)(*[_ld(o) for o in outs])
-    _lib.check(fn(_p(table), _ld(table), N, F, _lib.REDUCE[reduce], nb, idx_arr, bits or 64, nsrc_arr, fan_arr, out_arr,
-                  ldo_arr, _stream_ptr()), "gnn_gather_reduce_multi")
+    _lib.check(fn(*head, _lib.REDUCE[reduce], nb, idx_arr, bits or 64, nsrc_arr, fan_arr, out_arr, ldo_arr,
+                  _stream_ptr()), "gnn_gather_reduce_multi")
     return outs
 
 
-def gather_reduce_multi_split_raw(table: torch.Tensor, blocks, reduce: str, outs_hi, lo_off: int):
+def gather_reduce_multi_split_raw(table, blocks, reduce: str, outs_hi, lo_off: int):
     """gnn_gather_reduce_multi_f32_split: like gather_reduce_multi_raw on an fp32 table, but every reduced value x
     is written as hi = fp16(x) into `outs_hi[b]` (fp16 [n_src, F] views) and lo = fp16(x - hi) `lo_off` fp16
-    elements further along the row.  Raises GnnError(unsupported) off the TMA path."""
+    elements further along the row.  Raises GnnError(unsupported) off the TMA path.  `table`: a tensor or a
+    partition.ShardedTable."""
     import ctypes as C
-    _require_cuda(table, *[b[0] for b in blocks])
+    _require_cuda(*[b[0] for b in blocks])
     lib = _lib.load()
-    table = _rowmajor(table)
     if table.dtype != torch.float32:
         raise _lib.GnnError("gather_reduce_multi_split: fp32 table only")
-    N, F = table.shape
+    fn, head = _table_head(table, {torch.float32: lib.gnn_gather_reduce_multi_f32_split},
+                           {torch.float32: lib.gnn_gather_reduce_multi_sharded_f32_split})
     nb = len(blocks)
     idxs, bits = [], None
     for idx, n_src, fanout in blocks:
@@ -414,9 +434,8 @@ def gather_reduce_multi_split_raw(table: torch.Tensor, blocks, reduce: str, outs
     out_arr = (C.c_void_p * nb)(*[_p(o) for o in outs_hi])
     ldo_arr = (C.c_int64 * nb)(*[_ld(o) for o in outs_hi])
     lo_arr = (C.c_int64 * nb)(*[int(lo_off)] * nb)
-    _lib.check(lib.gnn_gather_reduce_multi_f32_split(_p(table), _ld(table), N, F, _lib.REDUCE[reduce], nb, idx_arr,
-                                                     bits or 64, nsrc_arr, fan_arr, out_arr, ldo_arr, lo_arr,
-                                                     _stream_ptr()), "gnn_gather_reduce_multi_f32_split")
+    _lib.check(fn(*head, _lib.REDUCE[reduce], nb, idx_arr, bits or 64, nsrc_arr, fan_arr, out_arr, ldo_arr, lo_arr,
+                  _stream_ptr()), "gnn_gather_reduce_multi_f32_split")
 
 
 def sample_neighbors(g: CSRGraph, src: torch.Tensor, k: int, seed: int, out_dtype=torch.int32,

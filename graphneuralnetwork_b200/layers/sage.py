@@ -16,7 +16,9 @@ from torch import nn
 import torch.nn.functional as F
 
 from .. import _lib
-from ..functional import gather_reduce, gather_reduce_multi_raw, gather_reduce_multi_split_raw, pad_table
+from ..functional import (_padded_empty, gather_reduce, gather_reduce_multi_raw, gather_reduce_multi_split_raw,
+                          pad_table)
+from ..partition import ShardedTable
 
 
 class SampledBlock:
@@ -139,7 +141,10 @@ class GraphSage(nn.Module):
         `node_id_blocks` = the id lists `multihop_sampling` returns (lengths B, B·f1, B·f1·f2, …)
         as int32/int64 device tensors.  Same arithmetic as `forward` on
         `[table[ids] for ids in node_id_blocks]`, without materialising the gathers of the
-        outermost hop: layer 0 reads neighbours straight from the table."""
+        outermost hop: layer 0 reads neighbours straight from the table.
+        `table` may be a `partition.ShardedTable` (rows spread over the GPUs of a node): the
+        logits and every weight gradient are then bit-identical to those over the concatenated
+        tensor table (but for the sign of zero noted in `_layer0_sharded`)."""
         L, fan, layer0 = self.num_layers, self.num_neighbors_list, self.gcn[0]
         assert len(node_id_blocks) == L + 1
         fused = (not (torch.is_grad_enabled() and table.requires_grad)) and L <= 4 \
@@ -148,6 +153,8 @@ class GraphSage(nn.Module):
         if fused and no_grad and 2 * L <= 4 and layer0.aggr_hidden_method == "sum" and not layer0.aggregator.use_bias \
                 and table.dtype == torch.float32:
             return self._upper_layers(self._layer0_one_launch_one_gemm(table, node_id_blocks))
+        if isinstance(table, ShardedTable):
+            return self._upper_layers(self._layer0_sharded(table, node_id_blocks))
         if fused:
             # every hop of layer 0 aggregates from the same table: ONE launch for all of them
             pooled = gather_reduce_multi_raw(table, [(node_id_blocks[hop + 1], node_id_blocks[hop].numel(), fan[hop])
@@ -156,6 +163,23 @@ class GraphSage(nn.Module):
             pooled = [SampledBlock(table, node_id_blocks[hop + 1], fan[hop]) for hop in range(L)]
         hidden = [layer0(table.index_select(0, node_id_blocks[hop].to(torch.int64)), pooled[hop]) for hop in range(L)]
         return self._upper_layers(hidden)
+
+    def _layer0_sharded(self, table, node_id_blocks):
+        """Layer 0 over a ShardedTable outside the one-launch inference form (training, L > 2, ...): the neighbour
+        reduce of every hop and, as fanout-1 blocks, the hop's own rows (what `table.index_select` gives a tensor
+        table: an exact copy, but -0.0 becomes +0.0 under mean/sum) come from the shards, four blocks per launch.
+        The own rows land in a contiguous [n, F] buffer and the reduces in padded ones, the shapes and strides the
+        tensor path hands the products, so both paths run the same GEMMs."""
+        L, fan, layer0 = self.num_layers, self.num_neighbors_list, self.gcn[0]
+        F = table.shape[1]
+        n_hop = [node_id_blocks[hop].numel() for hop in range(L)]
+        blocks = [(node_id_blocks[hop + 1], n_hop[hop], fan[hop]) for hop in range(L)] + \
+                 [(node_id_blocks[hop], n_hop[hop], 1) for hop in range(L)]
+        outs = [_padded_empty(n, F, table.dtype, table.device) for n in n_hop] + \
+               [torch.empty((n, F), dtype=table.dtype, device=table.device) for n in n_hop]
+        for i in range(0, len(blocks), 4):
+            gather_reduce_multi_raw(table, blocks[i:i + 4], layer0.aggr_neighbor_method, outs=outs[i:i + 4])
+        return [layer0(outs[L + hop], outs[hop]) for hop in range(L)]
 
     def _layer0_one_launch_one_gemm(self, table, node_id_blocks):
         """Inference form of layer 0 for all hops at once (SageGCN.py:23-27 on every hop of GraphSage.py:24-27):
@@ -206,6 +230,8 @@ class GraphSage(nn.Module):
 
     def _table_fits_fp16(self, table):
         """max|table| < 3e4 (an aggregate of rows never exceeds it): cached per table tensor (one host read)."""
+        if isinstance(table, ShardedTable):  # read-only, its max computed once at construction
+            return table.abs_max < 3.0e4
         key = (table.data_ptr(), table._version, tuple(table.shape))
         hit = getattr(self, "_fp16_ok", None)
         if hit is None or hit[0] != key:

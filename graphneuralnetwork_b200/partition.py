@@ -1119,6 +1119,193 @@ class PartitionedGraph:
         self.ops = {}
 
 
+# ---- a feature table sharded across ranks ---------------------------------------------------
+_TABLE_DTYPES = {torch.float32: 4, torch.bfloat16: 2}
+
+
+def shard_bounds(n_rows: int, world: int) -> List[int]:
+    """Row-balanced contiguous blocks: shard p holds the rows [n*p // world, n*(p+1) // world) (empty shards when
+    n_rows < world)."""
+    n_rows, world = int(n_rows), int(world)
+    if n_rows < 0 or world < 1:
+        raise ValueError(f"shard_bounds: bad size (rows={n_rows}, world={world})")
+    return [n_rows * p // world for p in range(world + 1)]
+
+
+def locate_rows(ids: torch.Tensor, bounds: List[int]):
+    """(shard, row within the shard) of every global id, by the sharded gather's rule: the last shard s with
+    bounds[s] <= id.  Ids outside [0, bounds[-1]) get shard -1 (the gather skips them)."""
+    ids = ids.to(torch.int64)
+    b = torch.tensor(bounds, dtype=torch.int64, device=ids.device)
+    s = torch.searchsorted(b, ids, right=True) - 1
+    valid = (ids >= 0) & (ids < b[-1])
+    s = torch.where(valid, s.clamp(0, len(bounds) - 2), torch.full_like(s, -1))
+    local = torch.where(valid, ids - b[s.clamp(min=0)], torch.full_like(ids, -1))
+    return s, local
+
+
+def agree_layout(F: int, ld: int, dtype, bounds, error: Optional[str], rank: int, world: int, group=None):
+    """The first step of building a ShardedTable (a collective): every rank states its block's width, padded row
+    stride, dtype and the row bounds of all shards, plus any local refusal, and every rank raises the same GnnError
+    if a rank refused or the ranks disagree — no rank is left waiting in a later collective, and no rank addresses
+    a peer's shard by bounds the peer does not hold."""
+    mine = (int(F), int(ld), str(dtype), tuple(int(b) for b in bounds), error)
+    every = [None] * world
+    dist.all_gather_object(every, mine, group=group)
+    problems = [f"rank {q}: {v[-1]}" for q, v in enumerate(every) if v[-1]]
+    if len({v[:3] for v in every}) > 1:
+        problems.append("ranks disagree on (F, ld, dtype): " +
+                        ", ".join(f"rank {q} {tuple(v[:3])}" for q, v in enumerate(every)))
+    if len({v[3] for v in every}) > 1:
+        problems.append("ranks disagree on the bounds: " +
+                        ", ".join(f"rank {q} {list(v[3])}" for q, v in enumerate(every)))
+    if problems:
+        raise _lib.GnnError("ShardedTable: " + "; ".join(problems))
+
+
+def _table_refusal(X: torch.Tensor) -> Optional[str]:
+    if not torch.is_tensor(X) or X.dim() != 2:
+        return "a 2-D feature tensor is needed"
+    if not X.is_cuda:
+        return "the table is on the CPU (the sharded gather reads device memory)"
+    if X.dtype not in _TABLE_DTYPES:
+        return f"dtype {X.dtype} (float32 or bfloat16)"
+    if X.requires_grad:
+        return "the table requires grad (features are inputs: there is no backward into a sharded table)"
+    return None
+
+
+class ShardedTable:
+    """A read-only feature table split into contiguous row blocks (shards), one per rank: the table argument of
+    `functional.gather_reduce_multi_raw` / `gather_reduce_multi_split_raw` and of `GraphSage.forward_sampled`, in
+    place of a tensor too large for one GPU.  Shard s holds the global rows [bounds[s], bounds[s+1]); the gather
+    reads each sampled row from its owner's memory (a peer's through a CUDA IPC mapping, over NVLink), and every
+    reduced row is bit-identical to the same gather over the concatenated table.
+
+    `ShardedTable(X_block, bounds, rank, world)` (a collective: every rank of `group` calls it) copies this rank's
+    rows into a peer-mapped buffer of 16-byte aligned rows and maps every peer's; `from_global` cuts the block out of
+    a table every rank holds; `local([t0, t1, ...])` builds the same object from tensors of one process on one
+    device, without IPC.  Like a tensor it has `shape` (global rows, F), `dtype`, `device`, `stride()` and
+    `requires_grad` (always False); `abs_max` is max |x| over the whole table."""
+
+    def __init__(self, X_block: torch.Tensor, bounds, rank: int, world: int, group=None):
+        self.bounds, self.rank, self.world, self.group = [int(b) for b in bounds], int(rank), int(world), group
+        if self.world > _lib.MAX_SHARDS:
+            raise _lib.GnnError(f"ShardedTable: {self.world} shards, at most {_lib.MAX_SHARDS}")
+        err = _table_refusal(X_block)
+        if err is None and (len(self.bounds) != self.world + 1 or
+                            X_block.shape[0] != self.bounds[self.rank + 1] - self.bounds[self.rank]):
+            err = f"block of {X_block.shape[0]} rows does not match bounds {self.bounds}"
+        F = int(X_block.shape[1]) if torch.is_tensor(X_block) and X_block.dim() == 2 else -1
+        dtype = X_block.dtype if torch.is_tensor(X_block) else None
+        ld = self._padded_ld(F, dtype)
+        agree_layout(F, ld, dtype, self.bounds, err, self.rank, self.world, group)
+        self._set_layout(F, ld, dtype, X_block.device)
+        n = X_block.shape[0]
+        self._buf = _PeerBuffer(n * ld * _TABLE_DTYPES[dtype], self.rank, self.world, group)
+        # the local fill either succeeds on every rank or every rank frees its buffer and raises (no rank is left in
+        # a collective the others skipped)
+        err = None
+        try:
+            if n:  # pad columns are zero, as pad_table leaves them: a 16-byte store of the gather may carry them out
+                full = self._view(self._buf.own, n)
+                full[:, F:].zero_()
+                full[:, :F].copy_(X_block)
+            amax = X_block.detach().abs().max().float() if n else torch.zeros((), device=self.device)
+            amax = amax.reshape(1).clone()
+            torch.cuda.synchronize(self.device)
+        except Exception as e:
+            err = f"{type(e).__name__}: {e}"
+        every = [None] * self.world
+        dist.all_gather_object(every, err, group=group)
+        failed = [f"rank {q}: {e}" for q, e in enumerate(every) if e]
+        if failed:
+            self._buf.close()
+            raise _lib.GnnError("ShardedTable: filling the shards failed: " + "; ".join(failed))
+        dist.all_reduce(amax, op=dist.ReduceOp.MAX, group=group)
+        self.abs_max = float(amax.item())
+        dist.barrier(group=group)  # no rank reads a shard before its owner has written it
+        self._keep = []
+        self._make_desc(self._buf.ptrs)
+
+    @classmethod
+    def from_global(cls, X: torch.Tensor, rank: int, world: int, group=None) -> "ShardedTable":
+        """This rank's rows of a table every rank holds, row-balanced bounds (`shard_bounds`)."""
+        bounds = shard_bounds(X.shape[0], world)
+        return cls(X[bounds[rank]:bounds[rank + 1]], bounds, rank, world, group)
+
+    @classmethod
+    def local(cls, shards) -> "ShardedTable":
+        """The shards as tensors of this process on one device (copied into 16-byte aligned rows; no IPC, no
+        collective).  The kernel cannot tell these allocations from peer mappings."""
+        from .functional import pad_table
+        shards = list(shards)
+        if not 1 <= len(shards) <= _lib.MAX_SHARDS:
+            raise _lib.GnnError(f"ShardedTable: {len(shards)} shards, 1 to {_lib.MAX_SHARDS}")
+        for t in shards:
+            err = _table_refusal(t)
+            if err:
+                raise _lib.GnnError("ShardedTable: " + err)
+        if len({(t.shape[1], t.dtype, t.device) for t in shards}) != 1:
+            raise _lib.GnnError("ShardedTable: the shards differ in F, dtype or device")
+        self = cls.__new__(cls)
+        self.rank, self.world, self.group, self._buf = 0, 1, None, None
+        self.bounds = [0]
+        for t in shards:
+            self.bounds.append(self.bounds[-1] + int(t.shape[0]))
+        F, dtype = int(shards[0].shape[1]), shards[0].dtype
+        self._set_layout(F, self._padded_ld(F, dtype), dtype, shards[0].device)
+        self._keep = [pad_table(t.detach()) if t.shape[0] else None for t in shards]  # row stride self.ld
+        self.abs_max = max([float(t.abs().max()) for t in self._keep if t is not None] or [0.0])
+        self._make_desc([0 if t is None else t.data_ptr() for t in self._keep])
+        return self
+
+    @staticmethod
+    def _padded_ld(F: int, dtype) -> int:
+        per16 = 16 // _TABLE_DTYPES.get(dtype, 4)
+        return (max(F, 0) + per16 - 1) // per16 * per16
+
+    def _set_layout(self, F, ld, dtype, device):
+        self.F, self.ld, self.dtype, self.device = int(F), int(ld), dtype, torch.device(device)
+        self.shape = torch.Size((self.bounds[-1], self.F))
+        self.requires_grad = False
+
+    def _view(self, ptr: int, rows: int) -> torch.Tensor:
+        """[rows, ld] torch view of a shard buffer."""
+        t = torch.as_tensor(_RawCudaBuffer(ptr, (rows, self.ld), _TORCH_TYPESTR[self.dtype]), device=self.device)
+        return t.view(self.dtype) if self.dtype != torch.float32 else t
+
+    def _make_desc(self, ptrs):
+        d = _lib.ShardedTableDesc()
+        d.struct_size = C.sizeof(_lib.ShardedTableDesc)
+        d.n_shards = len(self.bounds) - 1
+        for s, p in enumerate(ptrs):
+            d.base[s] = p or None
+        for s, b in enumerate(self.bounds):
+            d.row_begin[s] = b
+        self.desc = d
+
+    @property
+    def n_shards(self) -> int:
+        return len(self.bounds) - 1
+
+    def stride(self, dim: Optional[int] = None):
+        return (self.ld, 1) if dim is None else (self.ld, 1)[dim]
+
+    def close(self):
+        """Unmap and free the shard buffers (collective for a table built across ranks, like
+        PartitionedGraph.close)."""
+        if self._buf is not None:
+            # gathers are asynchronous: this rank's last ones may still read peer shards, and peers may still read
+            # this rank's shard, so every rank finishes its work before any mapping is closed or buffer freed
+            torch.cuda.synchronize(self.device)
+            dist.barrier(group=self.group)
+            self._buf.close()
+            self._buf = None
+        self._keep = []
+        self.desc = None
+
+
 # ---- training across ranks ------------------------------------------------------------------
 # A model holds replicated weights and rank-local activations.  With the loss rule below, the SUM over the ranks of
 # the per-rank gradients is the 1-GPU gradient, so one SUM all_reduce of the gradients before the optimizer step

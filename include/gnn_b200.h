@@ -251,6 +251,36 @@ int gnn_gather_reduce_multi_f32_split(const float* table, int64_t ld_table, int6
                                       const int64_t* n_src_host, const int32_t* fanout_host,
                                       void* const* out_hi_host, const int64_t* ld_out_host,
                                       const int64_t* lo_off_host, gnn_stream_t stream);
+/* A feature table split into contiguous row blocks (shards), e.g. one per GPU of a node: shard s holds the global
+ * rows [row_begin[s], row_begin[s+1]) at device address base[s] (this device's memory or a peer's gnn_peer_open
+ * mapping).  All shards share ld_table, F and the element type.  row_begin[0] = 0, non-decreasing,
+ * row_begin[n_shards] = global row count; base[s] may be NULL for an empty shard, else 16-byte aligned.
+ * struct_size = sizeof(gnn_sharded_table) (ABI versioning). */
+#define GNN_MAX_SHARDS 8
+typedef struct gnn_sharded_table {
+  int32_t struct_size;
+  int32_t n_shards; /* 1..GNN_MAX_SHARDS */
+  const void* base[GNN_MAX_SHARDS];
+  int64_t row_begin[GNN_MAX_SHARDS + 1];
+} gnn_sharded_table;
+/* gnn_gather_reduce_multi_{f32,bf16,f32_split} over a sharded table.  Same blocks and semantics (ids < 0 or >= the
+ * global row count contribute nothing); each output row is the same ordered sum as over the concatenated table, bit
+ * for bit: only the address each row is copied from differs.  TMA path only: ld_table * elem % 16 == 0 and rows of
+ * 256 bytes or more (GNN_ERR_MISALIGNED / GNN_ERR_UNSUPPORTED otherwise).  The table is validated before anything
+ * is launched. */
+int gnn_gather_reduce_multi_sharded_f32(const gnn_sharded_table* table, int64_t ld_table, int32_t F, int reduce,
+                                        int32_t n_blocks, const void* const* idx_host, int idx_bits,
+                                        const int64_t* n_src_host, const int32_t* fanout_host,
+                                        void* const* out_host, const int64_t* ld_out_host, gnn_stream_t stream);
+int gnn_gather_reduce_multi_sharded_bf16(const gnn_sharded_table* table, int64_t ld_table, int32_t F, int reduce,
+                                         int32_t n_blocks, const void* const* idx_host, int idx_bits,
+                                         const int64_t* n_src_host, const int32_t* fanout_host,
+                                         void* const* out_host, const int64_t* ld_out_host, gnn_stream_t stream);
+int gnn_gather_reduce_multi_sharded_f32_split(const gnn_sharded_table* table, int64_t ld_table, int32_t F,
+                                              int reduce, int32_t n_blocks, const void* const* idx_host,
+                                              int idx_bits, const int64_t* n_src_host, const int32_t* fanout_host,
+                                              void* const* out_hi_host, const int64_t* ld_out_host,
+                                              const int64_t* lo_off_host, gnn_stream_t stream);
 /* Edge-type axis (GATNE): table [n_nodes, n_types, F] (ld_row = stride between (node,type)
  * rows), idx [n_src, n_types, fanout]; out[(b*n_types+t), :] = reduce_k table[idx[b,t,k], t, :]
  * — the per-type neighbour aggregation of GATNE_Pytorch/models/GATNE.py:57-77 (`torch.cat` of T
