@@ -46,6 +46,10 @@ SIGNATURES = {
     "gnn_semantic_combine_f32": (cint, [ptr, ptr, i64, i32, i32, ptr, ptr]),
     "gnn_semantic_combine_bwd_f32": (cint, [ptr, ptr, ptr, i64, i32, i32, ptr, ptr, ptr, i64, ptr]),
     "gnn_semantic_scores_bwd_f32": (cint, [ptr, i64, ptr, ptr, ptr, i64, i32, i32, ptr, i64, ptr, ptr, ptr, i64, ptr]),
+    "gnn_semantic_scores_partial_f32": (cint, [ptr, i64, ptr, ptr, i64, i32, i32, ptr, ptr, i64, ptr]),
+    "gnn_semantic_scores_finalize_f32": (cint, [ptr, i64, i32, ptr, ptr, ptr]),
+    "gnn_semantic_combine_bwd_partial_f32": (cint, [ptr, ptr, ptr, i64, i32, i32, ptr, ptr, ptr, i64, ptr]),
+    "gnn_semantic_combine_bwd_finalize_f32": (cint, [ptr, ptr, i64, i32, ptr, ptr]),
     "gnn_gather_reduce_f32": (cint, [ptr, i64, i64, ptr, cint, i64, i32, i32, cint, ptr, i64, ptr, ptr]),
     "gnn_gather_reduce_bf16": (cint, [ptr, i64, i64, ptr, cint, i64, i32, i32, cint, ptr, i64, ptr, ptr]),
     "gnn_gather_reduce_multi_f32": (cint, [ptr, i64, i64, i32, cint, i32, ptr, cint, ptr, ptr, ptr, ptr, ptr]),
@@ -68,6 +72,11 @@ SIGNATURES = {
     "gnn_gat_fused_bwd_ex_f32": (cint, [ptr, ptr, ptr, ptr, ptr, ptr, i64, ptr, ptr, ptr, ptr, ptr, ptr, i64, i64, i64,
                                         i32, i32, f32, cint, ptr, ptr, i64, ptr, ptr, ptr, i64, ptr, i64, ptr, i64, i64,
                                         cint, ptr, ptr, ptr]),
+    "gnn_gat_fused_fwd_batch_f32": (cint, [ptr, ptr, ptr, i64, ptr, ptr, i64, i32, i32, f32, cint, cint, ptr, ptr, ptr,
+                                           ptr, i64, ptr, ptr, ptr, i64, i64, ptr, ptr]),
+    "gnn_gat_fused_bwd_batch_f32": (cint, [ptr, ptr, ptr, ptr, ptr, ptr, i64, ptr, ptr, ptr, ptr, ptr, ptr, i64, i32,
+                                           i32, f32, cint, ptr, ptr, i64, ptr, ptr, ptr, i64, ptr, i64, ptr, i64, i64,
+                                           cint, ptr, ptr, ptr, ptr]),
     "gnn_gat_fused_fwd_train_f32": (cint, [ptr, ptr, ptr, i64, ptr, ptr, i64, i64, i32, i32, f32, cint, cint, ptr, ptr,
                                            ptr, ptr, ptr, i64, ptr, ptr, ptr, i64, i64, i64, ptr]),
     "gnn_gat_fused_fwd_train_bf16": (cint, [ptr, ptr, ptr, i64, ptr, ptr, i64, i64, i32, i32, f32, cint, cint, ptr, ptr,
@@ -108,6 +117,12 @@ class SpmmOpts(C.Structure):
 class GatDropout(C.Structure):
     """gnn_gat_dropout of include/gnn_b200.h."""
     _fields_ = [("struct_size", i32), ("p", f32), ("seed", u64), ("seed_dev", ptr), ("edge_slot_base", i64)]
+
+
+class GatBatch(C.Structure):
+    """gnn_gat_batch of include/gnn_b200.h."""
+    _fields_ = [("struct_size", i32), ("n_graphs", i32), ("rows_per_graph", i64), ("cols_per_graph", i64),
+                ("slot_shift", ptr)]
 
 
 MAX_SHARDS = 8

@@ -69,6 +69,12 @@ struct GatArgs {
   // launch, which walks row_list (nullable: row = blockIdx.x)
   const int64_t* row_list;
   int64_t skip_deg_gt;
+  // batched AND rectangular (RB kernels, a rank's block of M metapaths): batch_n is the stride of this launch's rows
+  // (graph gm = row / batch_n, own row = row - gm * batch_n) and col_stride the stride of its column ids (graph gm's
+  // ids start at gm * col_stride) — the forward rows' and the table rows' counts, swapped in the transposed pass.
+  // slot_shift[gm] (nullable) moves graph gm's seeded-dropout slots.
+  int64_t col_stride;
+  const int64_t* slot_shift;
 };
 
 __device__ __forceinline__ bool aligned_to_dev(const void* p, size_t a) { return (reinterpret_cast<uintptr_t>(p) % a) == 0; }
@@ -172,7 +178,7 @@ struct GatBlock {
   static constexpr int kWarps = (W == 1) ? kGatWarps : W;
 };
 
-template <typename T, int CPL, int W, int HT, int PK>
+template <typename T, int CPL, int W, int HT, int PK, bool RB = false>
 __global__ void __launch_bounds__(GatBlock<W>::kWarps * 32) gat_fwd_kernel(const GatArgs a) {
   constexpr int BW = GatBlock<W>::kWarps;
   extern __shared__ float sm[];
@@ -207,12 +213,15 @@ __global__ void __launch_bounds__(GatBlock<W>::kWarps * 32) gat_fwd_kernel(const
   const int64_t d = e1 - e0;
   if (W == 1 && a.skip_deg_gt > 0 && d > a.skip_deg_gt) return;  // a long row: the CTA-per-row launch owns it
   const int64_t gm = a.batch_n ? i / a.batch_n : 0;      // graph of this row (batched launch)
-  const int64_t joff = gm * a.batch_n;                    // its col ids are offset by joff
+  const int64_t joff = gm * (RB ? a.col_stride : a.batch_n);  // its col ids are offset by joff
+  const int64_t roff = RB ? gm * a.batch_n : joff;        // its output row is i - roff
   const int64_t coff = gm * a.HF;                         // its feature columns start at coff
-  T* orow = reinterpret_cast<T*>(a.out) + (i - joff) * a.ldo + coff;
-  T* arow = a.out_act ? reinterpret_cast<T*>(a.out_act) + (i - joff) * a.ldo + coff : nullptr;
+  T* orow = reinterpret_cast<T*>(a.out) + (i - roff) * a.ldo + coff;
+  T* arow = a.out_act ? reinterpret_cast<T*>(a.out_act) + (i - roff) * a.ldo + coff : nullptr;
   const bool seeded = a.keep == nullptr && a.keep_prob > 0.f;
-  const uint64_t dseed = seeded ? drop_seed_of(a) : 0;
+  uint64_t dseed = seeded ? drop_seed_of(a) : 0;
+  // slot e + shift under seed s is slot e under seed s + shift*H*golden (see set_dropout)
+  if (RB && seeded && a.slot_shift) dseed += (uint64_t)__ldg(a.slot_shift + gm) * (uint64_t)a.H * 0x9E3779B97F4A7C15ULL;
   const uint32_t thresh24 = (uint32_t)(a.keep_prob * 16777216.f);
   if (d == 0) {
     // GAT/models/layers.py:28-30: an all -9e15 row soft-maxes to the uniform 1/N over ALL nodes
@@ -496,7 +505,7 @@ __host__ __device__ inline int gat_bwd_warp_floats(int SE, int H, int HF, bool t
 //   TR = false: rows of the forward CSR (destination i); gathers Wh_j and t_j.
 //   TR = true : rows of the transposed CSR (source j); gathers dOut_i and rowstat_i; `perm` maps its slots to the
 //               forward edge slots for the dropout factors.
-template <typename T, int CPL, int W, int HT, bool TR, int PK>
+template <typename T, int CPL, int W, int HT, bool TR, int PK, bool RB = false>
 __global__ void __launch_bounds__(GatBlock<W>::kWarps * 32) gat_bwd2_kernel(const GatArgs a) {
   constexpr int BW = GatBlock<W>::kWarps;
   constexpr int NA = TR ? 2 : 1;  // accumulators per column
@@ -511,7 +520,8 @@ __global__ void __launch_bounds__(GatBlock<W>::kWarps * 32) gat_bwd2_kernel(cons
   if (W == 1 && a.skip_deg_gt > 0 && d > a.skip_deg_gt) return;
   const int H = HT ? HT : a.H, Hp = HT ? HT : a.Hp, SE = a.SE, HF = a.HF, Fp = a.Fp;
   const int64_t gm = a.batch_n ? r / a.batch_n : 0;
-  const int64_t joff = gm * a.batch_n;
+  const int64_t joff = gm * (RB ? a.col_stride : a.batch_n);
+  const int64_t roff = RB ? gm * a.batch_n : joff;
   const int64_t coff = gm * a.HF;
   const int PW = gat_bwd_warp_floats(SE, H, HF, TR);
   float* w2s = sm + (size_t)warp * PW;
@@ -549,7 +559,8 @@ __global__ void __launch_bounds__(GatBlock<W>::kWarps * 32) gat_bwd2_kernel(cons
   }
   const bool vec4 = HT && (HT % 4 == 0) && aligned_to_dev(TR ? (const void*)a.rowstat : (const void*)a.t, 16);
   const bool seeded = a.keep == nullptr && a.keep_prob > 0.f;
-  const uint64_t dseed = seeded ? drop_seed_of(a) : 0;
+  uint64_t dseed = seeded ? drop_seed_of(a) : 0;
+  if (RB && seeded && a.slot_shift) dseed += (uint64_t)__ldg(a.slot_shift + gm) * (uint64_t)a.H * 0x9E3779B97F4A7C15ULL;
   const uint32_t thresh24 = (uint32_t)(a.keep_prob * 16777216.f);
   const int ngrp = 32 / Hp;
   const int hsub = lane % Hp, g = lane / Hp;
@@ -691,13 +702,13 @@ __global__ void __launch_bounds__(GatBlock<W>::kWarps * 32) gat_bwd2_kernel(cons
   // finalize (one warp): the head-wise contraction of the accumulated vector with this row's own vector
   float* buf = w2s;  // [HF] scratch (this warp's staging area is free now)
   __syncwarp();
-  const T* own = reinterpret_cast<const T*>(TR ? a.Wh : a.d_out) + (r - joff) * (TR ? a.ldw : a.ldo) + coff;
+  const T* own = reinterpret_cast<const T*>(TR ? a.Wh : a.d_out) + (r - roff) * (TR ? a.ldw : a.ldo) + coff;
 #pragma unroll
   for (int c = 0; c < CPL; ++c)
     if (cv[c]) {
       const int ci = col_of<PK>(lane, c);
       buf[ci] = acc2[c] * ldv<T>(own + ci);
-      if (TR) stv(reinterpret_cast<T*>(a.d_Wh) + (r - joff) * a.ld_dwh + coff + ci, acc1[c]);
+      if (TR) stv(reinterpret_cast<T*>(a.d_Wh) + (r - roff) * a.ld_dwh + coff + ci, acc1[c]);
     }
   __syncwarp();
   if (lane < H) {
@@ -744,15 +755,15 @@ size_t gat_smem_bytes(int SE, int H, int HF, int cpl) {
 }
 
 // forward launch: picks the compile-time head count when there is one
-template <typename T, int CPL, int W>
+template <typename T, int CPL, int W, bool RB>
 int gat_fwd_launch(const GatArgs& a, unsigned grid, size_t smem, cudaStream_t st) {
   constexpr int thr = GatBlock<W>::kWarps * 32;
 #define GNN_GAT_FWD_PK(HT, PKV)                                                                                 \
   do {                                                                                                          \
     if (smem > 48 * 1024)                                                                                       \
-      GNN_CUDA(cudaFuncSetAttribute(gat_fwd_kernel<T, CPL, W, HT, PKV>,                                         \
+      GNN_CUDA(cudaFuncSetAttribute(gat_fwd_kernel<T, CPL, W, HT, PKV, RB>,                                     \
                                     cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                   \
-    gat_fwd_kernel<T, CPL, W, HT, PKV><<<grid, thr, smem, st>>>(a);                                             \
+    gat_fwd_kernel<T, CPL, W, HT, PKV, RB><<<grid, thr, smem, st>>>(a);                                         \
   } while (0)
 #define GNN_GAT_FWD(HT)                                              \
   do {                                                               \
@@ -772,16 +783,16 @@ int gat_fwd_launch(const GatArgs& a, unsigned grid, size_t smem, cudaStream_t st
   return GNN_OK;
 }
 
-template <typename T, int W>
+template <typename T, int W, bool RB>
 int gat_fwd_dispatch(const GatArgs& a, int cpl, unsigned grid, cudaStream_t st) {
   int cplr = cpl <= 1 ? 1 : cpl <= 2 ? 2 : cpl <= 4 ? 4 : 8;
   if (a.packed && cplr < 2) cplr = 2;  // a packed lane owns column pairs
   const size_t smem = gat_smem_bytes<W>(a.SE, a.H, a.HF, cplr);
   switch (cplr) {
-    case 1: return gat_fwd_launch<T, 1, W>(a, grid, smem, st);
-    case 2: return gat_fwd_launch<T, 2, W>(a, grid, smem, st);
-    case 4: return gat_fwd_launch<T, 4, W>(a, grid, smem, st);
-    default: return gat_fwd_launch<T, 8, W>(a, grid, smem, st);
+    case 1: return gat_fwd_launch<T, 1, W, RB>(a, grid, smem, st);
+    case 2: return gat_fwd_launch<T, 2, W, RB>(a, grid, smem, st);
+    case 4: return gat_fwd_launch<T, 4, W, RB>(a, grid, smem, st);
+    default: return gat_fwd_launch<T, 8, W, RB>(a, grid, smem, st);
   }
 }
 
@@ -809,12 +820,28 @@ inline int set_dropout(GatArgs& a, const float* edge_keep, const gnn_gat_dropout
   return GNN_OK;
 }
 
+// cooperative, or the listed hub rows first and then one warp per row
+template <typename T, bool RB>
+int gat_fwd_schedule(GatArgs& a, int cpl, int64_t n, int64_t nnz, const int64_t* long_rows, int64_t n_long,
+                     int64_t long_threshold, cudaStream_t st) {
+  if (cooperative(n, nnz)) return gat_fwd_dispatch<T, kGatWarps, RB>(a, cpl, (unsigned)n, st);
+  if (n_long > 0) {  // hub rows: one 16-warp CTA each, launched first so the short rows fill in behind
+    a.row_list = long_rows;
+    int rc = gat_fwd_dispatch<T, 16, RB>(a, cpl, (unsigned)n_long, st);
+    if (rc != GNN_OK) return rc;
+    a.row_list = nullptr;
+    a.skip_deg_gt = long_threshold;
+  }
+  return gat_fwd_dispatch<T, 1, RB>(a, cpl, (unsigned)((n + kGatWarps - 1) / kGatWarps), st);
+}
+
 template <typename T>
 int gat_fwd_impl(const int64_t* rowptr, const int32_t* col, const T* Wh, int64_t ldw, const float* s, const float* t,
                  int64_t n, int64_t nnz, int32_t H, int32_t Fp, float alpha, int mode, int apply_elu,
                  const float* col_mean, const float* edge_keep, T* out, int64_t ldo, float* row_max, float* row_sum,
                  const int64_t* long_rows, int64_t n_long, int64_t long_threshold, cudaStream_t st,
-                 T* out_act = nullptr, const gnn_gat_dropout* drop = nullptr, int64_t batch_nodes = 0) {
+                 T* out_act = nullptr, const gnn_gat_dropout* drop = nullptr, int64_t batch_nodes = 0,
+                 const gnn_gat_batch* rb = nullptr) {
   int rc = check_common(n, H, Fp);
   if (rc != GNN_OK) return rc;
   if (n == 0) return GNN_OK;
@@ -855,18 +882,18 @@ int gat_fwd_impl(const int64_t* rowptr, const int32_t* col, const T* Wh, int64_t
   a.packed = sizeof(T) == 2 && Fp % 2 == 0 && ldw % 2 == 0 && aligned_to(Wh, 4);
   const int cpl = (HF + 31) / 32;
   GNN_REQUIRE(n_long == 0 || (long_rows && long_threshold > 0), GNN_ERR_BAD_ARG, "inconsistent long-row list");
-  if (cooperative(n, nnz)) return gat_fwd_dispatch<T, kGatWarps>(a, cpl, (unsigned)n, st);
-  if (n_long > 0) {  // hub rows: one 16-warp CTA each, launched first so the short rows fill in behind
-    a.row_list = long_rows;
-    rc = gat_fwd_dispatch<T, 16>(a, cpl, (unsigned)n_long, st);
-    if (rc != GNN_OK) return rc;
-    a.row_list = nullptr;
-    a.skip_deg_gt = long_threshold;
+  if (rb) {
+    if constexpr (sizeof(T) == 4) {
+      a.col_stride = rb->cols_per_graph;
+      a.slot_shift = rb->slot_shift;
+      return gat_fwd_schedule<T, true>(a, cpl, n, nnz, long_rows, n_long, long_threshold, st);
+    }
   }
-  return gat_fwd_dispatch<T, 1>(a, cpl, (unsigned)((n + kGatWarps - 1) / kGatWarps), st);
+  GNN_REQUIRE(!rb, GNN_ERR_UNSUPPORTED, "batched rectangular graphs are fp32 only");
+  return gat_fwd_schedule<T, false>(a, cpl, n, nnz, long_rows, n_long, long_threshold, st);
 }
 
-template <typename T, int CPLV, int WV, bool TR>
+template <typename T, int CPLV, int WV, bool TR, bool RB>
 int gat_bwd2_launch(const GatArgs& a, unsigned grid, cudaStream_t st) {
   constexpr int BW = GatBlock<WV>::kWarps;
   size_t f = (size_t)BW * gat_bwd_warp_floats(a.SE, a.H, a.HF, TR);
@@ -876,9 +903,9 @@ int gat_bwd2_launch(const GatArgs& a, unsigned grid, cudaStream_t st) {
 #define GNN_BWD2_PK(HTV, PKV)                                                                                  \
   do {                                                                                                         \
     if (smem > 48 * 1024)                                                                                      \
-      GNN_CUDA(cudaFuncSetAttribute(gat_bwd2_kernel<T, CPLV, WV, HTV, TR, PKV>,                                \
+      GNN_CUDA(cudaFuncSetAttribute(gat_bwd2_kernel<T, CPLV, WV, HTV, TR, PKV, RB>,                            \
                                     cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                  \
-    gat_bwd2_kernel<T, CPLV, WV, HTV, TR, PKV><<<grid, thrv, smem, st>>>(a);                                   \
+    gat_bwd2_kernel<T, CPLV, WV, HTV, TR, PKV, RB><<<grid, thrv, smem, st>>>(a);                               \
   } while (0)
 #define GNN_BWD2(HTV)                                                \
   do {                                                               \
@@ -898,14 +925,63 @@ int gat_bwd2_launch(const GatArgs& a, unsigned grid, cudaStream_t st) {
   return GNN_OK;
 }
 
-template <typename T, int WV, bool TR>
+template <typename T, int WV, bool TR, bool RB>
 int gat_bwd2_dispatch(const GatArgs& a, int cplr, unsigned grid, cudaStream_t st) {
   switch (cplr) {
-    case 1: return gat_bwd2_launch<T, 1, WV, TR>(a, grid, st);
-    case 2: return gat_bwd2_launch<T, 2, WV, TR>(a, grid, st);
-    case 4: return gat_bwd2_launch<T, 4, WV, TR>(a, grid, st);
-    default: return gat_bwd2_launch<T, 8, WV, TR>(a, grid, st);
+    case 1: return gat_bwd2_launch<T, 1, WV, TR, RB>(a, grid, st);
+    case 2: return gat_bwd2_launch<T, 2, WV, TR, RB>(a, grid, st);
+    case 4: return gat_bwd2_launch<T, 4, WV, TR, RB>(a, grid, st);
+    default: return gat_bwd2_launch<T, 8, WV, TR, RB>(a, grid, st);
   }
+}
+
+// pass 1 over the forward CSR (d_s), then pass 2 over the transposed CSR (d_Wh, d_t).  W: 1 warp per row, 4 = every
+// row a CTA (dense graphs), 16 = listed hub rows.  a.rowptr / a.col hold the forward CSR on entry.
+template <typename T, bool RB>
+int gat_bwd_passes(GatArgs& a, int cplr, int64_t n, int64_t n_cols, int64_t nnz, const int64_t* rowptr_t,
+                   const int32_t* col_t, const int64_t* perm_t, const int64_t* long_rows, int64_t n_long,
+                   const int64_t* long_rows_t, int64_t n_long_t, int64_t long_threshold, cudaStream_t st) {
+  int rc;
+  // the row-record kernel and pass 1 walk the n forward rows; pass 2 the n_cols table rows (its own schedule)
+  const bool coop = cooperative(n, nnz), coop_t = cooperative(n_cols, nnz);
+  const unsigned grid1 = (unsigned)((n + kGatWarps - 1) / kGatWarps);
+  const unsigned grid1_t = (unsigned)((n_cols + kGatWarps - 1) / kGatWarps);
+  if (n == 0) {
+    // no forward row: the table rows get zero gradients from pass 2 (every transposed row is empty)
+  } else if (coop) {
+    rc = gat_bwd2_dispatch<T, 4, false, RB>(a, cplr, (unsigned)n, st);
+    if (rc != GNN_OK) return rc;
+  } else {
+    if (n_long > 0) {
+      a.row_list = long_rows;
+      rc = gat_bwd2_dispatch<T, 16, false, RB>(a, cplr, (unsigned)n_long, st);
+      if (rc != GNN_OK) return rc;
+      a.row_list = nullptr;
+      a.skip_deg_gt = long_threshold;
+    }
+    rc = gat_bwd2_dispatch<T, 1, false, RB>(a, cplr, grid1, st);
+    if (rc != GNN_OK) return rc;
+  }
+  a.rowptr = rowptr_t;
+  a.col = col_t;
+  a.perm = perm_t;
+  a.n = n_cols;
+  a.row_list = nullptr;
+  a.skip_deg_gt = 0;
+  if (RB) {  // transposed rows are table rows (per graph: col_stride of them); their ids are forward rows
+    const int64_t rows = a.batch_n;
+    a.batch_n = a.col_stride;
+    a.col_stride = rows;
+  }
+  if (coop_t) return gat_bwd2_dispatch<T, 4, true, RB>(a, cplr, (unsigned)n_cols, st);
+  if (n_long_t > 0) {
+    a.row_list = long_rows_t;
+    rc = gat_bwd2_dispatch<T, 16, true, RB>(a, cplr, (unsigned)n_long_t, st);
+    if (rc != GNN_OK) return rc;
+    a.row_list = nullptr;
+    a.skip_deg_gt = long_threshold;
+  }
+  return gat_bwd2_dispatch<T, 1, true, RB>(a, cplr, grid1_t, st);
 }
 
 template <typename T>
@@ -916,14 +992,15 @@ int gat_bwd_impl(const int64_t* rowptr, const int32_t* col, const int64_t* rowpt
                  float alpha, int mode, const float* edge_keep, T* d_Wh, int64_t ld_dwh, float* d_s, float* d_t,
                  float* row_scratch, int64_t nnz, const int64_t* long_rows, int64_t n_long, const int64_t* long_rows_t,
                  int64_t n_long_t, int64_t long_threshold, cudaStream_t st, int apply_elu = 0, T* d_pre = nullptr,
-                 const gnn_gat_dropout* drop = nullptr, int64_t batch_nodes = 0) {
+                 const gnn_gat_dropout* drop = nullptr, int64_t batch_nodes = 0,
+                 const gnn_gat_batch* rb = nullptr) {
   int rc = check_common(n, H, Fp);
   if (rc != GNN_OK) return rc;
   rc = check_common(n_cols, H, Fp);
   if (rc != GNN_OK) return rc;
   GNN_REQUIRE(n_cols >= n, GNN_ERR_BAD_ARG, "n_cols (%lld) below the forward row count (%lld)", (long long)n_cols,
               (long long)n);
-  GNN_REQUIRE(n_cols == n || batch_nodes == 0, GNN_ERR_UNSUPPORTED, "batched graphs are square (n_cols == n)");
+  GNN_REQUIRE(n_cols == n || batch_nodes == 0 || rb, GNN_ERR_UNSUPPORTED, "batched graphs are square (n_cols == n)");
   if (n == 0 && n_cols == 0) return GNN_OK;
   GNN_REQUIRE(rowptr && rowptr_t && Wh && s && t && row_max && row_sum && out_pre && d_out && d_Wh && d_s && d_t &&
                   row_scratch,
@@ -978,48 +1055,37 @@ int gat_bwd_impl(const int64_t* rowptr, const int32_t* col, const int64_t* rowpt
   const int cpl = (HF + 31) / 32;
   int cplr = cpl <= 1 ? 1 : cpl <= 2 ? 2 : cpl <= 4 ? 4 : 8;
   if (a.packed && cplr < 2) cplr = 2;
-  // the row-record kernel and pass 1 walk the n forward rows; pass 2 the n_cols table rows (its own schedule)
-  const bool coop = cooperative(n, nnz), coop_t = cooperative(n_cols, nnz);
-  const unsigned grid1 = (unsigned)((n + kGatWarps - 1) / kGatWarps);
-  const unsigned grid1_t = (unsigned)((n_cols + kGatWarps - 1) / kGatWarps);
   GNN_REQUIRE((n_long == 0 || long_rows) && (n_long_t == 0 || long_rows_t) &&
                   ((n_long == 0 && n_long_t == 0) || long_threshold > 0),
               GNN_ERR_BAD_ARG, "inconsistent long-row lists");
-  // pass 1 over the forward CSR: d_s.  W: 1 warp per row, 4 = every row a CTA (dense graphs), 16 = listed hub rows
   a.rowptr = rowptr;
   a.col = col;
-  if (n == 0) {
-    // no forward row: the table rows get zero gradients from pass 2 (every transposed row is empty)
-  } else if (coop) {
-    rc = gat_bwd2_dispatch<T, 4, false>(a, cplr, (unsigned)n, st);
-    if (rc != GNN_OK) return rc;
-  } else {
-    if (n_long > 0) {
-      a.row_list = long_rows;
-      rc = gat_bwd2_dispatch<T, 16, false>(a, cplr, (unsigned)n_long, st);
-      if (rc != GNN_OK) return rc;
-      a.row_list = nullptr;
-      a.skip_deg_gt = long_threshold;
+  if (rb) {
+    GNN_REQUIRE(sizeof(T) == 4, GNN_ERR_UNSUPPORTED, "batched rectangular graphs are fp32 only");
+    if constexpr (sizeof(T) == 4) {
+      a.col_stride = rb->cols_per_graph;
+      a.slot_shift = rb->slot_shift;
+      return gat_bwd_passes<T, true>(a, cplr, n, n_cols, nnz, rowptr_t, col_t, perm_t, long_rows, n_long, long_rows_t,
+                                     n_long_t, long_threshold, st);
     }
-    rc = gat_bwd2_dispatch<T, 1, false>(a, cplr, grid1, st);
-    if (rc != GNN_OK) return rc;
   }
-  // pass 2 over the transposed CSR: d_Wh and d_t
-  a.rowptr = rowptr_t;
-  a.col = col_t;
-  a.perm = perm_t;
-  a.n = n_cols;
-  a.row_list = nullptr;
-  a.skip_deg_gt = 0;
-  if (coop_t) return gat_bwd2_dispatch<T, 4, true>(a, cplr, (unsigned)n_cols, st);
-  if (n_long_t > 0) {
-    a.row_list = long_rows_t;
-    rc = gat_bwd2_dispatch<T, 16, true>(a, cplr, (unsigned)n_long_t, st);
-    if (rc != GNN_OK) return rc;
-    a.row_list = nullptr;
-    a.skip_deg_gt = long_threshold;
-  }
-  return gat_bwd2_dispatch<T, 1, true>(a, cplr, grid1_t, st);
+  return gat_bwd_passes<T, false>(a, cplr, n, n_cols, nnz, rowptr_t, col_t, perm_t, long_rows, n_long, long_rows_t,
+                                  n_long_t, long_threshold, st);
+}
+
+// the batched-rectangular description: n_rows / n_cols are the launch's forward rows and table rows
+int check_batch(const gnn_gat_batch* b, int64_t* n_rows, int64_t* n_cols) {
+  GNN_REQUIRE(b, GNN_ERR_BAD_ARG, "null gnn_gat_batch");
+  GNN_REQUIRE(b->struct_size == (int32_t)sizeof(gnn_gat_batch), GNN_ERR_BAD_ARG,
+              "gnn_gat_batch struct_size mismatch (header/library version skew)");
+  GNN_REQUIRE(b->n_graphs >= 1 && b->n_graphs <= 32, GNN_ERR_UNSUPPORTED, "n_graphs=%d outside 1..32", b->n_graphs);
+  GNN_REQUIRE(b->rows_per_graph >= 0 && b->cols_per_graph >= b->rows_per_graph, GNN_ERR_BAD_ARG,
+              "need 0 <= rows_per_graph <= cols_per_graph (got %lld, %lld)", (long long)b->rows_per_graph,
+              (long long)b->cols_per_graph);
+  GNN_REQUIRE(b->cols_per_graph * b->n_graphs < 0x7fffffffLL, GNN_ERR_UNSUPPORTED, "column ids do not fit int32");
+  *n_rows = b->rows_per_graph * b->n_graphs;
+  *n_cols = b->cols_per_graph * b->n_graphs;
+  return GNN_OK;
 }
 
 }  // namespace
@@ -1128,6 +1194,39 @@ int gnn_gat_fused_bwd_ex_f32(const int64_t* rowptr, const int32_t* col, const in
                              n_rows, n_cols, H, Fp, alpha, mode, edge_keep, d_Wh, ld_dwh, d_s, d_t, row_scratch, nnz,
                              long_rows, n_long, long_rows_t, n_long_t, long_threshold, (cudaStream_t)stream, apply_elu,
                              d_pre, dropout, 0);
+}
+
+int gnn_gat_fused_fwd_batch_f32(const int64_t* rowptr, const int32_t* col, const float* Wh, int64_t ldw,
+                                const float* s, const float* t, int64_t nnz, int32_t H, int32_t Fp, float alpha,
+                                int mode, int apply_elu, const float* edge_keep, const gnn_gat_dropout* dropout,
+                                float* out_pre, float* out_act, int64_t ldo, float* row_max, float* row_sum,
+                                const int64_t* long_rows, int64_t n_long, int64_t long_threshold,
+                                const gnn_gat_batch* batch, gnn_stream_t stream) {
+  int64_t n = 0, n_cols = 0;
+  int rc = check_batch(batch, &n, &n_cols);
+  if (rc != GNN_OK) return rc;
+  GNN_REQUIRE(out_act || apply_elu == 0, GNN_ERR_BAD_ARG, "apply_elu > 0 needs out_act");
+  if (n == 0) return GNN_OK;
+  return gat_fwd_impl<float>(rowptr, col, Wh, ldw, s, t, n, nnz, H, Fp, alpha, mode, apply_elu, nullptr, edge_keep,
+                             out_pre, ldo, row_max, row_sum, long_rows, n_long, long_threshold, (cudaStream_t)stream,
+                             apply_elu > 0 ? out_act : nullptr, dropout, batch->rows_per_graph, batch);
+}
+
+int gnn_gat_fused_bwd_batch_f32(const int64_t* rowptr, const int32_t* col, const int64_t* rowptr_t, const int32_t* col_t,
+                                const int64_t* perm_t, const float* Wh, int64_t ldw, const float* s, const float* t,
+                                const float* row_max, const float* row_sum, const float* out_pre, const float* d_out,
+                                int64_t ldo, int32_t H, int32_t Fp, float alpha, int mode, const float* edge_keep,
+                                float* d_Wh, int64_t ld_dwh, float* d_s, float* d_t, float* row_scratch, int64_t nnz,
+                                const int64_t* long_rows, int64_t n_long, const int64_t* long_rows_t, int64_t n_long_t,
+                                int64_t long_threshold, int apply_elu, float* d_pre, const gnn_gat_dropout* dropout,
+                                const gnn_gat_batch* batch, gnn_stream_t stream) {
+  int64_t n = 0, n_cols = 0;
+  int rc = check_batch(batch, &n, &n_cols);
+  if (rc != GNN_OK) return rc;
+  return gat_bwd_impl<float>(rowptr, col, rowptr_t, col_t, perm_t, Wh, ldw, s, t, row_max, row_sum, out_pre, d_out, ldo,
+                             n, n_cols, H, Fp, alpha, mode, edge_keep, d_Wh, ld_dwh, d_s, d_t, row_scratch, nnz,
+                             long_rows, n_long, long_rows_t, n_long_t, long_threshold, (cudaStream_t)stream, apply_elu,
+                             d_pre, dropout, batch->rows_per_graph, batch);
 }
 
 }  // extern "C"

@@ -73,12 +73,9 @@ __device__ inline bool reduce_over_grid_m(float acc, int M, float* partial, unsi
   return true;
 }
 
-__global__ void __launch_bounds__(kSemThreads) semantic_scores_kernel(const float* __restrict__ P, int64_t ldp,
-                                                                      const float* __restrict__ b,
-                                                                      const float* __restrict__ q, int64_t N, int M,
-                                                                      int K, float* scores, float* beta, float* partial,
-                                                                      unsigned int* counter) {
-  __shared__ float tot[32];
+// this thread's warp's share of sum_n sum_k q_k tanh(P[n,m,k] + b_k), metapath m in lane m
+__device__ __forceinline__ float scores_warp_acc(const float* __restrict__ P, int64_t ldp, const float* __restrict__ b,
+                                                 const float* __restrict__ q, int64_t N, int M, int K) {
   const int lane = threadIdx.x & 31;
   const int64_t gw = ((int64_t)blockIdx.x * kSemThreads + threadIdx.x) >> 5;
   const int64_t nw = ((int64_t)gridDim.x * kSemThreads) >> 5;
@@ -92,21 +89,53 @@ __global__ void __launch_bounds__(kSemThreads) semantic_scores_kernel(const floa
       if (lane == m) acc += v;
     }
   }
-  if (!reduce_over_grid_m(acc, M, partial, counter, tot)) return;
-  if (threadIdx.x == 0) {
-    float mx = -INFINITY;
-    for (int m = 0; m < M; ++m) {
-      tot[m] = tot[m] / (float)N;
-      scores[m] = tot[m];
-      mx = fmaxf(mx, tot[m]);
-    }
-    float sum = 0.f;
-    for (int m = 0; m < M; ++m) {
-      tot[m] = expf(tot[m] - mx);
-      sum += tot[m];
-    }
-    for (int m = 0; m < M; ++m) beta[m] = tot[m] / sum;
+  return acc;
+}
+
+// one thread: tot (the node sums, overwritten) -> scores = tot / N, beta = softmax_M(scores)
+__device__ __forceinline__ void scores_finalize(float* tot, int64_t N, int M, float* scores, float* beta) {
+  float mx = -INFINITY;
+  for (int m = 0; m < M; ++m) {
+    tot[m] = tot[m] / (float)N;
+    scores[m] = tot[m];
+    mx = fmaxf(mx, tot[m]);
   }
+  float sum = 0.f;
+  for (int m = 0; m < M; ++m) {
+    tot[m] = expf(tot[m] - mx);
+    sum += tot[m];
+  }
+  for (int m = 0; m < M; ++m) beta[m] = tot[m] / sum;
+}
+
+__global__ void __launch_bounds__(kSemThreads) semantic_scores_kernel(const float* __restrict__ P, int64_t ldp,
+                                                                      const float* __restrict__ b,
+                                                                      const float* __restrict__ q, int64_t N, int M,
+                                                                      int K, float* scores, float* beta, float* partial,
+                                                                      unsigned int* counter) {
+  __shared__ float tot[32];
+  const float acc = scores_warp_acc(P, ldp, b, q, N, M, K);
+  if (!reduce_over_grid_m(acc, M, partial, counter, tot)) return;
+  if (threadIdx.x == 0) scores_finalize(tot, N, M, scores, beta);
+}
+
+// the node sums of semantic_scores_kernel over this part's rows, before the division by N
+__global__ void __launch_bounds__(kSemThreads) semantic_scores_partial_kernel(const float* __restrict__ P, int64_t ldp,
+                                                                              const float* __restrict__ b,
+                                                                              const float* __restrict__ q, int64_t N,
+                                                                              int M, int K, float* sums, float* partial,
+                                                                              unsigned int* counter) {
+  __shared__ float tot[32];
+  const float acc = scores_warp_acc(P, ldp, b, q, N, M, K);
+  if (!reduce_over_grid_m(acc, M, partial, counter, tot)) return;
+  if (threadIdx.x < M) sums[threadIdx.x] = tot[threadIdx.x];
+}
+
+__global__ void semantic_scores_finalize_kernel(const float* __restrict__ sums, int64_t n_total, int M, float* scores,
+                                                float* beta) {
+  __shared__ float tot[32];
+  for (int m = 0; m < M; ++m) tot[m] = sums[m];
+  scores_finalize(tot, n_total, M, scores, beta);
 }
 
 __global__ void __launch_bounds__(kSemThreads) semantic_combine_kernel(const float* __restrict__ beta,
@@ -123,13 +152,11 @@ __global__ void __launch_bounds__(kSemThreads) semantic_combine_kernel(const flo
   }
 }
 
-__global__ void __launch_bounds__(kSemThreads) semantic_combine_bwd_kernel(const float* __restrict__ d_out,
-                                                                           const float* __restrict__ z,
-                                                                           const float* __restrict__ beta, int64_t N,
-                                                                           int M, int D, float* __restrict__ dz,
-                                                                           float* d_scores_over_n, float* partial,
-                                                                           unsigned int* counter) {
-  __shared__ float tot[32];
+// writes the direct term dz = beta_m dOut of this thread's rows; returns its warp's share of
+// dbeta_m = sum_n <dOut_n, z_nm>, metapath m in lane m
+__device__ __forceinline__ float combine_bwd_warp_acc(const float* __restrict__ d_out, const float* __restrict__ z,
+                                                      const float* __restrict__ beta, int64_t N, int M, int D,
+                                                      float* __restrict__ dz) {
   const int lane = threadIdx.x & 31;
   const int64_t gw = ((int64_t)blockIdx.x * kSemThreads + threadIdx.x) >> 5;
   const int64_t nw = ((int64_t)gridDim.x * kSemThreads) >> 5;
@@ -150,12 +177,41 @@ __global__ void __launch_bounds__(kSemThreads) semantic_combine_bwd_kernel(const
       if (lane == m) acc += v;
     }
   }
+  return acc;
+}
+
+// one thread: the softmax backward over M, divided by the node count N
+__device__ __forceinline__ void combine_bwd_finalize(const float* tot, const float* beta, int64_t N, int M,
+                                                     float* d_scores_over_n) {
+  float dotp = 0.f;  // Σ_j beta_j dbeta_j
+  for (int m = 0; m < M; ++m) dotp = fmaf(beta[m], tot[m], dotp);
+  for (int m = 0; m < M; ++m) d_scores_over_n[m] = beta[m] * (tot[m] - dotp) / (float)N;
+}
+
+__global__ void __launch_bounds__(kSemThreads) semantic_combine_bwd_kernel(const float* __restrict__ d_out,
+                                                                           const float* __restrict__ z,
+                                                                           const float* __restrict__ beta, int64_t N,
+                                                                           int M, int D, float* __restrict__ dz,
+                                                                           float* d_scores_over_n, float* partial,
+                                                                           unsigned int* counter) {
+  __shared__ float tot[32];
+  const float acc = combine_bwd_warp_acc(d_out, z, beta, N, M, D, dz);
   if (!reduce_over_grid_m(acc, M, partial, counter, tot)) return;
-  if (threadIdx.x == 0) {
-    float dotp = 0.f;  // Σ_j beta_j dbeta_j
-    for (int m = 0; m < M; ++m) dotp = fmaf(beta[m], tot[m], dotp);
-    for (int m = 0; m < M; ++m) d_scores_over_n[m] = beta[m] * (tot[m] - dotp) / (float)N;
-  }
+  if (threadIdx.x == 0) combine_bwd_finalize(tot, beta, N, M, d_scores_over_n);
+}
+
+__global__ void __launch_bounds__(kSemThreads) semantic_combine_bwd_partial_kernel(
+    const float* __restrict__ d_out, const float* __restrict__ z, const float* __restrict__ beta, int64_t N, int M,
+    int D, float* __restrict__ dz, float* dbeta, float* partial, unsigned int* counter) {
+  __shared__ float tot[32];
+  const float acc = combine_bwd_warp_acc(d_out, z, beta, N, M, D, dz);
+  if (!reduce_over_grid_m(acc, M, partial, counter, tot)) return;
+  if (threadIdx.x < M) dbeta[threadIdx.x] = tot[threadIdx.x];
+}
+
+__global__ void semantic_combine_bwd_finalize_kernel(const float* __restrict__ dbeta, const float* __restrict__ beta,
+                                                     int64_t n_total, int M, float* d_scores_over_n) {
+  combine_bwd_finalize(dbeta, beta, n_total, M, d_scores_over_n);
 }
 
 __global__ void __launch_bounds__(kSemThreads) semantic_scores_bwd_kernel(const float* __restrict__ P, int64_t ldp,
@@ -295,6 +351,60 @@ int gnn_semantic_scores_bwd_f32(const float* P, int64_t ldp, const float* bias, 
   semantic_scores_bwd_kernel<<<grid_for(rows_per_iter * 64, N * M), kSemThreads, 0, (cudaStream_t)stream>>>(
       P, ldp, bias, q, d_scores_over_n, N * M, M, K, dP, lddp, dq, dbias, ws + 4,
       reinterpret_cast<unsigned int*>(ws));
+  GNN_LAUNCH_CHECK();
+  return GNN_OK;
+}
+
+int gnn_semantic_scores_partial_f32(const float* P, int64_t ldp, const float* bias, const float* q, int64_t N,
+                                    int32_t M, int32_t K, float* sums, void* workspace, int64_t workspace_bytes,
+                                    void* stream) {
+  int rc = check_sem(N, M, K, "gnn_semantic_scores_partial");
+  if (rc != GNN_OK) return rc;
+  GNN_REQUIRE(K <= kSemMaxK, GNN_ERR_UNSUPPORTED, "hidden width %d exceeds %d", K, kSemMaxK);
+  GNN_REQUIRE((P || N == 0) && q && sums && workspace, GNN_ERR_BAD_ARG, "null pointer");
+  GNN_REQUIRE(ldp >= K, GNN_ERR_BAD_ARG, "ldp smaller than K");
+  GNN_REQUIRE(workspace_bytes >= sem_ws_bytes(K) && aligned_to(workspace, 16), GNN_ERR_BAD_ARG,
+              "workspace too small or misaligned (gnn_semantic_workspace_size)");
+  float* ws = static_cast<float*>(workspace);
+  semantic_scores_partial_kernel<<<grid_for(kSemWarps * 8, N), kSemThreads, 0, (cudaStream_t)stream>>>(
+      P, ldp, bias, q, N, M, K, sums, ws + 4, reinterpret_cast<unsigned int*>(ws));
+  GNN_LAUNCH_CHECK();
+  return GNN_OK;
+}
+
+int gnn_semantic_scores_finalize_f32(const float* sums, int64_t n_total, int32_t M, float* scores, float* beta,
+                                     void* stream) {
+  int rc = check_sem(n_total, M, 1, "gnn_semantic_scores_finalize");
+  if (rc != GNN_OK) return rc;
+  GNN_REQUIRE(n_total > 0, GNN_ERR_BAD_ARG, "semantic attention over zero nodes (mean over an empty axis)");
+  GNN_REQUIRE(sums && scores && beta, GNN_ERR_BAD_ARG, "null pointer");
+  semantic_scores_finalize_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(sums, n_total, M, scores, beta);
+  GNN_LAUNCH_CHECK();
+  return GNN_OK;
+}
+
+int gnn_semantic_combine_bwd_partial_f32(const float* d_out, const float* z, const float* beta, int64_t N, int32_t M,
+                                         int32_t D, float* dz, float* dbeta, void* workspace, int64_t workspace_bytes,
+                                         void* stream) {
+  int rc = check_sem(N, M, D, "gnn_semantic_combine_bwd_partial");
+  if (rc != GNN_OK) return rc;
+  GNN_REQUIRE(((d_out && z && dz) || N == 0) && beta && dbeta && workspace, GNN_ERR_BAD_ARG, "null pointer");
+  GNN_REQUIRE(workspace_bytes >= sem_ws_bytes(kSemMaxM) && aligned_to(workspace, 16), GNN_ERR_BAD_ARG,
+              "workspace too small or misaligned (gnn_semantic_workspace_size)");
+  float* ws = static_cast<float*>(workspace);
+  semantic_combine_bwd_partial_kernel<<<grid_for(kSemWarps * 8, N), kSemThreads, 0, (cudaStream_t)stream>>>(
+      d_out, z, beta, N, M, D, dz, dbeta, ws + 4, reinterpret_cast<unsigned int*>(ws));
+  GNN_LAUNCH_CHECK();
+  return GNN_OK;
+}
+
+int gnn_semantic_combine_bwd_finalize_f32(const float* dbeta, const float* beta, int64_t n_total, int32_t M,
+                                          float* d_scores_over_n, void* stream) {
+  int rc = check_sem(n_total, M, 1, "gnn_semantic_combine_bwd_finalize");
+  if (rc != GNN_OK) return rc;
+  GNN_REQUIRE(n_total > 0, GNN_ERR_BAD_ARG, "semantic attention over zero nodes");
+  GNN_REQUIRE(dbeta && beta && d_scores_over_n, GNN_ERR_BAD_ARG, "null pointer");
+  semantic_combine_bwd_finalize_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(dbeta, beta, n_total, M, d_scores_over_n);
   GNN_LAUNCH_CHECK();
   return GNN_OK;
 }

@@ -606,12 +606,17 @@ class AttentionDropout:
     seed and a device int64 tensor mixed into it (so a captured CUDA graph draws a fresh mask per replay).  The
     kernels recompute the keep factor of every (edge, head) from the stream — no [nnz, H] mask is materialised.
     edge_slot_base: local edge slot e draws the factor of slot e + edge_slot_base (a row block of a larger CSR passes
-    its first global slot and draws the whole graph's mask for its edges)."""
+    its first global slot and draws the whole graph's mask for its edges).
+    slot_shift (device int64 [M], batched-rectangular graphs only): graph m's slots are moved by slot_shift[m] as
+    well (partition.PartitionedMetapaths.attention)."""
 
-    def __init__(self, p: float, seed: int, seed_dev: Optional[torch.Tensor] = None, edge_slot_base: int = 0):
+    def __init__(self, p: float, seed: int, seed_dev: Optional[torch.Tensor] = None, edge_slot_base: int = 0,
+                 slot_shift: Optional[torch.Tensor] = None):
         self.p, self.seed, self.seed_dev = float(p), int(seed) & 0xFFFFFFFFFFFFFFFF, seed_dev
         self.edge_slot_base = int(edge_slot_base)
+        self.slot_shift = slot_shift
         assert seed_dev is None or (seed_dev.dtype == torch.int64 and seed_dev.is_cuda and seed_dev.numel() == 1)
+        assert slot_shift is None or (slot_shift.dtype == torch.int64 and slot_shift.is_cuda)
 
     def c_struct(self):
         import ctypes as C
@@ -685,7 +690,10 @@ def gat_fwd_raw(g: CSRGraph, Wh, s, t, H, Fp, alpha, mode=_lib.GAT_SOFTMAX, elu=
     batch = M > 1: `g` is the block diagonal of M graphs over the same N nodes (CSRGraph.block_diagonal), Wh / out are
     [N, M*H*Fp] (graph m's columns at m*H*Fp), s / t are [M*N, H] (batched-row major) — HAN's metapaths in one launch.
     Rectangular `g` (n_cols > n_rows, a row block whose columns address [own rows ; halo rows]): Wh and t have n_cols
-    rows, s and out n_rows; fp32, one graph, H*Fp <= 256 and no row without edges."""
+    rows, s and out n_rows; fp32, H*Fp <= 256 and no row without edges.  With batch = M > 1 as well, `g` is the block
+    diagonal of M such blocks over one combined table (partition.PartitionedMetapaths.attention): Wh is
+    [n_cols / M, M*H*Fp], t [n_cols, H], s [n_rows, H], out [n_rows / M, M*H*Fp]; `dropout.slot_shift` moves each
+    graph's dropout slots."""
     _require_cuda(Wh, s, t, keep)
     lib = _lib.load()
     Wh = _rowmajor(Wh)
@@ -700,8 +708,8 @@ def gat_fwd_raw(g: CSRGraph, Wh, s, t, H, Fp, alpha, mode=_lib.GAT_SOFTMAX, elu=
             or t.shape != (nc, H)):
         raise _lib.GnnError(f"gat: Wh {tuple(Wh.shape)} / s {tuple(s.shape)} / t {tuple(t.shape)} do not match graph "
                             f"rows={n}, cols={nc}, batch={M}, H*Fp={H * Fp}")
-    if nc != n and (M > 1 or H * Fp > 256 or Wh.dtype != torch.float32):
-        raise _lib.GnnError("gat: a rectangular graph (table rows != rows) takes one fp32 graph of H*Fp <= 256")
+    if nc != n and (H * Fp > 256 or Wh.dtype != torch.float32):
+        raise _lib.GnnError("gat: a rectangular graph (table rows != rows) takes fp32 features and H*Fp <= 256")
     if M > 1 and H * Fp > 256:
         raise _lib.GnnError("gat: batched graphs need H*Fp <= 256 per graph")
     if out is None:
@@ -720,6 +728,20 @@ def gat_fwd_raw(g: CSRGraph, Wh, s, t, H, Fp, alpha, mode=_lib.GAT_SOFTMAX, elu=
     bn = nodes if M > 1 else 0
     lr, thr = g.gat_long_rows()
     f32 = Wh.dtype == torch.float32
+    import ctypes as C
+    if _batched_rect(g, M, dropout):
+        # batched and rectangular: one fp32 group, the training entry (it writes the activated form to out_act)
+        if Wh.dtype != torch.float32:
+            raise _lib.GnnError("gat: batched rectangular graphs take fp32 features")
+        pre_buf, act_buf = (out, out_act) if (out_act is not None or elu == 0) else (torch.empty_like(out), out)
+        dstruct = dropout.c_struct() if (dropout is not None and dropout.p > 0.0) else None
+        bstruct = _batch_struct(M, nodes, nc // M, dropout)
+        _lib.check(lib.gnn_gat_fused_fwd_batch_f32(
+            _p(g.rowptr), _p(g.col), _p(Wh), _ld(Wh), _p(s), _p(t), g.nnz, H, Fp, float(alpha), mode,
+            elu if act_buf is not None else 0, _p(keep), C.byref(dstruct) if dstruct is not None else None,
+            _p(pre_buf), _p(act_buf), _ld(out), _p(row_max), _p(row_sum), _p(lr), lr.numel(), thr, C.byref(bstruct),
+            _stream_ptr()), "gnn_gat_fused_fwd_batch_f32")
+        return out, row_max, row_sum
     train = out_act is not None or (dropout is not None and dropout.p > 0.0)
     pre_buf, act_buf = out, out_act
     if train and out_act is None and elu > 0:
@@ -735,7 +757,6 @@ def gat_fwd_raw(g: CSRGraph, Wh, s, t, H, Fp, alpha, mode=_lib.GAT_SOFTMAX, elu=
         # a head group restarts the head index at 0: materialise the stream once so every group sees its own heads
         keep, dropout = attention_keep_mask_from_seed(g, H, dropout), None
     dstruct = dropout.c_struct() if (dropout is not None and dropout.p > 0.0) else None
-    import ctypes as C
     for h0, h1, f0, f1 in groups:
         whole = len(groups) == 1
         Hg, Fg = h1 - h0, f1 - f0
@@ -761,6 +782,25 @@ def gat_fwd_raw(g: CSRGraph, Wh, s, t, H, Fp, alpha, mode=_lib.GAT_SOFTMAX, elu=
             row_max[:, h0:h1] = rm
             row_sum[:, h0:h1] = rs
     return out, row_max, row_sum
+
+
+def _batched_rect(g: CSRGraph, M: int, dropout: Optional[AttentionDropout]) -> bool:
+    """The batched-rectangular entries serve a batched graph whose table rows differ from its rows, or whose seeded
+    dropout carries per-graph slot shifts (a rank's block without halo rows is square)."""
+    shifted = dropout is not None and dropout.p > 0.0 and dropout.slot_shift is not None
+    return M > 1 and (g.n_cols != g.n_rows or shifted)
+
+
+def _batch_struct(M: int, rows: int, cols: int, dropout: Optional[AttentionDropout]):
+    b = _lib.GatBatch()
+    import ctypes as C
+    b.struct_size = C.sizeof(_lib.GatBatch)
+    b.n_graphs, b.rows_per_graph, b.cols_per_graph = int(M), int(rows), int(cols)
+    shift = None if (dropout is None or dropout.p <= 0.0) else dropout.slot_shift
+    if shift is not None and (shift.numel() != M or not shift.is_contiguous()):
+        raise _lib.GnnError(f"gat: slot_shift must be a contiguous [{M}] int64 tensor")
+    b.slot_shift = _p(shift)
+    return b
 
 
 class _GatFn(torch.autograd.Function):
@@ -812,7 +852,17 @@ class _GatFn(torch.autograd.Function):
         groups = list(_gat_groups(H, Fp))
         esz = Wh.element_size()
         need_perm = keep is not None or drop is not None
-        if nc != n:  # rectangular (one fp32 group, checked by the forward): table rows get d_Wh / d_t
+        if _batched_rect(g, M, drop):  # batched and rectangular (one fp32 group, no empty row: checked by the forward)
+            row_scratch = torch.empty((n, 4, H), dtype=torch.float32, device=dev)
+            bstruct = _batch_struct(M, n // M, nc // M, drop)
+            _lib.check(lib.gnn_gat_fused_bwd_batch_f32(
+                _p(g.rowptr), _p(g.col), _p(gt.rowptr), _p(gt.col), _p(g.perm_t) if need_perm else None, _p(Wh), _ld(Wh),
+                _p(s), _p(t), _p(row_max), _p(row_sum), _p(out), _p(d_out), _ld(out), H, Fp, alpha, mode,
+                _p(keep), _p(d_Wh), _ld(d_Wh), _p(d_s), _p(d_t), _p(row_scratch), g.nnz, _p(lr), lr.numel(), _p(lrt),
+                lrt.numel(), thr, elu, _p(d_pre), C.byref(dstruct) if dstruct is not None else None, C.byref(bstruct),
+                _stream_ptr()), "gnn_gat_fused_bwd_batch_f32")
+            groups = []
+        elif nc != n:  # rectangular (one fp32 group, checked by the forward): table rows get d_Wh / d_t
             row_scratch = torch.empty((n, 4, H), dtype=torch.float32, device=dev)
             _lib.check(lib.gnn_gat_fused_bwd_ex_f32(
                 _p(g.rowptr), _p(g.col), _p(gt.rowptr), _p(gt.col), _p(g.perm_t) if need_perm else None, _p(Wh), _ld(Wh),
@@ -968,3 +1018,94 @@ def semantic_attention(z: torch.Tensor, W1: torch.Tensor, b1: Optional[torch.Ten
             W1.shape[1] != z.shape[2] or q.numel() != W1.shape[0] or z.shape[0] == 0:
         raise _lib.GnnError(f"semantic_attention: unsupported shapes z {tuple(z.shape)} W1 {tuple(W1.shape)} q {tuple(q.shape)}")
     return _SemanticFn.apply(z, W1, b1, q)
+
+
+def _rank_ordered_sum(x: torch.Tensor, world: int, group) -> torch.Tensor:
+    """Σ over the ranks of x, added in rank order starting from rank 0's tensor (one all_gather): the same bits on
+    every rank whatever the backend's reduction algorithm, and x itself at world 1."""
+    if world == 1:
+        return x
+    import torch.distributed as dist
+    parts = [torch.empty_like(x) for _ in range(world)]
+    dist.all_gather(parts, x.contiguous(), group=group)
+    acc = parts[0]
+    for p in parts[1:]:
+        acc = acc + p
+    return acc
+
+
+class _SemanticPartitionedFn(torch.autograd.Function):
+    """_SemanticFn over a rank's rows of a row-partitioned node set: the node sums behind mean_N (forward) and dβ
+    (backward) are split at the rank boundary — partial over the own rows, a rank-ordered sum of the [M] partials,
+    then finalize with the global node count.  Collective in both directions."""
+
+    @staticmethod
+    def forward(ctx, z, W1, b1, q, n_total, world, group):
+        lib = _lib.load()
+        N, M, D = z.shape
+        K = W1.shape[0]
+        z = z.contiguous()
+        W1c, qv = W1.contiguous(), q.reshape(-1).contiguous()
+        b1c = None if b1 is None else b1.contiguous()
+        P = torch.mm(z.view(N * M, D), W1c.t())                      # [N*M, K]
+        ws = _semantic_workspace(K, z.device)
+        dev = z.device
+        sums = torch.empty(M, dtype=torch.float32, device=dev)
+        st = _stream_ptr()
+        _lib.check(lib.gnn_semantic_scores_partial_f32(_p(P), P.stride(0), _p(b1c), _p(qv), N, M, K, _p(sums), _p(ws),
+                                                       ws.numel(), st), "gnn_semantic_scores_partial_f32")
+        sums = _rank_ordered_sum(sums, world, group)
+        scores = torch.empty(M, dtype=torch.float32, device=dev)
+        beta = torch.empty(M, dtype=torch.float32, device=dev)
+        _lib.check(lib.gnn_semantic_scores_finalize_f32(_p(sums), n_total, M, _p(scores), _p(beta), st),
+                   "gnn_semantic_scores_finalize_f32")
+        out = torch.empty((N, D), dtype=torch.float32, device=dev)
+        _lib.check(lib.gnn_semantic_combine_f32(_p(beta), _p(z), N, M, D, _p(out), st), "gnn_semantic_combine_f32")
+        ctx.save_for_backward(z, W1c, b1c if b1c is not None else z.new_empty(0), qv, P, beta)
+        ctx.has_bias, ctx.q_shape, ctx.dist = b1 is not None, tuple(q.shape), (n_total, world, group)
+        return out
+
+    @staticmethod
+    def backward(ctx, d_out):
+        lib = _lib.load()
+        z, W1, b1, qv, P, beta = ctx.saved_tensors
+        n_total, world, group = ctx.dist
+        N, M, D = z.shape
+        K = W1.shape[0]
+        d_out = d_out.contiguous()
+        dev = z.device
+        ws = _semantic_workspace(K, dev)
+        dz = torch.empty_like(z)
+        dbeta = torch.empty(M, dtype=torch.float32, device=dev)
+        st = _stream_ptr()
+        _lib.check(lib.gnn_semantic_combine_bwd_partial_f32(_p(d_out), _p(z), _p(beta), N, M, D, _p(dz), _p(dbeta),
+                                                            _p(ws), ws.numel(), st),
+                   "gnn_semantic_combine_bwd_partial_f32")
+        dbeta = _rank_ordered_sum(dbeta, world, group)
+        dsn = torch.empty(M, dtype=torch.float32, device=dev)
+        _lib.check(lib.gnn_semantic_combine_bwd_finalize_f32(_p(dbeta), _p(beta), n_total, M, _p(dsn), st),
+                   "gnn_semantic_combine_bwd_finalize_f32")
+        dq = torch.zeros(K, dtype=torch.float32, device=dev)
+        db = torch.zeros(K, dtype=torch.float32, device=dev) if ctx.has_bias else None
+        dP = torch.empty_like(P)
+        if N > 0:  # the rank's share of the column sums dq / db (partition.allreduce_gradients adds the ranks')
+            _lib.check(lib.gnn_semantic_scores_bwd_f32(_p(P), P.stride(0), _p(b1) if ctx.has_bias else None, _p(qv),
+                                                       _p(dsn), N, M, K, _p(dP), dP.stride(0), _p(dq), _p(db), _p(ws),
+                                                       ws.numel(), st), "gnn_semantic_scores_bwd_f32")
+        z2 = z.view(N * M, D)
+        dW1 = torch.mm(dP.t(), z2) if ctx.needs_input_grad[1] else None
+        dz = torch.addmm(dz.view(N * M, D), dP, W1).view(N, M, D) if ctx.needs_input_grad[0] else None
+        return dz, dW1, db, dq.view(ctx.q_shape), None, None, None
+
+
+def semantic_attention_partitioned(z: torch.Tensor, W1: torch.Tensor, b1: Optional[torch.Tensor], q: torch.Tensor,
+                                   n_total: int, world: int, group=None) -> torch.Tensor:
+    """`semantic_attention` over this rank's rows z [n_local, M, D] of a row-partitioned node set of n_total nodes:
+    β is the one of all n_total nodes, identical on every rank (rank-ordered sums of the per-rank node sums).
+    Collective, forward and backward; at world 1 it computes the same bits as `semantic_attention`."""
+    _require_cuda(z, W1, q)
+    if z.dtype != torch.float32 or z.dim() != 3 or z.shape[1] > SEMANTIC_MAX_M or W1.shape[0] > SEMANTIC_MAX_K or \
+            W1.shape[1] != z.shape[2] or q.numel() != W1.shape[0] or n_total <= 0:
+        raise _lib.GnnError(f"semantic_attention: unsupported shapes z {tuple(z.shape)} W1 {tuple(W1.shape)} "
+                            f"q {tuple(q.shape)} n_total {n_total}")
+    return _SemanticPartitionedFn.apply(z, W1, b1, q, int(n_total), int(world), group)

@@ -22,10 +22,10 @@ from torch import nn
 import torch.nn.functional as F
 
 from .. import _lib
-from ..functional import (SEMANTIC_MAX_K, SEMANTIC_MAX_M, gat_aggregate, next_attention_dropout,
-                          semantic_attention)
+from ..functional import (SEMANTIC_MAX_K, SEMANTIC_MAX_M, AttentionDropout, gat_aggregate, halo_exchange,
+                          next_attention_dropout, semantic_attention, semantic_attention_partitioned)
 from ..graph import CSRGraph, adj_cache
-from ..partition import PartitionedGraph
+from ..partition import PartitionedGraph, PartitionedMetapaths
 from .gat import GraphAttentionLayer, _fused_heads
 from . import gat as _gat
 
@@ -138,7 +138,57 @@ class HANLayer(nn.Module):
             z = F.elu(F.dropout(z, p, training=training))  # NodeAttention.py:60-62, all metapaths at once
         return z.view(n, M, H * Fp)
 
+    def _batched_partitioned(self, pm, h):
+        """`_batched` on this rank's row block of a PartitionedMetapaths (h = the own rows): the per-metapath h·W_m on
+        the own rows, ONE halo exchange of the stacked Wh, s of the own rows and t of all table rows, one batched-
+        rectangular attention launch (forward and backward) and semantic attention over the global node count.
+        Feature dropout (GATConv.dropout, NodeAttention.py:59-60) draws on the own rows; the attention dropout
+        (the heads' GraphAttentionLayer.dropout, NodeAttention.py:31 — equal to it when built by the constructor)
+        draws the whole set's mask for the block's edges."""
+        convs = list(self.gat_layers)
+        M = len(convs)
+        heads0 = list(convs[0].attentions)
+        H, Fp, alpha = len(heads0), heads0[0].out_features, heads0[0].alpha
+        lin = self.semantic_attention.project[0]
+        # the refusals depend on the replicated model and the features' dtype only: every rank raises together
+        if M != len(pm):
+            raise _lib.GnnError(f"HANLayer: {M} metapath models for {len(pm)} metapath graphs")
+        if any(c.num_class is not None for c in convs) or h.dtype != torch.float32 or H * Fp > 256 or \
+                M > SEMANTIC_MAX_M or lin.out_features > SEMANTIC_MAX_K:
+            raise _lib.GnnError("HANLayer on PartitionedMetapaths: needs num_class None, fp32 features, H*F' <= 256, "
+                                f"M <= {SEMANTIC_MAX_M} and a semantic hidden width <= {SEMANTIC_MAX_K} (got "
+                                f"{h.dtype}, H*F' = {H * Fp}, M = {M}, K = {lin.out_features})")
+        g, shift = pm.attention()
+        n = pm.n_local
+        p, p_att, training = convs[0].dropout, heads0[0].dropout, self.training
+        drop_active = training and p > 0.0
+        Ws = [torch.cat([hd.W for hd in conv.attentions], dim=1) for conv in convs]
+        Wh = torch.cat([torch.mm(F.dropout(h, p, training=True) if drop_active else h, W) for W in Ws], dim=1)
+        Wh = halo_exchange(pm.union, Wh)                                                         # [n_comb, M*H*Fp]
+        nc = Wh.shape[0]
+        a = torch.stack([torch.stack([hd.a[:, 0] for hd in conv.attentions]) for conv in convs])  # [M, H, 2*Fp]
+        Wh4 = Wh.view(nc, M, H, Fp).float()
+        s = (Wh4[:n] * a[None, :, :, :Fp].float()).sum(-1).permute(1, 0, 2).reshape(M * n, H)
+        t = (Wh4 * a[None, :, :, Fp:].float()).sum(-1).permute(1, 0, 2).reshape(M * nc, H)
+        keep = drop = None
+        if training and p_att > 0.0:
+            if _gat.EXPLICIT_DROPOUT_MASK:
+                keep = _gat.attention_keep_mask(g, H, p_att)
+            else:
+                d = next_attention_dropout(p_att, Wh.device)
+                drop = AttentionDropout(d.p, d.seed, d.seed_dev, slot_shift=shift)  # the whole set's mask
+        double_elu = not drop_active
+        z = gat_aggregate(g, Wh, s, t, H, Fp, alpha, mode=_lib.GAT_SOFTMAX, elu=2 if double_elu else 1, keep=keep,
+                          dropout=drop, batch=M)                                                 # [n, M*H*Fp]
+        if not double_elu:
+            z = F.elu(F.dropout(z, p, training=training))
+        sem = self.semantic_attention
+        return semantic_attention_partitioned(z.view(n, M, H * Fp), lin.weight, lin.bias, sem.project[2].weight,
+                                              pm.n_total, pm.world, pm.group)
+
     def forward(self, gs, h):
+        if isinstance(gs, PartitionedMetapaths):
+            return self._batched_partitioned(gs, h)
         if any(isinstance(g, PartitionedGraph) for g in gs):
             raise _lib.GnnError("HANLayer: metapath graphs on a PartitionedGraph are not supported (the batched "
                                 "metapath attention runs on one GPU)")
@@ -167,7 +217,11 @@ class HANModel(nn.Module):
         self.predict = nn.Linear(widths[-1], out_size)
 
     def forward(self, g, h):
-        graphs = [a if isinstance(a, PartitionedGraph) else adj_cache.get(a) for a in g]  # dense float64 masks -> CSR, once per graph
+        """g: the M metapath adjacencies, or a PartitionedMetapaths (h = this rank's rows; so is the result)."""
+        if isinstance(g, PartitionedMetapaths):
+            graphs = g
+        else:
+            graphs = [a if isinstance(a, PartitionedGraph) else adj_cache.get(a) for a in g]  # dense float64 masks -> CSR, once per graph
         for layer in self.layers:
             h = layer(graphs, h)
         return self.predict(h)

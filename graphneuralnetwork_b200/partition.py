@@ -1119,6 +1119,203 @@ class PartitionedGraph:
         self.ops = {}
 
 
+# ---- HAN's metapath graphs over one row partition ---------------------------------------------
+
+def union_block(rowptrs, cols, n_global: int):
+    """Per-row union of the columns of M row blocks over the same rows (GLOBAL column ids): the block whose halo
+    plan serves all M metapaths with one exchange.  Returns (rowptr, col int64), columns ascending per row."""
+    n_loc = int(rowptrs[0].numel()) - 1
+    dev = cols[0].device
+    keys = []
+    for rp, c in zip(rowptrs, cols):
+        rows = torch.repeat_interleave(torch.arange(n_loc, dtype=torch.int64, device=dev), rp[1:] - rp[:-1],
+                                       output_size=int(c.numel()))
+        keys.append(rows * n_global + c.to(torch.int64))
+    key = torch.unique(torch.cat(keys), sorted=True)
+    rowptr = torch.zeros(n_loc + 1, dtype=torch.int64, device=dev)
+    torch.cumsum(torch.bincount(key // n_global, minlength=n_loc), 0, out=rowptr[1:])
+    return rowptr, key % n_global
+
+
+@dataclass
+class MetapathView:
+    """This rank's row block of M metapath graphs in ONE combined column space, that of the union block's halo plan:
+    local column c -> c - lo, remote column -> n_local + its slot in the union halo.  The M renamed blocks are stacked
+    as a block diagonal (graph m's rows at m * n_local, its column ids at m * n_comb), which the batched-rectangular
+    attention kernels walk in one launch; every row keeps its metapath's global edge order.
+    slot_shift[m]: global batched edge slot (the block diagonal of the M whole graphs, as one GPU numbers them) minus
+    local batched slot, for graph m's edges — the seeded attention dropout of the block is then the whole set's."""
+    rowptr: torch.Tensor          # [M * n_local + 1]
+    col: torch.Tensor             # int32 batched combined column ids
+    n_graphs: int
+    n_local: int
+    n_comb: int                   # n_local + n_halo of the union plan
+    slot_shift: List[int]
+    any_empty_row: bool           # some row of some metapath, on any rank, has no edge
+    halo_rows_per_graph: List[int]  # distinct remote columns of each metapath's block (what it alone would fetch)
+
+    def require_edges(self):
+        """GAT's rule for a row without edges is the mean over ALL N nodes; the flag is global, so every rank raises
+        together."""
+        if self.any_empty_row:
+            raise _lib.GnnError("HAN on PartitionedMetapaths: a metapath graph has rows without edges (their output "
+                                "is the mean over all nodes, not supported across ranks); add self-loops")
+
+
+def build_metapath_view(plan: HaloPlan, rowptrs, cols, group=None) -> MetapathView:
+    """The view of M row blocks (rowptr over the rank's rows, GLOBAL column ids) in the combined column space of
+    `plan`, the union block's plan (its halo must hold every remote column of every block).  Collective when
+    world > 1: one all_gather of (per-metapath nnz, has-empty-row) per rank."""
+    lo, hi = plan.bounds[plan.rank], plan.bounds[plan.rank + 1]
+    n_loc, M = hi - lo, len(rowptrs)
+    n_comb = n_loc + plan.n_halo
+    dev = cols[0].device
+    halo_ids = plan.halo_ids.to(dev)
+    order = torch.argsort(halo_ids)
+    sorted_ids = halo_ids[order]
+    parts_rp, parts_col, halo_m, nnz_loc, off = [], [], [], [], 0
+    empty = False
+    for m, (rp, c) in enumerate(zip(rowptrs, cols)):
+        c64 = c.to(dev).to(torch.int64)
+        is_loc = (c64 >= lo) & (c64 < hi)
+        rem = c64[~is_loc]
+        pos = torch.searchsorted(sorted_ids, rem)
+        if rem.numel() and (sorted_ids.numel() == 0 or
+                            not torch.equal(sorted_ids[pos.clamp_max(sorted_ids.numel() - 1)], rem)):
+            raise ValueError("build_metapath_view: a remote column is missing from the plan's halo")
+        comb = torch.empty_like(c64)
+        comb[is_loc] = c64[is_loc] - lo
+        comb[~is_loc] = order[pos] + n_loc
+        parts_rp.append(rp.to(dev)[:-1] + off)
+        parts_col.append(comb + m * n_comb)
+        halo_m.append(int(torch.unique(rem).numel()))
+        nnz_loc.append(int(c.numel()))
+        off += int(c.numel())
+        empty = empty or (n_loc > 0 and bool((rp[1:] == rp[:-1]).any().item()))
+    parts_rp.append(torch.tensor([off], dtype=torch.int64, device=dev))
+    rowptr = torch.cat(parts_rp)
+    col = torch.cat(parts_col).to(torch.int32)
+    if plan.world > 1:
+        mine = torch.tensor(nnz_loc + [int(empty)], dtype=torch.int64, device=dev)
+        every = [torch.empty_like(mine) for _ in range(plan.world)]
+        dist.all_gather(every, mine, group=group)
+        every = [[int(x) for x in e.tolist()] for e in every]
+    else:
+        every = [nnz_loc + [int(empty)]]
+    nnz_glob = [sum(e[m] for e in every) for m in range(M)]
+    shift = []
+    for m in range(M):
+        before = sum(e[m] for e in every[:plan.rank])  # the whole graph m's rowptr[lo]
+        shift.append(sum(nnz_glob[k] - nnz_loc[k] for k in range(m)) + before)
+    return MetapathView(rowptr, col, M, n_loc, n_comb, shift, any(e[M] for e in every), halo_m)
+
+
+class PartitionedMetapaths:
+    """This rank's share of HAN's M metapath graphs over the same N nodes, row-partitioned, in the form
+    `HANModel.forward(pm, X_local)` takes (X_local = the rank's own rows).  A sequence of length M, as the list of
+    graphs it replaces.
+
+    The row bounds are common to all metapaths, balanced on Σ_m rowptr_m (every rank's attention work is the sum over
+    the metapaths).  ONE halo serves them all: `union`, a `PartitionedGraph` over the per-row union of the M blocks'
+    columns, whose operators exchange the stacked Wh_local [n_local, M*H*F'] once per layer (`widths` lists every
+    layer's M*H*F').  The union moves some rows for metapaths that do not read them: `halo_rows` against
+    `halo_rows_per_graph` (Σ over the metapaths) shows that cost.  `attention()` is the batched block in the union's
+    combined column space (MetapathView) and the per-graph dropout slot shifts.
+
+    Collective construction; the lock-step rule of PartitionedGraph holds.  Constructors: from the rank's own row
+    blocks (rowptr over its rows, GLOBAL column ids) or `from_global(graphs, ...)` for graphs every rank holds."""
+
+    def __init__(self, rowptrs, cols, bounds: List[int], rank: int, world: int, widths, device=None, group=None,
+                 **kw):
+        if not 1 <= len(rowptrs) == len(cols):
+            raise ValueError("PartitionedMetapaths: one (rowptr, col) block per metapath")
+        dev = torch.device(device) if device is not None else cols[0].device
+        rowptrs = [r.to(dev) for r in rowptrs]
+        cols = [c.to(dev) for c in cols]
+        self.n_total = int(bounds[-1])
+        rp_u, col_u = union_block(rowptrs, cols, max(self.n_total, 1))
+        self.union = PartitionedGraph(rp_u, col_u, None, bounds, rank, world, widths, device=dev, group=group, **kw)
+        try:
+            self._view = build_metapath_view(self.union.plan, rowptrs, cols, group)
+        except Exception:
+            self.union.close()
+            raise
+        self.rank, self.world, self.group, self.bounds = self.union.rank, self.union.world, group, self.union.bounds
+        self._graph = None
+        self._shift = None
+
+    @classmethod
+    def from_global(cls, graphs, rank: int, world: int, widths, group=None, **kw) -> "PartitionedMetapaths":
+        """From M whole `CSRGraph`s over the same N nodes that every rank holds: bounds balanced on Σ_m rowptr_m."""
+        graphs = list(graphs)
+        n = graphs[0].n_rows
+        if any(g.n_rows != n or g.n_cols != n for g in graphs):
+            raise ValueError("PartitionedMetapaths: square metapath graphs over the same nodes")
+        bounds = balanced_bounds(sum(g.rowptr for g in graphs), world)
+        lo, hi = bounds[rank], bounds[rank + 1]
+        rows = torch.arange(lo, hi, dtype=torch.int64, device=graphs[0].rowptr.device)
+        blocks = [select_rows(g.rowptr, g.col, None, rows)[:2] for g in graphs]
+        return cls([b[0] for b in blocks], [b[1] for b in blocks], bounds, rank, world, widths,
+                   device=kw.pop("device", graphs[0].rowptr.device), group=group, **kw)
+
+    def __len__(self) -> int:
+        return self._view.n_graphs
+
+    def __getitem__(self, m: int):
+        """Metapath m's block in the combined column space: (rowptr [n_local + 1], int32 col in [0, n_comb))."""
+        v = self._view
+        if not 0 <= m < v.n_graphs:
+            raise IndexError(m)
+        r = v.n_local
+        rp = v.rowptr[m * r:(m + 1) * r + 1]
+        return rp - rp[0], v.col[int(rp[0]):int(rp[-1])] - m * v.n_comb
+
+    @property
+    def n_local(self) -> int:
+        return self.union.n_local
+
+    @property
+    def row_range(self):
+        return self.union.row_range
+
+    @property
+    def halo_rows(self) -> int:
+        return self.union.plan.n_halo
+
+    @property
+    def halo_rows_per_graph(self) -> List[int]:
+        return list(self._view.halo_rows_per_graph)
+
+    @property
+    def slot_shift(self) -> List[int]:
+        return list(self._view.slot_shift)
+
+    def op(self, F: int) -> PartitionedSpmm:
+        return self.union.op(F)
+
+    def attention(self):
+        """(batched CSRGraph [M*n_local, M*n_comb] in the combined column space, device int64 [M] slot shifts) for the
+        batched-rectangular attention kernels.  Raises on every rank when some metapath row has no edge."""
+        from .graph import CSRGraph
+        self._view.require_edges()
+        if self._graph is None:
+            v = self._view
+            g = CSRGraph(v.rowptr, v.col, None, v.n_graphs * v.n_local, v.n_graphs * v.n_comb)
+            g.transpose()      # built once with the block: the backward's pass 2 walks it
+            g.gat_long_rows()
+            g.transpose().gat_long_rows()
+            self._graph = g
+            self._shift = torch.tensor(v.slot_shift, dtype=torch.int64, device=v.rowptr.device)
+        return self._graph, self._shift
+
+    def local_index(self, idx_global: torch.Tensor) -> torch.Tensor:
+        return self.union.local_index(idx_global)
+
+    def close(self):
+        """Free the union's peer buffers (collective: every rank calls it)."""
+        self.union.close()
+
+
 # ---- a feature table sharded across ranks ---------------------------------------------------
 _TABLE_DTYPES = {torch.float32: 4, torch.bfloat16: 2}
 

@@ -441,6 +441,49 @@ int gnn_gat_fused_bwd_ex_f32(const int64_t* rowptr, const int32_t* col,
                              const int64_t* long_rows_t, int64_t n_long_t, int64_t long_threshold,
                              int apply_elu, float* d_pre, const gnn_gat_dropout* dropout /*nullable*/,
                              gnn_stream_t stream);
+
+/* Batched AND rectangular graphs (fp32): a rank's row block of HAN's M metapath graphs, each renamed into one shared
+ * combined column space of cols_per_graph >= rows_per_graph table rows ([own rows ; halo rows]).  The CSR is the
+ * block diagonal of the M blocks: n = n_graphs*rows_per_graph rows, row r = graph r / rows_per_graph, and graph m's
+ * column ids lie in [m*cols_per_graph, (m+1)*cols_per_graph), addressing row c - m*cols_per_graph of Wh's column block
+ * m.  Wh is [cols_per_graph, ldw] and t [n_graphs*cols_per_graph, H]; s, the row statistics and d_s are
+ * [n_graphs*rows_per_graph, H]; out / out_pre / d_out are [rows_per_graph, ldo] with graph m's columns at m*H*Fp;
+ * d_Wh / d_t follow Wh / t.  The backward's transposed CSR has n_graphs*cols_per_graph rows (transposed row r is
+ * graph r / cols_per_graph).
+ * slot_shift (device int64 [n_graphs], nullable): the seeded dropout of graph m's local edge slot e is the one of slot
+ * e + slot_shift[m] (after any edge_slot_base), so a row block draws exactly the mask of the whole batched graph
+ * (on one GPU: Σ_{m'<m} nnz_{m'} + rowptr_m[lo] - the block's own first slot of graph m).  An explicit edge_keep
+ * mask is in local slots.  Every row must have an edge (the rule for an empty row needs all N nodes).
+ * struct_size = sizeof(gnn_gat_batch); 1 <= n_graphs <= 32, H*Fp <= 256.  With cols_per_graph == rows_per_graph and
+ * no shift these entries compute the same bits as gnn_gat_fused_{fwd_train,bwd}_f32 with batch_nodes. */
+typedef struct gnn_gat_batch {
+  int32_t struct_size;
+  int32_t n_graphs;
+  int64_t rows_per_graph;
+  int64_t cols_per_graph;
+  const int64_t* slot_shift;
+} gnn_gat_batch;
+int gnn_gat_fused_fwd_batch_f32(const int64_t* rowptr, const int32_t* col, const float* Wh, int64_t ldw,
+                                const float* s, const float* t, int64_t nnz, int32_t H, int32_t Fp,
+                                float alpha, int mode, int apply_elu,
+                                const float* edge_keep, const gnn_gat_dropout* dropout,
+                                float* out_pre, float* out_act /*nullable when apply_elu == 0*/, int64_t ldo,
+                                float* row_max, float* row_sum,
+                                const int64_t* long_rows, int64_t n_long, int64_t long_threshold,
+                                const gnn_gat_batch* batch, gnn_stream_t stream);
+int gnn_gat_fused_bwd_batch_f32(const int64_t* rowptr, const int32_t* col,
+                                const int64_t* rowptr_t, const int32_t* col_t, const int64_t* perm_t /*nullable*/,
+                                const float* Wh, int64_t ldw, const float* s, const float* t,
+                                const float* row_max, const float* row_sum,
+                                const float* out_pre, const float* d_out, int64_t ldo,
+                                int32_t H, int32_t Fp, float alpha, int mode,
+                                const float* edge_keep,
+                                float* d_Wh, int64_t ld_dwh, float* d_s, float* d_t, float* row_scratch,
+                                int64_t nnz,
+                                const int64_t* long_rows, int64_t n_long,
+                                const int64_t* long_rows_t, int64_t n_long_t, int64_t long_threshold,
+                                int apply_elu, float* d_pre, const gnn_gat_dropout* dropout /*nullable*/,
+                                const gnn_gat_batch* batch, gnn_stream_t stream);
 /* bf16-feature variants (north_star: "bf16-feature variants within 1e-2"): Wh, out, out_pre, d_out and
  * d_Wh are bf16; the scores s/t, the softmax statistics and every accumulation stay fp32.
  * Same reference call site (GAT/models/layers.py:22-37). */
@@ -493,6 +536,24 @@ int gnn_semantic_scores_bwd_f32(const float* P, int64_t ldp, const float* bias, 
                                 const float* d_scores_over_n, int64_t N, int32_t M, int32_t K,
                                 float* dP, int64_t lddp, float* dq /*[K]*/, float* dbias /*[K]*/,
                                 void* workspace, int64_t workspace_bytes, gnn_stream_t stream);
+/* The two node sums split at the rank boundary (rows of one rank; N = its row count, 0 allowed): the caller adds
+ * the ranks' [M] partials in rank order and finalizes with the GLOBAL node count n_total.  With one part, partial +
+ * finalize computes the same bits as the fused entry.
+ *   scores_partial:   sums[m] = sum_n sum_k q[k] tanh(P[n*M+m, k] + bias[k]) (the fused entry's sum before / N)
+ *   scores_finalize:  scores = sums / n_total, beta = softmax_M(scores)
+ *   combine_bwd_partial:  dz[n, m, :] = beta[m] d_out[n, :], dbeta[m] = sum_n <d_out[n], z[n, m]>
+ *   combine_bwd_finalize: d_scores_over_n[m] = beta[m] (dbeta[m] - sum_j beta[j] dbeta[j]) / n_total
+ * gnn_semantic_scores_bwd_f32 then takes d_scores_over_n over the rank's rows (its dq / dbias are the rank's share). */
+int gnn_semantic_scores_partial_f32(const float* P, int64_t ldp, const float* bias, const float* q, int64_t N,
+                                    int32_t M, int32_t K, float* sums /*[M]*/, void* workspace,
+                                    int64_t workspace_bytes, gnn_stream_t stream);
+int gnn_semantic_scores_finalize_f32(const float* sums, int64_t n_total, int32_t M, float* scores, float* beta,
+                                     gnn_stream_t stream);
+int gnn_semantic_combine_bwd_partial_f32(const float* d_out, const float* z, const float* beta, int64_t N, int32_t M,
+                                         int32_t D, float* dz, float* dbeta /*[M]*/, void* workspace,
+                                         int64_t workspace_bytes, gnn_stream_t stream);
+int gnn_semantic_combine_bwd_finalize_f32(const float* dbeta, const float* beta, int64_t n_total, int32_t M,
+                                          float* d_scores_over_n, gnn_stream_t stream);
 
 /* ---- synthetic graphs for the benchmark shapes (SURVEY.md §8d) ---------------- */
 /* Power-law CSR generated on the device, row by row, from a counter-based hash of
