@@ -129,6 +129,36 @@ struct VecIO<__nv_bfloat16, 8> {
   }
 };
 
+// The first n columns of a VEC-wide vector of a row (n counts from p to the row's F): a whole vector when it lies
+// inside the F columns, else element by element.  A row's last, partial vector thus never touches the caller's
+// columns past F (a padded or sliced output's neighbours), and the accumulate load reads none of them.
+template <typename T, int VEC>
+__device__ __forceinline__ void store_cols(T* p, const float (&v)[VEC], int n) {
+  if (n >= VEC) {
+    VecIO<T, VEC>::store(p, v);
+    return;
+  }
+#pragma unroll
+  for (int i = 0; i < VEC; ++i)
+    if (i < n) {
+      const float o[1] = {v[i]};
+      VecIO<T, 1>::store(p + i, o);
+    }
+}
+template <typename T, int VEC>
+__device__ __forceinline__ void load_cols(const T* p, float (&v)[VEC], int n) {
+  if (n >= VEC) {
+    VecIO<T, VEC>::load(p, v);
+    return;
+  }
+#pragma unroll
+  for (int i = 0; i < VEC; ++i) {
+    float o[1] = {0.f};
+    if (i < n) VecIO<T, 1>::load(p + i, o);
+    v[i] = o[0];
+  }
+}
+
 // ---- raw (still packed) vector staging: keeps bf16 rows at half the registers while the
 // gathers are in flight; unpacked only when they are consumed --------------------------------
 template <typename T, int VEC>

@@ -74,7 +74,11 @@ __global__ void __launch_bounds__(kRowReduceThreads) row_reduce_kernel(const Row
     float v = 0.f;
     if (k < e) {
       if (a.col32) c = __ldg(a.col32 + k);
-      else if (a.col64) c = (int32_t)__ldg(a.col64 + k);
+      else if (a.col64) {
+        // an id outside int32 is invalid (>= every table's rows): -1, not its low 32 bits, which may name a real row
+        const int64_t c64 = __ldg(a.col64 + k);
+        c = (c64 >= 0 && c64 <= 0x7fffffffLL) ? (int32_t)c64 : -1;
+      }
       else c = (int32_t)k;
       if (a.src_div > 0 && c >= 0) c /= a.src_div;
       if (a.src_mul > 0 && c >= 0) c = c * a.src_mul + (int32_t)(row % a.src_mul);
@@ -129,7 +133,7 @@ __global__ void __launch_bounds__(kRowReduceThreads) row_reduce_kernel(const Row
       float o[VEC];
 #pragma unroll
       for (int i = 0; i < VEC; ++i) o[i] = (OP == 1) ? acc[ch][i] : acc[ch][i] * a.scale;
-      VecIO<T, VEC>::store(yr + col0, o);
+      store_cols<T, VEC>(yr + col0, o, a.F - col0);  // columns >= F stay untouched
       if (OP == 1 && a.argmax) {
 #pragma unroll
         for (int i = 0; i < VEC; ++i)

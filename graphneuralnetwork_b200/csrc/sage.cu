@@ -345,7 +345,7 @@ __global__ void __launch_bounds__(kSageThreads, (sage_min_ctas<T, NV, OP, SH>())
                   }
               }
             } else if (a.out_vec16[b]) {
-              VecIO<T, E>::store(orow + col0, o);
+              store_cols<T, E>(orow + col0, o, a.F - col0);  // columns >= F stay untouched
             } else {
 #pragma unroll
               for (int i = 0; i < E; ++i)

@@ -114,15 +114,15 @@ __global__ void __launch_bounds__(kSpmmThreads, MINB) spmm_rbs_kernel(const Spmm
 #pragma unroll
     for (int ch = 0; ch < CHUNKS; ++ch) {
       const int col0 = (gl + ch * GROUP) * VEC;
-      if (col0 < a.F) {
+      if (col0 < a.F) {  // columns >= F of Y are neither read nor written
         if (accum) {
           float prev[VEC];
-          VecIO<T, VEC>::load(yr + col0, prev);
+          load_cols<T, VEC>(yr + col0, prev, a.F - col0);
 #pragma unroll
           for (int i = 0; i < VEC; ++i) acc[ch][i] += prev[i];
         }
         if (EPI && (!SKIP || (r0 + r) >= a.epi_skip)) spmm_epilogue<VEC>(acc[ch], a.bias, a.relu, col0, a.F);
-        VecIO<T, VEC>::store(yr + col0, acc[ch]);
+        store_cols<T, VEC>(yr + col0, acc[ch], a.F - col0);
       }
 #pragma unroll
       for (int i = 0; i < VEC; ++i) acc[ch][i] = 0.f;
