@@ -77,6 +77,14 @@ SIGNATURES = {
     "gnn_gat_fused_bwd_batch_f32": (cint, [ptr, ptr, ptr, ptr, ptr, ptr, i64, ptr, ptr, ptr, ptr, ptr, ptr, i64, i32,
                                            i32, f32, cint, ptr, ptr, i64, ptr, ptr, ptr, i64, ptr, i64, ptr, i64, i64,
                                            cint, ptr, ptr, ptr, ptr]),
+    "gnn_gat_fused_bwd_ex_bf16": (cint, [ptr, ptr, ptr, ptr, ptr, ptr, i64, ptr, ptr, ptr, ptr, ptr, ptr, i64, i64, i64,
+                                         i32, i32, f32, cint, ptr, ptr, i64, ptr, ptr, ptr, i64, ptr, i64, ptr, i64, i64,
+                                         cint, ptr, ptr, ptr]),
+    "gnn_gat_fused_fwd_batch_bf16": (cint, [ptr, ptr, ptr, i64, ptr, ptr, i64, i32, i32, f32, cint, cint, ptr, ptr, ptr,
+                                            ptr, i64, ptr, ptr, ptr, i64, i64, ptr, ptr]),
+    "gnn_gat_fused_bwd_batch_bf16": (cint, [ptr, ptr, ptr, ptr, ptr, ptr, i64, ptr, ptr, ptr, ptr, ptr, ptr, i64, i32,
+                                            i32, f32, cint, ptr, ptr, i64, ptr, ptr, ptr, i64, ptr, i64, ptr, i64, i64,
+                                            cint, ptr, ptr, ptr, ptr]),
     "gnn_gat_fused_fwd_train_f32": (cint, [ptr, ptr, ptr, i64, ptr, ptr, i64, i64, i32, i32, f32, cint, cint, ptr, ptr,
                                            ptr, ptr, ptr, i64, ptr, ptr, ptr, i64, i64, i64, ptr]),
     "gnn_gat_fused_fwd_train_bf16": (cint, [ptr, ptr, ptr, i64, ptr, ptr, i64, i64, i32, i32, f32, cint, cint, ptr, ptr,

@@ -883,13 +883,12 @@ int gat_fwd_impl(const int64_t* rowptr, const int32_t* col, const T* Wh, int64_t
   const int cpl = (HF + 31) / 32;
   GNN_REQUIRE(n_long == 0 || (long_rows && long_threshold > 0), GNN_ERR_BAD_ARG, "inconsistent long-row list");
   if (rb) {
-    if constexpr (sizeof(T) == 4) {
-      a.col_stride = rb->cols_per_graph;
-      a.slot_shift = rb->slot_shift;
-      return gat_fwd_schedule<T, true>(a, cpl, n, nnz, long_rows, n_long, long_threshold, st);
-    }
+    // packed bf16 (PK = 2): graph gm's columns start at gm * HF (even, since Fp is) and its rows move by whole
+    // rows of even ldw / ldo, so every staged 32-bit word stays 4-byte aligned under the RB offsets
+    a.col_stride = rb->cols_per_graph;
+    a.slot_shift = rb->slot_shift;
+    return gat_fwd_schedule<T, true>(a, cpl, n, nnz, long_rows, n_long, long_threshold, st);
   }
-  GNN_REQUIRE(!rb, GNN_ERR_UNSUPPORTED, "batched rectangular graphs are fp32 only");
   return gat_fwd_schedule<T, false>(a, cpl, n, nnz, long_rows, n_long, long_threshold, st);
 }
 
@@ -1061,13 +1060,10 @@ int gat_bwd_impl(const int64_t* rowptr, const int32_t* col, const int64_t* rowpt
   a.rowptr = rowptr;
   a.col = col;
   if (rb) {
-    GNN_REQUIRE(sizeof(T) == 4, GNN_ERR_UNSUPPORTED, "batched rectangular graphs are fp32 only");
-    if constexpr (sizeof(T) == 4) {
-      a.col_stride = rb->cols_per_graph;
-      a.slot_shift = rb->slot_shift;
-      return gat_bwd_passes<T, true>(a, cplr, n, n_cols, nnz, rowptr_t, col_t, perm_t, long_rows, n_long, long_rows_t,
-                                     n_long_t, long_threshold, st);
-    }
+    a.col_stride = rb->cols_per_graph;
+    a.slot_shift = rb->slot_shift;
+    return gat_bwd_passes<T, true>(a, cplr, n, n_cols, nnz, rowptr_t, col_t, perm_t, long_rows, n_long, long_rows_t,
+                                   n_long_t, long_threshold, st);
   }
   return gat_bwd_passes<T, false>(a, cplr, n, n_cols, nnz, rowptr_t, col_t, perm_t, long_rows, n_long, long_rows_t,
                                   n_long_t, long_threshold, st);
@@ -1196,6 +1192,21 @@ int gnn_gat_fused_bwd_ex_f32(const int64_t* rowptr, const int32_t* col, const in
                              d_pre, dropout, 0);
 }
 
+int gnn_gat_fused_bwd_ex_bf16(const int64_t* rowptr, const int32_t* col, const int64_t* rowptr_t, const int32_t* col_t,
+                              const int64_t* perm_t, const void* Wh, int64_t ldw, const float* s, const float* t,
+                              const float* row_max, const float* row_sum, const void* out_pre, const void* d_out,
+                              int64_t ldo, int64_t n_rows, int64_t n_cols, int32_t H, int32_t Fp, float alpha, int mode,
+                              const float* edge_keep, void* d_Wh, int64_t ld_dwh, float* d_s, float* d_t,
+                              float* row_scratch, int64_t nnz, const int64_t* long_rows, int64_t n_long,
+                              const int64_t* long_rows_t, int64_t n_long_t, int64_t long_threshold, int apply_elu,
+                              void* d_pre, const gnn_gat_dropout* dropout, gnn_stream_t stream) {
+  return gat_bwd_impl<__nv_bfloat16>(rowptr, col, rowptr_t, col_t, perm_t, (const __nv_bfloat16*)Wh, ldw, s, t, row_max,
+                                     row_sum, (const __nv_bfloat16*)out_pre, (const __nv_bfloat16*)d_out, ldo, n_rows,
+                                     n_cols, H, Fp, alpha, mode, edge_keep, (__nv_bfloat16*)d_Wh, ld_dwh, d_s, d_t,
+                                     row_scratch, nnz, long_rows, n_long, long_rows_t, n_long_t, long_threshold,
+                                     (cudaStream_t)stream, apply_elu, (__nv_bfloat16*)d_pre, dropout, 0);
+}
+
 int gnn_gat_fused_fwd_batch_f32(const int64_t* rowptr, const int32_t* col, const float* Wh, int64_t ldw,
                                 const float* s, const float* t, int64_t nnz, int32_t H, int32_t Fp, float alpha,
                                 int mode, int apply_elu, const float* edge_keep, const gnn_gat_dropout* dropout,
@@ -1227,6 +1238,44 @@ int gnn_gat_fused_bwd_batch_f32(const int64_t* rowptr, const int32_t* col, const
                              n, n_cols, H, Fp, alpha, mode, edge_keep, d_Wh, ld_dwh, d_s, d_t, row_scratch, nnz,
                              long_rows, n_long, long_rows_t, n_long_t, long_threshold, (cudaStream_t)stream, apply_elu,
                              d_pre, dropout, batch->rows_per_graph, batch);
+}
+
+int gnn_gat_fused_fwd_batch_bf16(const int64_t* rowptr, const int32_t* col, const void* Wh, int64_t ldw,
+                                 const float* s, const float* t, int64_t nnz, int32_t H, int32_t Fp, float alpha,
+                                 int mode, int apply_elu, const float* edge_keep, const gnn_gat_dropout* dropout,
+                                 void* out_pre, void* out_act, int64_t ldo, float* row_max, float* row_sum,
+                                 const int64_t* long_rows, int64_t n_long, int64_t long_threshold,
+                                 const gnn_gat_batch* batch, gnn_stream_t stream) {
+  int64_t n = 0, n_cols = 0;
+  int rc = check_batch(batch, &n, &n_cols);
+  if (rc != GNN_OK) return rc;
+  GNN_REQUIRE(out_act || apply_elu == 0, GNN_ERR_BAD_ARG, "apply_elu > 0 needs out_act");
+  if (n == 0) return GNN_OK;
+  return gat_fwd_impl<__nv_bfloat16>(rowptr, col, (const __nv_bfloat16*)Wh, ldw, s, t, n, nnz, H, Fp, alpha, mode,
+                                     apply_elu, nullptr, edge_keep, (__nv_bfloat16*)out_pre, ldo, row_max, row_sum,
+                                     long_rows, n_long, long_threshold, (cudaStream_t)stream,
+                                     apply_elu > 0 ? (__nv_bfloat16*)out_act : nullptr, dropout, batch->rows_per_graph,
+                                     batch);
+}
+
+int gnn_gat_fused_bwd_batch_bf16(const int64_t* rowptr, const int32_t* col, const int64_t* rowptr_t,
+                                 const int32_t* col_t, const int64_t* perm_t, const void* Wh, int64_t ldw,
+                                 const float* s, const float* t, const float* row_max, const float* row_sum,
+                                 const void* out_pre, const void* d_out, int64_t ldo, int32_t H, int32_t Fp,
+                                 float alpha, int mode, const float* edge_keep, void* d_Wh, int64_t ld_dwh, float* d_s,
+                                 float* d_t, float* row_scratch, int64_t nnz, const int64_t* long_rows, int64_t n_long,
+                                 const int64_t* long_rows_t, int64_t n_long_t, int64_t long_threshold, int apply_elu,
+                                 void* d_pre, const gnn_gat_dropout* dropout, const gnn_gat_batch* batch,
+                                 gnn_stream_t stream) {
+  int64_t n = 0, n_cols = 0;
+  int rc = check_batch(batch, &n, &n_cols);
+  if (rc != GNN_OK) return rc;
+  return gat_bwd_impl<__nv_bfloat16>(rowptr, col, rowptr_t, col_t, perm_t, (const __nv_bfloat16*)Wh, ldw, s, t, row_max,
+                                     row_sum, (const __nv_bfloat16*)out_pre, (const __nv_bfloat16*)d_out, ldo, n, n_cols,
+                                     H, Fp, alpha, mode, edge_keep, (__nv_bfloat16*)d_Wh, ld_dwh, d_s, d_t,
+                                     row_scratch, nnz, long_rows, n_long, long_rows_t, n_long_t, long_threshold,
+                                     (cudaStream_t)stream, apply_elu, (__nv_bfloat16*)d_pre, dropout,
+                                     batch->rows_per_graph, batch);
 }
 
 }  // extern "C"

@@ -255,17 +255,32 @@ class _PartitionedGcnAggregateFn(torch.autograd.Function):
         dZ = dZ.contiguous()
         # always run: the backward exchange is a collective every rank takes part in
         dS = ctx.op.backward(dZ)
-        db = dZ.sum(dim=0) if (ctx.has_bias and ctx.needs_input_grad[1]) else None
+        db = dZ.sum(dim=0, dtype=torch.float32) if (ctx.has_bias and ctx.needs_input_grad[1]) else None  # bias is fp32
         return (dS if ctx.needs_input_grad[0] else None), db, None, None
+
+
+_DTYPE_NAME = {torch.float32: "fp32", torch.bfloat16: "bf16"}
+
+
+def require_partition_dtype(pg, X: torch.Tensor, what: str):
+    """A partition's peer buffers are built for one feature dtype (`pg.dtype`, the `dtype=` of its constructor): a
+    tensor of another dtype is refused.  The refusal depends on the dtypes only, so every rank raises together."""
+    if X.dtype != pg.dtype:
+        name = _DTYPE_NAME.get(pg.dtype, str(pg.dtype))
+        raise _lib.GnnError(f"{what}: the partition was built for {name} features "
+                            f"(dtype={pg.dtype}), got {X.dtype}")
 
 
 def partitioned_gcn_aggregate(pg, S: torch.Tensor, bias: Optional[torch.Tensor] = None,
                               relu: bool = False) -> torch.Tensor:
     """relu?(Â·S + bias)[own rows] with autograd into S and bias, over a partition.PartitionedGraph `pg`; S = the
-    rank's own rows (fp32).  Collective: every rank calls it, and its backward, in the same order."""
+    rank's own rows, of the partition's dtype (fp32 or bf16); the bias is applied in fp32 (cast as in
+    `gcn_aggregate`) and its gradient reduced in fp32.  Collective: every rank calls it, and its backward, in the same
+    order."""
     _require_cuda(S, bias)
-    if S.dtype != torch.float32 or (bias is not None and bias.dtype != torch.float32):
-        raise _lib.GnnError("partitioned_gcn_aggregate: fp32 features and bias expected")
+    require_partition_dtype(pg, S, "partitioned_gcn_aggregate")
+    if bias is not None and bias.dtype != torch.float32:
+        bias = bias.float()
     if S.dim() != 2 or S.shape[0] != pg.n_local:
         raise _lib.GnnError(f"partitioned_gcn_aggregate: S must be [{pg.n_local}, F] (this rank's rows), "
                             f"got {tuple(S.shape)}")
@@ -288,13 +303,13 @@ class _HaloExchangeFn(torch.autograd.Function):
 
 
 def halo_exchange(pg, X_local: torch.Tensor) -> torch.Tensor:
-    """[X_local ; halo] ([n_local + n_halo, F], fp32) over a partition.PartitionedGraph `pg`: the table whose rows the
-    combined column ids of `pg.attention()` address, as a private copy (its backward needs the halo rows after
-    later exchanges may have reused the peer buffer).  Collective, with autograd: every rank calls it, and its
-    backward, in the same order."""
+    """[X_local ; halo] ([n_local + n_halo, F], the partition's dtype: fp32 or bf16) over a partition.PartitionedGraph
+    `pg`: the table whose rows the combined column ids of `pg.attention()` address, as a private copy (its backward
+    needs the halo rows after later exchanges may have reused the peer buffer).  Collective, with autograd: every
+    rank calls it, and its backward, in the same order.  In bf16 the halo rows travel as bf16 and the returned
+    gradient rows are bf16 partials that the owner adds in fp32, rounding once per row (PartitionedSpmm)."""
     _require_cuda(X_local)
-    if X_local.dtype != torch.float32:
-        raise _lib.GnnError("halo_exchange: fp32 features expected")
+    require_partition_dtype(pg, X_local, "halo_exchange")
     if X_local.dim() != 2 or X_local.shape[0] != pg.n_local:
         raise _lib.GnnError(f"halo_exchange: X_local must be [{pg.n_local}, F] (this rank's rows), "
                             f"got {tuple(X_local.shape)}")
@@ -690,8 +705,8 @@ def gat_fwd_raw(g: CSRGraph, Wh, s, t, H, Fp, alpha, mode=_lib.GAT_SOFTMAX, elu=
     batch = M > 1: `g` is the block diagonal of M graphs over the same N nodes (CSRGraph.block_diagonal), Wh / out are
     [N, M*H*Fp] (graph m's columns at m*H*Fp), s / t are [M*N, H] (batched-row major) — HAN's metapaths in one launch.
     Rectangular `g` (n_cols > n_rows, a row block whose columns address [own rows ; halo rows]): Wh and t have n_cols
-    rows, s and out n_rows; fp32, H*Fp <= 256 and no row without edges.  With batch = M > 1 as well, `g` is the block
-    diagonal of M such blocks over one combined table (partition.PartitionedMetapaths.attention): Wh is
+    rows, s and out n_rows; fp32 or bf16, H*Fp <= 256 and no row without edges.  With batch = M > 1 as well, `g` is
+    the block diagonal of M such blocks over one combined table (partition.PartitionedMetapaths.attention): Wh is
     [n_cols / M, M*H*Fp], t [n_cols, H], s [n_rows, H], out [n_rows / M, M*H*Fp]; `dropout.slot_shift` moves each
     graph's dropout slots."""
     _require_cuda(Wh, s, t, keep)
@@ -708,8 +723,8 @@ def gat_fwd_raw(g: CSRGraph, Wh, s, t, H, Fp, alpha, mode=_lib.GAT_SOFTMAX, elu=
             or t.shape != (nc, H)):
         raise _lib.GnnError(f"gat: Wh {tuple(Wh.shape)} / s {tuple(s.shape)} / t {tuple(t.shape)} do not match graph "
                             f"rows={n}, cols={nc}, batch={M}, H*Fp={H * Fp}")
-    if nc != n and (H * Fp > 256 or Wh.dtype != torch.float32):
-        raise _lib.GnnError("gat: a rectangular graph (table rows != rows) takes fp32 features and H*Fp <= 256")
+    if nc != n and H * Fp > 256:
+        raise _lib.GnnError("gat: a rectangular graph (table rows != rows) takes H*Fp <= 256")
     if M > 1 and H * Fp > 256:
         raise _lib.GnnError("gat: batched graphs need H*Fp <= 256 per graph")
     if out is None:
@@ -730,17 +745,16 @@ def gat_fwd_raw(g: CSRGraph, Wh, s, t, H, Fp, alpha, mode=_lib.GAT_SOFTMAX, elu=
     f32 = Wh.dtype == torch.float32
     import ctypes as C
     if _batched_rect(g, M, dropout):
-        # batched and rectangular: one fp32 group, the training entry (it writes the activated form to out_act)
-        if Wh.dtype != torch.float32:
-            raise _lib.GnnError("gat: batched rectangular graphs take fp32 features")
+        # batched and rectangular: one group, the training entry (it writes the activated form to out_act)
         pre_buf, act_buf = (out, out_act) if (out_act is not None or elu == 0) else (torch.empty_like(out), out)
         dstruct = dropout.c_struct() if (dropout is not None and dropout.p > 0.0) else None
         bstruct = _batch_struct(M, nodes, nc // M, dropout)
-        _lib.check(lib.gnn_gat_fused_fwd_batch_f32(
+        fb = lib.gnn_gat_fused_fwd_batch_f32 if f32 else lib.gnn_gat_fused_fwd_batch_bf16
+        _lib.check(fb(
             _p(g.rowptr), _p(g.col), _p(Wh), _ld(Wh), _p(s), _p(t), g.nnz, H, Fp, float(alpha), mode,
             elu if act_buf is not None else 0, _p(keep), C.byref(dstruct) if dstruct is not None else None,
             _p(pre_buf), _p(act_buf), _ld(out), _p(row_max), _p(row_sum), _p(lr), lr.numel(), thr, C.byref(bstruct),
-            _stream_ptr()), "gnn_gat_fused_fwd_batch_f32")
+            _stream_ptr()), "gnn_gat_fused_fwd_batch")
         return out, row_max, row_sum
     train = out_act is not None or (dropout is not None and dropout.p > 0.0)
     pre_buf, act_buf = out, out_act
@@ -852,24 +866,27 @@ class _GatFn(torch.autograd.Function):
         groups = list(_gat_groups(H, Fp))
         esz = Wh.element_size()
         need_perm = keep is not None or drop is not None
-        if _batched_rect(g, M, drop):  # batched and rectangular (one fp32 group, no empty row: checked by the forward)
+        f32 = Wh.dtype == torch.float32
+        if _batched_rect(g, M, drop):  # batched and rectangular (one group, no empty row: checked by the forward)
             row_scratch = torch.empty((n, 4, H), dtype=torch.float32, device=dev)
             bstruct = _batch_struct(M, n // M, nc // M, drop)
-            _lib.check(lib.gnn_gat_fused_bwd_batch_f32(
+            fb = lib.gnn_gat_fused_bwd_batch_f32 if f32 else lib.gnn_gat_fused_bwd_batch_bf16
+            _lib.check(fb(
                 _p(g.rowptr), _p(g.col), _p(gt.rowptr), _p(gt.col), _p(g.perm_t) if need_perm else None, _p(Wh), _ld(Wh),
                 _p(s), _p(t), _p(row_max), _p(row_sum), _p(out), _p(d_out), _ld(out), H, Fp, alpha, mode,
                 _p(keep), _p(d_Wh), _ld(d_Wh), _p(d_s), _p(d_t), _p(row_scratch), g.nnz, _p(lr), lr.numel(), _p(lrt),
                 lrt.numel(), thr, elu, _p(d_pre), C.byref(dstruct) if dstruct is not None else None, C.byref(bstruct),
-                _stream_ptr()), "gnn_gat_fused_bwd_batch_f32")
+                _stream_ptr()), "gnn_gat_fused_bwd_batch")
             groups = []
-        elif nc != n:  # rectangular (one fp32 group, checked by the forward): table rows get d_Wh / d_t
+        elif nc != n:  # rectangular (one group, checked by the forward): table rows get d_Wh / d_t
             row_scratch = torch.empty((n, 4, H), dtype=torch.float32, device=dev)
-            _lib.check(lib.gnn_gat_fused_bwd_ex_f32(
+            fx = lib.gnn_gat_fused_bwd_ex_f32 if f32 else lib.gnn_gat_fused_bwd_ex_bf16
+            _lib.check(fx(
                 _p(g.rowptr), _p(g.col), _p(gt.rowptr), _p(gt.col), _p(g.perm_t) if need_perm else None, _p(Wh), _ld(Wh),
                 _p(s), _p(t), _p(row_max), _p(row_sum), _p(out), _p(d_out), _ld(out), n, nc, H, Fp, alpha, mode,
                 _p(keep), _p(d_Wh), _ld(d_Wh), _p(d_s), _p(d_t), _p(row_scratch), g.nnz, _p(lr), lr.numel(), _p(lrt),
                 lrt.numel(), thr, elu, _p(d_pre), C.byref(dstruct) if dstruct is not None else None, _stream_ptr()),
-                "gnn_gat_fused_bwd_ex_f32")
+                "gnn_gat_fused_bwd_ex")
             groups = []
         for gi, (h0, h1, f0, f1) in enumerate(groups):
             whole = len(groups) == 1

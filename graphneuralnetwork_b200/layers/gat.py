@@ -13,7 +13,8 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from .. import _lib
-from ..functional import attention_keep_mask, gat_aggregate, halo_exchange, next_attention_dropout, spmm_values
+from ..functional import (attention_keep_mask, gat_aggregate, halo_exchange, next_attention_dropout,
+                          require_partition_dtype, spmm_values)
 from ..graph import CSRGraph, adj_cache
 from ..partition import PartitionedGraph
 
@@ -94,11 +95,12 @@ def _fused_heads_partitioned(x, pg, Ws, a_srcs, a_dsts, alpha, mode, elu, dropou
     """`_fused_heads` on this rank's row block: Wh of the own rows, the halo rows' Wh from their owners
     (functional.halo_exchange), s of the own rows, t of all table rows, and the fused kernels over the block in the
     combined column space.  The backward returns d Wh of the halo rows (from the aggregation and from t) to their
-    owners; d a_src / d a_dst are this rank's share, summed over the ranks by partition.allreduce_gradients."""
+    owners; d a_src / d a_dst are this rank's share, summed over the ranks by partition.allreduce_gradients.
+    x has the partition's dtype (fp32 or bf16); s / t are fp32 from the same expression as `_fused_heads`, so one rank
+    computes the bits of one GPU in either dtype."""
     H = len(Ws)
     Fp = Ws[0].shape[1]
-    if x.dtype != torch.float32:
-        raise _lib.GnnError(f"GAT on a PartitionedGraph: fp32 features only (got {x.dtype})")
+    require_partition_dtype(pg, x, "GAT on a PartitionedGraph")
     if H * Fp > 256:
         raise _lib.GnnError(f"GAT on a PartitionedGraph: H*F' = {H * Fp} exceeds the 256 columns of one fused "
                             "attention call")
@@ -108,8 +110,8 @@ def _fused_heads_partitioned(x, pg, Ws, a_srcs, a_dsts, alpha, mode, elu, dropou
     Wh3 = Wh.view(-1, H, Fp)
     a_src = a_srcs[0].view(1, Fp) if H == 1 else torch.stack(list(a_srcs), dim=0)
     a_dst = a_dsts[0].view(1, Fp) if H == 1 else torch.stack(list(a_dsts), dim=0)
-    s = (Wh3[:pg.n_local] * a_src.unsqueeze(0)).sum(-1)  # [n_local, H]
-    t = (Wh3 * a_dst.unsqueeze(0)).sum(-1)               # [n_local + n_halo, H]
+    s = (Wh3[:pg.n_local].float() * a_src.float().unsqueeze(0)).sum(-1)  # [n_local, H]
+    t = (Wh3.float() * a_dst.float().unsqueeze(0)).sum(-1)               # [n_local + n_halo, H]
     keep = drop = None
     if training and dropout > 0.0:
         if EXPLICIT_DROPOUT_MASK:

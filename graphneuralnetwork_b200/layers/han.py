@@ -23,7 +23,8 @@ import torch.nn.functional as F
 
 from .. import _lib
 from ..functional import (SEMANTIC_MAX_K, SEMANTIC_MAX_M, AttentionDropout, gat_aggregate, halo_exchange,
-                          next_attention_dropout, semantic_attention, semantic_attention_partitioned)
+                          next_attention_dropout, require_partition_dtype, semantic_attention,
+                          semantic_attention_partitioned)
 from ..graph import CSRGraph, adj_cache
 from ..partition import PartitionedGraph, PartitionedMetapaths
 from .gat import GraphAttentionLayer, _fused_heads
@@ -144,7 +145,12 @@ class HANLayer(nn.Module):
         rectangular attention launch (forward and backward) and semantic attention over the global node count.
         Feature dropout (GATConv.dropout, NodeAttention.py:59-60) draws on the own rows; the attention dropout
         (the heads' GraphAttentionLayer.dropout, NodeAttention.py:31 — equal to it when built by the constructor)
-        draws the whole set's mask for the block's edges."""
+        draws the whole set's mask for the block's edges.
+        h has the partition's dtype (fp32 or bf16).  In bf16 the halo exchange moves bf16 rows and the node-level
+        attention runs in the bf16 batched-rectangular kernels; the split semantic kernels are fp32 only, so they take
+        z and the projection weights as fp32 views (autograd casts the gradients back) and the result is cast to h's
+        dtype.  This differs from the 1-GPU bf16 HAN, whose semantic attention is the plain torch formula in bf16:
+        the two agree to bf16 tolerance, not bit for bit."""
         convs = list(self.gat_layers)
         M = len(convs)
         heads0 = list(convs[0].attentions)
@@ -153,11 +159,12 @@ class HANLayer(nn.Module):
         # the refusals depend on the replicated model and the features' dtype only: every rank raises together
         if M != len(pm):
             raise _lib.GnnError(f"HANLayer: {M} metapath models for {len(pm)} metapath graphs")
-        if any(c.num_class is not None for c in convs) or h.dtype != torch.float32 or H * Fp > 256 or \
+        require_partition_dtype(pm, h, "HANLayer on PartitionedMetapaths")
+        if any(c.num_class is not None for c in convs) or H * Fp > 256 or \
                 M > SEMANTIC_MAX_M or lin.out_features > SEMANTIC_MAX_K:
-            raise _lib.GnnError("HANLayer on PartitionedMetapaths: needs num_class None, fp32 features, H*F' <= 256, "
+            raise _lib.GnnError("HANLayer on PartitionedMetapaths: needs num_class None, H*F' <= 256, "
                                 f"M <= {SEMANTIC_MAX_M} and a semantic hidden width <= {SEMANTIC_MAX_K} (got "
-                                f"{h.dtype}, H*F' = {H * Fp}, M = {M}, K = {lin.out_features})")
+                                f"H*F' = {H * Fp}, M = {M}, K = {lin.out_features})")
         g, shift = pm.attention()
         n = pm.n_local
         p, p_att, training = convs[0].dropout, heads0[0].dropout, self.training
@@ -183,8 +190,10 @@ class HANLayer(nn.Module):
         if not double_elu:
             z = F.elu(F.dropout(z, p, training=training))
         sem = self.semantic_attention
-        return semantic_attention_partitioned(z.view(n, M, H * Fp), lin.weight, lin.bias, sem.project[2].weight,
-                                              pm.n_total, pm.world, pm.group)
+        b1 = None if lin.bias is None else lin.bias.float()
+        out = semantic_attention_partitioned(z.view(n, M, H * Fp).float(), lin.weight.float(), b1,
+                                             sem.project[2].weight.float(), pm.n_total, pm.world, pm.group)
+        return out.to(h.dtype)
 
     def forward(self, gs, h):
         if isinstance(gs, PartitionedMetapaths):

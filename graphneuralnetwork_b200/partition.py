@@ -1004,7 +1004,9 @@ class PartitionedSpmm:
 
     def _return_add(self, out: torch.Tensor):
         """out[r] += the received rows of local row r, in (peer, slot) order; frees the receive buffer for the
-        peers' next step."""
+        peers' next step.  bf16: the partial rows travel as bf16, and out[r] plus its received rows is summed in fp32
+        and rounded once per row (the accumulating SpMM row flush) — the 1-GPU bf16 rule of fp32 accumulation with
+        one rounding at the end, applied to the owner's add."""
         from .functional import spmm_ex
         if self._R.n_rows > 0:
             spmm_ex(self._R, self.back, out, row_map=self._R._row_map, accumulate=True)
@@ -1047,6 +1049,7 @@ class PartitionedGraph:
                  **op_kw):
         self.bounds, self.rank, self.world, self.group = [int(b) for b in bounds], int(rank), int(world), group
         self.dev = torch.device(device) if device is not None else col.device
+        self.dtype = dtype  # the feature dtype of every operator and exchange (fp32 or bf16)
         widths = sorted({int(w) for w in widths})
         if not widths or widths[0] <= 0:
             raise ValueError("PartitionedGraph: at least one positive feature width is needed")
@@ -1277,6 +1280,10 @@ class PartitionedMetapaths:
     @property
     def row_range(self):
         return self.union.row_range
+
+    @property
+    def dtype(self) -> torch.dtype:
+        return self.union.dtype
 
     @property
     def halo_rows(self) -> int:
@@ -1518,20 +1525,30 @@ def broadcast_parameters(module: torch.nn.Module, group=None):
 
 def allreduce_gradients(module: torch.nn.Module, group=None):
     """SUM every parameter's .grad over the ranks: one all_reduce of the gradients flattened in parameter order
-    (a missing .grad counts as zeros).  Call between backward() and optimizer.step()."""
+    (a missing .grad counts as zeros).  Call between backward() and optimizer.step().
+    When any gradient is narrower than fp32 (a bf16 model), the flattened gradients are reduced in fp32 (or wider, if
+    some gradient is) and each sum is rounded once to its parameter's dtype: a bf16 ring sum would round at every hop.
+    A model whose gradients are all fp32 (or all fp64) is reduced as is."""
     params = [p for p in module.parameters() if p.requires_grad]
     if not params:
         return
-    flat = torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).reshape(-1) for p in params])
+    grads = [(p.grad if p.grad is not None else torch.zeros_like(p)).reshape(-1) for p in params]
+    if all(g.dtype.itemsize >= 4 for g in grads):
+        flat = torch.cat(grads)
+    else:
+        acc = torch.float32
+        for g in grads:
+            acc = torch.promote_types(acc, g.dtype)
+        flat = torch.cat([g.to(acc) for g in grads])
     dist.all_reduce(flat, group=group)
     off = 0
     for p in params:
         n = p.numel()
         g = flat[off:off + n].view_as(p)
         if p.grad is None:
-            p.grad = g.clone()
+            p.grad = g.to(p.dtype, copy=True)
         else:
-            p.grad.copy_(g)
+            p.grad.copy_(g)  # rounds once when the gradient is not fp32
         off += n
 
 

@@ -442,7 +442,7 @@ int gnn_gat_fused_bwd_ex_f32(const int64_t* rowptr, const int32_t* col,
                              int apply_elu, float* d_pre, const gnn_gat_dropout* dropout /*nullable*/,
                              gnn_stream_t stream);
 
-/* Batched AND rectangular graphs (fp32): a rank's row block of HAN's M metapath graphs, each renamed into one shared
+/* Batched AND rectangular graphs (fp32; bf16 below): a rank's row block of HAN's M metapath graphs, each renamed into one shared
  * combined column space of cols_per_graph >= rows_per_graph table rows ([own rows ; halo rows]).  The CSR is the
  * block diagonal of the M blocks: n = n_graphs*rows_per_graph rows, row r = graph r / rows_per_graph, and graph m's
  * column ids lie in [m*cols_per_graph, (m+1)*cols_per_graph), addressing row c - m*cols_per_graph of Wh's column block
@@ -507,6 +507,46 @@ int gnn_gat_fused_bwd_bf16(const int64_t* rowptr, const int32_t* col,
                            const int64_t* long_rows_t, int64_t n_long_t, int64_t long_threshold,
                            int apply_elu, void* d_pre, const gnn_gat_dropout* dropout, int64_t batch_nodes,
                            gnn_stream_t stream);
+/* bf16 rectangular and batched-rectangular forms (a rank's row block of a bf16 PartitionedGraph /
+ * PartitionedMetapaths): the same argument lists and semantics as gnn_gat_fused_bwd_ex_f32 and
+ * gnn_gat_fused_{fwd,bwd}_batch_f32, with the feature buffers bf16.  The non-batched rectangular forward is
+ * gnn_gat_fused_fwd{,_train}_bf16 itself (Wh and t are read only through col).  With cols_per_graph ==
+ * rows_per_graph and no shift the batched entries compute the same bits as gnn_gat_fused_{fwd_train,bwd}_bf16 with
+ * batch_nodes. */
+int gnn_gat_fused_bwd_ex_bf16(const int64_t* rowptr, const int32_t* col,
+                              const int64_t* rowptr_t, const int32_t* col_t, const int64_t* perm_t /*nullable*/,
+                              const void* Wh, int64_t ldw, const float* s, const float* t,
+                              const float* row_max, const float* row_sum,
+                              const void* out_pre, const void* d_out, int64_t ldo,
+                              int64_t n_rows, int64_t n_cols, int32_t H, int32_t Fp, float alpha, int mode,
+                              const float* edge_keep,
+                              void* d_Wh, int64_t ld_dwh, float* d_s, float* d_t, float* row_scratch,
+                              int64_t nnz,
+                              const int64_t* long_rows, int64_t n_long,
+                              const int64_t* long_rows_t, int64_t n_long_t, int64_t long_threshold,
+                              int apply_elu, void* d_pre, const gnn_gat_dropout* dropout /*nullable*/,
+                              gnn_stream_t stream);
+int gnn_gat_fused_fwd_batch_bf16(const int64_t* rowptr, const int32_t* col, const void* Wh, int64_t ldw,
+                                 const float* s, const float* t, int64_t nnz, int32_t H, int32_t Fp,
+                                 float alpha, int mode, int apply_elu,
+                                 const float* edge_keep, const gnn_gat_dropout* dropout,
+                                 void* out_pre, void* out_act /*nullable when apply_elu == 0*/, int64_t ldo,
+                                 float* row_max, float* row_sum,
+                                 const int64_t* long_rows, int64_t n_long, int64_t long_threshold,
+                                 const gnn_gat_batch* batch, gnn_stream_t stream);
+int gnn_gat_fused_bwd_batch_bf16(const int64_t* rowptr, const int32_t* col,
+                                 const int64_t* rowptr_t, const int32_t* col_t, const int64_t* perm_t /*nullable*/,
+                                 const void* Wh, int64_t ldw, const float* s, const float* t,
+                                 const float* row_max, const float* row_sum,
+                                 const void* out_pre, const void* d_out, int64_t ldo,
+                                 int32_t H, int32_t Fp, float alpha, int mode,
+                                 const float* edge_keep,
+                                 void* d_Wh, int64_t ld_dwh, float* d_s, float* d_t, float* row_scratch,
+                                 int64_t nnz,
+                                 const int64_t* long_rows, int64_t n_long,
+                                 const int64_t* long_rows_t, int64_t n_long_t, int64_t long_threshold,
+                                 int apply_elu, void* d_pre, const gnn_gat_dropout* dropout /*nullable*/,
+                                 const gnn_gat_batch* batch, gnn_stream_t stream);
 
 /* ---- HAN semantic attention: everything around its one GEMM -------------------- */
 /* HAN/models/SemanticAttention.py:15-20:

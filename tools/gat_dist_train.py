@@ -3,7 +3,7 @@
 `partition.PartitionedGraph`, replicated weights, the global loss rule and one gradient all-reduce per step.
 One JSON line per rank and configuration on stdout.
 
-    torchrun --nproc-per-node N tools/gat_dist_train.py --check [--transports p2p ce nccl]
+    torchrun --nproc-per-node N tools/gat_dist_train.py --check [--dtype fp32|bf16] [--transports p2p ce nccl]
     torchrun --nproc-per-node N tools/gat_dist_train.py --time [--nodes 20000000] [--features 128 --heads 8 --hidden 8]
 
 --check (small graphs every rank holds, with self-loops: a Cora-like graph and a 200 k-row power-law graph; 8 heads x 8,
@@ -12,11 +12,13 @@ One JSON line per rank and configuration on stdout.
   repeated and must be bit-identical.  Feature dropout is off (`model.dropout = 0`); the attention dropout of the
   heads stays 0.6.  Both runs draw identical attention-dropout streams: the host seed (torch.manual_seed) and the
   per-device counters of functional._drop_counters are reset before every run, and each rank's block draws the
-  whole graph's mask for its edges (edge_slot_base).
+  whole graph's mask for its edges (edge_slot_base).  --dtype bf16: the model, the features and the partition are
+  bf16 and the 1-GPU model is the same seeded bf16 model, under gcn_dist_train.CHECK_BOUNDS["bf16"].
 --time (large power-law graph plus self-loops, each rank generates only its own row block): ms per training step
   (forward + backward + gradient all-reduce + Adam) and per forward, ms of the two halo exchanges alone
-  (`exchange_only`, widths H*F' and classes), and a float64 spot check of sampled first-layer output rows.  Device
-  name and power limit are read in the same run."""
+  (`exchange_only`, widths H*F' and classes), and a float64 spot check of sampled first-layer output rows.  The fp32
+  and the bf16 model are timed at the same size in one run, their steps alternated; one line per dtype with its halo
+  bytes and the peak memory of its step.  Device name and power limit are read in the same run."""
 import argparse
 import json
 import os
@@ -36,7 +38,7 @@ from graphneuralnetwork_b200.layers import GAT, SpGAT  # noqa: E402
 from graphneuralnetwork_b200.layers.gat import _fused_heads  # noqa: E402
 from graphneuralnetwork_b200.partition import (PartitionedGraph, allreduce_gradients, broadcast_parameters,  # noqa: E402
                                                global_count, partitioned_cross_entropy)
-from gcn_dist_train import device_info, rel  # noqa: E402
+from gcn_dist_train import DTYPES, check_metrics, device_info, halo_bytes, peak_step_gb, timed_ms  # noqa: E402
 
 MODELS = {"GAT": GAT, "SpGAT": SpGAT}
 
@@ -109,25 +111,26 @@ def run_check(a, rank, world, dev):
     for name, n, make, F_in in graphs:
         g = make()
         gen = torch.Generator().manual_seed(11)
-        X = (torch.rand(n, F_in, generator=gen) * 2 - 1).to(dev)
+        dt = DTYPES[a.dtype]
+        X = (torch.rand(n, F_in, generator=gen) * 2 - 1).to(dev).to(dt)
         labels = torch.randint(0, a.classes, (n,), generator=gen).to(dev)
         idx_train = torch.randperm(n, generator=gen)[: max(n * 2 // 5, 1)].sort().values.to(dev)
         for cls in a.models:
             torch.manual_seed(0)
-            ref = make_model(cls, F_in, a).to(dev)
+            ref = make_model(cls, F_in, a).to(dev).to(dt)
             init = {k: v.clone() for k, v in ref.state_dict().items()}
             reset_streams()
             r_logits, r_grads, r_w = train(ref, X, g, labels, idx_train, None, 3)
             for transport in (a.transports if world > 1 else ["none"]):
                 pg = PartitionedGraph.from_global(g, rank, world, widths=[a.heads * a.hidden, a.classes],
-                                                  transport=transport if world > 1 else "p2p")
+                                                  transport=transport if world > 1 else "p2p", dtype=dt)
                 lo, hi = pg.row_range
                 X_loc, y_loc = X[lo:hi].contiguous(), labels[lo:hi]
                 idx_loc = pg.local_index(idx_train)
                 n_train = global_count(idx_loc.numel(), dev) if world > 1 else idx_loc.numel()
                 runs = []
                 for _ in range(2):
-                    model = make_model(cls, F_in, a).to(dev)
+                    model = make_model(cls, F_in, a).to(dev).to(dt)
                     if rank == 0:
                         model.load_state_dict(init)
                     if world > 1:
@@ -140,15 +143,11 @@ def run_check(a, rank, world, dev):
                 line = {"mode": "check", "model": cls, "graph": name, "n": n, "nnz": g.nnz,
                         "widths": [F_in, a.heads * a.hidden, a.classes], "world": world, "rank": rank,
                         "transport": pg.ops[a.classes].transport, "edge_slot_base": pg.edge_slot_base,
-                        "n_halo": pg.plan.n_halo,
-                        "logits_rel_err": rel(logits, r_logits[lo:hi]),
-                        "grad_rel_err": max(rel(grads[k], r_grads[k]) for k in r_grads),
-                        "weights_rel_err": max(rel(w[k], r_w[k]) for k in r_w),
-                        "bitwise_repeat": bool(torch.equal(logits, logits_b)
-                                               and all(torch.equal(grads[k], grads_b[k]) for k in grads)
-                                               and all(torch.equal(w[k], w_b[k]) for k in w))}
-                line["ok"] = (line["logits_rel_err"] <= 1e-5 and line["grad_rel_err"] <= 2e-5
-                              and line["weights_rel_err"] <= 1e-4 and line["bitwise_repeat"])
+                        "n_halo": pg.plan.n_halo}
+                line.update(check_metrics(a.dtype, logits, r_logits[lo:hi], grads, r_grads, w, r_w,
+                                          torch.equal(logits, logits_b)
+                                          and all(torch.equal(grads[k], grads_b[k]) for k in grads)
+                                          and all(torch.equal(w[k], w_b[k]) for k in w)))
                 print(json.dumps(line), flush=True)
                 pg.close()
                 del pg, runs
@@ -181,81 +180,83 @@ def run_time(a, rank, world, dev):
     rp, cc = with_self_loops(csr0.rowptr, csr0.col, lo)
     del csr0
     csr = CSRGraph(rp, cc, None, n_loc, a.nodes)
-    X = S.hashed_feature_block(lo, hi, F_in, dev)
+    X32 = S.hashed_feature_block(lo, hi, F_in, dev)
     labels = (torch.arange(lo, hi, device=dev) * 2654435761 % C).to(torch.int64)
     idx_loc = torch.arange(0, n_loc, 3, device=dev)  # every third row trains
-    pg = PartitionedGraph(csr.rowptr, csr.col, None, bounds, rank, world, widths=[H * Fp, C], device=dev, waves=1,
-                          transport=a.transport)
-    torch.manual_seed(0)
-    model = GAT(F_in, Fp, C, 0.6, 0.2, H).to(dev)
-    model.dropout = 0.0
-    if world > 1:
-        broadcast_parameters(model)
     n_train = global_count(idx_loc.numel(), dev) if world > 1 else idx_loc.numel()
-    opt = torch.optim.Adam(model.parameters(), lr=0.005)
-
-    def step():
-        opt.zero_grad(set_to_none=True)
-        out = model(X, pg)
-        partitioned_cross_entropy(out[idx_loc], labels[idx_loc], n_train).backward()
+    runs = {}
+    for name in a.time_dtypes:
+        dt = DTYPES[name]
+        pg = PartitionedGraph(csr.rowptr, csr.col, None, bounds, rank, world, widths=[H * Fp, C], device=dev, waves=1,
+                              transport=a.transport, dtype=dt)
+        torch.manual_seed(0)
+        model = GAT(F_in, Fp, C, 0.6, 0.2, H).to(dev).to(dt)
+        model.dropout = 0.0
         if world > 1:
-            allreduce_gradients(model)
-        opt.step()
+            broadcast_parameters(model)
+        opt = torch.optim.Adam(model.parameters(), lr=0.005)
+        X = X32.to(dt)
 
-    def forward():
+        def step(model=model, opt=opt, X=X, pg=pg):
+            model.train()
+            opt.zero_grad(set_to_none=True)
+            out = model(X, pg)
+            partitioned_cross_entropy(out[idx_loc].float(), labels[idx_loc], n_train).backward()
+            if world > 1:
+                allreduce_gradients(model)
+            opt.step()
+
+        def forward(model=model, X=X, pg=pg):
+            model.train()
+            with torch.no_grad():
+                model(X, pg)
+
+        Wh1, Wh2 = torch.randn(n_loc, H * Fp, device=dev).to(dt), torch.randn(n_loc, C, device=dev).to(dt)
+
+        def exchange(pg=pg, Wh1=Wh1, Wh2=Wh2):
+            pg.op(H * Fp).exchange_only(Wh1)
+            pg.op(C).exchange_only(Wh2)
+
+        runs[name] = {"pg": pg, "model": model, "X": X, "step": step, "forward": forward, "exchange": exchange,
+                      "train_step_ms": [], "forward_ms": [], "exchange_only_ms": []}
+    for r in runs.values():  # warm every shape before the first timed window
+        r["step"]()
+        r["forward"]()
+    for _ in range(2):  # the dtypes alternate: fp32 steps, bf16 steps, fp32 steps, ...
+        for r in runs.values():
+            r["train_step_ms"].append(timed_ms(r["step"], a.steps, a.warmup, world, dev))
+            r["forward_ms"].append(timed_ms(r["forward"], a.steps, a.warmup, world, dev))
+            if world > 1:
+                r["exchange_only_ms"].append(timed_ms(r["exchange"], a.steps, a.warmup, world, dev))
+    rows = S.spmm_check_rows(csr, 256, 17 + rank)
+    for name, r in runs.items():
+        pg, model = r["pg"], r["model"]
+        r["peak_step_gb"] = peak_step_gb(r["step"], dev)
+        # float64 spot check of sampled first-layer rows (eval mode: no dropout)
+        model.eval()
+        heads = list(model.attentions)
         with torch.no_grad():
-            model(X, pg)
-
-    Wh1 = torch.randn(n_loc, H * Fp, device=dev)
-    Wh2 = torch.randn(n_loc, C, device=dev)
-
-    def exchange():
-        pg.op(H * Fp).exchange_only(Wh1)
-        pg.op(C).exchange_only(Wh2)
-
-    def timed(fn, steps, warmup):
-        for _ in range(warmup):
-            fn()
-        torch.cuda.synchronize()
-        if world > 1:
-            dist.barrier()
-        t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        t0.record()
-        for _ in range(steps):
-            fn()
-        t1.record()
-        torch.cuda.synchronize()
-        t = torch.tensor([t0.elapsed_time(t1) / steps], dtype=torch.float64, device=dev)
-        if world > 1:
-            dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return round(float(t.item()), 3)
-
-    step_ms = timed(step, a.steps, a.warmup)
-    model.train()
-    fwd_ms = timed(forward, a.steps, a.warmup)
-    exch_ms = timed(exchange, a.steps, a.warmup) if world > 1 else None
-    # float64 spot check of sampled first-layer rows (eval mode: no dropout)
-    model.eval()
-    heads = list(model.attentions)
-    with torch.no_grad():
-        halves = [h._halves() for h in heads]
-        Y1 = _fused_heads(X, pg, [h.W for h in heads], [x[0] for x in halves], [x[1] for x in halves], 0.2,
-                          model._mode, 1, 0.0, False)
-        rows = S.spmm_check_rows(csr, 256, 17 + rank)
-        W = torch.cat([h.W for h in heads], dim=1)
-        ref = layer1_reference(csr, rows, lo, W, torch.stack([x[0] for x in halves]), torch.stack([x[1] for x in halves]),
-                               H, Fp, F_in)
-        err = float((Y1[rows].double() - ref).abs().max().item()) / max(float(ref.abs().max().item()), 1e-30)
-    for o in pg.ops.values():
-        o.check_status()
-    line = {"mode": "time", "world": world, "rank": rank, **info, "n": a.nodes, "nnz": nnz_total + a.nodes,
-            "rows_local": n_loc, "widths": [F_in, H * Fp, C], "heads": H, "transport": a.transport,
-            "n_halo": pg.plan.n_halo, "edge_slot_base": pg.edge_slot_base,
-            "peak_mem_gb": round(torch.cuda.max_memory_allocated(dev) / 1e9, 2),
-            "train_step_ms": step_ms, "forward_ms": fwd_ms, "exchange_only_ms": exch_ms,
-            "layer1_sampled_rel_err": err, "layer1_ok": err <= 1e-5}
-    print(json.dumps(line), flush=True)
-    pg.close()
+            halves = [h._halves() for h in heads]
+            Y1 = _fused_heads(r["X"], pg, [h.W for h in heads], [x[0] for x in halves], [x[1] for x in halves], 0.2,
+                              model._mode, 1, 0.0, False)
+            W = torch.cat([h.W for h in heads], dim=1)
+            ref = layer1_reference(csr, rows, lo, W, torch.stack([x[0] for x in halves]),
+                                   torch.stack([x[1] for x in halves]), H, Fp, F_in)
+            err = float((Y1[rows].double() - ref).abs().max().item()) / max(float(ref.abs().max().item()), 1e-30)
+        for o in pg.ops.values():
+            o.check_status()
+        line = {"mode": "time", "dtype": name, "world": world, "rank": rank, **info, "n": a.nodes,
+                "nnz": nnz_total + a.nodes, "rows_local": n_loc, "widths": [F_in, H * Fp, C], "heads": H,
+                "transport": a.transport, "n_halo": pg.plan.n_halo, "edge_slot_base": pg.edge_slot_base,
+                "halo_bytes_per_exchange": halo_bytes(pg),
+                "peak_mem_gb": round(torch.cuda.max_memory_allocated(dev) / 1e9, 2), "peak_step_gb": r["peak_step_gb"],
+                "train_step_ms": min(r["train_step_ms"]), "forward_ms": min(r["forward_ms"]),
+                "exchange_only_ms": min(r["exchange_only_ms"]) if r["exchange_only_ms"] else None,
+                "rounds_ms": {k: r[k] for k in ("train_step_ms", "forward_ms", "exchange_only_ms")},
+                "layer1_sampled_rel_err": err, "layer1_ok": err <= (1e-5 if name == "fp32" else 1e-2)}
+        print(json.dumps(line), flush=True)
+    for r in runs.values():
+        r["pg"].close()
 
 
 def main():
@@ -274,6 +275,9 @@ def main():
     ap.add_argument("--classes", type=int, default=41)
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=2)
+    ap.add_argument("--dtype", choices=sorted(DTYPES), default="fp32", help="--check: the features' and model's dtype")
+    ap.add_argument("--time-dtypes", nargs="+", choices=sorted(DTYPES), default=["fp32", "bf16"],
+                    help="--time: the dtypes whose steps alternate in one run")
     a = ap.parse_args()
     rank, world, local = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0))
     dev = torch.device("cuda", local)

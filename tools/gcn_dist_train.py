@@ -3,18 +3,22 @@
 `partition.PartitionedGraph`, replicated weights, the global loss rule and one gradient all-reduce per step.
 One JSON line per rank and configuration on stdout.
 
-    torchrun --nproc-per-node N tools/gcn_dist_train.py --check [--transports p2p ce nccl] [--configs 1:auto 4:2 auto:auto]
+    torchrun --nproc-per-node N tools/gcn_dist_train.py --check [--dtype fp32|bf16] [--transports p2p ce nccl]
+                                                        [--configs 1:auto 4:2 auto:auto]
     torchrun --nproc-per-node N tools/gcn_dist_train.py --time [--nodes 20000000] [--features 128 --hidden 64 --classes 41]
 
 --check (small graphs every rank holds: a Cora-like graph and a 200 k-row power-law graph, odd widths, dropout 0):
   every rank also trains the same seeded GCN_Model on its GPU over the WHOLE graph and compares its own rows of the
   logits, every gradient at step 1 (after the all-reduce) and the weights after 3 Adam steps; the 3-step run is
-  repeated and must be bit-identical.
+  repeated and must be bit-identical.  --dtype bf16: the model, the features and the partition are bf16 and the 1-GPU
+  model is the same seeded bf16 model; the bounds are then bf16's (CHECK_BOUNDS).
 --time (large graph, each rank generates only its own row block, as bench.py's partitioned-SpMM config does): ms per
   training step (forward + backward + gradient all-reduce + Adam) and per forward, the schedule chosen, a float64
   spot check of sampled first-layer output rows, and the fused bias/ReLU epilogue against the unfused
-  `op.forward` + torch bias + ReLU on the same plan, alternated in one run.  Device name and power limit are read
-  in the same run."""
+  `op.forward` + torch bias + ReLU on the same plan, alternated in one run.  The fp32 and the bf16 model (features,
+  weights and partition in that dtype) are timed at the same size in one run, their steps alternated; one line per
+  dtype with its halo bytes and the peak memory of its step.  Device name and power limit are read in the same
+  run."""
 import argparse
 import json
 import os
@@ -45,6 +49,67 @@ def device_info(dev):
     except Exception as e:  # the numbers stay valid, their context is then incomplete
         info["power_limit"] = f"unavailable ({type(e).__name__})"
     return info
+
+
+DTYPES = {"fp32": torch.float32, "bf16": torch.bfloat16}
+# --check bounds per dtype.  fp32: max-normalised errors against the 1-GPU fp32 model.  bf16: logits 1e-2 and step-1
+# gradients 3e-2 (the bf16 tolerances of the single-GPU parity tests); the weights after 3 Adam steps are bounded in
+# norm, ‖w - w_ref‖₂ / ‖w_ref‖₂ <= 5e-2 over all parameters.  Adam's first steps move a weight by about lr whatever the
+# size of its gradient, so an entry whose gradient is near zero may step in opposite directions in two bf16 runs that
+# reduce in different orders: such entries set the max-normalised error (reported as weights_rel_err, up to
+# 2·steps·lr / max|w|) but contribute little to the norm.
+CHECK_BOUNDS = {"fp32": {"logits": 1e-5, "grad": 2e-5, "weights": 1e-4, "weights_norm": None},
+                "bf16": {"logits": 1e-2, "grad": 3e-2, "weights": None, "weights_norm": 5e-2}}
+
+
+def check_metrics(dtype, logits, r_logits, grads, r_grads, w, r_w, repeat):
+    """The --check fields of one run against the 1-GPU run, with `ok` under CHECK_BOUNDS[dtype]."""
+    b = CHECK_BOUNDS[dtype]
+    num = sum(float((w[k].double() - r_w[k].double()).pow(2).sum()) for k in r_w)
+    den = sum(float(r_w[k].double().pow(2).sum()) for k in r_w)
+    m = {"dtype": dtype, "logits_rel_err": rel(logits, r_logits),
+         "grad_rel_err": max(rel(grads[k], r_grads[k]) for k in r_grads),
+         "weights_rel_err": max(rel(w[k], r_w[k]) for k in r_w),
+         "weights_norm_rel_err": (num / max(den, 1e-300)) ** 0.5, "bitwise_repeat": bool(repeat)}
+    m["weights_bound"] = b["weights_norm"] if b["weights"] is None else b["weights"]
+    w_ok = (m["weights_rel_err"] <= b["weights"]) if b["weights"] is not None else \
+        (m["weights_norm_rel_err"] <= b["weights_norm"])
+    m["ok"] = m["logits_rel_err"] <= b["logits"] and m["grad_rel_err"] <= b["grad"] and w_ok and m["bitwise_repeat"]
+    return m
+
+
+def timed_ms(fn, steps, warmup, world, dev):
+    """Mean ms per call over `steps` calls after `warmup` (CUDA events; the slowest rank's figure)."""
+    for _ in range(warmup):
+        fn()
+    torch.cuda.synchronize()
+    if world > 1:
+        dist.barrier()
+    t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    t0.record()
+    for _ in range(steps):
+        fn()
+    t1.record()
+    torch.cuda.synchronize()
+    t = torch.tensor([t0.elapsed_time(t1) / steps], dtype=torch.float64, device=dev)
+    if world > 1:
+        dist.all_reduce(t, op=dist.ReduceOp.MAX)
+    return round(float(t.item()), 3)
+
+
+def peak_step_gb(fn, dev):
+    """Peak memory while `fn` runs, above what was allocated before it (GB): the step's own working set."""
+    torch.cuda.synchronize()
+    base = torch.cuda.memory_allocated(dev)
+    torch.cuda.reset_peak_memory_stats(dev)
+    fn()
+    torch.cuda.synchronize()
+    return round((torch.cuda.max_memory_allocated(dev) - base) / 1e9, 3)
+
+
+def halo_bytes(pg):
+    """Bytes one exchange moves into this rank, per feature width (forward; the gradient return moves as many)."""
+    return {str(F): op.halo_bytes_received if hasattr(op, "halo_bytes_received") else 0 for F, op in pg.ops.items()}
 
 
 def parse_config(cfg):
@@ -100,26 +165,28 @@ def run_check(a, rank, world, dev):
     for name, n, make, F_in in graphs:
         g = make()
         gen = torch.Generator().manual_seed(11)
-        X = (torch.rand(n, F_in, generator=gen) * 2 - 1).to(dev)
+        dt = DTYPES[a.dtype]
+        X = (torch.rand(n, F_in, generator=gen) * 2 - 1).to(dev).to(dt)
         labels = torch.randint(0, F_CLS, (n,), generator=gen).to(dev)
         idx_train = torch.randperm(n, generator=gen)[: max(n * 2 // 5, 1)].sort().values.to(dev)
         for layers in a.layers:
             torch.manual_seed(0)
-            ref = GCN_Model(F_in, F_HID, F_CLS, layers, 0.0).to(dev)
+            ref = GCN_Model(F_in, F_HID, F_CLS, layers, 0.0).to(dev).to(dt)
             init = {k: v.clone() for k, v in ref.state_dict().items()}
             r_logits, r_grads, r_w = train(ref, X, g, labels, idx_train, None, 3)
             for transport in (a.transports if world > 1 else ["none"]):
                 for cfg in (a.configs if world > 1 else ["1:auto"]):
                     K, c0 = parse_config(cfg)
                     pg = PartitionedGraph.from_global(g, rank, world, widths=[F_HID, F_CLS], waves=K,
-                                                      two_pass_chunks=c0, transport=transport if world > 1 else "p2p")
+                                                      two_pass_chunks=c0, transport=transport if world > 1 else "p2p",
+                                                      dtype=dt)
                     lo, hi = pg.row_range
                     X_loc, y_loc = X[lo:hi].contiguous(), labels[lo:hi]
                     idx_loc = pg.local_index(idx_train)
                     n_train = global_count(idx_loc.numel(), dev) if world > 1 else idx_loc.numel()
                     runs = []
                     for _ in range(2):
-                        model = GCN_Model(F_in, F_HID, F_CLS, layers, 0.0).to(dev)
+                        model = GCN_Model(F_in, F_HID, F_CLS, layers, 0.0).to(dev).to(dt)
                         if rank == 0:
                             model.load_state_dict(init)
                         if world > 1:
@@ -131,15 +198,11 @@ def run_check(a, rank, world, dev):
                     line = {"mode": "check", "graph": name, "n": n, "nnz": int(g.rowptr[-1].item()), "layers": layers,
                             "widths": [F_in, F_HID, F_CLS], "world": world, "rank": rank, "transport": pg.ops[F_HID].transport,
                             "config": cfg, "waves": pg.plan.waves, "two_pass_chunks": pg.plan.two_pass_chunks,
-                            "p1_epilogue_skip": 0 if pg.plan.p1 is None else pg.plan.p1.epilogue_skip,
-                            "logits_rel_err": rel(logits, r_logits[lo:hi]),
-                            "grad_rel_err": max(rel(grads[k], r_grads[k]) for k in r_grads),
-                            "weights_rel_err": max(rel(w[k], r_w[k]) for k in r_w),
-                            "bitwise_repeat": bool(torch.equal(logits, logits_b)
-                                                   and all(torch.equal(grads[k], grads_b[k]) for k in grads)
-                                                   and all(torch.equal(w[k], w_b[k]) for k in w))}
-                    line["ok"] = (line["logits_rel_err"] <= 1e-5 and line["grad_rel_err"] <= 2e-5
-                                  and line["weights_rel_err"] <= 1e-4 and line["bitwise_repeat"])
+                            "p1_epilogue_skip": 0 if pg.plan.p1 is None else pg.plan.p1.epilogue_skip}
+                    line.update(check_metrics(a.dtype, logits, r_logits[lo:hi], grads, r_grads, w, r_w,
+                                              torch.equal(logits, logits_b)
+                                              and all(torch.equal(grads[k], grads_b[k]) for k in grads)
+                                              and all(torch.equal(w[k], w_b[k]) for k in w)))
                     print(json.dumps(line), flush=True)
                     pg.close()
                     del pg, runs
@@ -154,68 +217,95 @@ def run_time(a, rank, world, dev):
     csr, bounds, nnz_total = build_rank_block(a.nodes, a.deg, rank, world, dev)
     lo, hi = bounds[rank], bounds[rank + 1]
     n_loc = hi - lo
-    X = S.hashed_feature_block(lo, hi, F_in, dev)
+    X32 = S.hashed_feature_block(lo, hi, F_in, dev)
     labels = (torch.arange(lo, hi, device=dev) * 2654435761 % C).to(torch.int64)
     idx_loc = torch.arange(0, n_loc, 3, device=dev)  # every third row trains
-    # footprint of one rank, 2 layers (4-byte elements): the CSR and its two transposes (backward), X, and per
-    # layer S = XWᵀ, Y (saved for the ReLU mask), their gradients and the halo buffers; the largest share is 1/world
+    n_train = global_count(idx_loc.numel(), dev) if world > 1 else idx_loc.numel()
     nnz_loc = int(csr.rowptr[-1].item())
     gb = lambda b: round(b / 1e9, 2)  # noqa: E731
-    foot = {"csr_gb": gb(nnz_loc * 8 + (n_loc + 1) * 8), "transposes_gb": gb(2 * (nnz_loc * 8 + (n_loc + 1) * 8)),
-            "x_gb": gb(n_loc * F_in * 4), "activations_gb": gb(n_loc * (4 * H + 4 * C) * 4)}
-    foot["total_gb"] = round(sum(foot.values()), 2)
-    pg = PartitionedGraph(csr.rowptr, csr.col, csr.val, bounds, rank, world, widths=[H, C], device=dev, waves=None,
-                          transport=a.transport)
-    torch.manual_seed(0)
-    model = GCN_Model(F_in, H, C, 2, 0.0).to(dev)
-    if world > 1:
-        broadcast_parameters(model)
-    n_train = global_count(idx_loc.numel(), dev) if world > 1 else idx_loc.numel()
-    opt = torch.optim.Adam(model.parameters(), lr=0.01)
-
-    def step():
-        opt.zero_grad(set_to_none=True)
-        out = model(X, pg)
-        partitioned_cross_entropy(out[idx_loc], labels[idx_loc], n_train).backward()
-        if world > 1:
-            allreduce_gradients(model)
-        opt.step()
-
-    def forward():
-        with torch.no_grad():
-            model(X, pg)
-
-    def timed(fn, steps, warmup):
-        for _ in range(warmup):
-            fn()
-        torch.cuda.synchronize()
-        if world > 1:
-            dist.barrier()
-        t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        t0.record()
-        for _ in range(steps):
-            fn()
-        t1.record()
-        torch.cuda.synchronize()
-        t = torch.tensor([t0.elapsed_time(t1) / steps], dtype=torch.float64, device=dev)
-        if world > 1:
-            dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return round(float(t.item()), 3)
-
-    step_ms = timed(step, a.steps, a.warmup)
-    fwd_ms = timed(forward, a.steps, a.warmup)
-    # float64 spot check of sampled first-layer rows: relu((Â·X)[rows] Wᵀ + b), Â·X recomputed from the global ids
-    layer0 = model.gcn_blocks.gcn0
-    with torch.no_grad():
-        Y1 = layer0(X, pg, fused_relu=True)
     rows = S.spmm_check_rows(csr, 2048, 17 + rank)
     ax = S.spmm_sampled_reference(csr, rows, F_in)  # the block's CSR holds global column ids
-    ref = torch.clamp_min(ax @ layer0.dense.weight.detach().double().T + layer0.bias.detach().double(), 0.0)
-    err = float((Y1[rows].double() - ref).abs().max().item()) / max(float(ref.abs().max().item()), 1e-30)
-    del csr, ax, ref
-    # fused epilogue vs op.forward + torch bias + ReLU on the same plan, alternating
-    op = pg.op(H)
-    Sx = layer0.dense(X).detach()
+    runs = {}
+    for name in a.time_dtypes:
+        dt = DTYPES[name]
+        esz = 4 if dt == torch.float32 else 2
+        # footprint of one rank, 2 layers: the CSR and its two transposes (backward), X, and per layer S = XWᵀ,
+        # Y (saved for the ReLU mask), their gradients and the halo buffers; the largest share is 1/world
+        foot = {"csr_gb": gb(nnz_loc * 8 + (n_loc + 1) * 8), "transposes_gb": gb(2 * (nnz_loc * 8 + (n_loc + 1) * 8)),
+                "x_gb": gb(n_loc * F_in * esz), "activations_gb": gb(n_loc * (4 * H + 4 * C) * esz)}
+        foot["total_gb"] = round(sum(foot.values()), 2)
+        pg = PartitionedGraph(csr.rowptr, csr.col, csr.val, bounds, rank, world, widths=[H, C], device=dev, waves=None,
+                              transport=a.transport, dtype=dt)
+        torch.manual_seed(0)
+        model = GCN_Model(F_in, H, C, 2, 0.0).to(dev).to(dt)
+        if world > 1:
+            broadcast_parameters(model)
+        opt = torch.optim.Adam(model.parameters(), lr=0.01)
+        X = X32.to(dt)
+
+        def step(model=model, opt=opt, X=X, pg=pg):
+            opt.zero_grad(set_to_none=True)
+            out = model(X, pg)
+            partitioned_cross_entropy(out[idx_loc].float(), labels[idx_loc], n_train).backward()
+            if world > 1:
+                allreduce_gradients(model)
+            opt.step()
+
+        def forward(model=model, X=X, pg=pg):
+            with torch.no_grad():
+                model(X, pg)
+
+        Sh, Sc = torch.randn(n_loc, H, device=dev).to(dt), torch.randn(n_loc, C, device=dev).to(dt)
+
+        def exchange(pg=pg, Sh=Sh, Sc=Sc):
+            pg.op(H).exchange_only(Sh)
+            pg.op(C).exchange_only(Sc)
+
+        runs[name] = {"pg": pg, "model": model, "X": X, "step": step, "forward": forward, "exchange": exchange,
+                      "foot": foot, "train_step_ms": [], "forward_ms": [], "exchange_only_ms": []}
+    for r in runs.values():  # warm every shape before the first timed window
+        r["step"]()
+        r["forward"]()
+    for _ in range(2):  # the dtypes alternate: fp32 steps, bf16 steps, fp32 steps, ...
+        for r in runs.values():
+            r["train_step_ms"].append(timed_ms(r["step"], a.steps, a.warmup, world, dev))
+            r["forward_ms"].append(timed_ms(r["forward"], a.steps, a.warmup, world, dev))
+            if world > 1:
+                r["exchange_only_ms"].append(timed_ms(r["exchange"], a.steps, a.warmup, world, dev))
+    for name, r in runs.items():
+        pg, model = r["pg"], r["model"]
+        r["peak_step_gb"] = peak_step_gb(r["step"], dev)
+        # float64 spot check of sampled first-layer rows: relu((Â·X)[rows] Wᵀ + b), Â·X recomputed from the global ids
+        layer0 = model.gcn_blocks.gcn0
+        with torch.no_grad():
+            Y1 = layer0(r["X"], pg, fused_relu=True)
+        ref = torch.clamp_min(ax @ layer0.dense.weight.detach().double().T + layer0.bias.detach().double(), 0.0)
+        err = float((Y1[rows].double() - ref).abs().max().item()) / max(float(ref.abs().max().item()), 1e-30)
+        for o in pg.ops.values():
+            o.check_status()
+        line = {"mode": "time", "dtype": name, "world": world, "rank": rank, **info, "n": a.nodes, "nnz": nnz_total,
+                "rows_local": n_loc, "widths": [F_in, H, C], "transport": a.transport, "waves": pg.plan.waves,
+                "two_pass_chunks": pg.plan.two_pass_chunks,
+                "p1_epilogue_skip": 0 if pg.plan.p1 is None else pg.plan.p1.epilogue_skip,
+                "halo_bytes_per_exchange": halo_bytes(pg), "footprint_rank": r["foot"],
+                "peak_mem_gb": round(torch.cuda.max_memory_allocated(dev) / 1e9, 2), "peak_step_gb": r["peak_step_gb"],
+                "train_step_ms": min(r["train_step_ms"]), "forward_ms": min(r["forward_ms"]),
+                "exchange_only_ms": min(r["exchange_only_ms"]) if r["exchange_only_ms"] else None,
+                "rounds_ms": {k: r[k] for k in ("train_step_ms", "forward_ms", "exchange_only_ms")},
+                "layer1_sampled_rel_err": err, "layer1_ok": err <= (1e-5 if name == "fp32" else 1e-2)}
+        print(json.dumps(line), flush=True)
+    if "fp32" in runs:
+        epilogue_ab(a, runs["fp32"], world, dev)
+    for r in runs.values():
+        r["pg"].close()
+
+
+def epilogue_ab(a, r, world, dev):
+    """The fused bias/ReLU epilogue against op.forward + torch bias + ReLU on the same fp32 plan, alternated."""
+    H = a.hidden
+    layer0 = r["model"].gcn_blocks.gcn0
+    op = r["pg"].op(H)
+    Sx = layer0.dense(r["X"]).detach()
     b = layer0.bias.detach()
 
     def fused():
@@ -227,20 +317,13 @@ def run_time(a, rank, world, dev):
 
     ab = {"fused_ms": [], "unfused_ms": []}
     for _ in range(3):
-        ab["fused_ms"].append(timed(fused, a.steps, 1))
-        ab["unfused_ms"].append(timed(unfused, a.steps, 1))
+        ab["fused_ms"].append(timed_ms(fused, a.steps, 1, world, dev))
+        ab["unfused_ms"].append(timed_ms(unfused, a.steps, 1, world, dev))
     yf, yu = op.forward(Sx, bias=b, relu=True), op.forward(Sx)
     yu = torch.relu(yu + b)
-    for o in pg.ops.values():
-        o.check_status()
-    line = {"mode": "time", "world": world, "rank": rank, **info, "n": a.nodes, "nnz": nnz_total, "rows_local": n_loc,
-            "widths": [F_in, H, C], "transport": a.transport, "waves": pg.plan.waves,
-            "two_pass_chunks": pg.plan.two_pass_chunks, "p1_epilogue_skip": 0 if pg.plan.p1 is None else pg.plan.p1.epilogue_skip,
-            "footprint_rank": foot, "peak_mem_gb": round(torch.cuda.max_memory_allocated(dev) / 1e9, 2),
-            "train_step_ms": step_ms, "forward_ms": fwd_ms, "layer1_sampled_rel_err": err,
-            "layer1_ok": err <= 1e-5, "epilogue_ab_ms": ab, "fused_vs_unfused_max_abs_diff": float((yf - yu).abs().max().item())}
-    print(json.dumps(line), flush=True)
-    pg.close()
+    print(json.dumps({"mode": "epilogue_ab", "dtype": "fp32", "world": world,
+                      "rank": dist.get_rank() if world > 1 else 0, "epilogue_ab_ms": ab, "fused_vs_unfused_max_abs_diff": float((yf - yu).abs().max().item())}),
+          flush=True)
 
 
 def main():
@@ -259,6 +342,9 @@ def main():
     ap.add_argument("--classes", type=int, default=41)
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=2)
+    ap.add_argument("--dtype", choices=sorted(DTYPES), default="fp32", help="--check: the features' and model's dtype")
+    ap.add_argument("--time-dtypes", nargs="+", choices=sorted(DTYPES), default=["fp32", "bf16"],
+                    help="--time: the dtypes whose steps alternate in one run")
     a = ap.parse_args()
     rank, world, local = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0))
     dev = torch.device("cuda", local)
