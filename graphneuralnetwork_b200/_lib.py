@@ -29,6 +29,11 @@ SIGNATURES = {
     "gnn_dense_mask_count_workspace_size": (size_t, [i64]),
     "gnn_dense_mask_count": (cint, [ptr, cint, i64, i64, i64, ptr, ptr, size_t, ptr]),
     "gnn_dense_mask_fill": (cint, [ptr, cint, i64, i64, i64, ptr, ptr, ptr]),
+    "gnn_pattern_product_count_workspace_size": (size_t, [i64]),
+    "gnn_pattern_product_count": (cint, [ptr, ptr, i64, i64, ptr, ptr, i64, i64, i64, cint, ptr, ptr, ptr, size_t,
+                                         ptr]),
+    "gnn_pattern_product_fill": (cint, [ptr, ptr, i64, i64, ptr, ptr, i64, i64, i64, cint, ptr, ptr, ptr, size_t,
+                                        ptr]),
     "gnn_csr_transpose_workspace_size": (size_t, [i64, i64, i64]),
     "gnn_csr_transpose": (cint, [ptr, ptr, ptr, i64, i64, i64, ptr, ptr, ptr, ptr, ptr, size_t, ptr]),
     "gnn_index_block_transpose_workspace_size": (size_t, [i64, i64]),

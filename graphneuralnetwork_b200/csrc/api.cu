@@ -49,6 +49,9 @@ static std::map<std::string, int>& tune_map() {
       {"gat.bwd_stage_edges", 64},  // edges staged per warp pass of the backward kernels
       {"gat.coop_min_avg_deg", 256},  // nnz/n at which every row gets a whole CTA
       {"gat.long_row", 1024},        // rows above this get a CTA in the otherwise warp-per-row schedule
+      {"metapath.small_max", 256},   // product rows with at most this many products: one warp sorts them (cap 256)
+      {"metapath.medium_max", 8192}, // ... at most this many: one CTA sorts them (cap 8192); longer rows: bitmap
+      {"metapath.tile_cols", 0},     // columns per bitmap tile of the hub-row path (0 = as many as shared memory holds)
   };
   return m;
 }

@@ -258,6 +258,94 @@ class CSRGraph:
                    "gnn_dense_mask_fill")
         return CSRGraph(rowptr, col, None, n_rows, n_cols)
 
+    @staticmethod
+    def pattern_product(A: "CSRGraph", B: "CSRGraph", row_range=None, self_loops: bool = False,
+                        max_nnz: Optional[int] = None, validate: bool = True,
+                        path_rows: Optional[torch.Tensor] = None) -> "CSRGraph":
+        """Pattern of A·B (values ignored), rows `row_range` = (lo, hi) of A (default all): row r lists, once each and
+        ascending, every column j some x connects, (lo + r, x) in A and (x, j) in B (gnn_pattern_product_count/fill).
+        That is scipy's ((A_bool @ B_bool) > 0) after sort_indices(), the metapath adjacency HAN builds densely
+        (HAN/utils/data_utils.py:85-89).  self_loops adds column i to row i (square products only).  Column ids
+        stay global.  One host read of nnz sizes `col`; nnz above `max_nnz` raises GnnError before it is allocated.
+        validate: ids outside A's or B's columns raise IndexError (one host read).  path_rows: an int64[3] CUDA
+        tensor that receives the rows each kernel path took (warp sort, CTA sort, bitmap)."""
+        lo, hi = _pattern_args(A, B, row_range, validate)
+        rowptr = _pattern_count(A, B, lo, hi, self_loops, path_rows)
+        nnz = int(rowptr[-1].item())  # one host read: nnz sizes the col array
+        if max_nnz is not None and nnz > max_nnz:
+            raise _lib.GnnError(f"pattern_product: the product has {nnz} entries, more than max_nnz = {max_nnz} "
+                                f"({4 * nnz + 8 * (hi - lo + 1)} bytes for col and rowptr)")
+        return CSRGraph(rowptr, _pattern_fill(A, B, lo, hi, self_loops, rowptr, nnz), None, hi - lo, B.n_cols)
+
+    @staticmethod
+    def metapath(R: "CSRGraph", self_loops: bool = False, max_nnz: Optional[int] = None) -> "CSRGraph":
+        """Metapath adjacency pattern(R·Rᵀ) of a relation R [N x X] (paper x author, paper x subject), with
+        `self_loops` the (R·Rᵀ + I) > 0 HAN trains on.  Rᵀ is R's cached `transpose()`."""
+        _require_ids_in_range(R)  # before the transpose, which sorts by column id
+        return CSRGraph.pattern_product(R, R.transpose(), self_loops=self_loops, max_nnz=max_nnz, validate=False)
+
+
+def _pattern_args(A: CSRGraph, B: CSRGraph, row_range, validate: bool):
+    """(lo, hi) of a pattern product after the checks the kernels rely on."""
+    _require_cuda(A.rowptr, B.rowptr)
+    if A.n_cols != B.n_rows:
+        raise ValueError(f"pattern_product: A is [{A.n_rows}, {A.n_cols}] but B has {B.n_rows} rows")
+    lo, hi = (0, A.n_rows) if row_range is None else (int(row_range[0]), int(row_range[1]))
+    if not 0 <= lo <= hi <= A.n_rows:
+        raise IndexError(f"pattern_product: row range [{lo}, {hi}) outside the {A.n_rows} rows of A")
+    if validate:
+        _require_ids_in_range(A, B)
+    return lo, hi
+
+
+def _require_ids_in_range(*graphs: CSRGraph) -> None:
+    """IndexError if a column id of one of `graphs` lies outside its columns (one host read)."""
+    bad = [((g.col < 0) | (g.col >= g.n_cols)).any() for g in graphs if g.nnz]
+    if bad and bool(torch.stack(bad).any().item()):
+        raise IndexError("pattern_product: a column id outside [0, n_cols) of " +
+                         " or ".join(f"a [{g.n_rows}, {g.n_cols}] graph" for g in graphs))
+
+
+def _col_or_dummy(g: CSRGraph) -> torch.Tensor:
+    # an empty tensor has no address; the kernels read no column of a graph without entries
+    return g.col if g.nnz else torch.zeros(1, dtype=torch.int32, device=g.device)
+
+
+def _pattern_ws(n_rows: int, dev) -> torch.Tensor:
+    return torch.empty(_lib.load().gnn_pattern_product_count_workspace_size(n_rows), dtype=torch.uint8, device=dev)
+
+
+def _pattern_count(A: CSRGraph, B: CSRGraph, lo: int, hi: int, self_loops: bool,
+                   path_rows: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """int64 rowptr [hi - lo + 1] of rows [lo, hi) of pattern(A·B) (no host read)."""
+    _require_cuda(path_rows)
+    if path_rows is not None and (path_rows.dtype != torch.int64 or path_rows.numel() != 3
+                                  or not path_rows.is_contiguous()):
+        raise ValueError("pattern_product: path_rows must be a contiguous int64 tensor of 3 elements")
+    lib = _lib.load()
+    rowptr = torch.empty(hi - lo + 1, dtype=torch.int64, device=A.device)
+    ws = _pattern_ws(hi - lo, A.device)
+    _lib.check(lib.gnn_pattern_product_count(_p(A.rowptr), _p(_col_or_dummy(A)), A.n_rows, A.n_cols, _p(B.rowptr),
+                                             _p(_col_or_dummy(B)), B.n_cols, lo, hi, int(self_loops), _p(rowptr),
+                                             _p(path_rows), _p(ws), ws.numel(), _stream_ptr()),
+               "gnn_pattern_product_count")
+    return rowptr
+
+
+def _pattern_fill(A: CSRGraph, B: CSRGraph, lo: int, hi: int, self_loops: bool, rowptr: torch.Tensor,
+                  nnz: int) -> torch.Tensor:
+    """int32 col [nnz] of rows [lo, hi) of pattern(A·B), given their rowptr (global column ids)."""
+    col = torch.empty(nnz, dtype=torch.int32, device=A.device)
+    if nnz == 0:
+        return col
+    lib = _lib.load()
+    ws = _pattern_ws(hi - lo, A.device)
+    _lib.check(lib.gnn_pattern_product_fill(_p(A.rowptr), _p(_col_or_dummy(A)), A.n_rows, A.n_cols, _p(B.rowptr),
+                                            _p(_col_or_dummy(B)), B.n_cols, lo, hi, int(self_loops),
+                                            _p(rowptr.contiguous()), _p(col), _p(ws), ws.numel(), _stream_ptr()),
+               "gnn_pattern_product_fill")
+    return col
+
 
 class _AdjCache:
     """Converts an adjacency tensor to CSR once and reuses it while the tensor is unchanged

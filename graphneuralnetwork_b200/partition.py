@@ -1213,6 +1213,44 @@ def build_metapath_view(plan: HaloPlan, rowptrs, cols, group=None) -> MetapathVi
     return MetapathView(rowptr, col, M, n_loc, n_comb, shift, any(e[M] for e in every), halo_m)
 
 
+def metapath_row_plan(count, n: int, M: int, rank: int, world: int, max_nnz_per_rank: Optional[int] = None,
+                      group=None):
+    """Row bounds of M metapath graphs over n nodes that no rank holds whole, and this rank's block rowptrs.
+
+    `count(m, lo, hi)` returns the int64 rowptr [hi - lo + 1] of rows [lo, hi) of metapath m.  Each rank counts its
+    rows of an even split (`shard_bounds`) for every metapath; one all_gather in rank order gives every rank all
+    M·N per-row counts (8·M·N bytes), hence the global rowptr_m and bounds = balanced_bounds(Σ_m rowptr_m, world),
+    the bounds `PartitionedMetapaths.from_global` would choose.  If some rank's block holds more than
+    `max_nnz_per_rank` entries, every rank raises the same GnnError (they all see every count).
+    Returns (bounds, [rowptr_m of this rank's block, starting at 0])."""
+    even = shard_bounds(n, world)
+    lo, hi = even[rank], even[rank + 1]
+    mine = [count(m, lo, hi) for m in range(M)]
+    deg = torch.stack([rp[1:] - rp[:-1] for rp in mine]) if hi > lo else None
+    dev = mine[0].device
+    width = max(even[p + 1] - even[p] for p in range(world))
+    if world > 1:
+        send = torch.zeros(M, width, dtype=torch.int64, device=dev)
+        if deg is not None:
+            send[:, :hi - lo] = deg
+        every = [torch.empty_like(send) for _ in range(world)]
+        dist.all_gather(every, send, group=group)
+        deg_all = torch.cat([e[:, :even[p + 1] - even[p]] for p, e in enumerate(every)], dim=1)
+    else:
+        deg_all = deg if deg is not None else torch.zeros(M, 0, dtype=torch.int64, device=dev)
+    rowptr = torch.zeros(M, n + 1, dtype=torch.int64, device=dev)
+    torch.cumsum(deg_all, 1, out=rowptr[:, 1:])
+    bounds = balanced_bounds(rowptr.sum(0), world)
+    block_nnz = [int(x) for x in (rowptr[:, bounds[1:]] - rowptr[:, bounds[:-1]]).sum(0).tolist()]
+    if max_nnz_per_rank is not None and max(block_nnz) > max_nnz_per_rank:
+        over = ", ".join(f"rank {p}: {v}" for p, v in enumerate(block_nnz) if v > max_nnz_per_rank)
+        raise _lib.GnnError(f"PartitionedMetapaths.from_relations: a rank's block has more than max_nnz_per_rank = "
+                            f"{max_nnz_per_rank} entries over the {M} metapaths ({over}; "
+                            f"{4 * max(block_nnz)} bytes of column ids)")
+    b_lo, b_hi = bounds[rank], bounds[rank + 1]
+    return bounds, [(rowptr[m, b_lo:b_hi + 1] - rowptr[m, b_lo]).contiguous() for m in range(M)]
+
+
 class PartitionedMetapaths:
     """This rank's share of HAN's M metapath graphs over the same N nodes, row-partitioned, in the form
     `HANModel.forward(pm, X_local)` takes (X_local = the rank's own rows).  A sequence of length M, as the list of
@@ -1260,6 +1298,32 @@ class PartitionedMetapaths:
         blocks = [select_rows(g.rowptr, g.col, None, rows)[:2] for g in graphs]
         return cls([b[0] for b in blocks], [b[1] for b in blocks], bounds, rank, world, widths,
                    device=kw.pop("device", graphs[0].rowptr.device), group=group, **kw)
+
+    @classmethod
+    def from_relations(cls, relations, rank: int, world: int, widths, self_loops: bool = True,
+                       max_nnz_per_rank: Optional[int] = None, group=None, **kw) -> "PartitionedMetapaths":
+        """From M relation CSRs R_m [N x X_m] (paper x author, paper x subject) that every rank holds: metapath m is
+        pattern(R_m·R_mᵀ) (+ I with self_loops), composed on the device (`CSRGraph.metapath`), but each rank fills
+        only its own row block.  Collective: the ranks count the rows of an even split and exchange the per-row
+        counts (`metapath_row_plan`: M·N int64 on every rank), which gives exactly the bounds `from_global` chooses
+        for the composed graphs; a block of more than `max_nnz_per_rank` entries raises on every rank.  The result
+        equals `from_global([CSRGraph.metapath(R, self_loops) for R in relations], ...)` bit for bit."""
+        from .graph import _pattern_count, _pattern_fill, _require_cuda, _require_ids_in_range
+        rels = list(relations)
+        if not rels or any(R.n_rows != rels[0].n_rows for R in rels):
+            raise ValueError("PartitionedMetapaths.from_relations: relations over the same N nodes")
+        _require_cuda(*[R.rowptr for R in rels])
+        _require_ids_in_range(*rels)  # every rank holds the same relations: a refusal is every rank's
+        pairs = [(R, R.transpose()) for R in rels]
+
+        def count(m, lo, hi):
+            return _pattern_count(pairs[m][0], pairs[m][1], lo, hi, self_loops)
+
+        bounds, rowptrs = metapath_row_plan(count, rels[0].n_rows, len(rels), rank, world, max_nnz_per_rank, group)
+        lo, hi = bounds[rank], bounds[rank + 1]
+        cols = [_pattern_fill(R, Rt, lo, hi, self_loops, rp, int(rp[-1].item())) for (R, Rt), rp in zip(pairs, rowptrs)]
+        return cls(rowptrs, cols, bounds, rank, world, widths, device=kw.pop("device", rels[0].rowptr.device),
+                   group=group, **kw)
 
     def __len__(self) -> int:
         return self._view.n_graphs

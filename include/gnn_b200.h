@@ -87,6 +87,33 @@ int gnn_dense_mask_count(const void* adj, int adj_dtype, int64_t n_rows, int64_t
 int gnn_dense_mask_fill(const void* adj, int adj_dtype, int64_t n_rows, int64_t n_cols, int64_t ld,
                         const int64_t* rowptr, int32_t* col /*[nnz]*/, gnn_stream_t stream);
 
+/* Pattern product C = pattern(A·B) of two pattern CSRs, A [n_a x k] and B [k x n_b]
+ * (replaces HeteroGraph.get_mate_path_graph, HAN/utils/data_utils.py:85-89: the metapath
+ * adjacency (P·Pᵀ > 0) of a relation matrix P, there a dense float64 N x N array).  Values are
+ * ignored; column ids within a row may be unsorted or repeated, and ids outside [0, k) of A or
+ * [0, n_b) of B are skipped.  Rows [row_lo, row_hi) of A: output row r lists, once each and
+ * ascending, every global column j with (row_lo+r, x) in A and (x, j) in B -- scipy's
+ * ((A_bool @ B_bool) > 0) after sort_indices(), the adj.nonzero() order of the dense mask.
+ * self_loops (only when n_a == n_b) adds column i to row i, as (P·Pᵀ + I) > 0.
+ * Two steps because nnz is only known after the count.  Both take a workspace of
+ * gnn_pattern_product_count_workspace_size(row_hi - row_lo) bytes and route each row by its
+ * product count to one of three paths (tuning keys "metapath.small_max", "metapath.medium_max",
+ * "metapath.tile_cols"); path_rows (nullable int64[3]) receives the rows each path took
+ * (warp sort, CTA sort, shared-memory bitmap).  No floating point; the integer atomics of the
+ * bitmap path produce an order-independent set, so the output is the same bits on every run. */
+size_t gnn_pattern_product_count_workspace_size(int64_t n_rows);
+int gnn_pattern_product_count(const int64_t* a_rowptr, const int32_t* a_col, int64_t n_a, int64_t k,
+                              const int64_t* b_rowptr, const int32_t* b_col, int64_t n_b,
+                              int64_t row_lo, int64_t row_hi, int self_loops,
+                              int64_t* rowptr /*[row_hi-row_lo+1], out, starts at 0*/,
+                              int64_t* path_rows /*nullable int64[3], out*/,
+                              void* workspace, size_t workspace_bytes, gnn_stream_t stream);
+int gnn_pattern_product_fill(const int64_t* a_rowptr, const int32_t* a_col, int64_t n_a, int64_t k,
+                             const int64_t* b_rowptr, const int32_t* b_col, int64_t n_b,
+                             int64_t row_lo, int64_t row_hi, int self_loops,
+                             const int64_t* rowptr /*the count's*/, int32_t* col /*[rowptr[row_hi-row_lo]]*/,
+                             void* workspace, size_t workspace_bytes, gnn_stream_t stream);
+
 /* CSR -> CSR of the transpose (the structure the deterministic backward walks:
  * autograd of GCN/GCN.py:43 is Âᵀ·dY; GAT/models/layers.py:63 is aᵀ·dY).
  * Stable in the original row order, so each transposed row lists its sources in
