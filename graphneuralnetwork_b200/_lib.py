@@ -68,6 +68,8 @@ SIGNATURES = {
     "gnn_gather_reduce_bwd_f32": (cint, [ptr, ptr, i64, i32, f32, ptr, i64, ptr, i64, i32, ptr]),
     "gnn_gather_reduce_bwd_dense_f32": (cint, [ptr, i64, ptr, i64, i32, i32, f32, ptr, ptr]),
     "gnn_sample_neighbors": (cint, [ptr, ptr, ptr, cint, i64, i32, u64, ptr, ptr, cint, ptr]),
+    "gnn_node_union_workspace_size": (cint, [i64, i64, C.POINTER(size_t)]),
+    "gnn_node_union": (cint, [ptr, i64, ptr, i64, cint, ptr, ptr, ptr, ptr, ptr, size_t, ptr]),
     "gnn_gat_scores_f32": (cint, [ptr, i64, ptr, ptr, i64, i32, i32, ptr, ptr, ptr]),
     "gnn_gat_fused_fwd_f32": (cint, [ptr, ptr, ptr, i64, ptr, ptr, i64, i64, i32, i32, f32, cint, cint, ptr, ptr, ptr,
                                      i64, ptr, ptr, ptr, i64, i64, i64, ptr]),

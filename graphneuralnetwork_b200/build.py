@@ -20,7 +20,7 @@ CSRC = PKG / "csrc"
 OBJ = PKG / "csrc" / "build"
 LIB = PKG / "libgnn_b200.so"
 SOURCES = ["api.cu", "spmm.cu", "sage.cu", "gat.cu", "graph.cu", "peer.cu", "sampler.cu", "sddmm.cu", "semantic.cu",
-           "metapath.cu"]
+           "metapath.cu", "node_union.cu"]
 HEADERS = ["common.cuh", "rowreduce.cuh", "spmm_kernels.cuh", "../../include/gnn_b200.h"]
 
 NVCC_FLAGS = [

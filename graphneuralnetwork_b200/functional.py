@@ -480,6 +480,103 @@ def multihop_sampling(g: CSRGraph, src_nodes: torch.Tensor, sample_nums, seed: i
     return result
 
 
+def node_union(ids_a: torch.Tensor, ids_b: torch.Tensor):
+    """gnn_node_union: (out_ids, count_dev, map_a, map_b).  out_ids [n_a + n_b] holds the ascending unique ids of
+    ids_a ∪ {ids_b >= 0} followed by -1 padding; map_a / map_b (int64) give each input's position in it, -1 for a
+    negative id; count_dev is a device int64 [1].  ids_a and ids_b share one dtype, int32 or int64."""
+    _require_cuda(ids_a, ids_b)
+    lib = _lib.load()
+    ids_a, ids_b = ids_a.contiguous().view(-1), ids_b.contiguous().view(-1)
+    if ids_a.dtype != ids_b.dtype or ids_a.dtype not in (torch.int32, torch.int64):
+        raise _lib.GnnError(f"node_union: ids must share int32 or int64, got {ids_a.dtype} and {ids_b.dtype}")
+    import ctypes as C
+    n_a, n_b = ids_a.numel(), ids_b.numel()
+    ws_bytes = C.c_size_t(0)
+    _lib.check(lib.gnn_node_union_workspace_size(n_a, n_b, C.byref(ws_bytes)), "gnn_node_union_workspace_size")
+    dev = ids_a.device
+    ws = torch.empty(max(ws_bytes.value, 1), dtype=torch.uint8, device=dev)
+    out_ids = torch.empty(n_a + n_b, dtype=ids_a.dtype, device=dev)
+    count = torch.empty(1, dtype=torch.int64, device=dev)
+    map_a = torch.empty(n_a, dtype=torch.int64, device=dev)
+    map_b = torch.empty(n_b, dtype=torch.int64, device=dev)
+    _lib.check(lib.gnn_node_union(_p(ids_a), n_a, _p(ids_b), n_b, 32 if ids_a.dtype == torch.int32 else 64,
+                                  _p(out_ids), _p(count), _p(map_a), _p(map_b), _p(ws), ws_bytes.value, _stream_ptr()),
+               "gnn_node_union")
+    return out_ids, count, map_a, map_b
+
+
+class DedupBatch:
+    """One minibatch of the de-duplicating GraphSAGE (GraphSAGE/data_utils.py:82-162), built on the device by
+    `dedup_layer_nodes`.  With L layers and S_{L-1} the batch, S_i = S_{i+1} ∪ samples(S_{i+1}):
+      nodes[l]      int64 [n_l]      S_l; the batch keeps its order, every other set is ascending global id;
+      counts[l]     int              n_l = |S_l| (host ints);
+      center_map    int64 [L-1, n_0] row i: the position in S_i of each node of S_{i+1}, then -1;
+      neigh_map     int64 [L-1, n_0, k] row r of map i: the positions in S_i of the k draws of node r of S_{i+1},
+                                     in draw order; rows past n_{i+1} are -1 (the reference's layout: `forward` takes it);
+      neighbors[l]  int64 [n_l, k]   the global ids drawn for S_l; neighbors[0] are the outermost neighbours, which
+                                     the layer gathers straight from the feature table (`outer_neighbors`)."""
+
+    def __init__(self, nodes, counts, center_map, neigh_map, neighbors):
+        self.nodes, self.counts, self.center_map, self.neigh_map, self.neighbors = (nodes, counts, center_map,
+                                                                                    neigh_map, neighbors)
+
+    @property
+    def outer_neighbors(self) -> torch.Tensor:
+        return self.neighbors[0]
+
+
+def dedup_layer_nodes(g: CSRGraph, batch_ids, num_layers: int, k: int, seed: int) -> DedupBatch:
+    """GraphSAGE/data_utils.py:82-117 (`get_layer_adj_nodes`) and the id half of its collate_fn (:154-162) on the
+    device.  For l = L-2 … 0: draw k neighbours of every node of S_{l+1} (`sample_neighbors`, seed mixed per layer
+    as `multihop_sampling` does) and unite S_{l+1} with them (`node_union`); then draw k neighbours of S_0 once more,
+    not de-duplicated, for the outermost gather.  Sets are ascending global id instead of the reference's CPython
+    set order (only which row sits where differs; the maps carry it).
+
+    Every set stays padded to its bound n_{l+1}·(k+1) with -1 ids until the end, so the layers need no host sizes;
+    ONE device-to-host read of the L-1 union counts per batch then gives the shapes: that is the one
+    synchronisation.  A batch given on the device costs one more, for the range check of its ids.
+    A graph with a row without edges is refused (GnnError): the reference's `random.sample` fails there."""
+    if num_layers < 1 or k < 1:
+        raise ValueError(f"num_layers and k must be positive (got {num_layers}, {k})")
+    if g.has_empty_rows():
+        raise _lib.GnnError("dedup_layer_nodes: the graph has a row without edges; the reference's random.sample "
+                            "cannot draw from it")
+    dev = g.device
+    batch = torch.as_tensor(batch_ids).view(-1)
+    if batch.numel() == 0:
+        raise ValueError("dedup_layer_nodes: empty batch")
+    lo, hi = torch.stack([batch.min(), batch.max()]).tolist()
+    if lo < 0 or hi >= g.n_rows:
+        raise IndexError(f"dedup_layer_nodes: batch ids must lie in [0, {g.n_rows}), got [{lo}, {hi}]")
+    batch = batch.to(device=dev, dtype=torch.int64)
+    L = num_layers
+
+    def layer_seed(l):
+        return seed + 0x9E3779B9 * (L - l)  # hop L-1-l of multihop_sampling
+
+    padded, draws, maps, count_devs = [batch], [], [], []
+    for l in range(L - 2, -1, -1):
+        d = sample_neighbors(g, padded[0], k, layer_seed(l + 1), torch.int64)
+        out_ids, count, map_a, map_b = node_union(padded[0], d)
+        padded.insert(0, out_ids)
+        draws.insert(0, d)
+        maps.insert(0, (map_a, map_b))
+        count_devs.insert(0, count)
+    counts = (torch.cat(count_devs).tolist() if count_devs else []) + [batch.numel()]
+    nodes = [p[:n] for p, n in zip(padded, counts)]
+    n0 = counts[0]
+    center_map = torch.full((L - 1, n0), -1, dtype=torch.int64, device=dev)
+    neigh_map = torch.full((L - 1, n0, k), -1, dtype=torch.int64, device=dev)
+    neighbors = [None] * L
+    for i, (map_a, map_b) in enumerate(maps):
+        n = counts[i + 1]
+        center_map[i, :n] = map_a[:n]
+        neigh_map[i, :n] = map_b.view(-1, k)[:n]
+        neighbors[i + 1] = draws[i].view(-1, k)[:n]
+    neighbors[0] = sample_neighbors(g, nodes[0], k, layer_seed(0), torch.int64).view(n0, k)
+    return DedupBatch(nodes, counts, center_map, neigh_map, neighbors)
+
+
 class _GatherReduceFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, table, idx, n_src, fanout, reduce):

@@ -340,6 +340,22 @@ int gnn_sample_neighbors(const int64_t* rowptr, const int32_t* col, const void* 
                          int64_t n_src, int32_t k, uint64_t seed, const int64_t* seed_offset_dev,
                          void* out, int out_bits, gnn_stream_t stream);
 
+/* Node-set union with remap (the `set(nodes) | set(samples)` and id -> position maps of the de-duplicating
+ * GraphSAGE collate, GraphSAGE/data_utils.py:100-116), ordered by ascending global id instead of CPython's set order:
+ *   out_ids[0..count)  = the ascending unique ids of ids_a ∪ {ids_b >= 0}; out_ids[count..n_a+n_b) = -1, so a padded
+ *                        set can be handed to gnn_sample_neighbors and to the next union as it is;
+ *   map_a[i] / map_b[j] = position in out_ids of ids_a[i] / ids_b[j], -1 where the id is negative;
+ *   *out_count_dev     = count (stays on the device).
+ * ids_a, ids_b and out_ids are int32 or int64 (id_bits), the maps int64.  One radix sort of (id, slot) pairs over
+ * n_a + n_b keys, a head flag per run, a scan and a scatter: O(n_a + n_b) work and memory, nothing over the node
+ * count.  No floating point, no atomics: the same input gives the same bits.  n_a + n_b == 0 writes a count of 0.
+ * Bad sizes (negative, or n_a + n_b >= 2^31) and null pointers return GNN_ERR_BAD_ARG before any CUDA call. */
+int gnn_node_union_workspace_size(int64_t n_a, int64_t n_b, size_t* bytes_host /*out*/);
+int gnn_node_union(const void* ids_a, int64_t n_a, const void* ids_b, int64_t n_b, int id_bits,
+                   void* out_ids /*[n_a+n_b]*/, int64_t* out_count_dev /*[1]*/,
+                   int64_t* map_a /*[n_a]*/, int64_t* map_b /*[n_b]*/,
+                   void* workspace, size_t workspace_bytes, gnn_stream_t stream);
+
 /* ---- GAT / HAN: fused multi-head attention aggregation ---------------------------- */
 /* Per-node, per-head halves of the edge score (GAT/models/layers.py:25-26 decomposes
  * exactly: a·[Wh_i || Wh_j] = a[:F']·Wh_i + a[F':]·Wh_j):
