@@ -34,6 +34,11 @@ SIGNATURES = {
                                          ptr]),
     "gnn_pattern_product_fill": (cint, [ptr, ptr, i64, i64, ptr, ptr, i64, i64, i64, cint, ptr, ptr, ptr, size_t,
                                         ptr]),
+    "gnn_spgemm_workspace_size": (size_t, [i64, i64]),
+    "gnn_spgemm_values_f32": (cint, [ptr, ptr, ptr, i64, i64, i64, ptr, ptr, ptr, ptr, i64, i64, ptr, ptr, ptr, i32, ptr,
+                                     ptr, size_t, ptr]),
+    "gnn_spgemm_values_bwd_f32": (cint, [ptr, ptr, ptr, i64, i64, i64, ptr, ptr, ptr, ptr, ptr, ptr, i64, i64, ptr, ptr,
+                                         ptr, ptr, ptr, ptr, i64, i32, ptr, ptr, ptr, ptr, size_t, ptr]),
     "gnn_csr_transpose_workspace_size": (size_t, [i64, i64, i64]),
     "gnn_csr_transpose": (cint, [ptr, ptr, ptr, i64, i64, i64, ptr, ptr, ptr, ptr, ptr, size_t, ptr]),
     "gnn_index_block_transpose_workspace_size": (size_t, [i64, i64]),

@@ -52,6 +52,8 @@ static std::map<std::string, int>& tune_map() {
       {"metapath.small_max", 256},   // product rows with at most this many products: one warp sorts them (cap 256)
       {"metapath.medium_max", 8192}, // ... at most this many: one CTA sorts them (cap 8192); longer rows: bitmap
       {"metapath.tile_cols", 0},     // columns per bitmap tile of the hub-row path (0 = as many as shared memory holds)
+      {"spgemm.warp_slots", 1024},   // masked value products: rows with at most this many output entries ...
+      {"spgemm.warp_list", 1024},    // ... and a left row of at most this many keys take a warp; the rest a whole CTA
   };
   return m;
 }

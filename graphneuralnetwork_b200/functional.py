@@ -200,6 +200,119 @@ def spmm_values(pattern: CSRGraph, val: torch.Tensor, X: torch.Tensor) -> torch.
     return _SpmmValuesFn.apply(val, X, pattern)
 
 
+def _col_or_dummy(g: CSRGraph) -> torch.Tensor:
+    # an empty tensor has no address; the kernels read no column of a graph without entries
+    return g.col if g.nnz else torch.zeros(1, dtype=torch.int32, device=g.device)
+
+
+def _nonempty(t: torch.Tensor) -> torch.Tensor:
+    # a permutation of a graph without entries has no address; the kernels read none of it
+    return t if t.numel() else torch.zeros(1, dtype=t.dtype, device=t.device)
+
+
+def _spgemm_ws(n_a: int, k: int, dev) -> torch.Tensor:
+    return torch.empty(max(_lib.load().gnn_spgemm_workspace_size(n_a, k), 1), dtype=torch.uint8, device=dev)
+
+
+def spgemm_values_raw(A: CSRGraph, a_val: torch.Tensor, B: CSRGraph, b_val: torch.Tensor, C_pattern: CSRGraph,
+                      path_rows: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Values [C_pattern.nnz, C] of A·B on C_pattern, channel by channel (gnn_spgemm_values_f32, no autograd).
+    B is read through its cached transpose.  path_rows: an int64[2] CUDA tensor that receives the rows each
+    kernel path took (warp, CTA)."""
+    lib = _lib.load()
+    C = a_val.shape[1]
+    c_val = torch.empty((C_pattern.nnz, C), dtype=torch.float32, device=a_val.device)
+    Bt = B.transpose()
+    ws = _spgemm_ws(A.n_rows, A.n_cols, a_val.device)
+    _lib.check(lib.gnn_spgemm_values_f32(
+        _p(A.rowptr), _p(_col_or_dummy(A)), _p(a_val), A.n_rows, A.n_cols, A.nnz,
+        _p(Bt.rowptr), _p(_col_or_dummy(Bt)), _p(_nonempty(B.perm_t)), _p(b_val), B.n_cols, B.nnz,
+        _p(C_pattern.rowptr), _p(_col_or_dummy(C_pattern)), _p(_nonempty(c_val)), C, _p(path_rows),
+        _p(ws), ws.numel(), _stream_ptr()), "gnn_spgemm_values_f32")
+    return c_val
+
+
+def spgemm_values_bwd_raw(A: CSRGraph, a_val: torch.Tensor, B: CSRGraph, b_val: torch.Tensor, C_pattern: CSRGraph,
+                          dc: torch.Tensor, need_a: bool = True, need_b: bool = True,
+                          path_rows: Optional[torch.Tensor] = None):
+    """(dA [A.nnz, C], dB [B.nnz, C]) of spgemm_values_raw for the output gradient dc, each restricted to its
+    operand's pattern (gnn_spgemm_values_bwd_f32; None where not asked for).  Aᵀ and Cᵀ are the cached transposes.
+    path_rows: an int64[4] CUDA tensor, the rows each path took for dA and then for dB."""
+    lib = _lib.load()
+    C = dc.shape[1]
+    dev = dc.device
+    da = torch.zeros((A.nnz, C), dtype=torch.float32, device=dev) if need_a else None
+    db = torch.zeros((B.nnz, C), dtype=torch.float32, device=dev) if need_b else None
+    da_k = None if da is None else _nonempty(da)  # rows without entries still take their path
+    db_k = None if db is None else _nonempty(db)
+    if da_k is None and db_k is None:
+        return da, db
+    At = A.transpose() if db_k is not None else None
+    Ct = C_pattern.transpose() if db_k is not None else None
+    ws = _spgemm_ws(A.n_rows, A.n_cols, dev)
+    _lib.check(lib.gnn_spgemm_values_bwd_f32(
+        _p(A.rowptr), _p(_col_or_dummy(A)), _p(a_val), A.n_rows, A.n_cols, A.nnz,
+        None if At is None else _p(At.rowptr), None if At is None else _p(_col_or_dummy(At)),
+        None if At is None else _p(_nonempty(A.perm_t)),
+        _p(B.rowptr), _p(_col_or_dummy(B)), _p(b_val), B.n_cols, B.nnz,
+        _p(C_pattern.rowptr), _p(_col_or_dummy(C_pattern)),
+        None if Ct is None else _p(Ct.rowptr), None if Ct is None else _p(_col_or_dummy(Ct)),
+        None if Ct is None else _p(_nonempty(C_pattern.perm_t)), _p(_nonempty(dc)), C_pattern.nnz, C,
+        _p(da_k), _p(db_k), _p(path_rows), _p(ws), ws.numel(), _stream_ptr()), "gnn_spgemm_values_bwd_f32")
+    return da, db
+
+
+class _SpgemmValuesFn(torch.autograd.Function):
+    """C = A·B with C channels of values on fixed patterns; gradients into both value tensors, on their patterns."""
+
+    @staticmethod
+    def forward(ctx, a_val, b_val, A: CSRGraph, B: CSRGraph, C_pattern: CSRGraph):
+        ctx.graphs = (A, B, C_pattern)
+        ctx.save_for_backward(a_val, b_val)
+        return spgemm_values_raw(A, a_val, B, b_val, C_pattern)
+
+    @staticmethod
+    def backward(ctx, dc):
+        a_val, b_val = ctx.saved_tensors
+        A, B, C_pattern = ctx.graphs
+        da, db = spgemm_values_bwd_raw(A, a_val, B, b_val, C_pattern, dc.contiguous(), ctx.needs_input_grad[0],
+                                       ctx.needs_input_grad[1])
+        return da, db, None, None, None
+
+
+def spgemm_values(A: CSRGraph, a_val: torch.Tensor, B: CSRGraph, b_val: torch.Tensor,
+                  C_pattern: CSRGraph) -> torch.Tensor:
+    """Values [C_pattern.nnz, C] of the sparse product A·B on the pattern C_pattern (from `CSRGraph.pattern_product`),
+    each of the C channels its own product: the learned metapath composition of GTN (GTN/models/GTLayer.py, there a
+    dense torch.bmm).  a_val [A.nnz, C] and b_val [B.nnz, C] are fp32 in CSR slot order; autograd reaches both.
+    The rows of A, B and C_pattern hold ascending unique column ids (what pattern products and the CSR builders
+    produce).  Every output entry is one sum in ascending order of the inner index: the same bits on every run."""
+    _require_cuda(a_val, b_val, A.rowptr, B.rowptr, C_pattern.rowptr)
+    if a_val.dtype != torch.float32 or b_val.dtype != torch.float32:
+        raise _lib.GnnError(f"spgemm_values: fp32 values expected, got {a_val.dtype} / {b_val.dtype}")
+    if a_val.dim() != 2 or b_val.dim() != 2 or a_val.shape != (A.nnz, a_val.shape[1]) \
+            or b_val.shape != (B.nnz, a_val.shape[1]):
+        raise _lib.GnnError(f"spgemm_values: values [A.nnz = {A.nnz}, C] and [B.nnz = {B.nnz}, C] expected, got "
+                            f"{tuple(a_val.shape)} / {tuple(b_val.shape)}")
+    if A.n_cols != B.n_rows or C_pattern.n_rows != A.n_rows or C_pattern.n_cols != B.n_cols:
+        raise _lib.GnnError(f"spgemm_values: [{A.n_rows}, {A.n_cols}]·[{B.n_rows}, {B.n_cols}] does not give the "
+                            f"[{C_pattern.n_rows}, {C_pattern.n_cols}] pattern")
+    return _SpgemmValuesFn.apply(a_val.contiguous(), b_val.contiguous(), A, B, C_pattern)
+
+
+def column_normalize(pattern: CSRGraph, val: torch.Tensor) -> torch.Tensor:
+    """val [nnz, C] on `pattern` with every column of every channel divided by its sum (inf -> 0), autograd into
+    val: the column normalisation of GTN's `norm` (GTN/models/GTN.py:7-19) on a pattern without its diagonal.  The
+    column sums are the ordered row sums of the cached transpose (one SpMM per channel), not an atomic scatter."""
+    t = pattern.transpose()
+    ones = torch.ones((pattern.n_rows, 1), dtype=torch.float32, device=val.device)
+    perm = pattern.perm_t
+    sums = torch.cat([spmm_values(t, val[:, c][perm].contiguous(), ones) for c in range(val.shape[1])], dim=1)
+    inv = sums.pow(-1)
+    inv = torch.where(torch.isinf(inv), torch.zeros_like(inv), inv)
+    return val * inv[pattern.col.long()]
+
+
 class _GcnAggregateFn(torch.autograd.Function):
     """Y = relu?(Â·S + b) in ONE launch: the aggregation (GCN/GCN.py:43), the bias add
     (GCN.py:44-45) and the ReLU that follows every hidden layer (GCN.py:12,19) fused into the

@@ -12,14 +12,20 @@ On the message-passing path (re-designed):
   * `norm(H, add)` keeps the reference's dense-in / dense-out contract for `GTN_Model.normalization`, as
     element-wise work: multiplying by a diagonal matrix is a row scaling, and adds only exact zeros, so the
     result is bit-identical to the reference's `torch.mm(deg_inv, H)`.
-Adjacent, kept as plain torch (out of scope: the dense N^3 metapath composition): `GTConv`, `GTLayer`.
+  * Sparse composition (DESIGN §4.10): `GTN_Model.forward` also takes a `RelationStack` where the reference passes
+    the dense [N, N, K] tensor.  GTConv's soft selection is then a [nnz_U, C] value tensor on the union pattern U
+    of the relations, every GTLayer product is `functional.spgemm_values` on a pattern built once per stack
+    (P_1 = pattern(U·U), P_{l+1} = pattern(offdiag(P_l)·U)), `norm` is `functional.column_normalize` on the
+    pattern without its diagonal, and the final `gcn_conv` runs on the cached pattern of (offdiag(H) + I)^T.
+    Same parameters and state_dict as the dense path, which a dense `A` still takes unchanged.
 """
 import torch
 from torch import nn
 import torch.nn.functional as F
 
-from ..functional import spmm_values
-from ..graph import CSRGraph
+from .. import _lib
+from ..functional import column_normalize, spgemm_values, spmm_values
+from ..graph import CSRGraph, _require_cuda, _require_ids_in_range
 
 
 def norm(H, add=False):
@@ -56,14 +62,125 @@ def gcn_conv(X, H, weight):
     also fills the structural zeros, but in GTN a zero of the composed adjacency is a zero of every factor
     product, so no parameter receives anything from them (the model-level gradients are identical)."""
     XW = torch.mm(X, weight)
-    n = H.shape[0]
     g, rows, cols = _pattern_of_learned_adjacency(H)
     diag = rows == cols
     vals = torch.where(diag, torch.ones((), device=H.device, dtype=H.dtype), H[cols, rows])  # (offdiag(H) + I)[i, j]
-    deg = torch.zeros(n, device=H.device, dtype=vals.dtype).index_add(0, rows, vals)        # column sums, by row of H^T
+    return _normalized_aggregate(g, vals.float(), XW)
+
+
+def _normalized_aggregate(g, vals, XW):
+    """The tail of `gcn_conv` on g = CSR of (offdiag(H) + I)^T with its values: divide by the column sums of
+    offdiag(H) + I (the row sums of g, an ordered SpMM against ones; inf -> 0) and aggregate XW, autograd into vals."""
+    ones = torch.ones((g.n_cols, 1), dtype=torch.float32, device=vals.device)
+    deg = spmm_values(g, vals, ones).view(-1)
     deg_inv = deg.pow(-1)
     deg_inv = torch.where(deg_inv == float('inf'), torch.zeros_like(deg_inv), deg_inv)
-    return spmm_values(g, (vals * deg_inv[rows]).float(), XW)
+    return spmm_values(g, vals * deg_inv[g.edge_rows().long()], XW)
+
+
+def _drop_diagonal(P):
+    """(pattern of P without its diagonal, int64 slots of P it keeps).  Setup only: one host read of the count."""
+    keep = P.edge_rows() != P.col
+    idx = torch.nonzero(keep).flatten()
+    cum = torch.zeros(P.nnz + 1, dtype=torch.int64, device=P.device)
+    torch.cumsum(keep.to(torch.int64), 0, out=cum[1:])
+    return CSRGraph(cum[P.rowptr], P.col[idx].contiguous(), None, P.n_rows, P.n_cols), idx
+
+
+class RelationStack:
+    """GTN's K edge-type adjacencies (the last one usually the identity GTN appends) as ONE union pattern U [N, N]
+    with values V [nnz_U, K] (0 where relation k lacks the entry), plus the patterns every layer count needs, built
+    once with the pattern-product kernels and cached:
+        P_1 = pattern(U·U),  D_l = P_l without its diagonal,  P_{l+1} = pattern(D_l·U),
+    and for the final gcn_conv the CSR of (D_L + I)^T.  Pass it to `GTN_Model.forward` in place of the dense
+    [N, N, K] tensor.  `max_nnz` bounds every composed pattern: a larger one raises GnnError before its column array
+    is allocated (`CSRGraph.pattern_product`)."""
+
+    def __init__(self, U: CSRGraph, V: torch.Tensor, max_nnz=None):
+        _require_cuda(U.rowptr, V)
+        if U.n_rows != U.n_cols:
+            raise ValueError(f"RelationStack: relations must be square, got [{U.n_rows}, {U.n_cols}]")
+        if V.dim() != 2 or V.shape[0] != U.nnz:
+            raise ValueError(f"RelationStack: V must be [nnz_U = {U.nnz}, K], got {tuple(V.shape)}")
+        _require_ids_in_range(U)
+        self.U, self.V = U, V.to(torch.float32).contiguous()
+        self.n, self.num_edge = U.n_rows, V.shape[1]
+        self.max_nnz = max_nnz
+        self._P, self._D, self._keep = [], [], []
+        self._gcn = {}
+
+    @staticmethod
+    def from_dense(A: torch.Tensor, max_nnz=None) -> "RelationStack":
+        """From the reference's dense input A [N, N, K] (GTN/main.py builds it with the identity as the last type)."""
+        _require_cuda(A)
+        if A.dim() != 3 or A.shape[0] != A.shape[1]:
+            raise ValueError(f"RelationStack.from_dense: A must be [N, N, K], got {tuple(A.shape)}")
+        U = CSRGraph.from_dense_mask((A != 0).any(dim=2).to(torch.float32))
+        rows, cols = U.edge_rows().long(), U.col.long()
+        return RelationStack(U, A[rows, cols].to(torch.float32), max_nnz)
+
+    @staticmethod
+    def from_relations(graphs, max_nnz=None) -> "RelationStack":
+        """From K value-carrying CSRGraphs [N, N] (val None: ones), in GTN's edge-type order.  Repeated entries of
+        one relation add up.  Ids outside [0, N) raise IndexError."""
+        graphs = list(graphs)
+        if not graphs:
+            raise ValueError("RelationStack.from_relations: no relations")
+        n = graphs[0].n_rows
+        for g in graphs:
+            _require_cuda(g.rowptr)
+            if g.n_rows != n or g.n_cols != n:
+                raise ValueError(f"RelationStack.from_relations: relations must be [{n}, {n}], got "
+                                 f"[{g.n_rows}, {g.n_cols}]")
+        _require_ids_in_range(*graphs)
+        dev = graphs[0].device
+        keys = torch.cat([g.edge_rows().long() * n + g.col.long() for g in graphs])
+        kind = torch.cat([torch.full((g.nnz,), k, dtype=torch.int64, device=dev) for k, g in enumerate(graphs)])
+        vals = torch.cat([torch.ones(g.nnz, device=dev) if g.val is None else g.val.float() for g in graphs])
+        ukeys, inv = torch.unique(keys, sorted=True, return_inverse=True)
+        V = torch.zeros((ukeys.numel(), len(graphs)), dtype=torch.float32, device=dev)
+        V.index_put_((inv, kind), vals, accumulate=True)
+        U, perm = CSRGraph.from_coo(ukeys // n, ukeys % n, None, n, n, return_perm=True, validate=False)
+        return RelationStack(U, V[perm], max_nnz)
+
+    def patterns(self, num_layers: int):
+        """([P_1 .. P_L], [D_1 .. D_{L-1}], [slots of P_l that D_l keeps]) for L = num_layers (built on first use)."""
+        while len(self._P) < num_layers:
+            A = self.U if not self._P else self._D[-1]
+            P = CSRGraph.pattern_product(A, self.U, max_nnz=self.max_nnz, validate=False)
+            D, keep = _drop_diagonal(P)
+            for g in (P, D):  # transposes the backward and the column sums walk, and their SpMM plans
+                _plan(g)
+                _plan(g.transpose())
+            self._P.append(P)
+            self._D.append(D)
+            self._keep.append(keep)
+        self.U.transpose()
+        return self._P[:num_layers], self._D[:num_layers - 1], self._keep[:num_layers - 1]
+
+    def gcn_pattern(self, num_layers: int):
+        """(g, src, diag) for the final gcn_conv on P_L: g the CSR of (D_L + I)^T, src the int64 slot of P_L each
+        edge of g reads (0 on the diagonal), diag the bool mask of the self-loops."""
+        if num_layers not in self._gcn:
+            self.patterns(num_layers)
+            D, idx = self._D[num_layers - 1], self._keep[num_layers - 1]
+            dev = D.device
+            rows = torch.cat([D.col.long(), torch.arange(self.n, device=dev)])          # j: row of H^T
+            cols = torch.cat([D.edge_rows().long(), torch.arange(self.n, device=dev)])  # i
+            g, perm = CSRGraph.from_coo(rows, cols, None, self.n, self.n, return_perm=True, validate=False)
+            diag = perm >= D.nnz
+            src = idx[torch.where(diag, torch.zeros_like(perm), perm)] if D.nnz else torch.zeros_like(perm)
+            _plan(g)
+            _plan(g.transpose())
+            self._gcn[num_layers] = (g, src, diag)
+        return self._gcn[num_layers]
+
+
+def _plan(g):
+    """Host-side SpMM plans of g, computed now so that a training step reads nothing back from the device."""
+    g.long_row_plan()
+    g.rows_per_team()
+    g.edge_rows()
 
 
 class GTConv(nn.Module):
@@ -80,6 +197,11 @@ class GTConv(nn.Module):
     def forward(self, A):
         return torch.sum(A * F.softmax(self.weight, dim=1), dim=1)
 
+    def forward_sparse(self, stack):
+        """The same soft selection on a RelationStack: values [nnz_U, out_channels] on its union pattern."""
+        s = F.softmax(self.weight, dim=1)[:, :, 0, 0]  # [C, K]
+        return torch.sum(stack.V.unsqueeze(1) * s.unsqueeze(0), dim=2)
+
 
 class GTLayer(nn.Module):
     """GTN/models/GTLayer.py: one metapath-composition step (dense bmm; out of scope, kept as the reference has it)."""
@@ -92,6 +214,18 @@ class GTLayer(nn.Module):
         self.conv1 = GTConv(in_channels, out_channels)
         if self.first:
             self.conv2 = GTConv(in_channels, out_channels)
+
+    def forward_sparse(self, stack, P, H_=None, D=None):
+        """One composition step on a RelationStack: H_ None gives a·b on P = pattern(U·U); else H_ holds the
+        normalised values on D (an earlier H without its diagonal) and the result is H_·a on P = pattern(D·U)."""
+        a = self.conv1.forward_sparse(stack)
+        if self.first:
+            H = spgemm_values(stack.U, a, stack.U, self.conv2.forward_sparse(stack), P)
+            W = [(F.softmax(self.conv1.weight, dim=1)).detach(), (F.softmax(self.conv2.weight, dim=1)).detach()]
+        else:
+            H = spgemm_values(D, H_, stack.U, a, P)
+            W = [(F.softmax(self.conv1.weight, dim=1)).detach()]
+        return H, W
 
     def forward(self, A, H_=None):
         if self.first:
@@ -137,6 +271,8 @@ class GTN_Model(nn.Module):
         return torch.stack([norm(H[i, :, :]) for i in range(self.num_channels)], dim=0)
 
     def forward(self, A, X, target_x):
+        if isinstance(A, RelationStack):
+            return self._forward_sparse(A, X, target_x)
         A = A.unsqueeze(0).permute(0, 3, 1, 2)
         Ws = []
         for i in range(self.num_layers):
@@ -147,6 +283,29 @@ class GTN_Model(nn.Module):
                 H, W = self.layers[i](A, H)
             Ws.append(W)
         X_ = torch.cat([F.relu(self.gcn_conv(X, H[i])) for i in range(self.num_channels)], dim=1)
+        X_ = F.relu(self.linear1(X_))
+        y = self.linear2(X_[target_x])
+        return y, Ws
+
+    def _forward_sparse(self, stack, X, target_x):
+        """forward() on a RelationStack: the same computation with every H a [nnz(P_l), C] value tensor."""
+        if stack.num_edge != self.num_edge:
+            raise ValueError(f"GTN_Model: the stack has {stack.num_edge} edge types, the model {self.num_edge}")
+        Ps, Ds, keeps = stack.patterns(self.num_layers)
+        Ws = []
+        H = None
+        for i in range(self.num_layers):
+            if i == 0:
+                H, W = self.layers[i].forward_sparse(stack, Ps[0])
+            else:
+                Hn = column_normalize(Ds[i - 1], H[keeps[i - 1]])  # norm(H): diagonal dropped, columns scaled
+                H, W = self.layers[i].forward_sparse(stack, Ps[i], Hn, Ds[i - 1])
+            Ws.append(W)
+        g, src, diag = stack.gcn_pattern(self.num_layers)
+        XW = torch.mm(X, self.weight)
+        one = torch.ones((), device=H.device, dtype=H.dtype)
+        X_ = torch.cat([F.relu(_normalized_aggregate(g, torch.where(diag, one, H[src, c]), XW))
+                        for c in range(self.num_channels)], dim=1)
         X_ = F.relu(self.linear1(X_))
         y = self.linear2(X_[target_x])
         return y, Ws

@@ -114,6 +114,46 @@ int gnn_pattern_product_fill(const int64_t* a_rowptr, const int32_t* a_col, int6
                              const int64_t* rowptr /*the count's*/, int32_t* col /*[rowptr[row_hi-row_lo]]*/,
                              void* workspace, size_t workspace_bytes, gnn_stream_t stream);
 
+/* Value-carrying sparse x sparse product on a known pattern (GTN's learned metapath composition,
+ * GTN/models/GTLayer.py: H = a·b, H = norm(H)·a, there a dense torch.bmm of [C, N, N]).  Values
+ * are fp32 with C channels per entry, entry-major ([nnz, C]), 1 <= C <= 8 (GNN_ERR_UNSUPPORTED
+ * above); each channel is its own product over the same patterns.  A is [n_a x k] with nnz_a
+ * entries, B is [k x n_b] with nnz_b entries, and c_rowptr / c_col is the pattern of A·B from
+ * gnn_pattern_product_* (or any superset of it: entries no product reaches are 0).
+ *   forward:  C[i, j, c] = Σ_x A[i, x, c]·B[x, j, c]
+ *   backward: dA[i, x, c] = Σ_{j ∈ B[x]} dC[i, j, c]·B[x, j, c]      on pattern(A)
+ *             dB[x, j, c] = Σ_{i : x ∈ A[i]} A[i, x, c]·dC[i, j, c]  on pattern(B)
+ * B enters the forward as its transpose (bt_*: gnn_csr_transpose's rowptr_t / col_t / perm_t, the
+ * values stay in B's slot order); the backward takes Aᵀ and Cᵀ the same way.  The rows of A, B
+ * and C must hold ascending, unique column ids (a transposed CSR has them); one thread owns one
+ * output entry and sums it in ascending order of the inner index, so the output is the same bits
+ * on every run.  Output rows with at most "spgemm.warp_slots" entries whose left operand row
+ * holds at most "spgemm.warp_list" ids take one warp each, the others one CTA each; path_rows
+ * (nullable int64[2] forward, [4] backward: dA then dB) receives the rows each path took (warp,
+ * CTA).  da_val / db_val are nullable.  Column ids of the output pattern outside the product
+ * and permutation entries outside the value arrays are skipped.  Bad sizes and null pointers
+ * return GNN_ERR_BAD_ARG, a workspace below gnn_spgemm_workspace_size(n_a, k) bytes
+ * GNN_ERR_WORKSPACE, both before any CUDA call. */
+size_t gnn_spgemm_workspace_size(int64_t n_a, int64_t k);
+int gnn_spgemm_values_f32(const int64_t* a_rowptr, const int32_t* a_col, const float* a_val /*[nnz_a, C]*/,
+                          int64_t n_a, int64_t k, int64_t nnz_a,
+                          const int64_t* bt_rowptr /*[n_b+1]*/, const int32_t* bt_col, const int64_t* bt_perm,
+                          const float* b_val /*[nnz_b, C], B's slot order*/, int64_t n_b, int64_t nnz_b,
+                          const int64_t* c_rowptr, const int32_t* c_col, float* c_val /*[nnz_c, C], out*/,
+                          int32_t C, int64_t* path_rows /*nullable int64[2]*/,
+                          void* workspace, size_t workspace_bytes, gnn_stream_t stream);
+int gnn_spgemm_values_bwd_f32(const int64_t* a_rowptr, const int32_t* a_col, const float* a_val,
+                              int64_t n_a, int64_t k, int64_t nnz_a,
+                              const int64_t* at_rowptr /*[k+1]*/, const int32_t* at_col, const int64_t* at_perm,
+                              const int64_t* b_rowptr, const int32_t* b_col, const float* b_val,
+                              int64_t n_b, int64_t nnz_b,
+                              const int64_t* c_rowptr, const int32_t* c_col,
+                              const int64_t* ct_rowptr /*[n_b+1]*/, const int32_t* ct_col, const int64_t* ct_perm,
+                              const float* dc_val /*[nnz_c, C]*/, int64_t nnz_c, int32_t C,
+                              float* da_val /*nullable [nnz_a, C], out*/, float* db_val /*nullable [nnz_b, C], out*/,
+                              int64_t* path_rows /*nullable int64[4]*/,
+                              void* workspace, size_t workspace_bytes, gnn_stream_t stream);
+
 /* CSR -> CSR of the transpose (the structure the deterministic backward walks:
  * autograd of GCN/GCN.py:43 is Âᵀ·dY; GAT/models/layers.py:63 is aᵀ·dY).
  * Stable in the original row order, so each transposed row lists its sources in
