@@ -119,6 +119,7 @@ SIGNATURES = {
     "gnn_halo_push_waves": (cint, [ptr, i64, i32, i32, ptr, ptr, i32, i32, i64, ptr, ptr, i32, i32, C.c_uint32, ptr, ptr]),
     "gnn_peer_signal": (cint, [ptr, i32, i32, i32, C.c_uint32, ptr]),
     "gnn_peer_wait": (cint, [ptr, i32, i32, C.c_uint32, ptr, i64, ptr]),
+    "gnn_peer_reduce_rows_f32": (cint, [ptr, i32, i64, i32, i64, i64, ptr, i64, i32, ptr]),
     "gnn_spmm_csr_ex_f32": (cint, [ptr, ptr, ptr, ptr, ptr, i64, i64, i32, i64, i64, ptr, ptr]),
     "gnn_spmm_csr_ex_bf16": (cint, [ptr, ptr, ptr, ptr, ptr, i64, i64, i32, i64, i64, ptr, ptr]),
 }

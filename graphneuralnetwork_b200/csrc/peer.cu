@@ -22,6 +22,9 @@
 //                    a rank signals each peer after its wave of rows has been pushed (stream order:
 //                    the mover kernel has completed), and the consumer of a wave waits only for that
 //                    wave's flags — no collective barrier on the data path.
+//   gnn_peer_reduce_rows_f32   out[r] = relu?(src[0][row_lo + r] + ... + src[P-1][row_lo + r]): the ordered
+//                    cross-rank sum of P row buffers (this rank's and the peers' mappings), read over NVLink,
+//                    added left to right in fp32 — every rank that reduces a row gets the same bits.
 #include "common.cuh"
 
 using namespace gnn;
@@ -379,6 +382,56 @@ __global__ void peer_wait_kernel(const uint32_t* flags, int n_slots, int skip, u
   }
 }
 
+// ---- ordered row reduction over P sources -------------------------------------------------------
+struct ReduceArgs {
+  const float* src[kMaxPeers];
+  int32_t n_src;
+  int64_t ld_src;
+  int64_t row_lo;
+  int64_t n_rows;
+  int32_t F;
+  int32_t n_vec;   // float4 columns per row (0 on the scalar path)
+  int32_t per_row; // work items per row: n_vec + (F - 4 * n_vec) scalar tail columns
+  float* out;
+  int64_t ld_out;
+  int32_t relu;
+};
+
+// One thread per (row, float4 column) or (row, tail column).  The P sources are added in slot order, starting from
+// src[0]: ((s0 + s1) + s2) + ..., with no reassociation (plain adds, nothing to contract).
+__global__ void peer_reduce_rows_kernel(const ReduceArgs a) {
+  const int64_t total = a.n_rows * a.per_row;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t r = i / a.per_row;
+    const int c = (int)(i - r * a.per_row);
+    const int64_t s_off = (a.row_lo + r) * a.ld_src;
+    float* o = a.out + r * a.ld_out;
+    if (c < a.n_vec) {
+      float4 acc = __ldcg(reinterpret_cast<const float4*>(a.src[0] + s_off) + c);
+      for (int q = 1; q < a.n_src; ++q) {
+        const float4 v = __ldcg(reinterpret_cast<const float4*>(a.src[q] + s_off) + c);
+        acc.x += v.x;
+        acc.y += v.y;
+        acc.z += v.z;
+        acc.w += v.w;
+      }
+      if (a.relu) {
+        acc.x = acc.x < 0.f ? 0.f : acc.x;
+        acc.y = acc.y < 0.f ? 0.f : acc.y;
+        acc.z = acc.z < 0.f ? 0.f : acc.z;
+        acc.w = acc.w < 0.f ? 0.f : acc.w;
+      }
+      reinterpret_cast<float4*>(o)[c] = acc;
+    } else {
+      const int col = 4 * a.n_vec + (c - a.n_vec);
+      float acc = __ldcg(a.src[0] + s_off + col);
+      for (int q = 1; q < a.n_src; ++q) acc += __ldcg(a.src[q] + s_off + col);
+      if (a.relu) acc = acc < 0.f ? 0.f : acc;
+      o[col] = acc;
+    }
+  }
+}
+
 }  // namespace
 
 extern "C" {
@@ -582,6 +635,40 @@ int gnn_halo_push(const void* X, int64_t ldx, int32_t F, int32_t elem_size, cons
       halo_push_kernel<uint16_t, 4><<<(unsigned)grid, warps * 32, smem > 48 * 1024 ? 0 : smem, st>>>(a);
     }
   }
+  GNN_LAUNCH_CHECK();
+  return GNN_OK;
+}
+
+int gnn_peer_reduce_rows_f32(const float* const* src_host, int32_t n_src, int64_t ld_src, int32_t F, int64_t row_lo,
+                             int64_t row_hi, float* out, int64_t ld_out, int32_t relu, gnn_stream_t stream) {
+  GNN_REQUIRE(src_host && out, GNN_ERR_BAD_ARG, "null pointer");
+  GNN_REQUIRE(n_src >= 1 && n_src <= kMaxPeers, GNN_ERR_BAD_ARG, "n_src=%d outside [1, %d]", n_src, kMaxPeers);
+  GNN_REQUIRE(F > 0 && ld_src >= F && ld_out >= F, GNN_ERR_BAD_ARG, "bad width / leading dimension");
+  GNN_REQUIRE(row_lo >= 0 && row_hi >= row_lo, GNN_ERR_BAD_ARG, "bad row range [%lld, %lld)", (long long)row_lo,
+              (long long)row_hi);
+  ReduceArgs a{};
+  bool v16 = ld_src % 4 == 0 && ld_out % 4 == 0 && aligned_to(out, 16);
+  for (int q = 0; q < n_src; ++q) {
+    GNN_REQUIRE(src_host[q] != nullptr, GNN_ERR_BAD_ARG, "null pointer (source %d)", q);
+    a.src[q] = src_host[q];
+    v16 = v16 && aligned_to(src_host[q], 16);
+  }
+  if (row_hi == row_lo) return GNN_OK;
+  a.n_src = n_src;
+  a.ld_src = ld_src;
+  a.row_lo = row_lo;
+  a.n_rows = row_hi - row_lo;
+  a.F = F;
+  a.n_vec = v16 ? F / 4 : 0;
+  a.per_row = a.n_vec + (F - 4 * a.n_vec);
+  a.out = out;
+  a.ld_out = ld_out;
+  a.relu = relu ? 1 : 0;
+  const int64_t total = a.n_rows * a.per_row;
+  int64_t grid = (total + 255) / 256;
+  const int64_t cap = (int64_t)num_sms() * 8;
+  grid = grid > cap ? cap : grid;
+  peer_reduce_rows_kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(a);
   GNN_LAUNCH_CHECK();
   return GNN_OK;
 }

@@ -300,17 +300,89 @@ def spgemm_values(A: CSRGraph, a_val: torch.Tensor, B: CSRGraph, b_val: torch.Te
     return _SpgemmValuesFn.apply(a_val.contiguous(), b_val.contiguous(), A, B, C_pattern)
 
 
-def column_normalize(pattern: CSRGraph, val: torch.Tensor) -> torch.Tensor:
+def column_normalize(pattern: CSRGraph, val: torch.Tensor, reduce=None) -> torch.Tensor:
     """val [nnz, C] on `pattern` with every column of every channel divided by its sum (inf -> 0), autograd into
     val: the column normalisation of GTN's `norm` (GTN/models/GTN.py:7-19) on a pattern without its diagonal.  The
-    column sums are the ordered row sums of the cached transpose (one SpMM per channel), not an atomic scatter."""
+    column sums are the ordered row sums of the cached transpose (one SpMM per channel), not an atomic scatter.
+    reduce: on a row block of the pattern (partition.PartitionedRelationStack) the sums are partial, and
+    `reduce([n_cols, C])` returns the sums over every rank's rows (`rank_all_reduce`); None keeps them as they are."""
     t = pattern.transpose()
     ones = torch.ones((pattern.n_rows, 1), dtype=torch.float32, device=val.device)
     perm = pattern.perm_t
     sums = torch.cat([spmm_values(t, val[:, c][perm].contiguous(), ones) for c in range(val.shape[1])], dim=1)
+    if reduce is not None:
+        sums = reduce(sums)
     inv = sums.pow(-1)
     inv = torch.where(torch.isinf(inv), torch.zeros_like(inv), inv)
     return val * inv[pattern.col.long()]
+
+
+def peer_reduce_rows_raw(src_ptrs, ld_src: int, F: int, row_lo: int, row_hi: int, out: torch.Tensor,
+                         relu: bool = False) -> torch.Tensor:
+    """out[r, :F] = relu?(Σ_q src_q[row_lo + r, :F]) over the fp32 row buffers at the device addresses `src_ptrs`
+    (this process' or peers' IPC mappings), added in list order in fp32 (gnn_peer_reduce_rows_f32, no autograd)."""
+    import ctypes as C
+    _require_cuda(out)
+    if out.dtype != torch.float32 or out.dim() != 2 or out.shape[0] < row_hi - row_lo or out.shape[1] < F \
+            or (out.shape[1] > 1 and out.stride(1) != 1):
+        raise _lib.GnnError(f"peer_reduce_rows: fp32 out of at least [{row_hi - row_lo}, {F}] expected, got "
+                            f"{out.dtype} {tuple(out.shape)}")
+    if row_hi == row_lo:
+        return out
+    src = (C.c_void_p * len(src_ptrs))(*[int(p) for p in src_ptrs])
+    _lib.check(_lib.load().gnn_peer_reduce_rows_f32(src, len(src_ptrs), ld_src, F, row_lo, row_hi, _p(out), _ld(out),
+                                                    1 if relu else 0, _stream_ptr()), "gnn_peer_reduce_rows_f32")
+    return out
+
+
+class _RankAllReduceFn(torch.autograd.Function):
+    """y = Σ over the ranks of x, added in rank order (partition.PeerRowReduce.all_reduce at `site`); every rank gets
+    the same bits.  Backward: the same all-reduce of dy (site + "_bwd"), since every rank's y depends on every x."""
+
+    @staticmethod
+    def forward(ctx, x, red, site: str):
+        ctx.red, ctx.site = red, site
+        return red.all_reduce(site, x.contiguous())
+
+    @staticmethod
+    def backward(ctx, dy):
+        # always run: the reduction is a collective every rank takes part in
+        return ctx.red.all_reduce(ctx.site + "_bwd", dy.contiguous()), None, None
+
+
+def rank_all_reduce(red, site: str, x: torch.Tensor) -> torch.Tensor:
+    """Σ over the ranks of the fp32 [rows, F] partial x, in rank order, with autograd (collective, both ways)."""
+    _require_cuda(x)
+    return _RankAllReduceFn.apply(x, red, site)
+
+
+class _RowReduceScatterFn(torch.autograd.Function):
+    """y = relu?(Σ over the ranks of x)[own rows] (partition.PeerRowReduce.reduce_scatter, ReLU fused into the reduce).
+    Backward: dz = dy ⊙ [y > 0], then the all-gather of every rank's dz (site + "_bwd"): each rank's x reaches every
+    output row."""
+
+    @staticmethod
+    def forward(ctx, x, red, site: str, relu: bool):
+        y = red.reduce_scatter(site, x.contiguous(), relu)
+        ctx.red, ctx.site, ctx.relu = red, site, relu
+        if relu:
+            ctx.save_for_backward(y)
+        return y
+
+    @staticmethod
+    def backward(ctx, dy):
+        dz = dy
+        if ctx.relu:
+            (y,) = ctx.saved_tensors
+            dz = dy * (y > 0).to(dy.dtype)
+        # always run: the all-gather is a collective every rank takes part in
+        return ctx.red.all_gather(ctx.site + "_bwd", dz.contiguous()), None, None, None
+
+
+def row_reduce_scatter(red, site: str, x: torch.Tensor, relu: bool = False) -> torch.Tensor:
+    """relu?(Σ over the ranks of the fp32 [N, F] partial x), this rank's rows only, with autograd (collective)."""
+    _require_cuda(x)
+    return _RowReduceScatterFn.apply(x, red, site, relu)
 
 
 class _GcnAggregateFn(torch.autograd.Function):

@@ -18,14 +18,19 @@ On the message-passing path (re-designed):
     (P_1 = pattern(U·U), P_{l+1} = pattern(offdiag(P_l)·U)), `norm` is `functional.column_normalize` on the
     pattern without its diagonal, and the final `gcn_conv` runs on the cached pattern of (offdiag(H) + I)^T.
     Same parameters and state_dict as the dense path, which a dense `A` still takes unchanged.
+  * Across GPUs (DESIGN §4.10): `GTN_Model.forward(ps, X_local, target_local)` takes a
+    `partition.PartitionedRelationStack`, one rank's row block of every composed H_l.  The composition stays local;
+    the column sums of `norm` and the degrees of the final gcn_conv are partial sums over the rank's rows that a
+    rank-ordered all-reduce completes, and the gcn_conv's partial output is reduce-scattered with its ReLU fused.
 """
 import torch
 from torch import nn
 import torch.nn.functional as F
 
 from .. import _lib
-from ..functional import column_normalize, spgemm_values, spmm_values
+from ..functional import column_normalize, rank_all_reduce, row_reduce_scatter, spgemm_values, spmm_values
 from ..graph import CSRGraph, _require_cuda, _require_ids_in_range
+from ..partition import PartitionedRelationStack
 
 
 def norm(H, add=False):
@@ -68,19 +73,33 @@ def gcn_conv(X, H, weight):
     return _normalized_aggregate(g, vals.float(), XW)
 
 
-def _normalized_aggregate(g, vals, XW):
+def _normalized_aggregate(g, vals, XW, reduce=None):
     """The tail of `gcn_conv` on g = CSR of (offdiag(H) + I)^T with its values: divide by the column sums of
-    offdiag(H) + I (the row sums of g, an ordered SpMM against ones; inf -> 0) and aggregate XW, autograd into vals."""
+    offdiag(H) + I (the row sums of g, an ordered SpMM against ones; inf -> 0) and aggregate XW, autograd into vals.
+    vals [nnz] is one channel; vals [nnz, C] gives the C channels' outputs side by side, [n_rows, C * w].
+    reduce: on a row block (partition.PartitionedRelationStack) the degrees are partial sums, and `reduce([n_rows, C])`
+    returns the sums over every rank's rows; None keeps them."""
+    if vals.dim() == 1:
+        ones = torch.ones((g.n_cols, 1), dtype=torch.float32, device=vals.device)
+        deg = spmm_values(g, vals, ones)
+        deg = (deg if reduce is None else reduce(deg)).view(-1)
+        deg_inv = deg.pow(-1)
+        deg_inv = torch.where(deg_inv == float('inf'), torch.zeros_like(deg_inv), deg_inv)
+        return spmm_values(g, vals * deg_inv[g.edge_rows().long()], XW)
     ones = torch.ones((g.n_cols, 1), dtype=torch.float32, device=vals.device)
-    deg = spmm_values(g, vals, ones).view(-1)
+    deg = torch.cat([spmm_values(g, vals[:, c].contiguous(), ones) for c in range(vals.shape[1])], dim=1)
+    if reduce is not None:
+        deg = reduce(deg)
     deg_inv = deg.pow(-1)
     deg_inv = torch.where(deg_inv == float('inf'), torch.zeros_like(deg_inv), deg_inv)
-    return spmm_values(g, vals * deg_inv[g.edge_rows().long()], XW)
+    rows = g.edge_rows().long()
+    return torch.cat([spmm_values(g, vals[:, c] * deg_inv[rows, c], XW) for c in range(vals.shape[1])], dim=1)
 
 
-def _drop_diagonal(P):
-    """(pattern of P without its diagonal, int64 slots of P it keeps).  Setup only: one host read of the count."""
-    keep = P.edge_rows() != P.col
+def _drop_diagonal(P, lo=0):
+    """(pattern of P without its diagonal, int64 slots of P it keeps).  P may be the row block [lo, lo + n_rows) of a
+    square pattern: its diagonal is then (r, lo + r).  Setup only: one host read of the count."""
+    keep = (P.edge_rows() + lo) != P.col if lo else P.edge_rows() != P.col
     idx = torch.nonzero(keep).flatten()
     cum = torch.zeros(P.nnz + 1, dtype=torch.int64, device=P.device)
     torch.cumsum(keep.to(torch.int64), 0, out=cum[1:])
@@ -163,17 +182,23 @@ class RelationStack:
         edge of g reads (0 on the diagonal), diag the bool mask of the self-loops."""
         if num_layers not in self._gcn:
             self.patterns(num_layers)
-            D, idx = self._D[num_layers - 1], self._keep[num_layers - 1]
-            dev = D.device
-            rows = torch.cat([D.col.long(), torch.arange(self.n, device=dev)])          # j: row of H^T
-            cols = torch.cat([D.edge_rows().long(), torch.arange(self.n, device=dev)])  # i
-            g, perm = CSRGraph.from_coo(rows, cols, None, self.n, self.n, return_perm=True, validate=False)
-            diag = perm >= D.nnz
-            src = idx[torch.where(diag, torch.zeros_like(perm), perm)] if D.nnz else torch.zeros_like(perm)
-            _plan(g)
-            _plan(g.transpose())
-            self._gcn[num_layers] = (g, src, diag)
+            self._gcn[num_layers] = _gcn_pattern(self._D[num_layers - 1], self._keep[num_layers - 1], self.n)
         return self._gcn[num_layers]
+
+
+def _gcn_pattern(D, idx, n, lo=0):
+    """(g, src, diag) of the final gcn_conv on the rows [lo, lo + D.n_rows) of D_L (kept slots `idx` of P_L): g the CSR
+    of (D_L + I)^T restricted to those rows, [n, D.n_rows] (columns = row index i - lo, self-loops for j in the block),
+    src the int64 slot of P_L each edge of g reads (0 on the diagonal), diag the bool mask of the self-loops."""
+    n_loc, dev = D.n_rows, D.device
+    rows = torch.cat([D.col.long(), torch.arange(lo, lo + n_loc, device=dev)])   # j: row of H^T
+    cols = torch.cat([D.edge_rows().long(), torch.arange(n_loc, device=dev)])    # i - lo
+    g, perm = CSRGraph.from_coo(rows, cols, None, n, n_loc, return_perm=True, validate=False)
+    diag = perm >= D.nnz
+    src = idx[torch.where(diag, torch.zeros_like(perm), perm)] if D.nnz else torch.zeros_like(perm)
+    _plan(g)
+    _plan(g.transpose())
+    return g, src, diag
 
 
 def _plan(g):
@@ -215,12 +240,15 @@ class GTLayer(nn.Module):
         if self.first:
             self.conv2 = GTConv(in_channels, out_channels)
 
-    def forward_sparse(self, stack, P, H_=None, D=None):
+    def forward_sparse(self, stack, P, H_=None, D=None, U_rows=None):
         """One composition step on a RelationStack: H_ None gives a·b on P = pattern(U·U); else H_ holds the
-        normalised values on D (an earlier H without its diagonal) and the result is H_·a on P = pattern(D·U)."""
+        normalised values on D (an earlier H without its diagonal) and the result is H_·a on P = pattern(D·U).
+        U_rows = (rows [lo, hi) of U as a CSRGraph, first slot, end slot): a·b of those rows only, on P = their
+        block of pattern(U·U)."""
         a = self.conv1.forward_sparse(stack)
         if self.first:
-            H = spgemm_values(stack.U, a, stack.U, self.conv2.forward_sparse(stack), P)
+            A, a_A = (stack.U, a) if U_rows is None else (U_rows[0], a[U_rows[1]:U_rows[2]])
+            H = spgemm_values(A, a_A, stack.U, self.conv2.forward_sparse(stack), P)
             W = [(F.softmax(self.conv1.weight, dim=1)).detach(), (F.softmax(self.conv2.weight, dim=1)).detach()]
         else:
             H = spgemm_values(D, H_, stack.U, a, P)
@@ -273,6 +301,8 @@ class GTN_Model(nn.Module):
     def forward(self, A, X, target_x):
         if isinstance(A, RelationStack):
             return self._forward_sparse(A, X, target_x)
+        if isinstance(A, PartitionedRelationStack):
+            return self._forward_partitioned(A, X, target_x)
         A = A.unsqueeze(0).permute(0, 3, 1, 2)
         Ws = []
         for i in range(self.num_layers):
@@ -308,4 +338,34 @@ class GTN_Model(nn.Module):
                         for c in range(self.num_channels)], dim=1)
         X_ = F.relu(self.linear1(X_))
         y = self.linear2(X_[target_x])
+        return y, Ws
+
+    def _forward_partitioned(self, ps, X_local, target_local):
+        """forward() on this rank's rows: X_local = X[lo:hi], target_local = ids local to the block; returns
+        (logits of target_local, Ws).  Collective: every rank runs it, and its backward, in the same order."""
+        if (ps.num_edge, ps.num_layers, ps.width) != (self.num_edge, self.num_layers, self.num_channels * self.w_out):
+            raise ValueError(f"GTN_Model: the partitioned stack has {ps.num_edge} edge types, {ps.num_layers} layers "
+                             f"and width {ps.width}; the model {self.num_edge}, {self.num_layers} and "
+                             f"{self.num_channels * self.w_out} (num_channels * w_out)")
+        if X_local.dim() != 2 or X_local.shape[0] != ps.n_local:
+            raise ValueError(f"GTN_Model: X_local must hold this rank's {ps.n_local} rows, got {tuple(X_local.shape)}")
+        red = ps.reduce
+        Ws = []
+        H = None
+        for i in range(self.num_layers):
+            if i == 0:
+                H, W = self.layers[i].forward_sparse(ps.stack, ps.P[0], U_rows=ps.U_rows)
+            else:
+                Hn = column_normalize(ps.D[i - 1], H[ps.keep[i - 1]],
+                                      reduce=lambda x, site=f"norm{i}": rank_all_reduce(red, site, x))
+                H, W = self.layers[i].forward_sparse(ps.stack, ps.P[i], Hn, ps.D[i - 1])
+            Ws.append(W)
+        g, src, diag = ps.gcn
+        XW = torch.mm(X_local, self.weight)
+        one = torch.ones((), device=H.device, dtype=H.dtype)
+        vals = torch.where(diag.unsqueeze(1), one, H[src])
+        Y = _normalized_aggregate(g, vals, XW, reduce=lambda x: rank_all_reduce(red, "deg", x))  # partial [N, C*w_out]
+        X_ = row_reduce_scatter(red, "out", Y, relu=True)
+        X_ = F.relu(self.linear1(X_))
+        y = self.linear2(X_[target_local])
         return y, Ws

@@ -1214,14 +1214,15 @@ def build_metapath_view(plan: HaloPlan, rowptrs, cols, group=None) -> MetapathVi
 
 
 def metapath_row_plan(count, n: int, M: int, rank: int, world: int, max_nnz_per_rank: Optional[int] = None,
-                      group=None):
+                      group=None, what: str = "PartitionedMetapaths.from_relations", items: str = "metapaths"):
     """Row bounds of M metapath graphs over n nodes that no rank holds whole, and this rank's block rowptrs.
 
     `count(m, lo, hi)` returns the int64 rowptr [hi - lo + 1] of rows [lo, hi) of metapath m.  Each rank counts its
     rows of an even split (`shard_bounds`) for every metapath; one all_gather in rank order gives every rank all
     M·N per-row counts (8·M·N bytes), hence the global rowptr_m and bounds = balanced_bounds(Σ_m rowptr_m, world),
     the bounds `PartitionedMetapaths.from_global` would choose.  If some rank's block holds more than
-    `max_nnz_per_rank` entries, every rank raises the same GnnError (they all see every count).
+    `max_nnz_per_rank` entries, every rank raises the same GnnError (they all see every count); `what` and `items`
+    name the caller and what its M graphs are in that message.
     Returns (bounds, [rowptr_m of this rank's block, starting at 0])."""
     even = shard_bounds(n, world)
     lo, hi = even[rank], even[rank + 1]
@@ -1244,8 +1245,8 @@ def metapath_row_plan(count, n: int, M: int, rank: int, world: int, max_nnz_per_
     block_nnz = [int(x) for x in (rowptr[:, bounds[1:]] - rowptr[:, bounds[:-1]]).sum(0).tolist()]
     if max_nnz_per_rank is not None and max(block_nnz) > max_nnz_per_rank:
         over = ", ".join(f"rank {p}: {v}" for p, v in enumerate(block_nnz) if v > max_nnz_per_rank)
-        raise _lib.GnnError(f"PartitionedMetapaths.from_relations: a rank's block has more than max_nnz_per_rank = "
-                            f"{max_nnz_per_rank} entries over the {M} metapaths ({over}; "
+        raise _lib.GnnError(f"{what}: a rank's block has more than max_nnz_per_rank = "
+                            f"{max_nnz_per_rank} entries over the {M} {items} ({over}; "
                             f"{4 * max(block_nnz)} bytes of column ids)")
     b_lo, b_hi = bounds[rank], bounds[rank + 1]
     return bounds, [(rowptr[m, b_lo:b_hi + 1] - rowptr[m, b_lo]).contiguous() for m in range(M)]
@@ -1385,6 +1386,248 @@ class PartitionedMetapaths:
     def close(self):
         """Free the union's peer buffers (collective: every rank calls it)."""
         self.union.close()
+
+
+# ---- GTN's learned metapath composition over one row partition ----------------------------------
+
+class PeerRowReduce:
+    """Ordered cross-rank sums of fp32 row buffers over NVLink peer memory, one peer-mapped buffer per reduce SITE
+    (a named place in a step that runs every step, in the same order on every rank).
+
+      all_reduce(site, x [N, F])               every rank gets Σ_q x_q, all N rows
+      reduce_scatter(site, x [N, F], relu)     this rank gets relu?(Σ_q x_q) of its own rows [lo, hi)
+      all_gather(site, x_local [n_local, F])   every rank gets the owners' blocks stacked in rank order, [N, F]
+
+    A call writes this rank's operand into its own buffer of the site, raises its arrival flag on every peer, waits
+    for theirs, and reduces with `gnn_peer_reduce_rows_f32`, which adds the ranks' rows in rank order 0..P-1 in fp32
+    (the all-gather copies the owners' blocks with `gnn_peer_copy_async` instead); then it raises its "consumed" flag.
+    A buffer is rewritten only after every peer has raised "consumed" for the previous call of that site.  Every wait
+    is bounded: a lost peer sets a status word (`check_status`) instead of hanging the GPU.  Nothing is read back to
+    the host.  At world 1 no buffer exists: the reduction is the same kernel over one source, a copy (or ReLU).
+
+    sites: {name: (rows, cols)} of this rank's buffer; every rank passes the same names.  Construction is collective
+    (the buffers are exported with CUDA IPC and mapped by every peer)."""
+
+    def __init__(self, sites: Dict[str, tuple], bounds: List[int], rank: int, world: int, device, group=None,
+                 timeout_ms: int = 20000):
+        self.bounds, self.rank, self.world, self.group = [int(b) for b in bounds], int(rank), int(world), group
+        self.dev, self.timeout_ms = torch.device(device), int(timeout_ms)
+        self._status = torch.zeros(1, dtype=torch.int32, device=self.dev)
+        self._sites: Dict[str, dict] = {}
+        self._bufs: List[_PeerBuffer] = []
+        if self.world == 1:
+            return
+        try:
+            self._flags = _PeerBuffer(len(sites) * 256, self.rank, self.world, group)  # 32 arrive + 32 consumed slots
+            self._bufs.append(self._flags)
+            for k, (name, (rows, cols)) in enumerate(sorted(sites.items())):
+                ld = (int(cols) + 3) // 4 * 4  # 16-byte rows: the reduce kernel reads float4 vectors
+                buf = _PeerBuffer(max(int(rows), 1) * ld * 4, self.rank, self.world, group)
+                self._bufs.append(buf)
+                self._sites[name] = {"buf": buf, "rows": int(rows), "cols": int(cols), "ld": ld, "flag": k * 256,
+                                     "step": 0}
+        except Exception:
+            self.close()
+            raise
+
+    def _flag_ptrs(self, off: int):
+        return (C.c_void_p * self.world)(*[p + off for p in self._flags.ptrs])
+
+    def _signal(self, off: int, value: int, stream):
+        _lib.check(_lib.load().gnn_peer_signal(self._flag_ptrs(off), self.world, self.rank, self.rank,
+                                               value & 0xFFFFFFFF, stream.cuda_stream), "gnn_peer_signal")
+
+    def _wait(self, off: int, value: int, stream):
+        _lib.check(_lib.load().gnn_peer_wait(self._flags.own + off, self.world, self.rank, value & 0xFFFFFFFF,
+                                             self._status.data_ptr(), self.timeout_ms, stream.cuda_stream),
+                   "gnn_peer_wait")
+
+    def _site(self, name: str, x: torch.Tensor) -> dict:
+        site = self._sites.get(name)
+        if site is None:
+            raise _lib.GnnError(f"PeerRowReduce: no reduce site {name!r} (built for {sorted(self._sites)})")
+        if x.dtype != torch.float32 or x.dim() != 2 or x.shape[0] > site["rows"] or x.shape[1] > site["cols"]:
+            raise _lib.GnnError(f"PeerRowReduce: site {name!r} holds fp32 [{site['rows']}, {site['cols']}], got "
+                                f"{x.dtype} {tuple(x.shape)}")
+        return site
+
+    def _publish(self, site: dict, x: torch.Tensor, stream):
+        """x into this rank's buffer of the site once every peer has read its previous contents; then the flags."""
+        s = site["step"]
+        if s > 0:
+            self._wait(site["flag"] + 128, s, stream)
+        if x.shape[0]:
+            t = torch.as_tensor(_RawCudaBuffer(site["buf"].own, (x.shape[0], site["ld"])), device=self.dev)
+            t[:, :x.shape[1]].copy_(x)
+        self._signal(site["flag"], s + 1, stream)
+        self._wait(site["flag"], s + 1, stream)
+
+    def _done(self, site: dict, stream):
+        site["step"] += 1
+        self._signal(site["flag"] + 128, site["step"], stream)
+
+    def _reduce(self, name: str, x: torch.Tensor, row_lo: int, row_hi: int, relu: bool) -> torch.Tensor:
+        from .functional import peer_reduce_rows_raw
+        F = int(x.shape[1])
+        out = torch.empty((row_hi - row_lo, F), dtype=torch.float32, device=self.dev)
+        if self.world == 1:
+            x = x.contiguous()
+            return peer_reduce_rows_raw([x.data_ptr()], F, F, row_lo, row_hi, out, relu)
+        site = self._site(name, x)
+        stream = torch.cuda.current_stream(self.dev)
+        self._publish(site, x, stream)
+        peer_reduce_rows_raw(site["buf"].ptrs, site["ld"], F, row_lo, row_hi, out, relu)
+        self._done(site, stream)
+        return out
+
+    def all_reduce(self, name: str, x: torch.Tensor) -> torch.Tensor:
+        return self._reduce(name, x, 0, int(x.shape[0]), False)
+
+    def reduce_scatter(self, name: str, x: torch.Tensor, relu: bool = False) -> torch.Tensor:
+        return self._reduce(name, x, self.bounds[self.rank], self.bounds[self.rank + 1], relu)
+
+    def all_gather(self, name: str, x_local: torch.Tensor) -> torch.Tensor:
+        F = int(x_local.shape[1])
+        if self.world == 1:
+            return x_local.contiguous().clone()
+        site = self._site(name, x_local)
+        if site["ld"] != site["cols"] or F != site["cols"]:
+            raise _lib.GnnError(f"PeerRowReduce.all_gather: site {name!r} needs contiguous rows of {F} columns")
+        stream = torch.cuda.current_stream(self.dev)
+        out = torch.empty((self.bounds[-1], F), dtype=torch.float32, device=self.dev)
+        self._publish(site, x_local, stream)
+        lib, row_bytes = _lib.load(), F * 4
+        for q in range(self.world):
+            rows = self.bounds[q + 1] - self.bounds[q]
+            if rows:
+                _lib.check(lib.gnn_peer_copy_async(out.data_ptr() + self.bounds[q] * row_bytes, site["buf"].ptrs[q],
+                                                   rows * row_bytes, stream.cuda_stream), "gnn_peer_copy_async")
+        self._done(site, stream)
+        return out
+
+    def check_status(self):
+        """Raise if a flag wait of an earlier call timed out (synchronises)."""
+        s = int(self._status.item())
+        if s:
+            raise _lib.GnnError(f"rank {self.rank}: timed out waiting for the reduce flag of peer {s - 1}")
+
+    def close(self):
+        """Free the peer buffers (collective)."""
+        if self._bufs:
+            torch.cuda.synchronize(self.dev)
+            if dist.is_initialized():
+                dist.barrier(group=self.group)
+            for b in self._bufs:
+                b.close()
+            self._bufs = []
+            self._sites = {}
+
+
+GTN_MAX_CHANNELS = 8  # gnn_spgemm_values_f32 takes up to 8 channels: the [N, C] reduce sites hold 8 columns
+
+
+class PartitionedRelationStack:
+    """One rank's share of a `layers.gtn.RelationStack` that every rank holds, for `GTN_Model.forward(ps, X_local,
+    target_local)`: rank p owns rows [lo, hi) of every composed H_l (the same bounds for all layers), of X and of the
+    output.  The union pattern U and its values V stay whole on every rank (they are small).
+
+      P_1 = pattern(U[lo:hi]·U),  D_l = P_l without the entries (r, lo + r),  P_{l+1} = pattern(D_l·U)
+      gcn   the CSR of (D_L + I)ᵀ restricted to the local rows: N rows, columns the local row index i - lo, self-loops
+            for j in [lo, hi)
+
+    The composition needs no communication.  GTN's column normalisation and the degrees of its final gcn_conv sum
+    along columns, so each rank computes partial [N, C] sums over its rows and `PeerRowReduce.all_reduce` adds them in
+    rank order; the gcn_conv aggregates only the local rows' XW into a partial [N, C·w_out], which a reduce-scatter with
+    the ReLU fused turns into this rank's rows (its backward is the all-gather of the output gradient).
+
+    Bounds: every rank builds the chain P_1 .. P_L for its rows of an even split (`shard_bounds`), filling
+    P_1 .. P_{L-1} and counting P_L; `metapath_row_plan` (one "metapath" per layer) exchanges the per-row counts and
+    returns bounds balanced on Σ_l rowptr_l and this rank's rowptrs of every layer, from which the final block is
+    filled layer by layer without counting again.  A block of more than `max_nnz_per_rank` entries over the L layers
+    raises the same GnnError on every rank.
+
+    width = num_channels * w_out of the model (it sizes the output sites).  Collective construction; every rank runs
+    the same sequence of forward and backward calls (the reduce sites count calls with flags in peer memory)."""
+
+    def __init__(self, stack, rank: int, world: int, num_layers: int, width: int, max_nnz_per_rank: Optional[int] = None,
+                 group=None, timeout_ms: int = 20000):
+        from .graph import CSRGraph, _pattern_count, _pattern_fill
+        from .layers.gtn import _drop_diagonal, _gcn_pattern, _plan
+        L, n = int(num_layers), stack.n
+        if L < 1 or int(width) <= 0:
+            raise ValueError(f"PartitionedRelationStack: num_layers >= 1 and width > 0 needed, got {L}, {width}")
+        if int(world) > 1 and int(width) % 4:
+            raise ValueError(f"PartitionedRelationStack: width {width} must be a multiple of 4 across ranks "
+                             "(the output's all-gather copies whole 16-byte rows)")
+        self.stack, self.rank, self.world, self.group = stack, int(rank), int(world), group
+        self.num_layers, self.width, self.num_edge, self.n = L, int(width), stack.num_edge, n
+        U = stack.U
+        U.transpose()  # B of every product is read through its transpose
+        chain = {}
+
+        def count(m, lo, hi):
+            """rowptr of rows [lo, hi) of P_{m+1}; P_1 .. P_{L-1} of the even split are filled for the next count."""
+            A, a_lo, a_hi = (U, lo, hi) if m == 0 else (chain["D"], 0, hi - lo)
+            rp = _pattern_count(A, U, a_lo, a_hi, False)
+            if m < L - 1:
+                P = CSRGraph(rp, _pattern_fill(A, U, a_lo, a_hi, False, rp, int(rp[-1].item())), None, hi - lo, n)
+                chain["D"] = _drop_diagonal(P, lo)[0]
+            return rp
+
+        self.bounds, rowptrs = metapath_row_plan(count, n, L, self.rank, self.world, max_nnz_per_rank, group,
+                                                 what="PartitionedRelationStack", items="layers")
+        chain.clear()  # the even split's fills are not needed any more
+        lo, hi = self.row_range
+        n_loc = hi - lo
+        u0, u1 = int(U.rowptr[lo].item()), int(U.rowptr[hi].item())
+        self.U_rows = (CSRGraph(U.rowptr[lo:hi + 1] - u0, U.col[u0:u1], None, n_loc, n), u0, u1)
+        _plan(self.U_rows[0])
+        _plan(self.U_rows[0].transpose())
+        self.P, self.D, self.keep = [], [], []
+        A, a_lo, a_hi = U, lo, hi
+        for rp in rowptrs:
+            P = CSRGraph(rp, _pattern_fill(A, U, a_lo, a_hi, False, rp, int(rp[-1].item())), None, n_loc, n)
+            D, keep = _drop_diagonal(P, lo)
+            for g in (P, D):  # transposes the backward and the column sums walk, and their SpMM plans
+                _plan(g)
+                _plan(g.transpose())
+            self.P.append(P)
+            self.D.append(D)
+            self.keep.append(keep)
+            A, a_lo, a_hi = D, 0, n_loc
+        self.gcn = _gcn_pattern(self.D[-1], self.keep[-1], n, lo)
+        sites = {"deg": (n, GTN_MAX_CHANNELS), "deg_bwd": (n, GTN_MAX_CHANNELS), "out": (n, self.width),
+                 "out_bwd": (max(self.bounds[p + 1] - self.bounds[p] for p in range(self.world)), self.width)}
+        for l in range(1, L):
+            sites[f"norm{l}"] = sites[f"norm{l}_bwd"] = (n, GTN_MAX_CHANNELS)
+        self.reduce = PeerRowReduce(sites, self.bounds, self.rank, self.world, U.device, group, timeout_ms)
+
+    @property
+    def row_range(self):
+        return self.bounds[self.rank], self.bounds[self.rank + 1]
+
+    @property
+    def n_local(self) -> int:
+        return self.bounds[self.rank + 1] - self.bounds[self.rank]
+
+    @property
+    def nnz_per_layer(self) -> List[int]:
+        """nnz of this rank's block of every P_l."""
+        return [P.nnz for P in self.P]
+
+    def local_index(self, idx_global: torch.Tensor) -> torch.Tensor:
+        """The global node ids of `idx_global` this rank owns, as local row indices."""
+        lo, hi = self.row_range
+        idx = idx_global.to(torch.int64)
+        return idx[(idx >= lo) & (idx < hi)] - lo
+
+    def check_status(self):
+        """Raise if a flag wait of an earlier step timed out (synchronises)."""
+        self.reduce.check_status()
+
+    def close(self):
+        """Free the peer buffers (collective: every rank calls it)."""
+        self.reduce.close()
 
 
 # ---- a feature table sharded across ranks ---------------------------------------------------

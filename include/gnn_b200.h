@@ -759,6 +759,19 @@ int gnn_peer_signal(uint32_t* const* peer_flags_host /*[n_peers] device ptrs*/, 
 int gnn_peer_wait(const uint32_t* flags, int32_t n_slots, int32_t skip_slot, uint32_t value,
                   uint32_t* status /*nullable device word*/, int64_t timeout_ms, gnn_stream_t stream);
 
+/* Ordered row reduction over n_src (1..16) fp32 row buffers of this address space (this rank's and the peers'
+ * gnn_peer_open mappings), each [*, ld_src] with F columns:
+ *   out[r][c] = relu?(src[0][row_lo + r][c] + src[1][row_lo + r][c] + ... + src[n_src - 1][row_lo + r][c])
+ * for r in [0, row_hi - row_lo), c in [0, F), out [*, ld_out].  The adds run left to right in fp32, so every rank
+ * that reduces a row gets the same bits; relu != 0 clamps the sum at 0.  Reads are 16-byte vectors when ld_src and
+ * ld_out are multiples of 4 and every pointer is 16-byte aligned (a scalar tail covers F % 4), scalar otherwise; no
+ * store leaves the output's F columns or rows.  One source is a plain copy (or ReLU).  The caller orders the reads
+ * after the sources are written (gnn_peer_wait).  Null pointers and bad sizes return GNN_ERR_BAD_ARG before any
+ * CUDA call; an empty row range launches nothing. */
+int gnn_peer_reduce_rows_f32(const float* const* src_host /*[n_src] device ptrs*/, int32_t n_src, int64_t ld_src,
+                             int32_t F, int64_t row_lo, int64_t row_hi, float* out, int64_t ld_out, int32_t relu,
+                             gnn_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif
