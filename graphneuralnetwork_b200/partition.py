@@ -37,6 +37,7 @@ from __future__ import annotations
 
 import ctypes as C
 from dataclasses import dataclass, field
+from itertools import accumulate
 from typing import Dict, List, Optional
 
 import torch
@@ -91,6 +92,17 @@ def split_columns(rowptr, col, val, lo: int, hi: int):
     val_loc = None if val is None else val[is_loc]
     val_rem = None if val is None else val[rem]
     return rowptr_loc, col_loc, val_loc, rowptr_rem, col_rem_global, val_rem
+
+
+def _offsets(counts) -> List[int]:
+    """Exclusive prefix sum of `counts`, with the total appended."""
+    return list(accumulate(counts, initial=0))
+
+
+def _local_index(idx: torch.Tensor, lo: int, hi: int) -> torch.Tensor:
+    """The ids of `idx` in [lo, hi) as row indices local to that block (ascending where idx is)."""
+    idx = idx.to(torch.int64)
+    return idx[(idx >= lo) & (idx < hi)] - lo
 
 
 def select_rows(rowptr: torch.Tensor, col: torch.Tensor, val: Optional[torch.Tensor], rows: torch.Tensor):
@@ -164,16 +176,10 @@ class HaloPlan:
         return int(self.halo_ids.numel())
 
     def send_off(self) -> List[int]:
-        off = [0]
-        for c in self.send_counts:
-            off.append(off[-1] + c)
-        return off
+        return _offsets(self.send_counts)
 
     def recv_off(self) -> List[int]:
-        off = [0]
-        for c in self.recv_counts:
-            off.append(off[-1] + c)
-        return off
+        return _offsets(self.recv_counts)
 
 
 def choose_two_pass_chunks(K: int, F: int, elem: int, nnz_p1_base: int, rows_interior: int, m_rows, m_nnz_loc, m_nnz_rem,
@@ -222,57 +228,68 @@ def choose_two_pass_chunks(K: int, F: int, elem: int, nnz_p1_base: int, rows_int
     return best[0], report
 
 
-def _auto_schedule(rowptr, col, bounds, rank, world, group, F, elem_size):
-    """(K, c0) for all ranks: statistics at the finest wave count, coarsened for the smaller K (the chunk
-    boundaries are nested), one all_reduce of the modelled step times."""
-    dev = col.device
-    lo, hi = bounds[rank], bounds[rank + 1]
-    n_loc = hi - lo
-    col = col.to(torch.int64)
-    KM = AUTO_MAX_WAVES
-    is_loc = (col >= lo) & (col < hi)
-    csum = torch.zeros(col.numel() + 1, dtype=torch.int64, device=dev)
-    torch.cumsum(is_loc.to(torch.int64), 0, out=csum[1:])
-    loc_deg = csum[rowptr[1:]] - csum[rowptr[:-1]]
-    deg = rowptr[1:] - rowptr[:-1]
-    rem_deg = deg - loc_deg
-    del csum
-    total = int(rowptr[-1].item())
-    tg = torch.tensor([total * k // KM for k in range(1, KM)], dtype=torch.int64, device=dev)
-    cuts = [0] + torch.searchsorted(rowptr, tg).clamp_(0, n_loc).tolist() + [n_loc]
-    for i in range(1, len(cuts)):
-        cuts[i] = max(cuts[i], cuts[i - 1])
+def _chunk_stats(chunk_bounds: List[int], rowptr_loc: torch.Tensor, rem_deg: torch.Tensor):
+    """The MIXED rows (rows with a remote column) of every row chunk: ([row count], [their local nnz], [their remote
+    nnz]), lists over the chunks; and the INTERIOR rows of the whole block: (row count, nnz)."""
+    loc_deg = rowptr_loc[1:] - rowptr_loc[:-1]
     mixed = rem_deg > 0
     m_rows, m_loc, m_rem = [], [], []
-    for w in range(KM):
-        a, b = cuts[w], cuts[w + 1]
+    for a, b in zip(chunk_bounds[:-1], chunk_bounds[1:]):
         mw = mixed[a:b]
         m_rows.append(int(mw.sum().item()))
         m_loc.append(int(loc_deg[a:b][mw].sum().item()))
         m_rem.append(int(rem_deg[a:b].sum().item()))
-    rows_interior = n_loc - sum(m_rows)
-    nnz_interior = int(loc_deg.sum().item()) - sum(m_loc)
-    # halo rows per finest wave (first chunk that needs them)
-    col_rem = col[~is_loc]
-    del is_loc
-    uniq, inverse = torch.unique(col_rem, sorted=True, return_inverse=True)
-    wave_rows = [0] * KM
-    if uniq.numel():
-        row_of_rem = torch.repeat_interleave(torch.arange(n_loc, dtype=torch.int64, device=dev), rem_deg,
-                                             output_size=int(col_rem.numel()))
-        chunk_of_rem = torch.bucketize(row_of_rem, torch.tensor(cuts[1:-1], dtype=torch.int64, device=dev), right=True)
-        first = torch.full((uniq.numel(),), KM, dtype=torch.int64, device=dev)
-        first.scatter_reduce_(0, inverse, chunk_of_rem, reduce="amin", include_self=True)
-        wave_rows = torch.bincount(first, minlength=KM).tolist()[:KM]
-        del row_of_rem, chunk_of_rem, first
-    del uniq, inverse, col_rem
+    return (m_rows, m_loc, m_rem), (rem_deg.numel() - sum(m_rows), int(loc_deg.sum().item()) - sum(m_loc))
+
+
+def _coarsen(per_chunk: List[int], K: int) -> List[int]:
+    """Per-chunk sums at K chunks from the sums at a multiple of K chunks cut by `balanced_bounds` (the cuts for K
+    are every (len/K)-th cut of the finer ones: total*k//K == total*(k*g)//(K*g))."""
+    g = len(per_chunk) // K
+    return [sum(per_chunk[w * g:(w + 1) * g]) for w in range(K)]
+
+
+def _first_chunk(chunk_bounds: List[int], rem_deg: torch.Tensor, inverse: torch.Tensor, n_uniq: int) -> torch.Tensor:
+    """For every distinct remote column (`inverse` maps each remote entry, in CSR order, to its index among the
+    n_uniq), the first row chunk that reads it."""
+    K, dev = len(chunk_bounds) - 1, rem_deg.device
+    if K == 1 or n_uniq == 0:
+        return torch.zeros(n_uniq, dtype=torch.int64, device=dev)
+    row_of_rem = torch.repeat_interleave(torch.arange(rem_deg.numel(), dtype=torch.int64, device=dev), rem_deg,
+                                         output_size=int(inverse.numel()))
+    chunk_of_rem = torch.bucketize(row_of_rem, torch.tensor(chunk_bounds[1:-1], dtype=torch.int64, device=dev),
+                                   right=True)
+    del row_of_rem
+    first = torch.full((n_uniq,), K, dtype=torch.int64, device=dev)
+    first.scatter_reduce_(0, inverse, chunk_of_rem, reduce="amin", include_self=True)
+    return first
+
+
+def _combined_columns(plan: "HaloPlan", col: torch.Tensor) -> torch.Tensor:
+    """The int32 column ids of the block `plan` was built from (GLOBAL ids `col`) in the COMBINED column space:
+    local column c -> c - lo, remote column -> n_local + its halo slot."""
+    lo, hi = plan.bounds[plan.rank], plan.bounds[plan.rank + 1]
+    col64 = col.to(torch.int64)
+    is_loc = (col64 >= lo) & (col64 < hi)
+    del col64
+    comb = torch.empty(col.numel(), dtype=torch.int32, device=col.device)
+    comb[is_loc] = plan.col_loc.to(col.device)
+    comb[~is_loc] = plan.col_rem.to(col.device) + (hi - lo)
+    return comb
+
+
+def _auto_schedule(per_chunk, interior, first_chunk, world, group, F, elem_size):
+    """(K, c0) for all ranks from this rank's statistics at the finest wave count (`_chunk_stats` and `_first_chunk`
+    at AUTO_MAX_WAVES chunks), coarsened for the smaller K, and one all_reduce of the modelled step times."""
+    KM = AUTO_MAX_WAVES
+    rows_interior, nnz_interior = interior
+    wave_rows = torch.bincount(first_chunk, minlength=KM).tolist()[:KM]  # halo rows per finest wave
     ks = [k for k in (1, 2, 4, 8) if k <= KM]
-    times = torch.full((len(ks), KM + 1), 1e9, dtype=torch.float64, device=dev)
+    times = torch.full((len(ks), KM + 1), 1e9, dtype=torch.float64, device=first_chunk.device)
     for ki, K in enumerate(ks):
-        gsz = KM // K
-        merge = lambda v: [sum(v[w * gsz:(w + 1) * gsz]) for w in range(K)]
-        _, rep_k = choose_two_pass_chunks(K, F, elem_size, nnz_interior, rows_interior, merge(m_rows), merge(m_loc),
-                                          merge(m_rem), [r * F * elem_size for r in merge(wave_rows)], world)
+        m_rows, m_loc, m_rem = (_coarsen(v, K) for v in per_chunk)
+        _, rep_k = choose_two_pass_chunks(K, F, elem_size, nnz_interior, rows_interior, m_rows, m_loc, m_rem,
+                                          [r * F * elem_size for r in _coarsen(wave_rows, K)], world)
         for c0 in range(K + 1):
             times[ki, c0] = rep_k[f"c0={c0}"]
     dist.all_reduce(times, group=group)
@@ -293,40 +310,29 @@ def build_halo_plan(rowptr: torch.Tensor, col: torch.Tensor, val: Optional[torch
       and the (K, c0) with the smallest sum is used by all of them.
     two_pass_chunks: c0 in [0, waves] (None: chosen by `choose_two_pass_chunks` for feature width F)."""
     dev = col.device
-    if waves is None and world > 1:
-        waves, two_pass_chunks, auto_report = _auto_schedule(rowptr, col, bounds, rank, world, group, F, elem_size)
-    else:
-        auto_report = None
-    K = max(int(waves or 1), 1) if world > 1 else 1
     lo, hi = bounds[rank], bounds[rank + 1]
     n_loc = hi - lo
     col = col.to(torch.int64)
     rowptr_loc, col_loc, val_loc, rowptr_rem, col_rem_g, val_rem = split_columns(rowptr, col, val, lo, hi)
-    # K row chunks of (nearly) equal nnz
-    total = int(rowptr[-1].item())
-    if K > 1:
-        tg = torch.tensor([total * k // K for k in range(1, K)], dtype=torch.int64, device=dev)
-        cuts = torch.searchsorted(rowptr, tg).clamp_(0, n_loc).tolist()
-    else:
-        cuts = []
-    chunk_bounds = [0] + [int(c) for c in cuts] + [n_loc]
-    for i in range(1, len(chunk_bounds)):
-        chunk_bounds[i] = max(chunk_bounds[i], chunk_bounds[i - 1])
     rem_deg = rowptr_rem[1:] - rowptr_rem[:-1]
     uniq, inverse = torch.unique(col_rem_g, sorted=True, return_inverse=True)  # de-duplicated halo
+    stats = None  # _chunk_stats at the plan's K, once known
+    if waves is None and world > 1:
+        cuts = balanced_bounds(rowptr, AUTO_MAX_WAVES)
+        per_chunk, interior = _chunk_stats(cuts, rowptr_loc, rem_deg)
+        first = _first_chunk(cuts, rem_deg, inverse, uniq.numel())
+        K, two_pass_chunks, auto_report = _auto_schedule(per_chunk, interior, first, world, group, F, elem_size)
+        g = AUTO_MAX_WAVES // K
+        chunk_bounds, first_wave = cuts[::g], first // g
+        stats = [_coarsen(v, K) for v in per_chunk], interior
+        del first
+    else:
+        auto_report = None
+        K = max(int(waves or 1), 1) if world > 1 else 1
+        chunk_bounds = balanced_bounds(rowptr, K)  # K row chunks of (nearly) equal nnz
+        first_wave = _first_chunk(chunk_bounds, rem_deg, inverse, uniq.numel())
     edges = torch.tensor(bounds[1:-1], dtype=torch.int64, device=dev)
     owner = torch.bucketize(uniq, edges, right=True) if world > 1 else torch.zeros_like(uniq)
-    if K > 1 and uniq.numel():
-        row_of_rem = torch.repeat_interleave(torch.arange(n_loc, dtype=torch.int64, device=dev), rem_deg,
-                                             output_size=int(col_rem_g.numel()))
-        cb = torch.tensor(chunk_bounds[1:-1], dtype=torch.int64, device=dev)
-        chunk_of_rem = torch.bucketize(row_of_rem, cb, right=True)
-        del row_of_rem
-        first_wave = torch.full((uniq.numel(),), K, dtype=torch.int64, device=dev)
-        first_wave.scatter_reduce_(0, inverse, chunk_of_rem, reduce="amin", include_self=True)
-        del chunk_of_rem
-    else:
-        first_wave = torch.zeros_like(uniq)
     key = owner * K + first_wave
     order = torch.argsort(key, stable=True)  # uniq is ascending: ties keep id order
     slot_of_uniq = torch.empty_like(order)
@@ -337,9 +343,7 @@ def build_halo_plan(rowptr: torch.Tensor, col: torch.Tensor, val: Optional[torch
                 torch.zeros(world * K, dtype=torch.int64, device=dev)).view(world, K)
     recv_wave_counts = [[int(x) for x in r] for r in counts2d.tolist()]
     recv_counts = [sum(r) for r in recv_wave_counts]
-    recv_off = [0]
-    for c in recv_counts:
-        recv_off.append(recv_off[-1] + c)
+    recv_off = _offsets(recv_counts)
     plan_kw = dict(rank=rank, world=world, bounds=bounds, waves=K, chunk_bounds=chunk_bounds, rowptr_loc=rowptr_loc,
                    col_loc=col_loc, val_loc=val_loc, rowptr_rem=rowptr_rem, col_rem=col_rem, val_rem=val_rem,
                    halo_ids=halo_ids, recv_counts=recv_counts, recv_wave_counts=recv_wave_counts)
@@ -359,10 +363,7 @@ def build_halo_plan(rowptr: torch.Tensor, col: torch.Tensor, val: Optional[torch
     req_in = torch.empty(int(sum(send_counts)), dtype=torch.int64, device=dev)
     dist.all_to_all_single(req_in, req_out, output_split_sizes=send_counts, input_split_sizes=recv_counts, group=group)
     # backward: owner q tells requester p where p's segment starts in q's send list
-    send_off = [0]
-    for c in send_counts:
-        send_off.append(send_off[-1] + c)
-    so_out = torch.tensor(send_off[:world], dtype=torch.int64, device=dev)
+    so_out = torch.tensor(_offsets(send_counts)[:world], dtype=torch.int64, device=dev)
     so_in = torch.empty_like(so_out)
     dist.all_to_all_single(so_in, so_out, group=group)
     plan = HaloPlan(two_pass_chunks=K, send_rows=req_in.to(torch.int32), send_counts=send_counts,
@@ -371,17 +372,9 @@ def build_halo_plan(rowptr: torch.Tensor, col: torch.Tensor, val: Optional[torch
     if not consumers:
         return plan
     # ---- row classes and the consumers of the step --------------------------------------------
-    mixed = rem_deg > 0
-    loc_deg = rowptr_loc[1:] - rowptr_loc[:-1]
-    m_rows, m_nnz_loc, m_nnz_rem = [], [], []
-    for w in range(K):
-        a, b = chunk_bounds[w], chunk_bounds[w + 1]
-        mw = mixed[a:b]
-        m_rows.append(int(mw.sum().item()))
-        m_nnz_loc.append(int(loc_deg[a:b][mw].sum().item()))
-        m_nnz_rem.append(int(rem_deg[a:b].sum().item()))
-    rows_interior = n_loc - sum(m_rows)
-    nnz_interior = int(loc_deg.sum().item()) - sum(m_nnz_loc)
+    if stats is None:
+        stats = _chunk_stats(chunk_bounds, rowptr_loc, rem_deg)
+    (m_rows, m_nnz_loc, m_nnz_rem), (rows_interior, nnz_interior) = stats
     row_b = F * elem_size
     wave_bytes = [max(sum(recv_wave_counts[q][w] for q in range(world)), sum(send_wave_counts[p][w] for p in range(world)))
                   * row_b for w in range(K)]
@@ -401,6 +394,7 @@ def build_halo_plan(rowptr: torch.Tensor, col: torch.Tensor, val: Optional[torch
     plan.model = dict(report, chosen=c0, model_choice=c0_model, rows_interior=rows_interior,
                       rows_mixed=sum(m_rows), nnz_interior=nnz_interior)
     cut_row = chunk_bounds[c0]  # mixed rows at or beyond this row are single-pass
+    mixed = rem_deg > 0
     all_rows = torch.arange(n_loc, dtype=torch.int64, device=dev)
     # P1: local columns of every row except the single-pass mixed rows.  The two-pass mixed rows come first (their
     # remote pass adds the rest, so a fused epilogue skips them: Consumer.epilogue_skip), then the interior rows.
@@ -415,14 +409,7 @@ def build_halo_plan(rowptr: torch.Tensor, col: torch.Tensor, val: Optional[torch
         rp, cc, vv = select_rows(rowptr_loc, col_loc, val_loc, rows)
         plan.p1 = (Consumer("local", rp, cc, vv, rows.to(torch.int32), n_loc, epilogue_skip=n_first)
                    if rows.numel() else None)
-    # combined column space of the single-pass rows: local col j -> j, remote -> n_loc + halo slot
-    col_comb = None
-    if c0 < K:
-        is_loc = (col >= lo) & (col < hi)
-        col_comb = torch.empty(col.numel(), dtype=torch.int32, device=dev)
-        col_comb[is_loc] = col_loc
-        col_comb[~is_loc] = col_rem + n_loc
-        del is_loc
+    col_comb = _combined_columns(plan, col) if c0 < K else None  # the column space of the single-pass rows
     plan.p2 = []
     for w in range(K):
         a, b = chunk_bounds[w], chunk_bounds[w + 1]
@@ -464,14 +451,8 @@ def build_attention_view(plan: HaloPlan, rowptr: torch.Tensor, col: torch.Tensor
     """The attention view of the block `plan` was built from (rowptr over the rank's rows, GLOBAL column ids).
     Collective when world > 1: one all_gather of (nnz, has-empty-row) per rank gives the exclusive scan of the
     ranks' nnz and the global empty-row flag."""
-    lo, hi = plan.bounds[plan.rank], plan.bounds[plan.rank + 1]
-    n_loc = hi - lo
-    col64 = col.to(torch.int64)
-    is_loc = (col64 >= lo) & (col64 < hi)
-    del col64
-    col_comb = torch.empty(col.numel(), dtype=torch.int32, device=col.device)
-    col_comb[is_loc] = plan.col_loc.to(col.device)
-    col_comb[~is_loc] = plan.col_rem.to(col.device) + n_loc
+    n_loc = plan.n_local
+    col_comb = _combined_columns(plan, col)
     empty = bool((rowptr[1:] == rowptr[:-1]).any().item()) if n_loc > 0 else False
     base, any_empty = 0, empty
     if plan.world > 1:
@@ -570,6 +551,55 @@ class _PeerBuffer:
 _TORCH_TYPESTR = {torch.float32: "<f4", torch.bfloat16: "<u2"}
 
 
+def _raw_view(ptr: int, rows: int, ld: int, dtype: torch.dtype, device) -> torch.Tensor:
+    """[rows, ld] tensor of `dtype` over the device memory at `ptr` (zero-copy)."""
+    t = torch.as_tensor(_RawCudaBuffer(ptr, (rows, ld), _TORCH_TYPESTR[dtype]), device=device)
+    return t.view(dtype) if dtype != torch.float32 else t
+
+
+def _close_peer_buffers(bufs: List[_PeerBuffer], device, group):
+    """Free peer buffers (collective): every rank finishes its queued work, which may read a peer's buffer or be read
+    from, before any mapping is closed."""
+    if bufs:
+        torch.cuda.synchronize(device)
+        if dist.is_initialized():
+            dist.barrier(group=group)
+        for b in bufs:
+            b.close()
+
+
+class _PeerFlags:
+    """Monotonic flags in peer memory: `n_arrays` arrays of 32 uint32 slots (128 bytes) in one peer buffer per rank,
+    slot q of an array written by rank q only.  `signal(a, v)` sets this rank's slot of array a to v on every rank;
+    `wait(a, v)` holds `stream` until every peer's slot of this rank's array a has reached v.  Values wrap at 2^32.
+    Every wait is bounded by timeout_ms: a lost peer sets the status word (`check_status`) instead of hanging the
+    GPU.  Construction is collective."""
+
+    def __init__(self, n_arrays: int, rank: int, world: int, group, device, timeout_ms: int):
+        self.rank, self.world, self.timeout_ms = rank, world, int(timeout_ms)
+        self.status = torch.zeros(1, dtype=torch.int32, device=device)
+        self.buf = _PeerBuffer(n_arrays * 128, rank, world, group)
+
+    def ptrs(self, array: int):
+        """Device pointers of flag array `array` on every rank."""
+        return (C.c_void_p * self.world)(*[p + array * 128 for p in self.buf.ptrs])
+
+    def signal(self, array: int, value: int, stream):
+        _lib.check(_lib.load().gnn_peer_signal(self.ptrs(array), self.world, self.rank, self.rank,
+                                               value & 0xFFFFFFFF, stream.cuda_stream), "gnn_peer_signal")
+
+    def wait(self, array: int, value: int, stream):
+        _lib.check(_lib.load().gnn_peer_wait(self.buf.own + array * 128, self.world, self.rank, value & 0xFFFFFFFF,
+                                             self.status.data_ptr(), self.timeout_ms, stream.cuda_stream),
+                   "gnn_peer_wait")
+
+    def check_status(self, what: str):
+        """Raise if a wait timed out (synchronises)."""
+        s = int(self.status.item())
+        if s:
+            raise _lib.GnnError(f"rank {self.rank}: timed out waiting for the {what} flag of peer {s - 1}")
+
+
 class PartitionedSpmm:
     """Executes Y_local = (Â·X)[own rows] (and dX_local = (Âᵀ·dY)[own rows]) for one rank.
 
@@ -605,9 +635,7 @@ class PartitionedSpmm:
             raise ValueError(f"unknown transport {transport!r}")
         self.mover = {"auto": 0, "vector": 1, "tma": 2}[mover]
         if int(mover_ctas) < 0:
-            model = getattr(plan, "model", None) or {}
-            exchange_bound = model.get("exchange_ms", 0.0) >= EXCHANGE_BOUND_RATIO * max(model.get("compute_ms", 0.0), 1e-9)
-            mover_ctas = 32 if (plan.two_pass_chunks == 0 or exchange_bound) else 48
+            mover_ctas = 32 if (plan.two_pass_chunks == 0 or plan.model.get("exchange_bound", False)) else 48
         if int(mover_warps) < 0:
             mover_warps = 4
         self.mover_ctas, self.mover_warps, self.dedicated = int(mover_ctas), int(mover_warps), int(dedicated_sms)
@@ -623,7 +651,7 @@ class PartitionedSpmm:
         self._t_loc = self._t_rem = self._R = None
         self._fstep = self._bstep = 0
         self._bufs: List[_PeerBuffer] = []
-        self._status = torch.zeros(1, dtype=torch.int32, device=self.dev)
+        self._flags: Optional[_PeerFlags] = None
         if plan.world == 1:
             return
         self.comm = torch.cuda.Stream(device=self.dev, priority=-1)  # halo traffic is scheduled first
@@ -634,10 +662,10 @@ class PartitionedSpmm:
         self._wave_cum_send = [[sum(r[:w]) for w in range(plan.waves + 1)] for r in plan.send_wave_counts]
         if self.transport in ("p2p", "ce"):
             self._halo_buf = _PeerBuffer(n_halo * self.ld * self.elem, plan.rank, plan.world, group)
-            self._flags = _PeerBuffer(4 * 32 * 4, plan.rank, plan.world, group)  # arrive/consumed x fwd/bwd
-            self._bufs += [self._halo_buf, self._flags]
-            self.halo = self._view(self._halo_buf.own, n_halo, self.ld)[:, :self.F]
-            self._wave_table = None
+            # flag arrays 0 arrive_fwd, 1 consumed_fwd, 2 arrive_bwd, 3 consumed_bwd
+            self._flags = _PeerFlags(4, plan.rank, plan.world, group, self.dev, self.timeout_ms)
+            self._bufs += [self._halo_buf, self._flags.buf]
+            self.halo = _raw_view(self._halo_buf.own, n_halo, self.ld, dtype, self.dev)[:, :self.F]
             R = _lib.load().gnn_halo_rows_per_stage(self.F * self.elem)
             if (self.transport == "p2p" and fused_signal and self.mover != 1 and self.dedicated == 0 and R > 0
                     and self.ld == self.F):
@@ -683,29 +711,10 @@ class PartitionedSpmm:
         return table, len(rows), chunk, done
 
     # -- helpers ---------------------------------------------------------------------------
-    def _view(self, ptr: int, rows: int, ld: int) -> torch.Tensor:
-        t = torch.as_tensor(_RawCudaBuffer(ptr, (rows, ld), _TORCH_TYPESTR[self.dtype]), device=self.dev)
-        return t.view(self.dtype) if self.dtype != torch.float32 else t
-
-    def _flag_ptrs(self, which: int):
-        """Device pointers of flag array `which` (0 arrive_fwd, 1 consumed_fwd, 2 arrive_bwd, 3 consumed_bwd)
-        on every rank."""
-        return (C.c_void_p * self.plan.world)(*[p + which * 128 for p in self._flags.ptrs])
-
-    def _signal(self, which: int, value: int, stream):
-        _lib.check(_lib.load().gnn_peer_signal(self._flag_ptrs(which), self.plan.world, self.plan.rank, self.plan.rank,
-                                               value & 0xFFFFFFFF, stream.cuda_stream), "gnn_peer_signal")
-
-    def _wait(self, which: int, value: int, stream):
-        _lib.check(_lib.load().gnn_peer_wait(self._flags.own + which * 128, self.plan.world, self.plan.rank,
-                                             value & 0xFFFFFFFF, self._status.data_ptr(), self.timeout_ms,
-                                             stream.cuda_stream), "gnn_peer_wait")
-
     def check_status(self):
         """Raise if a flag wait of an earlier step timed out (synchronises)."""
-        s = int(self._status.item())
-        if s:
-            raise _lib.GnnError(f"rank {self.plan.rank}: timed out waiting for the halo flag of peer {s - 1}")
+        if self._flags is not None:
+            self._flags.check_status("halo")
 
     def _graph(self, c: Consumer):
         from .graph import CSRGraph
@@ -747,21 +756,30 @@ class PartitionedSpmm:
         if self.transport == "p2p":
             self._push(X, self._halo_buf.ptrs, seg_begin, seg_rows, dst_row, self.ld, plan.send_rows, stream)
             return
-        lib = _lib.load()
-        row_bytes = self.ld * self.elem
         self._ev_packed.record(stream)
-        for s_i in range(1, W):  # rotated: rank r copies to r+1 first
+        self._copy_to_peers(self._copy_streams, self._ev_copied, self._ev_packed, stream, self._halo_buf.ptrs, dst_row,
+                            self._sendbuf.data_ptr(), seg_begin, seg_rows)
+
+    def _copy_to_peers(self, streams, done, ready, join, dst_ptrs, dst_row, src, src_row, rows, wait_join=False):
+        """One gnn_peer_copy_async of rows[q] rows (src row src_row[q] -> row dst_row[q] of dst_ptrs[q]) per peer q
+        with rows to send, in rotated order (rank r copies to r+1 first), dealt over the copy `streams`; each stream
+        first waits on the event `ready` (and on the stream `join` too with wait_join).  Then `join` waits on every
+        stream through the events `done`."""
+        plan, lib = self.plan, _lib.load()
+        W, row_bytes = plan.world, self.ld * self.elem
+        for s_i in range(1, W):
             q = (plan.rank + s_i) % W
-            if seg_rows[q] == 0:
+            if rows[q] == 0:
                 continue
-            st = self._copy_streams[s_i % len(self._copy_streams)]
-            st.wait_event(self._ev_packed)
-            _lib.check(lib.gnn_peer_copy_async(self._halo_buf.ptrs[q] + dst_row[q] * row_bytes,
-                                               self._sendbuf.data_ptr() + seg_begin[q] * row_bytes,
-                                               seg_rows[q] * row_bytes, st.cuda_stream), "gnn_peer_copy_async")
-        for k, st in enumerate(self._copy_streams):
-            self._ev_copied[k].record(st)
-            stream.wait_event(self._ev_copied[k])
+            st = streams[s_i % len(streams)]
+            st.wait_event(ready)
+            if wait_join:
+                st.wait_stream(join)
+            _lib.check(lib.gnn_peer_copy_async(dst_ptrs[q] + dst_row[q] * row_bytes, src + src_row[q] * row_bytes,
+                                               rows[q] * row_bytes, st.cuda_stream), "gnn_peer_copy_async")
+        for ev, st in zip(done, streams):
+            ev.record(st)
+            join.wait_event(ev)
 
     def _exchange(self, X: torch.Tensor, stream):
         """Whole exchange of one step on `stream` (waves in order, flags after every wave)."""
@@ -775,7 +793,7 @@ class PartitionedSpmm:
                                    group=self.group)
             return
         if s > 0:
-            self._wait(1, s, stream)  # every peer has consumed the halo of the previous step: safe to overwrite
+            self._flags.wait(1, s, stream)  # every peer has consumed the halo of the previous step: safe to overwrite
         if self.transport == "ce":
             # pack: the push kernel with this rank's own send buffer as every "peer" (rows land in send order)
             W = plan.world
@@ -788,12 +806,12 @@ class PartitionedSpmm:
             o.ctas, o.warps_per_cta = self.mover_ctas, self.mover_warps
             _lib.check(_lib.load().gnn_halo_push_waves(
                 X.data_ptr(), X.stride(0), self.F, self.elem, plan.send_rows.data_ptr(), table.data_ptr(), n_segs, K,
-                n_chunks, done.data_ptr(), self._flag_ptrs(0), plan.world, plan.rank, (s * K) & 0xFFFFFFFF, C.byref(o),
-                stream.cuda_stream), "gnn_halo_push_waves")
+                n_chunks, done.data_ptr(), self._flags.ptrs(0), plan.world, plan.rank, (s * K) & 0xFFFFFFFF,
+                C.byref(o), stream.cuda_stream), "gnn_halo_push_waves")
             return
         for w in range(K):
             self._exchange_wave(X, w, stream)
-            self._signal(0, s * K + w + 1, stream)
+            self._flags.signal(0, s * K + w + 1, stream)
 
     def _run(self, c: Consumer, X, halo, out, excl: int = 0, bias: Optional[torch.Tensor] = None, relu: bool = False):
         from .functional import spmm_ex
@@ -822,14 +840,14 @@ class PartitionedSpmm:
     def _exchange_wait(self, w: int, stream):
         """The halo rows of wave w are readable on `stream` (flags: per wave; nccl: the whole halo, at wave 0)."""
         if self.transport in ("p2p", "ce"):
-            self._wait(0, self._fstep * self.plan.waves + w + 1, stream)
+            self._flags.wait(0, self._fstep * self.plan.waves + w + 1, stream)
         elif w == 0:
             stream.wait_event(self._ev_halo)
 
     def _exchange_end(self, stream):
         """This rank is done reading its halo: the peers may overwrite it in the next step."""
         if self.transport in ("p2p", "ce"):
-            self._signal(1, self._fstep + 1, stream)
+            self._flags.signal(1, self._fstep + 1, stream)
         self._fstep += 1
 
     def forward(self, X: torch.Tensor, out: Optional[torch.Tensor] = None, overlap: bool = True,
@@ -883,8 +901,8 @@ class PartitionedSpmm:
         K, s = plan.waves, self._fstep
         self._exchange(X, main)
         if self.transport in ("p2p", "ce"):
-            self._wait(0, s * K + K, main)
-            self._signal(1, s + 1, main)
+            self._flags.wait(0, s * K + K, main)
+            self._flags.signal(1, s + 1, main)
         self._fstep += 1
 
     # -- backward --------------------------------------------------------------------------
@@ -920,7 +938,7 @@ class PartitionedSpmm:
         if self.transport in ("p2p", "ce"):
             self._back_buf = _PeerBuffer(max(n_send, 1) * self.ld * self.elem, plan.rank, plan.world, self.group)
             self._bufs.append(self._back_buf)
-            self.back = self._view(self._back_buf.own, max(n_send, 1), self.ld)[:, :self.F]
+            self.back = _raw_view(self._back_buf.own, max(n_send, 1), self.ld, self.dtype, self.dev)[:, :self.F]
             self._bcopy_streams = [torch.cuda.Stream(device=self.dev, priority=-1) for _ in range(4)]
             self._ev_partial = torch.cuda.Event()
             self._ev_bcopied = [torch.cuda.Event() for _ in range(4)]
@@ -964,9 +982,9 @@ class PartitionedSpmm:
         """Send the partial rows to their owners (copy engines + flags, or all_to_all); `local()` runs on the main
         stream while they travel.  On return the rows this rank receives are in `self.back`, visible to the main
         stream."""
-        plan, lib = self.plan, _lib.load()
+        plan = self.plan
         main = torch.cuda.current_stream()
-        s, W = self._bstep, plan.world
+        s = self._bstep
         if self.transport == "nccl":
             dist.all_to_all_single(self.back[:int(plan.send_rows.numel())], self._partial[:plan.n_halo].contiguous(),
                                    output_split_sizes=plan.send_counts, input_split_sizes=plan.recv_counts,
@@ -979,28 +997,14 @@ class PartitionedSpmm:
             comm.wait_event(self._ev_partial)
             with torch.cuda.stream(comm):
                 if s > 0:
-                    self._wait(3, s, comm)  # every owner has consumed the partials of the previous step
-                row_bytes = self.ld * self.elem
-                base = self._partial.data_ptr()
-                for s_i in range(1, W):
-                    q = (plan.rank + s_i) % W
-                    if plan.recv_counts[q] == 0:
-                        continue
-                    st = self._bcopy_streams[s_i % len(self._bcopy_streams)]
-                    st.wait_event(self._ev_partial)
-                    if s > 0:
-                        st.wait_stream(comm)
-                    _lib.check(lib.gnn_peer_copy_async(self._back_buf.ptrs[q] + plan.back_off[q] * row_bytes,
-                                                       base + self._recv_off[q] * row_bytes,
-                                                       plan.recv_counts[q] * row_bytes, st.cuda_stream),
-                               "gnn_peer_copy_async")
-                for k, st in enumerate(self._bcopy_streams):
-                    self._ev_bcopied[k].record(st)
-                    comm.wait_event(self._ev_bcopied[k])
-                self._signal(2, s + 1, comm)
+                    self._flags.wait(3, s, comm)  # every owner has consumed the partials of the previous step
+                self._copy_to_peers(self._bcopy_streams, self._ev_bcopied, self._ev_partial, comm, self._back_buf.ptrs,
+                                    plan.back_off, self._partial.data_ptr(), self._recv_off, plan.recv_counts,
+                                    wait_join=s > 0)
+                self._flags.signal(2, s + 1, comm)
             if local is not None:
                 local()
-            self._wait(2, s + 1, main)
+            self._flags.wait(2, s + 1, main)
 
     def _return_add(self, out: torch.Tensor):
         """out[r] += the received rows of local row r, in (peer, slot) order; frees the receive buffer for the
@@ -1011,17 +1015,12 @@ class PartitionedSpmm:
         if self._R.n_rows > 0:
             spmm_ex(self._R, self.back, out, row_map=self._R._row_map, accumulate=True)
         if self.transport != "nccl":
-            self._signal(3, self._bstep + 1, torch.cuda.current_stream())
+            self._flags.signal(3, self._bstep + 1, torch.cuda.current_stream())
         self._bstep += 1
 
     def close(self):
-        if self._bufs:
-            torch.cuda.synchronize(self.dev)
-            if dist.is_initialized():
-                dist.barrier(group=self.group)
-            for b in self._bufs:
-                b.close()
-            self._bufs = []
+        _close_peer_buffers(self._bufs, self.dev, self.group)
+        self._bufs = []
 
 
 class PartitionedGraph:
@@ -1111,9 +1110,7 @@ class PartitionedGraph:
     def local_index(self, idx_global: torch.Tensor) -> torch.Tensor:
         """The global node ids of `idx_global` (train / val / test ids) that this rank owns, as local row indices
         (ascending where idx_global is)."""
-        lo, hi = self.row_range
-        idx = idx_global.to(torch.int64)
-        return idx[(idx >= lo) & (idx < hi)] - lo
+        return _local_index(idx_global, *self.row_range)
 
     def close(self):
         """Free the peer buffers (collective: every rank calls it)."""
@@ -1412,35 +1409,24 @@ class PeerRowReduce:
                  timeout_ms: int = 20000):
         self.bounds, self.rank, self.world, self.group = [int(b) for b in bounds], int(rank), int(world), group
         self.dev, self.timeout_ms = torch.device(device), int(timeout_ms)
-        self._status = torch.zeros(1, dtype=torch.int32, device=self.dev)
         self._sites: Dict[str, dict] = {}
         self._bufs: List[_PeerBuffer] = []
+        self._flags: Optional[_PeerFlags] = None
         if self.world == 1:
             return
         try:
-            self._flags = _PeerBuffer(len(sites) * 256, self.rank, self.world, group)  # 32 arrive + 32 consumed slots
-            self._bufs.append(self._flags)
+            # flag arrays 2k (arrive) and 2k + 1 (consumed) for site k
+            self._flags = _PeerFlags(2 * len(sites), self.rank, self.world, group, self.dev, self.timeout_ms)
+            self._bufs.append(self._flags.buf)
             for k, (name, (rows, cols)) in enumerate(sorted(sites.items())):
                 ld = (int(cols) + 3) // 4 * 4  # 16-byte rows: the reduce kernel reads float4 vectors
                 buf = _PeerBuffer(max(int(rows), 1) * ld * 4, self.rank, self.world, group)
                 self._bufs.append(buf)
-                self._sites[name] = {"buf": buf, "rows": int(rows), "cols": int(cols), "ld": ld, "flag": k * 256,
+                self._sites[name] = {"buf": buf, "rows": int(rows), "cols": int(cols), "ld": ld, "flag": 2 * k,
                                      "step": 0}
         except Exception:
             self.close()
             raise
-
-    def _flag_ptrs(self, off: int):
-        return (C.c_void_p * self.world)(*[p + off for p in self._flags.ptrs])
-
-    def _signal(self, off: int, value: int, stream):
-        _lib.check(_lib.load().gnn_peer_signal(self._flag_ptrs(off), self.world, self.rank, self.rank,
-                                               value & 0xFFFFFFFF, stream.cuda_stream), "gnn_peer_signal")
-
-    def _wait(self, off: int, value: int, stream):
-        _lib.check(_lib.load().gnn_peer_wait(self._flags.own + off, self.world, self.rank, value & 0xFFFFFFFF,
-                                             self._status.data_ptr(), self.timeout_ms, stream.cuda_stream),
-                   "gnn_peer_wait")
 
     def _site(self, name: str, x: torch.Tensor) -> dict:
         site = self._sites.get(name)
@@ -1455,16 +1441,15 @@ class PeerRowReduce:
         """x into this rank's buffer of the site once every peer has read its previous contents; then the flags."""
         s = site["step"]
         if s > 0:
-            self._wait(site["flag"] + 128, s, stream)
+            self._flags.wait(site["flag"] + 1, s, stream)
         if x.shape[0]:
-            t = torch.as_tensor(_RawCudaBuffer(site["buf"].own, (x.shape[0], site["ld"])), device=self.dev)
-            t[:, :x.shape[1]].copy_(x)
-        self._signal(site["flag"], s + 1, stream)
-        self._wait(site["flag"], s + 1, stream)
+            _raw_view(site["buf"].own, x.shape[0], site["ld"], torch.float32, self.dev)[:, :x.shape[1]].copy_(x)
+        self._flags.signal(site["flag"], s + 1, stream)
+        self._flags.wait(site["flag"], s + 1, stream)
 
     def _done(self, site: dict, stream):
         site["step"] += 1
-        self._signal(site["flag"] + 128, site["step"], stream)
+        self._flags.signal(site["flag"] + 1, site["step"], stream)
 
     def _reduce(self, name: str, x: torch.Tensor, row_lo: int, row_hi: int, relu: bool) -> torch.Tensor:
         from .functional import peer_reduce_rows_raw
@@ -1507,18 +1492,13 @@ class PeerRowReduce:
 
     def check_status(self):
         """Raise if a flag wait of an earlier call timed out (synchronises)."""
-        s = int(self._status.item())
-        if s:
-            raise _lib.GnnError(f"rank {self.rank}: timed out waiting for the reduce flag of peer {s - 1}")
+        if self._flags is not None:
+            self._flags.check_status("reduce")
 
     def close(self):
         """Free the peer buffers (collective)."""
         if self._bufs:
-            torch.cuda.synchronize(self.dev)
-            if dist.is_initialized():
-                dist.barrier(group=self.group)
-            for b in self._bufs:
-                b.close()
+            _close_peer_buffers(self._bufs, self.dev, self.group)
             self._bufs = []
             self._sites = {}
 
@@ -1617,9 +1597,7 @@ class PartitionedRelationStack:
 
     def local_index(self, idx_global: torch.Tensor) -> torch.Tensor:
         """The global node ids of `idx_global` this rank owns, as local row indices."""
-        lo, hi = self.row_range
-        idx = idx_global.to(torch.int64)
-        return idx[(idx >= lo) & (idx < hi)] - lo
+        return _local_index(idx_global, *self.row_range)
 
     def check_status(self):
         """Raise if a flag wait of an earlier step timed out (synchronises)."""
@@ -1719,7 +1697,7 @@ class ShardedTable:
         err = None
         try:
             if n:  # pad columns are zero, as pad_table leaves them: a 16-byte store of the gather may carry them out
-                full = self._view(self._buf.own, n)
+                full = _raw_view(self._buf.own, n, ld, dtype, self.device)
                 full[:, F:].zero_()
                 full[:, :F].copy_(X_block)
             amax = X_block.detach().abs().max().float() if n else torch.zeros((), device=self.device)
@@ -1780,11 +1758,6 @@ class ShardedTable:
         self.F, self.ld, self.dtype, self.device = int(F), int(ld), dtype, torch.device(device)
         self.shape = torch.Size((self.bounds[-1], self.F))
         self.requires_grad = False
-
-    def _view(self, ptr: int, rows: int) -> torch.Tensor:
-        """[rows, ld] torch view of a shard buffer."""
-        t = torch.as_tensor(_RawCudaBuffer(ptr, (rows, self.ld), _TORCH_TYPESTR[self.dtype]), device=self.device)
-        return t.view(self.dtype) if self.dtype != torch.float32 else t
 
     def _make_desc(self, ptrs):
         d = _lib.ShardedTableDesc()
