@@ -65,15 +65,15 @@ def spmm_raw(g: CSRGraph, X: torch.Tensor, out: Optional[torch.Tensor] = None, p
     if planned or accumulate or bias is not None or relu:
         lr, thr, chunk_off, n_chunks, chunk, ws = plan if plan is not None else (None, 0, None, 0, 0, None)
         fn = lib.gnn_spmm_csr_planned_f32 if f32 else lib.gnn_spmm_csr_planned_bf16
-        _lib.check(fn(_p(g.rowptr), _p(g.col), _p(g.val), _p(X), _p(out), g.n_rows, g.n_cols, F, _ld(X), _ld(out),
-                      _p(lr), 0 if lr is None else lr.numel(), thr, _p(chunk_off), n_chunks, chunk,
+        _lib.check(fn(_p(g.rowptr), _p(g.col), _p(g.val), _p(_nonempty(X)), _p(out), g.n_rows, g.n_cols, F, _ld(X),
+                      _ld(out), _p(lr), 0 if lr is None else lr.numel(), thr, _p(chunk_off), n_chunks, chunk,
                       1 if accumulate else 0, g.rows_per_team() if planned else 0, _p(bias), 1 if relu else 0,
                       _p(ws), 0 if ws is None else ws.numel(), st),
                    "gnn_spmm_csr_planned")
     else:
         fn = lib.gnn_spmm_csr_f32 if f32 else lib.gnn_spmm_csr_bf16
-        _lib.check(fn(_p(g.rowptr), _p(g.col), _p(g.val), _p(X), _p(out), g.n_rows, g.n_cols, F, _ld(X), _ld(out), st),
-                   "gnn_spmm_csr")
+        _lib.check(fn(_p(g.rowptr), _p(g.col), _p(g.val), _p(_nonempty(X)), _p(out), g.n_rows, g.n_cols, F, _ld(X),
+                      _ld(out), st), "gnn_spmm_csr")
     return out
 
 
@@ -206,7 +206,8 @@ def _col_or_dummy(g: CSRGraph) -> torch.Tensor:
 
 
 def _nonempty(t: torch.Tensor) -> torch.Tensor:
-    # a permutation of a graph without entries has no address; the kernels read none of it
+    # an empty tensor (the permutation of a graph without entries, the X of a graph without columns) has no address;
+    # the kernels read none of it
     return t if t.numel() else torch.zeros(1, dtype=t.dtype, device=t.device)
 
 
@@ -1256,69 +1257,6 @@ def _semantic_workspace(K: int, device) -> torch.Tensor:
 SEMANTIC_MAX_M, SEMANTIC_MAX_K = 32, 256
 
 
-class _SemanticFn(torch.autograd.Function):
-    """out = sum_m softmax_M(mean_N(q . tanh(z W1^T + b)))_m z[:, m, :]: one GEMM + two launches forward, two
-    launches + two GEMMs backward (csrc/semantic.cu)."""
-
-    @staticmethod
-    def forward(ctx, z, W1, b1, q):
-        lib = _lib.load()
-        N, M, D = z.shape
-        K = W1.shape[0]
-        z = z.contiguous()
-        W1c, qv = W1.contiguous(), q.reshape(-1).contiguous()
-        b1c = None if b1 is None else b1.contiguous()
-        P = torch.mm(z.view(N * M, D), W1c.t())                      # [N*M, K], the library GEMM
-        ws = _semantic_workspace(K, z.device)
-        scores = torch.empty(M, dtype=torch.float32, device=z.device)
-        beta = torch.empty(M, dtype=torch.float32, device=z.device)
-        out = torch.empty((N, D), dtype=torch.float32, device=z.device)
-        st = _stream_ptr()
-        _lib.check(lib.gnn_semantic_scores_f32(_p(P), P.stride(0), _p(b1c), _p(qv), N, M, K, _p(scores), _p(beta), _p(ws),
-                                               ws.numel(), st), "gnn_semantic_scores_f32")
-        _lib.check(lib.gnn_semantic_combine_f32(_p(beta), _p(z), N, M, D, _p(out), st), "gnn_semantic_combine_f32")
-        ctx.save_for_backward(z, W1c, b1c if b1c is not None else z.new_empty(0), qv, P, beta)
-        ctx.has_bias, ctx.q_shape = b1 is not None, tuple(q.shape)
-        return out
-
-    @staticmethod
-    def backward(ctx, d_out):
-        lib = _lib.load()
-        z, W1, b1, qv, P, beta = ctx.saved_tensors
-        N, M, D = z.shape
-        K = W1.shape[0]
-        d_out = d_out.contiguous()
-        ws = _semantic_workspace(K, z.device)
-        dz = torch.empty_like(z)
-        dsn = torch.empty(M, dtype=torch.float32, device=z.device)
-        dP = torch.empty_like(P)
-        dq = torch.empty(K, dtype=torch.float32, device=z.device)
-        db = torch.empty(K, dtype=torch.float32, device=z.device) if ctx.has_bias else None
-        st = _stream_ptr()
-        _lib.check(lib.gnn_semantic_combine_bwd_f32(_p(d_out), _p(z), _p(beta), N, M, D, _p(dz), _p(dsn), _p(ws),
-                                                    ws.numel(), st), "gnn_semantic_combine_bwd_f32")
-        _lib.check(lib.gnn_semantic_scores_bwd_f32(_p(P), P.stride(0), _p(b1) if ctx.has_bias else None, _p(qv), _p(dsn),
-                                                   N, M, K, _p(dP), dP.stride(0), _p(dq), _p(db), _p(ws), ws.numel(), st),
-                   "gnn_semantic_scores_bwd_f32")
-        z2 = z.view(N * M, D)
-        dW1 = torch.mm(dP.t(), z2) if ctx.needs_input_grad[1] else None                 # [K, D]
-        if ctx.needs_input_grad[0]:
-            dz = torch.addmm(dz.view(N * M, D), dP, W1).view(N, M, D)                    # direct term + dP·W1
-        else:
-            dz = None
-        return dz, dW1, db, dq.view(ctx.q_shape)
-
-
-def semantic_attention(z: torch.Tensor, W1: torch.Tensor, b1: Optional[torch.Tensor], q: torch.Tensor) -> torch.Tensor:
-    """HAN semantic attention over z [N, M, D] with project = Linear(D,K; W1,b1) -> tanh -> Linear(K,1; q, no bias)
-    (SemanticAttention.py:8-20): returns [N, D].  fp32, M <= 32, K <= 256."""
-    _require_cuda(z, W1, q)
-    if z.dtype != torch.float32 or z.dim() != 3 or z.shape[1] > SEMANTIC_MAX_M or W1.shape[0] > SEMANTIC_MAX_K or \
-            W1.shape[1] != z.shape[2] or q.numel() != W1.shape[0] or z.shape[0] == 0:
-        raise _lib.GnnError(f"semantic_attention: unsupported shapes z {tuple(z.shape)} W1 {tuple(W1.shape)} q {tuple(q.shape)}")
-    return _SemanticFn.apply(z, W1, b1, q)
-
-
 def _rank_ordered_sum(x: torch.Tensor, world: int, group) -> torch.Tensor:
     """Σ over the ranks of x, added in rank order starting from rank 0's tensor (one all_gather): the same bits on
     every rank whatever the backend's reduction algorithm, and x itself at world 1."""
@@ -1333,68 +1271,101 @@ def _rank_ordered_sum(x: torch.Tensor, world: int, group) -> torch.Tensor:
     return acc
 
 
-class _SemanticPartitionedFn(torch.autograd.Function):
-    """_SemanticFn over a rank's rows of a row-partitioned node set: the node sums behind mean_N (forward) and dβ
-    (backward) are split at the rank boundary — partial over the own rows, a rank-ordered sum of the [M] partials,
-    then finalize with the global node count.  Collective in both directions."""
+class _SemanticFn(torch.autograd.Function):
+    """out = sum_m softmax_M(mean_N(q . tanh(z W1^T + b)))_m z[:, m, :]: one GEMM + two launches forward, two
+    launches + two GEMMs backward (csrc/semantic.cu).
+    dist = (n_total, world, group): z is a rank's rows of a row-partitioned node set, and the node sums behind mean_N
+    (forward) and dβ (backward) are split at the rank boundary: partial over the own rows, a rank-ordered sum of the
+    [M] partials, then finalize with the global node count.  Collective in both directions."""
 
     @staticmethod
-    def forward(ctx, z, W1, b1, q, n_total, world, group):
+    def forward(ctx, z, W1, b1, q, dist):
         lib = _lib.load()
         N, M, D = z.shape
         K = W1.shape[0]
+        dev = z.device
         z = z.contiguous()
         W1c, qv = W1.contiguous(), q.reshape(-1).contiguous()
         b1c = None if b1 is None else b1.contiguous()
-        P = torch.mm(z.view(N * M, D), W1c.t())                      # [N*M, K]
-        ws = _semantic_workspace(K, z.device)
-        dev = z.device
-        sums = torch.empty(M, dtype=torch.float32, device=dev)
-        st = _stream_ptr()
-        _lib.check(lib.gnn_semantic_scores_partial_f32(_p(P), P.stride(0), _p(b1c), _p(qv), N, M, K, _p(sums), _p(ws),
-                                                       ws.numel(), st), "gnn_semantic_scores_partial_f32")
-        sums = _rank_ordered_sum(sums, world, group)
+        P = torch.mm(z.view(N * M, D), W1c.t())                      # [N*M, K], the library GEMM
+        ws = _semantic_workspace(K, dev)
         scores = torch.empty(M, dtype=torch.float32, device=dev)
         beta = torch.empty(M, dtype=torch.float32, device=dev)
-        _lib.check(lib.gnn_semantic_scores_finalize_f32(_p(sums), n_total, M, _p(scores), _p(beta), st),
-                   "gnn_semantic_scores_finalize_f32")
+        st = _stream_ptr()
+        if dist is None:
+            _lib.check(lib.gnn_semantic_scores_f32(_p(P), P.stride(0), _p(b1c), _p(qv), N, M, K, _p(scores), _p(beta),
+                                                   _p(ws), ws.numel(), st), "gnn_semantic_scores_f32")
+        else:
+            n_total, world, group = dist
+            sums = torch.empty(M, dtype=torch.float32, device=dev)
+            _lib.check(lib.gnn_semantic_scores_partial_f32(_p(P), P.stride(0), _p(b1c), _p(qv), N, M, K, _p(sums),
+                                                           _p(ws), ws.numel(), st), "gnn_semantic_scores_partial_f32")
+            sums = _rank_ordered_sum(sums, world, group)
+            _lib.check(lib.gnn_semantic_scores_finalize_f32(_p(sums), n_total, M, _p(scores), _p(beta), st),
+                       "gnn_semantic_scores_finalize_f32")
         out = torch.empty((N, D), dtype=torch.float32, device=dev)
         _lib.check(lib.gnn_semantic_combine_f32(_p(beta), _p(z), N, M, D, _p(out), st), "gnn_semantic_combine_f32")
         ctx.save_for_backward(z, W1c, b1c if b1c is not None else z.new_empty(0), qv, P, beta)
-        ctx.has_bias, ctx.q_shape, ctx.dist = b1 is not None, tuple(q.shape), (n_total, world, group)
+        ctx.has_bias, ctx.q_shape, ctx.dist = b1 is not None, tuple(q.shape), dist
         return out
 
     @staticmethod
     def backward(ctx, d_out):
         lib = _lib.load()
         z, W1, b1, qv, P, beta = ctx.saved_tensors
-        n_total, world, group = ctx.dist
         N, M, D = z.shape
         K = W1.shape[0]
-        d_out = d_out.contiguous()
         dev = z.device
+        d_out = d_out.contiguous()
         ws = _semantic_workspace(K, dev)
         dz = torch.empty_like(z)
-        dbeta = torch.empty(M, dtype=torch.float32, device=dev)
-        st = _stream_ptr()
-        _lib.check(lib.gnn_semantic_combine_bwd_partial_f32(_p(d_out), _p(z), _p(beta), N, M, D, _p(dz), _p(dbeta),
-                                                            _p(ws), ws.numel(), st),
-                   "gnn_semantic_combine_bwd_partial_f32")
-        dbeta = _rank_ordered_sum(dbeta, world, group)
         dsn = torch.empty(M, dtype=torch.float32, device=dev)
-        _lib.check(lib.gnn_semantic_combine_bwd_finalize_f32(_p(dbeta), _p(beta), n_total, M, _p(dsn), st),
-                   "gnn_semantic_combine_bwd_finalize_f32")
-        dq = torch.zeros(K, dtype=torch.float32, device=dev)
-        db = torch.zeros(K, dtype=torch.float32, device=dev) if ctx.has_bias else None
+        st = _stream_ptr()
+        if ctx.dist is None:
+            _lib.check(lib.gnn_semantic_combine_bwd_f32(_p(d_out), _p(z), _p(beta), N, M, D, _p(dz), _p(dsn), _p(ws),
+                                                        ws.numel(), st), "gnn_semantic_combine_bwd_f32")
+        else:
+            n_total, world, group = ctx.dist
+            dbeta = torch.empty(M, dtype=torch.float32, device=dev)
+            _lib.check(lib.gnn_semantic_combine_bwd_partial_f32(_p(d_out), _p(z), _p(beta), N, M, D, _p(dz), _p(dbeta),
+                                                                _p(ws), ws.numel(), st),
+                       "gnn_semantic_combine_bwd_partial_f32")
+            dbeta = _rank_ordered_sum(dbeta, world, group)
+            _lib.check(lib.gnn_semantic_combine_bwd_finalize_f32(_p(dbeta), _p(beta), n_total, M, _p(dsn), st),
+                       "gnn_semantic_combine_bwd_finalize_f32")
+        # dq / db are column sums over the rows (on a partition the rank's share, which partition.allreduce_gradients
+        # adds up): the kernel writes them, and a rank without rows contributes zeros
+        alloc = torch.empty if N > 0 else torch.zeros
+        dq = alloc(K, dtype=torch.float32, device=dev)
+        db = alloc(K, dtype=torch.float32, device=dev) if ctx.has_bias else None
         dP = torch.empty_like(P)
-        if N > 0:  # the rank's share of the column sums dq / db (partition.allreduce_gradients adds the ranks')
+        if N > 0:
             _lib.check(lib.gnn_semantic_scores_bwd_f32(_p(P), P.stride(0), _p(b1) if ctx.has_bias else None, _p(qv),
                                                        _p(dsn), N, M, K, _p(dP), dP.stride(0), _p(dq), _p(db), _p(ws),
                                                        ws.numel(), st), "gnn_semantic_scores_bwd_f32")
         z2 = z.view(N * M, D)
-        dW1 = torch.mm(dP.t(), z2) if ctx.needs_input_grad[1] else None
-        dz = torch.addmm(dz.view(N * M, D), dP, W1).view(N, M, D) if ctx.needs_input_grad[0] else None
-        return dz, dW1, db, dq.view(ctx.q_shape), None, None, None
+        dW1 = torch.mm(dP.t(), z2) if ctx.needs_input_grad[1] else None                 # [K, D]
+        if ctx.needs_input_grad[0]:
+            dz = torch.addmm(dz.view(N * M, D), dP, W1).view(N, M, D)                    # direct term + dP·W1
+        else:
+            dz = None
+        return dz, dW1, db, dq.view(ctx.q_shape), None
+
+
+def _semantic(z: torch.Tensor, W1: torch.Tensor, b1: Optional[torch.Tensor], q: torch.Tensor, dist=None):
+    """The shape checks of both entries: dist None needs rows in z, a partition a positive global node count."""
+    _require_cuda(z, W1, q)
+    if z.dtype != torch.float32 or z.dim() != 3 or z.shape[1] > SEMANTIC_MAX_M or W1.shape[0] > SEMANTIC_MAX_K or \
+            W1.shape[1] != z.shape[2] or q.numel() != W1.shape[0] or (z.shape[0] if dist is None else dist[0]) <= 0:
+        raise _lib.GnnError(f"semantic_attention: unsupported shapes z {tuple(z.shape)} W1 {tuple(W1.shape)} "
+                            f"q {tuple(q.shape)}" + ("" if dist is None else f" n_total {dist[0]}"))
+    return _SemanticFn.apply(z, W1, b1, q, dist)
+
+
+def semantic_attention(z: torch.Tensor, W1: torch.Tensor, b1: Optional[torch.Tensor], q: torch.Tensor) -> torch.Tensor:
+    """HAN semantic attention over z [N, M, D] with project = Linear(D,K; W1,b1) -> tanh -> Linear(K,1; q, no bias)
+    (SemanticAttention.py:8-20): returns [N, D].  fp32, M <= 32, K <= 256."""
+    return _semantic(z, W1, b1, q)
 
 
 def semantic_attention_partitioned(z: torch.Tensor, W1: torch.Tensor, b1: Optional[torch.Tensor], q: torch.Tensor,
@@ -1402,9 +1373,4 @@ def semantic_attention_partitioned(z: torch.Tensor, W1: torch.Tensor, b1: Option
     """`semantic_attention` over this rank's rows z [n_local, M, D] of a row-partitioned node set of n_total nodes:
     β is the one of all n_total nodes, identical on every rank (rank-ordered sums of the per-rank node sums).
     Collective, forward and backward; at world 1 it computes the same bits as `semantic_attention`."""
-    _require_cuda(z, W1, q)
-    if z.dtype != torch.float32 or z.dim() != 3 or z.shape[1] > SEMANTIC_MAX_M or W1.shape[0] > SEMANTIC_MAX_K or \
-            W1.shape[1] != z.shape[2] or q.numel() != W1.shape[0] or n_total <= 0:
-        raise _lib.GnnError(f"semantic_attention: unsupported shapes z {tuple(z.shape)} W1 {tuple(W1.shape)} "
-                            f"q {tuple(q.shape)} n_total {n_total}")
-    return _SemanticPartitionedFn.apply(z, W1, b1, q, int(n_total), int(world), group)
+    return _semantic(z, W1, b1, q, (int(n_total), int(world), group))

@@ -13,8 +13,8 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from .. import _lib
-from ..functional import (attention_keep_mask, gat_aggregate, halo_exchange, next_attention_dropout,
-                          require_partition_dtype, spmm_values)
+from ..functional import (AttentionDropout, attention_keep_mask, gat_aggregate, halo_exchange,
+                          next_attention_dropout, require_partition_dtype, spmm_values)
 from ..graph import CSRGraph, adj_cache
 from ..partition import PartitionedGraph
 
@@ -66,60 +66,56 @@ class SpecialSpmm(nn.Module):
         return SpecialSpmmFunction.apply(indices, values, shape, b)
 
 
+def _attention_dropout(g, H, p, device, edge_slot_base=None, slot_shift=None):
+    """(keep, dropout) for `gat_aggregate`: post-softmax attention dropout p (layers.py:31) over g, as an explicit
+    [nnz, H] mask (EXPLICIT_DROPOUT_MASK) or as a seeded stream that materialises no mask.  On a rank's block the
+    stream draws the whole graph's mask for the block's edges: `edge_slot_base` for a block of one graph,
+    `slot_shift` for a block of a batched set (partition.PartitionedMetapaths)."""
+    if p <= 0.0:
+        return None, None
+    if EXPLICIT_DROPOUT_MASK:
+        return attention_keep_mask(g, H, p), None
+    drop = next_attention_dropout(p, device)
+    if edge_slot_base is not None:
+        drop = drop.with_slot_base(edge_slot_base)
+    if slot_shift is not None:
+        drop = AttentionDropout(drop.p, drop.seed, drop.seed_dev, slot_shift=slot_shift)
+    return None, drop
+
+
 def _fused_heads(x, adj, Ws, a_srcs, a_dsts, alpha, mode, elu, dropout, training, out=None):
     """All heads of one attention layer: x [N,in]; Ws list of [in,F']; a_* list of [F'].
-    adj may be a partition.PartitionedGraph: x is then the rank's own rows, and so is the result."""
-    if isinstance(adj, PartitionedGraph):
-        return _fused_heads_partitioned(x, adj, Ws, a_srcs, a_dsts, alpha, mode, elu, dropout, training)
-    g = adj_cache.get(adj)
+    adj may be a partition.PartitionedGraph: x (in the partition's dtype) is then the rank's own rows, and so is the
+    result.  The block's table is [own rows ; halo rows] (functional.halo_exchange) in the combined column space, s
+    comes from the own rows and t from all table rows, so one rank computes one GPU's bits in either dtype.  The
+    backward returns d Wh of the halo rows (from the aggregation and from t) to their owners; d a_src / d a_dst are
+    this rank's share, summed over the ranks by partition.allreduce_gradients.  `out`: one GPU, see `gat_aggregate`."""
     H = len(Ws)
     Fp = Ws[0].shape[1]
+    pg = adj if isinstance(adj, PartitionedGraph) else None
+    if pg is None:
+        # no slot base: it reads the device seed back, and a one-GPU step may run under CUDA-graph capture
+        g, slot_base = adj_cache.get(adj), None
+    else:
+        # refused before the exchange, the first collective: every rank raises together
+        require_partition_dtype(pg, x, "GAT on a PartitionedGraph")
+        if H * Fp > 256:
+            raise _lib.GnnError(f"GAT on a PartitionedGraph: H*F' = {H * Fp} exceeds the 256 columns of one fused "
+                                "attention call")
+        g, slot_base = pg.attention()
     W_cat = Ws[0] if H == 1 else torch.cat(list(Ws), dim=1)
     Wh = torch.mm(x, W_cat)  # [N, H*F']  (layers.py:23, all heads at once)
+    if pg is not None:
+        Wh = halo_exchange(pg, Wh)  # [n_local + n_halo, H*F']
     Wh3 = Wh.view(-1, H, Fp)
     a_src = a_srcs[0].view(1, Fp) if H == 1 else torch.stack(list(a_srcs), dim=0)
     a_dst = a_dsts[0].view(1, Fp) if H == 1 else torch.stack(list(a_dsts), dim=0)
+    own = Wh3 if pg is None else Wh3[:pg.n_local]  # the rows of s (no slice on one GPU: its backward copies)
     # scores are fp32 even for bf16 features (the softmax statistics live in fp32)
-    s = (Wh3.float() * a_src.float().unsqueeze(0)).sum(-1)  # [N,H] = Wh_i·a[:F']
-    t = (Wh3.float() * a_dst.float().unsqueeze(0)).sum(-1)  # [N,H] = Wh_j·a[F':]
-    keep = drop = None
-    if training and dropout > 0.0:  # post-softmax dropout, layers.py:31
-        if EXPLICIT_DROPOUT_MASK:
-            keep = attention_keep_mask(g, H, dropout)
-        else:
-            drop = next_attention_dropout(dropout, Wh.device)  # seeded: no [nnz, H] mask is materialised
+    s = (own.float() * a_src.float().unsqueeze(0)).sum(-1)  # [rows, H] = Wh_i·a[:F']
+    t = (Wh3.float() * a_dst.float().unsqueeze(0)).sum(-1)  # [table rows, H] = Wh_j·a[F':]
+    keep, drop = _attention_dropout(g, H, dropout if training else 0.0, Wh.device, edge_slot_base=slot_base)
     return gat_aggregate(g, Wh, s, t, H, Fp, alpha, mode=mode, elu=elu, keep=keep, out=out, dropout=drop)
-
-
-def _fused_heads_partitioned(x, pg, Ws, a_srcs, a_dsts, alpha, mode, elu, dropout, training):
-    """`_fused_heads` on this rank's row block: Wh of the own rows, the halo rows' Wh from their owners
-    (functional.halo_exchange), s of the own rows, t of all table rows, and the fused kernels over the block in the
-    combined column space.  The backward returns d Wh of the halo rows (from the aggregation and from t) to their
-    owners; d a_src / d a_dst are this rank's share, summed over the ranks by partition.allreduce_gradients.
-    x has the partition's dtype (fp32 or bf16); s / t are fp32 from the same expression as `_fused_heads`, so one rank
-    computes the bits of one GPU in either dtype."""
-    H = len(Ws)
-    Fp = Ws[0].shape[1]
-    require_partition_dtype(pg, x, "GAT on a PartitionedGraph")
-    if H * Fp > 256:
-        raise _lib.GnnError(f"GAT on a PartitionedGraph: H*F' = {H * Fp} exceeds the 256 columns of one fused "
-                            "attention call")
-    g, edge_slot_base = pg.attention()
-    W_cat = Ws[0] if H == 1 else torch.cat(list(Ws), dim=1)
-    Wh = halo_exchange(pg, torch.mm(x, W_cat))  # [n_local + n_halo, H*F']
-    Wh3 = Wh.view(-1, H, Fp)
-    a_src = a_srcs[0].view(1, Fp) if H == 1 else torch.stack(list(a_srcs), dim=0)
-    a_dst = a_dsts[0].view(1, Fp) if H == 1 else torch.stack(list(a_dsts), dim=0)
-    s = (Wh3[:pg.n_local].float() * a_src.float().unsqueeze(0)).sum(-1)  # [n_local, H]
-    t = (Wh3.float() * a_dst.float().unsqueeze(0)).sum(-1)               # [n_local + n_halo, H]
-    keep = drop = None
-    if training and dropout > 0.0:
-        if EXPLICIT_DROPOUT_MASK:
-            keep = attention_keep_mask(g, H, dropout)
-        else:
-            # the whole graph's mask for this block's edges
-            drop = next_attention_dropout(dropout, Wh.device).with_slot_base(edge_slot_base)
-    return gat_aggregate(g, Wh, s, t, H, Fp, alpha, mode=mode, elu=elu, keep=keep, dropout=drop)
 
 
 class GraphAttentionLayer(nn.Module):

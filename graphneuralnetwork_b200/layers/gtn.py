@@ -76,24 +76,26 @@ def gcn_conv(X, H, weight):
 def _normalized_aggregate(g, vals, XW, reduce=None):
     """The tail of `gcn_conv` on g = CSR of (offdiag(H) + I)^T with its values: divide by the column sums of
     offdiag(H) + I (the row sums of g, an ordered SpMM against ones; inf -> 0) and aggregate XW, autograd into vals.
-    vals [nnz] is one channel; vals [nnz, C] gives the C channels' outputs side by side, [n_rows, C * w].
+    vals [nnz, C] gives the C channels' outputs side by side, [n_rows, C * w]; vals [nnz] is one channel, [n_rows, w].
     reduce: on a row block (partition.PartitionedRelationStack) the degrees are partial sums, and `reduce([n_rows, C])`
     returns the sums over every rank's rows; None keeps them."""
-    if vals.dim() == 1:
-        ones = torch.ones((g.n_cols, 1), dtype=torch.float32, device=vals.device)
-        deg = spmm_values(g, vals, ones)
-        deg = (deg if reduce is None else reduce(deg)).view(-1)
-        deg_inv = deg.pow(-1)
-        deg_inv = torch.where(deg_inv == float('inf'), torch.zeros_like(deg_inv), deg_inv)
-        return spmm_values(g, vals * deg_inv[g.edge_rows().long()], XW)
+    V = vals if vals.dim() == 2 else vals.unsqueeze(1)  # not view(nnz, -1): a rank's empty block has nnz = 0
+    C = V.shape[1]
+
+    def channel(x, c):  # column c of x [rows, C]; one channel is x itself, without a copy forward or backward
+        return x.view(-1) if C == 1 else x[:, c]
+
+    def side_by_side(parts):
+        return parts[0] if C == 1 else torch.cat(parts, dim=1)
+
     ones = torch.ones((g.n_cols, 1), dtype=torch.float32, device=vals.device)
-    deg = torch.cat([spmm_values(g, vals[:, c].contiguous(), ones) for c in range(vals.shape[1])], dim=1)
+    deg = side_by_side([spmm_values(g, channel(V, c).contiguous(), ones) for c in range(C)])
     if reduce is not None:
         deg = reduce(deg)
     deg_inv = deg.pow(-1)
     deg_inv = torch.where(deg_inv == float('inf'), torch.zeros_like(deg_inv), deg_inv)
     rows = g.edge_rows().long()
-    return torch.cat([spmm_values(g, vals[:, c] * deg_inv[rows, c], XW) for c in range(vals.shape[1])], dim=1)
+    return side_by_side([spmm_values(g, channel(V, c) * channel(deg_inv, c)[rows], XW) for c in range(C)])
 
 
 def _drop_diagonal(P, lo=0):
@@ -299,10 +301,8 @@ class GTN_Model(nn.Module):
         return torch.stack([norm(H[i, :, :]) for i in range(self.num_channels)], dim=0)
 
     def forward(self, A, X, target_x):
-        if isinstance(A, RelationStack):
+        if isinstance(A, (RelationStack, PartitionedRelationStack)):
             return self._forward_sparse(A, X, target_x)
-        if isinstance(A, PartitionedRelationStack):
-            return self._forward_partitioned(A, X, target_x)
         A = A.unsqueeze(0).permute(0, 3, 1, 2)
         Ws = []
         for i in range(self.num_layers):
@@ -318,54 +318,45 @@ class GTN_Model(nn.Module):
         return y, Ws
 
     def _forward_sparse(self, stack, X, target_x):
-        """forward() on a RelationStack: the same computation with every H a [nnz(P_l), C] value tensor."""
-        if stack.num_edge != self.num_edge:
-            raise ValueError(f"GTN_Model: the stack has {stack.num_edge} edge types, the model {self.num_edge}")
-        Ps, Ds, keeps = stack.patterns(self.num_layers)
+        """forward() on a RelationStack: the same computation with every H a [nnz(P_l), C] value tensor.
+        On a PartitionedRelationStack, forward() on this rank's rows: X = X[lo:hi], target_x = ids local to the block;
+        returns (logits of target_x, Ws).  The column sums of norm and the gcn_conv degrees are then completed by
+        rank-ordered all-reduces, and the gcn_conv output by a reduce-scatter.  Collective: every rank runs it, and
+        its backward, in the same order."""
+        if isinstance(stack, PartitionedRelationStack):
+            ps = stack
+            if (ps.num_edge, ps.num_layers, ps.width) != (self.num_edge, self.num_layers, self.num_channels * self.w_out):
+                raise ValueError(f"GTN_Model: the partitioned stack has {ps.num_edge} edge types, {ps.num_layers} "
+                                 f"layers and width {ps.width}; the model {self.num_edge}, {self.num_layers} and "
+                                 f"{self.num_channels * self.w_out} (num_channels * w_out)")
+            if X.dim() != 2 or X.shape[0] != ps.n_local:
+                raise ValueError(f"GTN_Model: X_local must hold this rank's {ps.n_local} rows, got {tuple(X.shape)}")
+            stack, (Ps, Ds, keeps), (g, src, diag), U_rows = ps.stack, (ps.P, ps.D, ps.keep), ps.gcn, ps.U_rows
+            red = ps.reduce
+        else:
+            if stack.num_edge != self.num_edge:
+                raise ValueError(f"GTN_Model: the stack has {stack.num_edge} edge types, the model {self.num_edge}")
+            Ps, Ds, keeps = stack.patterns(self.num_layers)
+            g, src, diag = stack.gcn_pattern(self.num_layers)
+            red = U_rows = None
+
+        def reduce(site):  # the column sums over every rank's rows; None: one GPU's sums are whole
+            return None if red is None else (lambda x: rank_all_reduce(red, site, x))
         Ws = []
         H = None
         for i in range(self.num_layers):
             if i == 0:
-                H, W = self.layers[i].forward_sparse(stack, Ps[0])
+                H, W = self.layers[i].forward_sparse(stack, Ps[0], U_rows=U_rows)
             else:
-                Hn = column_normalize(Ds[i - 1], H[keeps[i - 1]])  # norm(H): diagonal dropped, columns scaled
+                # norm(H): diagonal dropped, columns scaled
+                Hn = column_normalize(Ds[i - 1], H[keeps[i - 1]], reduce=reduce(f"norm{i}"))
                 H, W = self.layers[i].forward_sparse(stack, Ps[i], Hn, Ds[i - 1])
             Ws.append(W)
-        g, src, diag = stack.gcn_pattern(self.num_layers)
         XW = torch.mm(X, self.weight)
         one = torch.ones((), device=H.device, dtype=H.dtype)
-        X_ = torch.cat([F.relu(_normalized_aggregate(g, torch.where(diag, one, H[src, c]), XW))
-                        for c in range(self.num_channels)], dim=1)
+        vals = torch.where(diag.unsqueeze(1), one, H[src])
+        Y = _normalized_aggregate(g, vals, XW, reduce=reduce("deg"))  # [N, C * w_out]; partial on a row block
+        X_ = F.relu(Y) if red is None else row_reduce_scatter(red, "out", Y, relu=True)
         X_ = F.relu(self.linear1(X_))
         y = self.linear2(X_[target_x])
-        return y, Ws
-
-    def _forward_partitioned(self, ps, X_local, target_local):
-        """forward() on this rank's rows: X_local = X[lo:hi], target_local = ids local to the block; returns
-        (logits of target_local, Ws).  Collective: every rank runs it, and its backward, in the same order."""
-        if (ps.num_edge, ps.num_layers, ps.width) != (self.num_edge, self.num_layers, self.num_channels * self.w_out):
-            raise ValueError(f"GTN_Model: the partitioned stack has {ps.num_edge} edge types, {ps.num_layers} layers "
-                             f"and width {ps.width}; the model {self.num_edge}, {self.num_layers} and "
-                             f"{self.num_channels * self.w_out} (num_channels * w_out)")
-        if X_local.dim() != 2 or X_local.shape[0] != ps.n_local:
-            raise ValueError(f"GTN_Model: X_local must hold this rank's {ps.n_local} rows, got {tuple(X_local.shape)}")
-        red = ps.reduce
-        Ws = []
-        H = None
-        for i in range(self.num_layers):
-            if i == 0:
-                H, W = self.layers[i].forward_sparse(ps.stack, ps.P[0], U_rows=ps.U_rows)
-            else:
-                Hn = column_normalize(ps.D[i - 1], H[ps.keep[i - 1]],
-                                      reduce=lambda x, site=f"norm{i}": rank_all_reduce(red, site, x))
-                H, W = self.layers[i].forward_sparse(ps.stack, ps.P[i], Hn, ps.D[i - 1])
-            Ws.append(W)
-        g, src, diag = ps.gcn
-        XW = torch.mm(X_local, self.weight)
-        one = torch.ones((), device=H.device, dtype=H.dtype)
-        vals = torch.where(diag.unsqueeze(1), one, H[src])
-        Y = _normalized_aggregate(g, vals, XW, reduce=lambda x: rank_all_reduce(red, "deg", x))  # partial [N, C*w_out]
-        X_ = row_reduce_scatter(red, "out", Y, relu=True)
-        X_ = F.relu(self.linear1(X_))
-        y = self.linear2(X_[target_local])
         return y, Ws

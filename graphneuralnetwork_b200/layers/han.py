@@ -22,9 +22,8 @@ from torch import nn
 import torch.nn.functional as F
 
 from .. import _lib
-from ..functional import (SEMANTIC_MAX_K, SEMANTIC_MAX_M, AttentionDropout, gat_aggregate, halo_exchange,
-                          next_attention_dropout, require_partition_dtype, semantic_attention,
-                          semantic_attention_partitioned)
+from ..functional import (SEMANTIC_MAX_K, SEMANTIC_MAX_M, gat_aggregate, halo_exchange, require_partition_dtype,
+                          semantic_attention, semantic_attention_partitioned)
 from ..graph import CSRGraph, adj_cache
 from ..partition import PartitionedGraph, PartitionedMetapaths
 from .gat import GraphAttentionLayer, _fused_heads
@@ -104,14 +103,22 @@ class HANLayer(nn.Module):
         self.semantic_attention = SemanticAttention(in_size=out_size * layer_num_heads)
         self._width = out_size * layer_num_heads
 
-    def _batched(self, gs, h):
-        """All M metapath GATConvs (HAN.py:16-21) in ONE attention launch over the block diagonal of the M graphs:
-        `z[:, m, :]` is metapath m's multi-head output — the tensor `torch.stack(semantic_embeddings, dim=1)` builds.
-        Per-metapath feature dropout (NodeAttention.py:59: every GATConv draws its own mask) is kept."""
+    def _batched(self, graphs, h):
+        """All M metapath GATConvs (HAN.py:16-21) in ONE attention launch, forward and backward: `z[:, m, :]` is
+        metapath m's multi-head output — the tensor `torch.stack(semantic_embeddings, dim=1)` builds.  `graphs` is the
+        list of M graphs, run as their block diagonal, or a PartitionedMetapaths with h its own rows: then ONE halo
+        exchange of the stacked Wh, and the batched-rectangular launch over the rank's blocks in the union's combined
+        column space, with s of the own rows and t of all table rows.
+        Per-metapath feature dropout (NodeAttention.py:59: every GATConv draws its own mask, on a partition over the own
+        rows) is kept.  The attention dropout takes the GATConvs' `dropout`, as GATConv.forward does; a rank's block
+        draws the whole set's mask for its edges."""
         convs = list(self.gat_layers)
-        M, n = len(convs), h.shape[0]
-        graphs = [adj_cache.get(g) for g in gs]
-        big = CSRGraph.block_diagonal(graphs)
+        M = len(convs)
+        pm = graphs if isinstance(graphs, PartitionedMetapaths) else None
+        if pm is None:
+            g, shift = CSRGraph.block_diagonal([adj_cache.get(a) for a in graphs]), None
+        else:
+            g, shift = pm.attention()
         heads0 = list(convs[0].attentions)
         H, Fp, alpha = len(heads0), heads0[0].out_features, heads0[0].alpha
         p, training = convs[0].dropout, self.training
@@ -122,89 +129,51 @@ class HANLayer(nn.Module):
         # perturbation of one score into a 1e-4 change of that edge's gradient: measured on the ACM-sized golden);
         # per-metapath feature dropout draws its own mask per GATConv as the reference does
         Wh = torch.cat([torch.mm(F.dropout(h, p, training=True) if drop_active else h, W) for W in Ws], dim=1)
+        if pm is not None:
+            Wh = halo_exchange(pm.union, Wh)                                                 # [n_comb, M*H*Fp]
+        n, nc = g.n_rows // M, Wh.shape[0]
         a = torch.stack([torch.stack([hd.a[:, 0] for hd in conv.attentions]) for conv in convs])  # [M, H, 2*Fp]
-        Wh4 = Wh.view(n, M, H, Fp).float()
-        s = (Wh4 * a[None, :, :, :Fp].float()).sum(-1).permute(1, 0, 2).reshape(M * n, H)     # batched-row major
-        t = (Wh4 * a[None, :, :, Fp:].float()).sum(-1).permute(1, 0, 2).reshape(M * n, H)
-        keep = drop = None
-        if drop_active:
-            if _gat.EXPLICIT_DROPOUT_MASK:
-                keep = _gat.attention_keep_mask(big, H, p)
-            else:
-                drop = next_attention_dropout(p, Wh.device)
+        Wh4 = Wh.view(nc, M, H, Fp).float()
+        own = Wh4 if pm is None else Wh4[:n]  # the rows of s (no slice on one GPU: its backward copies)
+        s = (own * a[None, :, :, :Fp].float()).sum(-1).permute(1, 0, 2).reshape(M * n, H)     # batched-row major
+        t = (Wh4 * a[None, :, :, Fp:].float()).sum(-1).permute(1, 0, 2).reshape(M * nc, H)
+        keep, drop = _gat._attention_dropout(g, H, p if training else 0.0, Wh.device, slot_shift=shift)
         double_elu = convs[0].num_class is None and not drop_active
-        z = gat_aggregate(big, Wh, s, t, H, Fp, alpha, mode=_lib.GAT_SOFTMAX, elu=2 if double_elu else 1, keep=keep,
-                          dropout=drop, batch=M)                                                 # [N, M*H*Fp]
+        z = gat_aggregate(g, Wh, s, t, H, Fp, alpha, mode=_lib.GAT_SOFTMAX, elu=2 if double_elu else 1, keep=keep,
+                          dropout=drop, batch=M)                                                 # [n, M*H*Fp]
         if not double_elu:
             z = F.elu(F.dropout(z, p, training=training))  # NodeAttention.py:60-62, all metapaths at once
         return z.view(n, M, H * Fp)
 
-    def _batched_partitioned(self, pm, h):
-        """`_batched` on this rank's row block of a PartitionedMetapaths (h = the own rows): the per-metapath h·W_m on
-        the own rows, ONE halo exchange of the stacked Wh, s of the own rows and t of all table rows, one batched-
-        rectangular attention launch (forward and backward) and semantic attention over the global node count.
-        Feature dropout (GATConv.dropout, NodeAttention.py:59-60) draws on the own rows; the attention dropout
-        (the heads' GraphAttentionLayer.dropout, NodeAttention.py:31 — equal to it when built by the constructor)
-        draws the whole set's mask for the block's edges.
-        h has the partition's dtype (fp32 or bf16).  In bf16 the halo exchange moves bf16 rows and the node-level
-        attention runs in the bf16 batched-rectangular kernels; the split semantic kernels are fp32 only, so they take
-        z and the projection weights as fp32 views (autograd casts the gradients back) and the result is cast to h's
-        dtype.  This differs from the 1-GPU bf16 HAN, whose semantic attention is the plain torch formula in bf16:
-        the two agree to bf16 tolerance, not bit for bit."""
-        convs = list(self.gat_layers)
-        M = len(convs)
-        heads0 = list(convs[0].attentions)
-        H, Fp, alpha = len(heads0), heads0[0].out_features, heads0[0].alpha
-        lin = self.semantic_attention.project[0]
-        # the refusals depend on the replicated model and the features' dtype only: every rank raises together
-        if M != len(pm):
-            raise _lib.GnnError(f"HANLayer: {M} metapath models for {len(pm)} metapath graphs")
-        require_partition_dtype(pm, h, "HANLayer on PartitionedMetapaths")
-        if any(c.num_class is not None for c in convs) or H * Fp > 256 or \
-                M > SEMANTIC_MAX_M or lin.out_features > SEMANTIC_MAX_K:
-            raise _lib.GnnError("HANLayer on PartitionedMetapaths: needs num_class None, H*F' <= 256, "
-                                f"M <= {SEMANTIC_MAX_M} and a semantic hidden width <= {SEMANTIC_MAX_K} (got "
-                                f"H*F' = {H * Fp}, M = {M}, K = {lin.out_features})")
-        g, shift = pm.attention()
-        n = pm.n_local
-        p, p_att, training = convs[0].dropout, heads0[0].dropout, self.training
-        drop_active = training and p > 0.0
-        Ws = [torch.cat([hd.W for hd in conv.attentions], dim=1) for conv in convs]
-        Wh = torch.cat([torch.mm(F.dropout(h, p, training=True) if drop_active else h, W) for W in Ws], dim=1)
-        Wh = halo_exchange(pm.union, Wh)                                                         # [n_comb, M*H*Fp]
-        nc = Wh.shape[0]
-        a = torch.stack([torch.stack([hd.a[:, 0] for hd in conv.attentions]) for conv in convs])  # [M, H, 2*Fp]
-        Wh4 = Wh.view(nc, M, H, Fp).float()
-        s = (Wh4[:n] * a[None, :, :, :Fp].float()).sum(-1).permute(1, 0, 2).reshape(M * n, H)
-        t = (Wh4 * a[None, :, :, Fp:].float()).sum(-1).permute(1, 0, 2).reshape(M * nc, H)
-        keep = drop = None
-        if training and p_att > 0.0:
-            if _gat.EXPLICIT_DROPOUT_MASK:
-                keep = _gat.attention_keep_mask(g, H, p_att)
-            else:
-                d = next_attention_dropout(p_att, Wh.device)
-                drop = AttentionDropout(d.p, d.seed, d.seed_dev, slot_shift=shift)  # the whole set's mask
-        double_elu = not drop_active
-        z = gat_aggregate(g, Wh, s, t, H, Fp, alpha, mode=_lib.GAT_SOFTMAX, elu=2 if double_elu else 1, keep=keep,
-                          dropout=drop, batch=M)                                                 # [n, M*H*Fp]
-        if not double_elu:
-            z = F.elu(F.dropout(z, p, training=training))
-        sem = self.semantic_attention
-        b1 = None if lin.bias is None else lin.bias.float()
-        out = semantic_attention_partitioned(z.view(n, M, H * Fp).float(), lin.weight.float(), b1,
-                                             sem.project[2].weight.float(), pm.n_total, pm.world, pm.group)
-        return out.to(h.dtype)
-
     def forward(self, gs, h):
+        convs = list(self.gat_layers)
+        heads0 = list(convs[0].attentions)
+        width = len(heads0) * heads0[0].out_features
         if isinstance(gs, PartitionedMetapaths):
-            return self._batched_partitioned(gs, h)
+            sem = self.semantic_attention
+            M, lin = len(convs), sem.project[0]
+            # the refusals depend on the replicated model and the features' dtype only: every rank raises together,
+            # before the first collective
+            if M != len(gs):
+                raise _lib.GnnError(f"HANLayer: {M} metapath models for {len(gs)} metapath graphs")
+            require_partition_dtype(gs, h, "HANLayer on PartitionedMetapaths")
+            if any(c.num_class is not None for c in convs) or width > 256 or \
+                    M > SEMANTIC_MAX_M or lin.out_features > SEMANTIC_MAX_K:
+                raise _lib.GnnError("HANLayer on PartitionedMetapaths: needs num_class None, H*F' <= 256, "
+                                    f"M <= {SEMANTIC_MAX_M} and a semantic hidden width <= {SEMANTIC_MAX_K} (got "
+                                    f"H*F' = {width}, M = {M}, K = {lin.out_features})")
+            # semantic attention over the global node count.  Its split kernels are fp32, so they take fp32 views
+            # (autograd casts the gradients back) and the result has h's dtype.  The 1-GPU bf16 HAN runs the plain
+            # torch formula in bf16 instead: the two agree to bf16 tolerance, not bit for bit
+            b1 = None if lin.bias is None else lin.bias.float()
+            out = semantic_attention_partitioned(self._batched(gs, h).float(), lin.weight.float(), b1,
+                                                 sem.project[2].weight.float(), gs.n_total, gs.world, gs.group)
+            return out.to(h.dtype)
         if any(isinstance(g, PartitionedGraph) for g in gs):
             raise _lib.GnnError("HANLayer: metapath graphs on a PartitionedGraph are not supported (the batched "
                                 "metapath attention runs on one GPU)")
-        convs = list(self.gat_layers)
-        heads0 = list(convs[0].attentions)
         if (getattr(self, "batched", True) and len(convs) > 1 and all(c.num_class is None for c in convs)
-                and len(heads0) * heads0[0].out_features <= 256 and h.dtype in (torch.float32, torch.bfloat16)):
+                and width <= 256 and h.dtype in (torch.float32, torch.bfloat16)):
             return self.semantic_attention(self._batched(gs, h))
         if torch.is_grad_enabled() and (h.requires_grad or any(p.requires_grad for p in self.parameters())):
             z = torch.stack([conv(h, g).flatten(1) for g, conv in zip(gs, convs)], dim=1)  # (N, M, H·F')

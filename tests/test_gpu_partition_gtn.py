@@ -127,6 +127,37 @@ def test_world_one_step_reads_nothing_back():
     torch.cuda.synchronize()
 
 
+@pytest.mark.parametrize("C", [1, 2])
+def test_empty_block_gcn_tail_takes_part_in_the_reduce(C):
+    """A rank whose row block is empty: its gcn_conv pattern is [n, 0] with [0, C] values.  The normalise-and-aggregate
+    tail still hands its (zero) partial degrees to the reduce, as every rank must, and returns a zero partial output;
+    the backward gives empty value and XW gradients.  norm's column sums over the empty D_l reach the reduce too."""
+    from graphneuralnetwork_b200.functional import column_normalize
+    from graphneuralnetwork_b200.graph import CSRGraph
+    from graphneuralnetwork_b200.layers.gtn import _gcn_pattern, _normalized_aggregate
+    n, w = 50, 8
+    D = CSRGraph(torch.zeros(1, dtype=torch.int64, device=DEV), torch.zeros(0, dtype=torch.int32, device=DEV), None,
+                 0, n)
+    g, src, diag = _gcn_pattern(D, torch.zeros(0, dtype=torch.int64, device=DEV), n, n)
+    assert (g.n_rows, g.n_cols, g.nnz, src.numel(), diag.numel()) == (n, 0, 0, 0, 0)
+    vals = torch.zeros((0, C), device=DEV, requires_grad=True)
+    XW = torch.zeros((0, w), device=DEV, requires_grad=True)
+    seen = []
+
+    def reduce(x):
+        seen.append(x.detach().clone())
+        return x
+
+    Y = _normalized_aggregate(g, vals, XW, reduce=reduce)
+    assert len(seen) == 1 and seen[0].shape == (n, C) and not seen[0].any()
+    assert Y.shape == (n, C * w) and not Y.any()
+    dv, dx = torch.autograd.grad(Y, (vals, XW), torch.randn_like(Y))
+    assert dv.shape == (0, C) and dx.shape == (0, w)
+    Hn = column_normalize(D, vals, reduce=reduce)
+    assert len(seen) == 2 and seen[1].shape == (n, C) and not seen[1].any() and Hn.shape == (0, C)
+    assert torch.autograd.grad(Hn.sum(), vals)[0].shape == (0, C)
+
+
 def test_refusals():
     stack, X, target, _, K, classes = _golden_stack()
     ps = PartitionedRelationStack(stack, 0, 1, 2, 16)

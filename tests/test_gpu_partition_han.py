@@ -387,8 +387,8 @@ def test_partitioned_han_refusals():
 
 @pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs on one node")
 def test_two_rank_han_training_all_transports_check():
-    """Two real ranks train HAN on PartitionedMetapaths (ACM-shaped metapaths, self-loops, 8 heads x 8, attention
-    dropout 0.6) over p2p, ce and nccl; every rank compares its rows of the logits, the step-1 gradients and the
+    """Two real ranks train HAN on PartitionedMetapaths (ACM-shaped metapaths, self-loops, 8 heads x 8, dropout
+    off) over p2p, ce and nccl; every rank compares its rows of the logits, the step-1 gradients and the
     weights after 3 Adam steps with the same model trained on one GPU, and repeats the run bit for bit."""
     import json
     import os

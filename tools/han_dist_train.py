@@ -10,15 +10,15 @@ One JSON line per rank and configuration on stdout.
   graph and a dense paper-subject-paper graph; 8 heads x 8, 3 classes): every rank also trains the same seeded
   HANModel on its GPU over the WHOLE graphs (one block holding every row, which the GPU tests hold bit-identical to
   HANModel over the plain graphs) and compares its own rows of the logits, every gradient at step 1 (after the
-  all-reduce) and the weights after 3 Adam steps; the 3-step run is repeated and must be bit-identical.  Attention
-  dropout is 0.6 and feature dropout off (a rank draws its feature masks over its own rows).  Both runs draw identical
-  attention-dropout streams: the host seed (torch.manual_seed) and functional._drop_counters are reset before every
-  run, and each rank's block draws the whole set's mask for its edges (per-metapath slot shifts).  --dtype bf16: the
-  model, the features and the partitions are bf16 and the 1-GPU run is the same seeded bf16 model over the whole
-  graphs as one block, under gcn_dist_train.CHECK_BOUNDS["bf16"].
+  all-reduce) and the weights after 3 Adam steps; the 3-step run is repeated and must be bit-identical.  Dropout is
+  off: a GATConv's one `dropout` sets its feature and its attention dropout, and a rank draws its feature masks over
+  its own rows.  (The GPU tests hold a rank block's attention-dropout mask to the whole set's, and HANModel on a
+  one-rank partition to one GPU with dropout 0.6.)  --dtype bf16: the model, the features and the partitions are
+  bf16 and the 1-GPU run is the same seeded bf16 model over the whole graphs as one block, under
+  gcn_dist_train.CHECK_BOUNDS["bf16"].
 --time (a synthetic set of power-law metapaths of different mean degrees plus self-loops, generated on the device on
-  every rank): ms per training step (forward + backward + gradient all-reduce + Adam) and per forward, ms of the
-  stacked-Wh halo exchange alone, peak memory, the union halo rows against Σ of the per-metapath halo rows, and a
+  every rank; dropout 0.6): ms per training step (forward + backward + gradient all-reduce + Adam) and per forward,
+  ms of the stacked-Wh halo exchange alone, peak memory, the union halo rows against Σ of the per-metapath halo rows, and a
   float64 spot check of sampled first-layer rows of metapath 0.  The fp32 and the bf16 model are timed at the same
   size in one run, their steps alternated; one line per dtype with its halo bytes and the peak memory of its step.
   Device name and power limit are read in the same run."""
@@ -84,14 +84,8 @@ def train(model, graphs, X, target, idx, n_train, steps, group=None):
     return logits1, grads1, {k: v.detach().clone() for k, v in model.state_dict().items()}
 
 
-def make_model(M, F_in, a):
-    """HANModel with attention dropout 0.6 and no feature dropout (the feature masks of a rank are drawn over its own
-    rows, so they cannot equal one GPU's)."""
-    m = HANModel(M, F_in, a.hidden, a.classes, [a.heads], 0.6)
-    for layer in m.layers:
-        for conv in layer.gat_layers:
-            conv.dropout = 0.0
-    return m
+def make_model(M, F_in, a, dropout):
+    return HANModel(M, F_in, a.hidden, a.classes, [a.heads], dropout)
 
 
 def run_check(a, rank, world, dev):
@@ -104,7 +98,7 @@ def run_check(a, rank, world, dev):
     labels = torch.randint(0, a.classes, (n,), generator=gen).to(dev)
     idx_train = torch.randperm(n, generator=gen)[: n // 5].sort().values.to(dev)
     torch.manual_seed(0)
-    ref = make_model(M, F_in, a).to(dev).to(dt)
+    ref = make_model(M, F_in, a, 0.0).to(dev).to(dt)
     init = {k: v.clone() for k, v in ref.state_dict().items()}
     # the 1-GPU run: the whole graphs as one block (tests/test_gpu_partition_han.py holds this equal, bit for bit, to
     # HANModel over the plain graphs in fp32; tests/test_gpu_partition_bf16.py within bf16 tolerance in bf16, whose
@@ -122,7 +116,7 @@ def run_check(a, rank, world, dev):
         n_train = global_count(idx_loc.numel(), dev) if world > 1 else idx_loc.numel()
         runs = []
         for _ in range(2):
-            model = make_model(M, F_in, a).to(dev).to(dt)
+            model = make_model(M, F_in, a, 0.0).to(dev).to(dt)
             if rank == 0:
                 model.load_state_dict(init)
             if world > 1:
@@ -181,7 +175,7 @@ def run_time(a, rank, world, dev):
         labels = (torch.arange(lo, hi, device=dev) * 2654435761 % C).to(torch.int64)
         idx_loc = torch.arange(0, n_loc, 3, device=dev)  # every third row trains
         torch.manual_seed(0)
-        model = make_model(M, F_in, a).to(dev).to(dt)
+        model = make_model(M, F_in, a, 0.6).to(dev).to(dt)
         if world > 1:
             broadcast_parameters(model)
         n_train = global_count(idx_loc.numel(), dev) if world > 1 else idx_loc.numel()
